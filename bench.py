@@ -2,7 +2,7 @@
 """Headline benchmark: MaxViT grid fields/sec of the 12hr MetNet3 model (BASELINE.json configs[1]:
 inference, bf16, batch 64 synthetic CMAQ grids = 768 fields per step per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
 
 * a "step" = one forward of `MetNet3` over one batch of B=64 synthetic CMAQ tensors (64*12 = 768 grid fields)
 * `value`  = fields/s with the inputs already resident in HBM (CUDA events, max over ranks)
@@ -18,6 +18,8 @@ inference, bf16, batch 64 synthetic CMAQ grids = 768 fields per step per GPU).
 * `train`  = BASELINE configs[2]: the training step (train-mode forward, Focal-R, backward, NCCL gradient all-reduce, fused
              AdamW), with its own roofline block for the kernel with the largest share of the step
 * `--config 3|4` = BASELINE configs[3] (512x512 domain, MaxViT depth 2) / configs[4] (512 channels, 32 x 64 heads, depth 4)
+* `--dump-outputs DIR` = rank 0 writes the predictions of the last timed inference step as DIR/prediction.npy (float32), so
+             that two builds can be compared output for output on identical seeded inputs
 N>1: one process per GPU (torchrun), batch-sharded, no data-path collective (inference) -> weak scaling.
 """
 import argparse
@@ -39,6 +41,21 @@ CONV_FLOPS_PER_FIELD = 2.0 * 84 * 70 * 128 * 1152          # algorithmic: unpadd
 ATTN_FLOPS_PER_FIELD = 2.0125e9                             # SURVEY 8d: qkv 1.2505 + QK^T 0.1726 + PV 0.1726 + out 0.4168 GF, 53-token count
 FWD_GFLOP_PER_FIELD_REF = 25.864                            # SURVEY F8 (reference graph, no lead-time dedup)
 FWD_GFLOP_PER_FIELD_EXEC = 17.516                           # with the stem computed once per sample (H5)
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory, **arrays):
+    """write each array as DIRECTORY/<name>.npy in float32.  When the arrays exceed DUMP_LIMIT_BYTES in all, each is replaced
+    by a fixed strided sample of its flattened values (the same elements on every run with the same arguments)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    total = sum(a.numel() for a in arrays.values())
+    stride = -(-total * 4 // (DUMP_LIMIT_BYTES - 4096 * len(arrays)))      # 4 KB per file for the .npy header
+    for name, a in arrays.items():
+        a = a.detach().float().cpu()
+        if stride > 1:
+            a = a.flatten()[::stride]
+        np.save(os.path.join(directory, f"{name}.npy"), a.numpy())
 
 
 class ClockSampler:
@@ -163,8 +180,10 @@ def run_reference(args, rank, world):
             metnet3_forward(x, ts, sd, cfg)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            metnet3_forward(x, ts, sd, cfg)
+            y = metnet3_forward(x, ts, sd, cfg)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, prediction=y)
     value = bs * cfg.L * args.steps / dt
     sample = f"B={bs} synthetic CMAQ tensor (12 fields) per step, fp32, eval, {threads} torch CPU threads"
     print(json.dumps({
@@ -209,7 +228,7 @@ def run_train(args, cfg, dev, rank, world, barrier, max_over_ranks):
     barrier()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     l0 = _lib.launch_count()
-    steps = max(20, args.steps)
+    steps = args.steps
     e0.record()
     for _ in range(steps):
         loss = step()
@@ -308,17 +327,20 @@ def run_other_config(args, dev, rank, world):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     with torch.no_grad():
         for _ in range(W):
-            model(x, timestamps=ts)
+            y = model(x, timestamps=ts)               # held like in the timed loop: the allocator sees the same pattern
         barrier()
         l0 = _lib.launch_count()
         with ClockSampler(dev.index or 0) as clk:
             e0.record()
             for _ in range(args.steps):
-                model(x, timestamps=ts)
+                y = model(x, timestamps=ts)
             e1.record()
             barrier()
         launches = (_lib.launch_count() - l0) // args.steps
         ms = max_over_ranks(e0.elapsed_time(e1))
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, prediction=y)
+        del y
         # end to end: pinned host tensor in, pinned host predictions out, synchronously per step (tiny batches: no pipelining)
         y_host = torch.empty(B, L, cfg.H, cfg.W, dtype=torch.float32).pin_memory()
         barrier()
@@ -408,7 +430,7 @@ def run_other_config(args, dev, rank, world):
             for _ in range(3):
                 step()
             barrier()
-            steps = max(5, args.steps)
+            steps = args.steps
             e0.record()
             for _ in range(steps):
                 loss = step()
@@ -441,7 +463,7 @@ def run_other_config(args, dev, rank, world):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10, help="timed steps of every leg")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--batch", type=int, default=64, help="CMAQ samples per GPU per step (x12 lead times = fields)")
@@ -457,7 +479,10 @@ def main():
     ap.add_argument("--e2e-input", default="bf16", choices=["bf16", "fp32"],
                     help="host format of the e2e leg's inputs: bf16 = batches packed by pipeline.pack_host (bit-identical "
                          "predictions, half the H2D bytes); fp32 = the reference's tensor; the other one is reported beside it")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the predictions of the last timed step to DIR/prediction.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -511,7 +536,7 @@ def main():
     with torch.no_grad():
         # ---------------- device-resident throughput
         for _ in range(W):
-            step_resident()
+            y = step_resident()                       # held like in the timed loop: the allocator sees the same pattern
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         launches0 = _lib.launch_count()
@@ -519,10 +544,13 @@ def main():
         with ClockSampler(local) as clk:
             e0.record()
             for _ in range(args.steps):
-                step_resident()
+                y = step_resident()
             e1.record()
             barrier()
         trace, _lib.TRACE = _lib.TRACE, None
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, prediction=y)
+        del y
         launches = (_lib.launch_count() - launches0) // args.steps
         ms_total = max_over_ranks(e0.elapsed_time(e1))
         # ---------------- end to end (host buffers in, host predictions out) through the package's streaming API:
