@@ -193,32 +193,26 @@ VG_API int vg_attn_out_fwd(int dtype, const void* attn, int inner, const void* W
                     int reg_per_field, float* reg_out, void* x_out, int N, int Hl, int Wl, int C, int win, int R,
                     int grid_mode, long long drop_seed, int drop_salt, int drop_thresh, float* scratch, long long scratch_elems,
                     void* stream);
-/* (both: drop_thresh T in [1,255] = the training dropout of vg_attn_fused_fwd -- same hash, same masks -- on the
+/* (both: drop_thresh T in [1,255] = the training dropout of vg_attn_fused2_fwd -- same hash, same masks -- on the
  * probabilities / on the to_out output before the residual; 0 = none) */
 
-/* maxvit.py:170-219 + 298-340 in ONE kernel (fp32 residual stream, tcgen05 kind::f16 QKV projection on fp16 operands, kind::tf32 QK^T / out-projection, bf16 PV):
+/* maxvit.py:170-219 + 298-340 in ONE kernel, IN PLACE on the fp32 residual stream: xio += to_out(attn(xio)).
  * gather + register tokens + LayerNorm + FiLM -> per head {QKV, QK-RMSNorm, QK^T + rel-pos bias, softmax, PV,
- * out-projection accumulated over heads} -> + residual -> inverse partition.  x/x_out: CL (N,Hl,Wl,128) fp32;
+ * out-projection accumulated over heads} -> + residual -> inverse partition.  xio: CL (N,Hl,Wl,128) fp32.
+ * The window / grid partition (maxvit.py:298 / :322) is the TMA tensor map itself -- block: boxes (32 ch, 7, 7) of the view
+ * (C, Wl, N*Hl); grid: boxes (32 ch, 1, 7, 1, 7) of the view (C, Y, 7, X, 7N) -- the token rows of the next tile are prefetched
+ * by the TMA warp, and the result returns through the same maps with cp.reduce.async.bulk.tensor (.add), which performs the
+ * residual add.  QKV projection, QK^T and PV run as tcgen05 kind::f16 (fp16 / bf16 operands), the out-projection as
+ * kind::tf32 on the O_h accumulator read in place from TMEM; two compute groups of 8 warps alternate heads.
  * wqkv_h: fp16 [heads][96][128] (per head the 32 q rows, 32 k rows, 32 v rows of to_qkv.weight, rounded to fp16:
  * the QKV projection runs as kind::f16 on fp16 operands -- tf32's 10-bit mantissa at twice the rate);
  * wout_h: fp32 [heads][128][32] (per head the 32 columns of to_out.0.weight); head_tab: fp32 [heads][1332] =
  * per head the relative-position bias times log2(e) as 7 pre-shifted copies [bi][row 0..12] (bi stride 180 floats, row stride
  * 12 floats, entry k = 0..6 of a row = table[(row*13 + bi+6-k)]; the strides make the kernel's reads bank-conflict-free),
- * table[169]*log2(e) x 8, 32*gamma_q*gamma_k [32], 32 unused.  Needs C=128, dim_head=32, win=7, R=4, heads >= 4.
+ * table[169]*log2(e) x 8, 32*gamma_q*gamma_k [32], 32 unused.  Needs C=128, dim_head=32, win=7, R=4, heads >= 4 and even.
  * Training: drop_thresh T in [1,255] enables nn.Dropout (maxvit.py:146,151) on the attention probabilities and on the
  * to_out output with drop probability T/256 (kept values scaled by 256/(256-T)); the masks are a counter-based hash of
- * (drop_seed, drop_salt = layer id, row, group) that the backward kernels regenerate.  T = 0: no dropout (eval). */
-VG_API int vg_attn_fused_fwd(const float* x, float* x_out, const float* reg_in, int reg_per_field, float* reg_out,
-                      const float* film, const void* wqkv_h, const float* wout_h, const float* head_tab, int N, int Hl, int Wl, int C, int win, int R,
-                      int grid_mode, int heads, int dh, float ln_eps, long long drop_seed, int drop_salt, int drop_thresh, void* stream);
-
-/* Second-generation fused attention (maxvit.py:170-219 + 298-340), IN PLACE on the fp32 residual stream: xio += to_out(attn(xio)).
- * The window / grid partition (maxvit.py:298 / :322) is the TMA tensor map itself -- block: boxes (32 ch, 7, 7) of the view
- * (C, Wl, N*Hl); grid: boxes (32 ch, 1, 7, 1, 7) of the view (C, Y, 7, X, 7N) -- the token rows of the next tile are prefetched
- * by the TMA warp, and the result returns through the same maps with cp.reduce.async.bulk.tensor (.add), which performs the
- * residual add.  QKV projection, QK^T and PV run as tcgen05 kind::f16 (fp16 / bf16 operands), the out-projection as
- * kind::tf32 on the O_h accumulator read in place from TMEM; two compute groups of 8 warps alternate heads.  Same operand
- * formats (wqkv_h, wout_h, head_tab), dropout hash and constraints as vg_attn_fused_fwd, plus: heads even.
+ * (drop_seed, drop_salt = layer id, row, group) that the backward kernels regenerate.  T = 0: no dropout (eval).
  * A caller that needs the input afterwards (training) copies it first and passes the copy.
  * logit_bound: 0, or a bound of |logit + bias| * log2(e) over all heads that the caller derived from the weights (q-hat and k-hat are
  * unit vectors, maxvit.py:26-30: |logit| <= dh * max|gamma_q * gamma_k|); at most 115 lets the kernel skip the running maximum of the
@@ -388,11 +382,11 @@ VG_API int vg_attn_out_bwd_gather(const float* dx_out, const float* dreg, float 
  * key slot), out_mask [n_windows][64][C] */
 VG_API int vg_dropout_mask_debug(long long drop_seed, int drop_salt, int drop_thresh, long long n_windows, int heads, int C,
                           void* prob_mask, void* out_mask, void* stream);
-/* per-(field, head) core backward: dqkv written; dq_gamma, dk_gamma, dbias_table accumulated.  use_tf32 = 1 / 2 / 3: tensor-core
- * kernel (1: tf32 mma; 2: bf16 mma + ldmatrix on fp32 tensors; 3: the same kernel with qkv, datt, dqkv and att_out as bf16
- * tensors; fp32 accumulate), which can also re-materialise the forward output att = softmax(.) V [rows][inner]
- * (att_out, or NULL) for the to_out weight gradient when the forward pass was the fused kernel; 0: exact-fp32 SIMT kernel.
- * drop_thresh > 0 (bf16 kernels only): the forward pass applied dropout to the probabilities with these parameters. */
+/* per-(field, head) core backward: dqkv written; dq_gamma, dk_gamma, dbias_table accumulated.  use_tf32 = 2 / 3: tensor-core
+ * kernel (2: bf16 mma + ldmatrix on fp32 tensors; 3: qkv, datt, dqkv and att_out as bf16 tensors; fp32 accumulate), which can
+ * also re-materialise the forward output att = softmax(.) V [rows][inner] (att_out, or NULL) for the to_out weight gradient
+ * when the forward pass was the fused kernel; 0: exact-fp32 SIMT kernel.  Any other mode is an error.
+ * drop_thresh > 0: the forward pass applied dropout to the probabilities with these parameters. */
 VG_API int vg_attn_core_bwd(const void* qkv, const void* datt, const float* q_gamma, const float* k_gamma,
                      const float* bias_table, int N, int Hl, int Wl, int win, int R, int heads, int dh, void* dqkv,
                      float* dq_gamma, float* dk_gamma, float* dbias_table, int use_tf32, void* att_out, long long drop_seed,

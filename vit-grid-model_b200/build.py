@@ -13,7 +13,7 @@ from concurrent.futures import ThreadPoolExecutor
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB_PATH = os.path.join(HERE, "libvitgrid.so")
-SOURCES = ["vg_api.cu", "vg_gemm.cu", "vg_mem.cu", "vg_attn.cu", "vg_attn_fused.cu", "vg_attn_fused2.cu", "vg_attn_bwd_tc.cu", "vg_wgrad.cu", "vg_bwd.cu", "vg_bwd_vit.cu", "vg_eval.cu"]
+SOURCES = ["vg_api.cu", "vg_gemm.cu", "vg_mem.cu", "vg_attn.cu", "vg_attn_fused2.cu", "vg_attn_bwd_tc.cu", "vg_wgrad.cu", "vg_bwd.cu", "vg_bwd_vit.cu", "vg_eval.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden"]
 

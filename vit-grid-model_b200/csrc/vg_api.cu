@@ -309,15 +309,6 @@ int vg_attn_out_fwd(int dtype, const void* attn, int inner, const void* Wt, cons
                   (cudaStream_t)stream);
 }
 
-int vg_attn_fused_fwd(const float* x, float* x_out, const float* reg_in, int reg_per_field, float* reg_out,
-                      const float* film, const void* wqkv_h, const float* wout_h, const float* head_tab, int N, int Hl, int Wl, int C, int win, int R,
-                      int grid_mode, int heads, int dh, float ln_eps, long long drop_seed, int drop_salt, int drop_thresh, void* stream) {
-  AttnGeom g;
-  if (make_attn_geom(g, N, Hl, Wl, C, win, R, grid_mode)) return 1;
-  return attn_fused_run(x, x_out, reg_in, reg_per_field, reg_out, film, wqkv_h, wout_h, head_tab, g,
-                        heads, dh, ln_eps, (unsigned)drop_seed, (unsigned)drop_salt, drop_thresh, (cudaStream_t)stream);
-}
-
 int vg_attn_fused2_fwd(float* xio, const float* reg_in, int reg_per_field, float* reg_out, const float* film, const void* wqkv_h,
                        const float* wout_h, const float* head_tab, int N, int Hl, int Wl, int C, int win, int R, int grid_mode, int heads,
                        int dh, float ln_eps, long long drop_seed, int drop_salt, int drop_thresh, float logit_bound, void* stream) {

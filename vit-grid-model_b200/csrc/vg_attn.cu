@@ -472,11 +472,10 @@ int attn_core_run(int dtype, const void* qkv, const float* qgamma, const float* 
   drop.seed = seed; drop.salt = salt; drop.thresh = drop_thresh; drop.scale = 256.0f / (256.0f - (float)drop_thresh);
   // dtype 2 = fp32 storage with 3xTF32 tensor-core products (the 'tf32_conv' precision of wide networks); dtype 4 = fp32 storage and
   // bf16 storage (0) take single tf32 products (the mixed-precision modes).  Shapes outside the mma kernel (S > 64, attention dropout) and exact fp32 (dtype 1) run the SIMT kernel.
-  static const bool mma_off = getenv("VG_ATTN_CORE_MMA") && atoi(getenv("VG_ATTN_CORE_MMA")) == 0;
   const int out_split = dtype == 6;                        // dtype 6 = 2 with the output rows as the split operand [hi | hi | lo]
   if (out_split) dtype = 2;
-  if (out_split && (mma_off || drop_thresh || g.S() > 64 || (dh != 32 && dh != 64))) return set_error("attn_core: the split output (dtype 6) needs the tensor-core kernel (S <= 64, dim_head 32 / 64, no dropout)");
-  if (dtype != 1 && !mma_off && drop_thresh == 0 && g.S() <= 64 && g.win <= 64) {
+  if (out_split && (drop_thresh || g.S() > 64 || (dh != 32 && dh != 64))) return set_error("attn_core: the split output (dtype 6) needs the tensor-core kernel (S <= 64, dim_head 32 / 64, no dropout)");
+  if (dtype != 1 && drop_thresh == 0 && g.S() <= 64 && g.win <= 64) {
     if (dh == 64) return dtype == 0 ? core_mma_launch<bf16, 64, false>(qkv, qgamma, kgamma, bias_table, g, heads, out, 0, st)
                        : dtype == 4 ? core_mma_launch<float, 64, false>(qkv, qgamma, kgamma, bias_table, g, heads, out, out_split, st)
                                     : core_mma_launch<float, 64, true>(qkv, qgamma, kgamma, bias_table, g, heads, out, out_split, st);

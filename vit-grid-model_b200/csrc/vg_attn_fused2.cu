@@ -47,7 +47,7 @@ constexpr int VT_OFF = QK_OFF + 2 * 16384;       // V (bf16, MN-major B operand 
 constexpr int RAW_OFF = VT_OFF + 2 * 8192;       // token rows of a tile: 4 channel planes x [128 rows x 128 B], SWIZZLE_128B
 constexpr int RAW_BYTES = 4 * 16384;
 constexpr int TAB_SR = 12, TAB_SB = 180, TAB_T169 = 7 * TAB_SB;
-constexpr int TAB_FLOATS = TAB_T169 + 8 + 64;    // same per-head table as the first-generation kernel (ops.pack_head_tables)
+constexpr int TAB_FLOATS = TAB_T169 + 8 + 64;    // the per-head table of ops.pack_head_tables
 constexpr int TAB_OFF = RAW_OFF + RAW_BYTES;     // 2 x TAB_FLOATS floats
 constexpr int FILM_OFF = TAB_OFF + 2 * TAB_FLOATS * 4;   // 2 windows x (gamma[128] | beta[128])
 constexpr int REGS_OFF = FILM_OFF + 2 * 1024;    // 2 windows x register-token rows [4][128]
@@ -898,9 +898,8 @@ int attn_fused2_run(float* xio, const float* reg_in, int reg_per_field, float* r
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   const long long n_tiles = (p.n_windows + 1) / 2;
   const int grid = (int)(n_tiles < sms ? n_tiles : sms);
-  // logit_bound: the caller's bound of |logit + bias| in the exp2 domain (0 = none given); VG_ATTN2_NOMAX=0 keeps the running maximum
-  static const bool nomax_off = getenv("VG_ATTN2_NOMAX") && atoi(getenv("VG_ATTN2_NOMAX")) == 0;
-  const bool nomax = !nomax_off && logit_bound > 0.f && logit_bound <= 115.f;
+  // logit_bound: the caller's bound of |logit + bias| in the exp2 domain (0 = none given: keep the running maximum)
+  const bool nomax = logit_bound > 0.f && logit_bound <= 115.f;
   if (drop_thresh) attn_fused2_kernel<true, false, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
   else if (p.dbg) attn_fused2_kernel<false, true, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
   else if (nomax) attn_fused2_kernel<false, false, true><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);

@@ -725,276 +725,17 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
 }
 
 // ------------------------------------------------------------------------------------------------
-// Tensor-core version of the core backward (tf32 mma.sync m16n8k8, fp32 accumulate) for the mixed-precision path.
+// Tensor-core version of the core backward for the mixed-precision path: bf16 mma.sync m16n8k16 (fp32 accumulate) with
+// ldmatrix operand fetch (transposed operands come for free from ldmatrix.trans).
 // Block = (field, head), 4 warps, looping over the field's windows (3 blocks per SM hide each other's load latency);
 // each warp owns 16 rows of the window:
-//   phase 1  load q,k,v,dO rows, RMSNorm -> Qh, Kh, V, dO in shared memory (row stride 36: conflict-free fragments)
+//   phase 1  load q,k,v,dO rows, RMSNorm -> Qh, Kh, V, dO in shared memory (row stride 80 B: conflict-free ldmatrix)
 //   phase 2  S = Qh Kh^T (+bias), row softmax in registers -> P (smem);  [att = P V, optional output]
-//            dP = dO V^T, dS = P*(dP - rowdot) -> dS (smem), bias-table gradient (smem atomics)
+//            dP = dO V^T, dS = P*(dP - rowdot) -> dS (smem), bias-table gradient
 //   phase 3  dV = P^T dO, dKh = dS^T Qh (rows = keys), dQh = dS Kh (rows = queries); RMSNorm backward on the
 //            accumulator fragments (raw q,k re-read from global) -> dqkv
-// The 53 valid tokens are padded to 64 with zero rows; padded keys are masked to -inf before the softmax.
-// ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void mma_tf32(float* c, const float* a, const float* b) {
-  asm volatile(
-      "mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
-      : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3])
-      : "r"(__float_as_uint(a[0])), "r"(__float_as_uint(a[1])), "r"(__float_as_uint(a[2])), "r"(__float_as_uint(a[3])),
-        "r"(__float_as_uint(b[0])), "r"(__float_as_uint(b[1])));
-}
-
-namespace cb {
-constexpr int DH = 32, SM = 64, LD = 36, LDP = 68;
-constexpr int SLOT_FLOATS = 4 * SM * LD + 2 * SM * LDP + 2 * SM;   // Qh Kh V dO | P dS | 1/|q| 1/|k|
-}  // namespace cb
-
-// C[16 x 8*NT] += A[16 x K] * B,  A element (r, k) at a[r*lda + k] (TRANS_A: at a[k*lda + r]);
-// B given as Bt (NT form: element (k, n) at b[n*ldb + k]) or B (NN form: element (k, n) at b[k*ldb + n]).
-template <int NT, int K, bool TRANS_A, bool NN>
-__device__ __forceinline__ void warp_mma(float (*acc)[4], const float* a, int lda, const float* b, int ldb, int lane) {
-  const int g = lane >> 2, t = lane & 3;
-#pragma unroll
-  for (int ks = 0; ks < K / 8; ++ks) {
-    float af[4];
-    if (!TRANS_A) {
-      af[0] = a[g * lda + ks * 8 + t]; af[1] = a[(g + 8) * lda + ks * 8 + t];
-      af[2] = a[g * lda + ks * 8 + t + 4]; af[3] = a[(g + 8) * lda + ks * 8 + t + 4];
-    } else {
-      af[0] = a[(ks * 8 + t) * lda + g]; af[1] = a[(ks * 8 + t) * lda + g + 8];
-      af[2] = a[(ks * 8 + t + 4) * lda + g]; af[3] = a[(ks * 8 + t + 4) * lda + g + 8];
-    }
-#pragma unroll
-    for (int nt = 0; nt < NT; ++nt) {
-      float bf[2];
-      if (!NN) { bf[0] = b[(nt * 8 + g) * ldb + ks * 8 + t]; bf[1] = b[(nt * 8 + g) * ldb + ks * 8 + t + 4]; }
-      else { bf[0] = b[(ks * 8 + t) * ldb + nt * 8 + g]; bf[1] = b[(ks * 8 + t + 4) * ldb + nt * 8 + g]; }
-      mma_tf32(acc[nt], af, bf);
-    }
-  }
-}
-
-__global__ void __launch_bounds__(128, 3) attn_core_bwd_mma_kernel(const AttnCoreBwdParams p, float* __restrict__ att_out) {
-  using namespace cb;
-  extern __shared__ float sm[];
-  const AttnGeom g_ = p.g;
-  const int S = g_.S(), nwin = g_.nwin(), W2 = 2 * g_.win - 1, nb = W2 * W2 + 1, R = g_.R, win = g_.win;
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int wl = warp;
-  const int g = lane >> 2, t = lane & 3;
-  float* base = sm;
-  float* sQ = base; float* sK = sQ + SM * LD; float* sV = sK + SM * LD; float* sdO = sV + SM * LD;
-  float* sP = sdO + SM * LD; float* sDS = sP + SM * LDP;
-  float* inq = sDS + SM * LDP; float* ink = inq + SM;
-  float* sbias = sm + SLOT_FLOATS;         // [nb]
-  float* dbias = sbias + nb;               // [nb]
-  float* gred = dbias + nb;                // [2][DH]
-  const int n = blockIdx.x / p.heads, hd = blockIdx.x - n * p.heads;
-  const int inner = p.heads * DH;
-  const float rs = sqrtf((float)DH);
-  for (int i = threadIdx.x; i < nb; i += 128) { sbias[i] = p.bias_table[i * p.heads + hd]; dbias[i] = 0.f; }
-  if (threadIdx.x < 2 * DH) gred[threadIdx.x] = 0.f;
-  const float gq_l = p.qgamma[hd * DH + lane], gk_l = p.kgamma[hd * DH + lane];
-  // per-thread gamma-gradient accumulators for the fragment columns d = nt*8 + 2t (+1)
-  float dgq[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, dgk[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
-  __syncthreads();
-  const int r0 = wl * 16;                  // first row (query or key) of this warp's m-tile
-  // relative-position-bias index of (query i, key j) = base(i) - off(j) for window tokens, nb-1 when either is a
-  // register token (maxvit.py:160-167).  This thread's two query rows and 16 key columns never change: hoist.
-  const int ia = r0 + g, ib = r0 + g + 8;
-  int base_a = -1, base_b = -1;            // -1: register / padded query row -> shared last entry
-  if (ia >= R && ia < S) { const int ti = ia - R, a = ti / win, b = ti - a * win; base_a = (a + win - 1) * W2 + (b + win - 1); }
-  if (ib >= R && ib < S) { const int ti = ib - R, a = ti / win, b = ti - a * win; base_b = (a + win - 1) * W2 + (b + win - 1); }
-  int offj[16];                            // key j = nt*8 + 2t + e  ->  off(j), or -1 for register / padded keys
-#pragma unroll
-  for (int k = 0; k < 16; ++k) {
-    const int j = (k >> 1) * 8 + 2 * t + (k & 1);
-    offj[k] = -1;
-    if (j >= R && j < S) { const int tj = j - R, a = tj / win, b = tj - a * win; offj[k] = a * W2 + b; }
-  }
-
-  for (int wi = 0; wi < nwin; ++wi) {
-    {
-      const long long row0 = ((long long)n * nwin + wi) * S;
-      // ---------------- phase 1: rows r0..r0+15, lane = d; all loads are issued before the first use
-      {
-        float qv[16], kv[16], vv[16], dov[16];
-#pragma unroll
-        for (int r = 0; r < 16; ++r) {
-          const int i = r0 + r;
-          qv[r] = kv[r] = vv[r] = dov[r] = 0.f;
-          if (i < S) {
-            const float* src = p.qkv + (row0 + i) * 3 * inner + hd * DH + lane;
-            qv[r] = __ldg(src); kv[r] = __ldg(src + inner); vv[r] = __ldg(src + 2 * inner);
-            dov[r] = __ldg(p.datt + (row0 + i) * inner + hd * DH + lane);
-          }
-        }
-#pragma unroll
-        for (int r = 0; r < 16; ++r) {
-          const int i = r0 + r;
-          const float nq = fmaxf(sqrtf(warp_sum(qv[r] * qv[r])), 1e-12f), nk = fmaxf(sqrtf(warp_sum(kv[r] * kv[r])), 1e-12f);
-          sQ[i * LD + lane] = qv[r] / nq * rs * gq_l; sK[i * LD + lane] = kv[r] / nk * rs * gk_l;
-          sV[i * LD + lane] = vv[r]; sdO[i * LD + lane] = dov[r];
-          if (lane == 0) { inq[i] = 1.0f / nq; ink[i] = 1.0f / nk; }
-        }
-      }
-      __syncthreads();
-      // ---------------- phase 2: my 16 query rows x 64 keys
-      float pr[8][4];
-#pragma unroll
-      for (int nt = 0; nt < 8; ++nt) pr[nt][0] = pr[nt][1] = pr[nt][2] = pr[nt][3] = 0.f;
-      warp_mma<8, DH, false, false>(pr, sQ + r0 * LD, LD, sK, LD, lane);
-      {
-        float ma = -INFINITY, mb = -INFINITY;
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const int j = nt * 8 + 2 * t + e;
-            if (j < S) {
-              const int oj = offj[nt * 2 + e];
-              const int bxa = (oj >= 0 && base_a >= 0) ? base_a - oj : nb - 1, bxb = (oj >= 0 && base_b >= 0) ? base_b - oj : nb - 1;
-              pr[nt][e] += sbias[bxa]; pr[nt][2 + e] += sbias[bxb];
-              ma = fmaxf(ma, pr[nt][e]); mb = fmaxf(mb, pr[nt][2 + e]);
-            } else { pr[nt][e] = -INFINITY; pr[nt][2 + e] = -INFINITY; }
-          }
-        ma = fmaxf(ma, __shfl_xor_sync(0xffffffffu, ma, 1)); ma = fmaxf(ma, __shfl_xor_sync(0xffffffffu, ma, 2));
-        mb = fmaxf(mb, __shfl_xor_sync(0xffffffffu, mb, 1)); mb = fmaxf(mb, __shfl_xor_sync(0xffffffffu, mb, 2));
-        float sa = 0.f, sb = 0.f;
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt)
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            pr[nt][e] = __expf(pr[nt][e] - ma); pr[nt][2 + e] = __expf(pr[nt][2 + e] - mb);
-            sa += pr[nt][e]; sb += pr[nt][2 + e];
-          }
-        sa += __shfl_xor_sync(0xffffffffu, sa, 1); sa += __shfl_xor_sync(0xffffffffu, sa, 2);
-        sb += __shfl_xor_sync(0xffffffffu, sb, 1); sb += __shfl_xor_sync(0xffffffffu, sb, 2);
-        const float ia_ = ia < S ? 1.0f / sa : 0.f, ib_ = ib < S ? 1.0f / sb : 0.f;    // padded query rows: P = 0
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-          pr[nt][0] *= ia_; pr[nt][1] *= ia_; pr[nt][2] *= ib_; pr[nt][3] *= ib_;
-          *reinterpret_cast<float2*>(sP + ia * LDP + nt * 8 + 2 * t) = make_float2(pr[nt][0], pr[nt][1]);
-          *reinterpret_cast<float2*>(sP + ib * LDP + nt * 8 + 2 * t) = make_float2(pr[nt][2], pr[nt][3]);
-        }
-        __syncwarp();
-        if (att_out) {                                              // att = P V (forward output, for the to_out weight gradient)
-          float av[4][4];
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) av[nt][0] = av[nt][1] = av[nt][2] = av[nt][3] = 0.f;
-          warp_mma<4, SM, false, true>(av, sP + r0 * LDP, LDP, sV, LD, lane);
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) {
-            if (ia < S) *reinterpret_cast<float2*>(att_out + (row0 + ia) * inner + hd * DH + nt * 8 + 2 * t) = make_float2(av[nt][0], av[nt][1]);
-            if (ib < S) *reinterpret_cast<float2*>(att_out + (row0 + ib) * inner + hd * DH + nt * 8 + 2 * t) = make_float2(av[nt][2], av[nt][3]);
-          }
-        }
-        // dP = dO V^T, dS = P * (dP - rowdot)
-        float dp[8][4];
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) dp[nt][0] = dp[nt][1] = dp[nt][2] = dp[nt][3] = 0.f;
-        warp_mma<8, DH, false, false>(dp, sdO + r0 * LD, LD, sV, LD, lane);
-        float da = 0.f, db = 0.f;
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) { da += pr[nt][0] * dp[nt][0] + pr[nt][1] * dp[nt][1]; db += pr[nt][2] * dp[nt][2] + pr[nt][3] * dp[nt][3]; }
-        da += __shfl_xor_sync(0xffffffffu, da, 1); da += __shfl_xor_sync(0xffffffffu, da, 2);
-        db += __shfl_xor_sync(0xffffffffu, db, 1); db += __shfl_xor_sync(0xffffffffu, db, 2);
-#pragma unroll
-        for (int nt = 0; nt < 8; ++nt) {
-#pragma unroll
-          for (int e = 0; e < 2; ++e) {
-            const int j = nt * 8 + 2 * t + e;
-            const float dsa = pr[nt][e] * (dp[nt][e] - da), dsb = pr[nt][2 + e] * (dp[nt][2 + e] - db);
-            dp[nt][e] = dsa; dp[nt][2 + e] = dsb;
-            if (j < S) {
-              const int oj = offj[nt * 2 + e];
-              const int bxa = (oj >= 0 && base_a >= 0) ? base_a - oj : nb - 1, bxb = (oj >= 0 && base_b >= 0) ? base_b - oj : nb - 1;
-              if (ia < S) atomicAdd(&dbias[bxa], dsa);
-              if (ib < S) atomicAdd(&dbias[bxb], dsb);
-            }
-          }
-          *reinterpret_cast<float2*>(sDS + ia * LDP + nt * 8 + 2 * t) = make_float2(dp[nt][0], dp[nt][1]);
-          *reinterpret_cast<float2*>(sDS + ib * LDP + nt * 8 + 2 * t) = make_float2(dp[nt][2], dp[nt][3]);
-        }
-      }
-      __syncthreads();
-      // ---------------- phase 3: rows r0..r0+15 as keys (dV, dKh) and as queries (dQh)
-      {
-        float acc[4][4];
-        // dV[j][d] = sum_i P[i][j] dO[i][d]
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
-        warp_mma<4, SM, true, true>(acc, sP + r0, LDP, sdO, LD, lane);
-#pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
-          if (ia < S) *reinterpret_cast<float2*>(p.dqkv + (row0 + ia) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t) = make_float2(acc[nt][0], acc[nt][1]);
-          if (ib < S) *reinterpret_cast<float2*>(p.dqkv + (row0 + ib) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t) = make_float2(acc[nt][2], acc[nt][3]);
-        }
-        // which = 0: dQh = dS Kh (rows = queries);  which = 1: dKh = dS^T Qh (rows = keys); then RMSNorm backward
-#pragma unroll
-        for (int which = 0; which < 2; ++which) {
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
-          if (which == 0) warp_mma<4, SM, false, true>(acc, sDS + r0 * LDP, LDP, sK, LD, lane);
-          else warp_mma<4, SM, true, true>(acc, sDS + r0, LDP, sQ, LD, lane);
-          const float* gam = which == 0 ? p.qgamma : p.kgamma;
-          const float* inv = which == 0 ? inq : ink;
-          float* dg = which == 0 ? dgq : dgk;
-          float ua[8], ub[8], ga[8], gb[8], dota = 0.f, dotb = 0.f;
-          const float inva = inv[ia], invb = inv[ib];
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) {
-            const int d = nt * 8 + 2 * t;
-            float2 xa = make_float2(0.f, 0.f), xb = make_float2(0.f, 0.f);
-            if (ia < S) xa = *reinterpret_cast<const float2*>(p.qkv + (row0 + ia) * 3 * inner + which * inner + hd * DH + d);
-            if (ib < S) xb = *reinterpret_cast<const float2*>(p.qkv + (row0 + ib) * 3 * inner + which * inner + hd * DH + d);
-            const float g0 = gam[hd * DH + d], g1 = gam[hd * DH + d + 1];
-            ua[2 * nt] = xa.x * inva; ua[2 * nt + 1] = xa.y * inva; ub[2 * nt] = xb.x * invb; ub[2 * nt + 1] = xb.y * invb;
-            dg[2 * nt] += (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs;
-            dg[2 * nt + 1] += (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
-            ga[2 * nt] = acc[nt][0] * rs * g0; ga[2 * nt + 1] = acc[nt][1] * rs * g1;
-            gb[2 * nt] = acc[nt][2] * rs * g0; gb[2 * nt + 1] = acc[nt][3] * rs * g1;
-            dota += ga[2 * nt] * ua[2 * nt] + ga[2 * nt + 1] * ua[2 * nt + 1];
-            dotb += gb[2 * nt] * ub[2 * nt] + gb[2 * nt + 1] * ub[2 * nt + 1];
-          }
-          dota += __shfl_xor_sync(0xffffffffu, dota, 1); dota += __shfl_xor_sync(0xffffffffu, dota, 2);
-          dotb += __shfl_xor_sync(0xffffffffu, dotb, 1); dotb += __shfl_xor_sync(0xffffffffu, dotb, 2);
-#pragma unroll
-          for (int nt = 0; nt < 4; ++nt) {
-            const int d = nt * 8 + 2 * t;
-            if (ia < S) *reinterpret_cast<float2*>(p.dqkv + (row0 + ia) * 3 * inner + which * inner + hd * DH + d) =
-                make_float2(inva * (ga[2 * nt] - ua[2 * nt] * dota), inva * (ga[2 * nt + 1] - ua[2 * nt + 1] * dota));
-            if (ib < S) *reinterpret_cast<float2*>(p.dqkv + (row0 + ib) * 3 * inner + which * inner + hd * DH + d) =
-                make_float2(invb * (gb[2 * nt] - ub[2 * nt] * dotb), invb * (gb[2 * nt + 1] - ub[2 * nt + 1] * dotb));
-          }
-        }
-      }
-      __syncthreads();
-    }
-  }
-  // gamma gradients: reduce over the 8 row groups of the warp (lanes with equal t), then over warps
-#pragma unroll
-  for (int k = 0; k < 8; ++k) {
-    float a = dgq[k], b = dgk[k];
-    a += __shfl_xor_sync(0xffffffffu, a, 4); a += __shfl_xor_sync(0xffffffffu, a, 8); a += __shfl_xor_sync(0xffffffffu, a, 16);
-    b += __shfl_xor_sync(0xffffffffu, b, 4); b += __shfl_xor_sync(0xffffffffu, b, 8); b += __shfl_xor_sync(0xffffffffu, b, 16);
-    if (g == 0) {
-      const int d = (k >> 1) * 8 + 2 * t + (k & 1);
-      atomicAdd(&gred[d], a); atomicAdd(&gred[DH + d], b);
-    }
-  }
-  __syncthreads();
-  if (threadIdx.x < 2 * DH) {
-    const int which = threadIdx.x / DH, d = threadIdx.x % DH;
-    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, gred[threadIdx.x]);
-  }
-  for (int i = threadIdx.x; i < nb; i += 128) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
-}
-
-// ------------------------------------------------------------------------------------------------
-// bf16 version of the tensor-core core backward: mma.sync m16n8k16 (fp32 accumulate) with ldmatrix operand fetch
-// (transposed operands come for free from ldmatrix.trans), half the shared memory of the tf32 kernel (4-5 blocks per SM)
-// and ~4x fewer instructions.  Same phases and work split as attn_core_bwd_mma_kernel.  The relative-position-bias
-// gradient of a thread's 32 fixed (query, key) pairs is accumulated in registers over the field's windows.
+// The 53 valid tokens are padded to 64 with zero rows; padded keys are masked to -inf before the softmax.  The
+// relative-position-bias gradient of a thread's 32 fixed (query, key) pairs is accumulated in registers over the field's windows.
 // ------------------------------------------------------------------------------------------------
 namespace cbh {
 constexpr int DH = 32, SM = 64;
@@ -1635,14 +1376,14 @@ int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma,
                          const AttnGeom& g, int heads, void* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                          void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
 
-// use_tf32: 0 exact-fp32 SIMT, 1 tf32 mma.sync, 2 bf16 mma.sync on fp32 tensors, 3 bf16 tensors (qkv, datt, dqkv, att_out): the
+// use_tf32: 0 exact-fp32 SIMT, 2 bf16 mma.sync on fp32 tensors, 3 bf16 tensors (qkv, datt, dqkv, att_out): the
 // tcgen05 kernel (vg_attn_bwd_tc.cu); VG_ATTN_BWD_TC=0 or a shape outside it selects the bf16 mma.sync kernel
 int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                       const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                       int use_tf32, float* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
   if (dh != 32) return set_error("attn_core_bwd: dim_head must be 32 (got %d)", dh);
   if (drop_thresh < 0 || drop_thresh > 255) return set_error("attn_core_bwd: dropout threshold %d outside [0, 255]", drop_thresh);
-  if (drop_thresh && use_tf32 == 1) return set_error("attn_core_bwd: dropout is built into the bf16 tensor-core kernels (modes 2, 3) and the exact-fp32 kernel (mode 0)");
+  if (use_tf32 != 0 && use_tf32 != 2 && use_tf32 != 3) return set_error("attn_core_bwd: mode %d (0 exact fp32, 2 bf16 mma on fp32 tensors, 3 bf16 tensors)", use_tf32);
   if (g.S() > 64) return set_error("attn_core_bwd: sequence %d > 64", g.S());
   const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
   if (use_tf32 == 3) {
@@ -1672,22 +1413,7 @@ int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, 
     else attn_core_bwd_bf16_kernel<false><<<g.N * heads, 128, smem3, st>>>(q, att_out, make_drop(seed, salt, drop_thresh));
     return check_launch("attn_core_bwd_bf16_kernel");
   }
-  if (use_tf32) {
-    const size_t smem2 = (size_t)(cb::SLOT_FLOATS + 2 * nb + 2 * cb::DH) * sizeof(float);
-    static PerDeviceSize attr2_pd;                  // depends on the window size: raise the limit when it grows
-    size_t& attr2 = attr2_pd.cur();
-    if (smem2 > attr2) {
-      cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2);
-      if (e != cudaSuccess) return set_error("attn_core_bwd_mma smem attr: %s", cudaGetErrorString(e));
-      attr2 = smem2;
-    }
-    AttnCoreBwdParams q;
-    q.qkv = qkv; q.datt = datt; q.qgamma = qgamma; q.kgamma = kgamma; q.bias_table = bias_table; q.dqkv = dqkv;
-    q.dqgamma = dqgamma; q.dkgamma = dkgamma; q.dbias_table = dbias_table; q.g = g; q.heads = heads;
-    attn_core_bwd_mma_kernel<<<g.N * heads, 128, smem2, st>>>(q, att_out);
-    return check_launch("attn_core_bwd_mma_kernel");
-  }
-  if (att_out) return set_error("attn_core_bwd: att_out is only produced by the tf32 kernel");
+  if (att_out) return set_error("attn_core_bwd: att_out is only produced by the tensor-core kernels (modes 2, 3)");
   const size_t smem = (size_t)(8 * 64 * 33 + 64 * 65 + 2 * nb + 128 + 8 * 2 * 32 + (drop_thresh ? 64 * 65 : 0)) * sizeof(float);
   static PerDeviceSize attr_pd;                  // depends on the window size: raise the limit when it grows
   size_t& attr = attr_pd.cur();

@@ -222,8 +222,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 // The generic kernel above re-reads the A operand from L2 once per tap (9x).  Here a tile of 256 output pixels loads
 // its input rows ONCE, with the halo of P+1 rows on each side, as two [HR rows x 128 B] channel-block tiles
 // (SWIZZLE_128B, written by TMA); tap (dy,dx) is then the same smem tile addressed through a UMMA descriptor whose
-// start address is shifted by (P+1 + dy*P + dx) rows (128 B each; the descriptor's base-offset field carries the
-// swizzle phase of the shifted start).  Only the weights (16 KiB per tap and channel block) stream through a ring.
+// start address is shifted by (P+1 + dy*P + dx) rows (128 B each; the descriptor's base-offset field stays 0: the 128B
+// swizzle is applied to absolute shared-memory address bits, so a row-shifted start into a 1024-B-aligned tile needs no
+// phase correction -- measured on B200).  Only the weights (16 KiB per tap and channel block) stream through a ring.
 // K order: channel block 0 taps 0..8, then channel block 1 taps 0..8, so each A half-buffer is reloaded for the next
 // tile while the other half is being consumed.  L2->SM traffic per 256-pixel tile: 100 KiB (A) + 288 KiB (B)
 // instead of 576 + 288 KiB.
@@ -233,15 +234,12 @@ constexpr int HB_STAGES = 3;                                  // weight ring
 constexpr int HALO_RES_BYTES = 8 * 2 * 4096;                  // per epilogue warp: two [32 rows][128 B] fp32 residual chunks (TMA)
 constexpr int HALO_A_BYTES = HALO_MAX_ROWS * 128;             // per channel block
 constexpr int HALO_SMEM_BYTES = 2 * HALO_A_BYTES + HB_STAGES * B_BYTES + HALO_RES_BYTES + PARAM_FLOATS * 4 + 1024 + 256;
-static int g_halo_base_offset = 0;   // measured on B200: the 128B swizzle is applied to absolute smem address bits, so a
-                                     // row-shifted start into a 1024-B-aligned tile needs base_offset = 0 (1 gives wrong results)
 
 struct HaloShape {
   long long M;          // flat pixels (rows of the [q][128] matrices)
   int num_tiles;        // 256-pixel tiles
   int P;                // row pitch (pixels)
   int HR;               // halo rows loaded per tile (multiple of 16)
-  int use_base_offset;
   int res_tma;          // the fp32 residual arrives through mapR (else: per-thread global loads)
   int flip;             // data gradient: tap t of the weights is applied with the input shift of tap 8 - t (the negated shift)
   int out2_tma;         // the fp32 copy of the output leaves through mapO (TMA tensor stores from the residual buffers)
@@ -332,8 +330,7 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             mbar_wait(full + stage, phase);
             tc_fence_after();
             if (elect_one()) {
-              uint64_t da0 = umma_desc_k128_shift(sa, r0), da1 = umma_desc_k128_shift(sa, r0 + 128);
-              if (hs.use_base_offset) { da0 |= (uint64_t)(r0 & 7) << 49; da1 |= (uint64_t)((r0 + 128) & 7) << 49; }
+              const uint64_t da0 = umma_desc_k128_shift(sa, r0), da1 = umma_desc_k128_shift(sa, r0 + 128);
               const uint64_t db = umma_desc_k128(smem_u32(sB + stage * B_BYTES));
 #pragma unroll
               for (int k = 0; k < 4; ++k) {
@@ -394,204 +391,6 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
   tc_fence_before();
   __syncthreads();
   if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, TMEM_COLS); }
-}
-
-// ------------------------------------------------------------------------------------------------
-// The same convolution on CTA PAIRS (tcgen05 cta_group::2), built to test whether the shared-memory port bounds the
-// single-CTA kernel (an M128 x N128 x K16 MMA needs 128 B/clk of operands, the port's width; per 256-pixel tile 1 152 KB of
-// operand reads + 392 KB of TMA writes).  Two CTAs of a cluster work on two adjacent 256-pixel tiles with ONE stream of
-// M256 x N128 instructions issued by the leader: each CTA supplies its own 128 A rows and HALF of the weight tile (64 of the
-// 128 output channels), so per CTA an instruction reads 4 + 2 KB instead of 4 + 4 KB and the weight ring carries 8 KB
-// stages.  Result on B200: bit-identical outputs, no speed-up (1.28 vs 1.18 ms) -- the port is not the bound; kept as an
-// opt-in (VG_CONV_PAIR=1) and as the base for wider tiles.  Protocol (after DeepGEMM / CUTLASS 2-SM kernels):
-//   * both CTAs run a TMA producer; every load signals the LEADER's full barrier (cta_group::2 TMA, peer bit of the barrier
-//     address cleared), which the leader arms with the bytes of both CTAs;
-//   * the leader's MMA thread issues for the pair; tcgen05.commit is multicast to the barriers of both CTAs (operand slots
-//     free, accumulator ready);
-//   * both CTAs run the epilogue on their own TMEM; "accumulator drained" arrivals of all 16 epilogue warps go to the leader.
-// ------------------------------------------------------------------------------------------------
-constexpr int HB2_STAGES = 6;                                 // weight ring, 8 KiB per stage and CTA
-constexpr int B2_BYTES = B_BYTES / 2;
-constexpr int HALO2_BAR_BYTES = 512;
-constexpr int HALO2_SMEM_BYTES = 2 * HALO_A_BYTES + HB2_STAGES * B2_BYTES + HALO_RES_BYTES + PARAM_FLOATS * 4 + 1024 + HALO2_BAR_BYTES;
-constexpr uint32_t PEER_BIT_MASK = 0xFEFFFFFFu;               // shared::cluster address -> the same offset in the pair's even CTA
-
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t* dst_smem, uint32_t ncols) {
-  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish2() { asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t ncols) {
-  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
-}
-// TMA load into THIS CTA's shared memory whose bytes are counted on the pair leader's mbarrier
-__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, uint64_t* bar, int c0, int c1) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-      ::"r"(smem_u32(dst)), "l"(m), "r"(smem_u32(bar) & PEER_BIT_MASK), "r"(c0), "r"(c1) : "memory");
-}
-__device__ __forceinline__ void tc_mma_bf16_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
-}
-// completion of all prior MMAs of the pair -> one arrival on the barrier at this offset in BOTH CTAs
-__device__ __forceinline__ void tc_commit_pair(uint64_t* bar) {
-  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"((unsigned short)3) : "memory");
-}
-// arrive on the LEADER's copy of a barrier (works from either CTA of the pair)
-__device__ __forceinline__ void mbar_arrive_leader(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(smem_u32(bar) & PEER_BIT_MASK) : "memory");
-}
-
-template <bool TRAIN>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-conv_halo2_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                  const __grid_constant__ CUtensorMap mapR, const HaloShape hs, const EpiParams ep) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint8_t* sB = smem + 2 * HALO_A_BYTES;
-  uint8_t* sres = sB + HB2_STAGES * B2_BYTES;
-  float* sparam = reinterpret_cast<float*>(sres + HALO_RES_BYTES);
-  uint64_t* full = reinterpret_cast<uint64_t*>(sres + HALO_RES_BYTES + PARAM_FLOATS * 4);
-  uint64_t* empty = full + HB2_STAGES;
-  uint64_t* a_full = empty + HB2_STAGES;   // [2]
-  uint64_t* a_free = a_full + 2;           // [2]
-  uint64_t* tfull = a_free + 2;            // [2]
-  uint64_t* tempty = tfull + 2;            // [2]  (the leader's copy is the live one: 16 arrivals)
-  uint64_t* res_full = tempty + 2;         // [8 epilogue warps][2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(res_full + 16);
-
-  const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
-  const int lane = threadIdx.x & 31;
-  const uint32_t rank = cluster_ctarank();
-  const int pair = blockIdx.x >> 1, npairs_grid = gridDim.x >> 1;
-  const int n_pair_tiles = (hs.num_tiles + 1) >> 1;
-
-  if (warp == 0 && lane == 0) { tma_prefetch_desc(&mapA); tma_prefetch_desc(&mapB); if (hs.res_tma) tma_prefetch_desc(&mapR); }
-  if (warp == 1 && lane == 0) {
-    for (int s = 0; s < HB2_STAGES; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(a_full + s, 1); mbar_init(a_free + s, 1); mbar_init(tfull + s, 1); mbar_init(tempty + s, 16); }
-    for (int s = 0; s < 16; ++s) mbar_init(res_full + s, 1);
-    fence_mbar_init();
-  }
-  if (warp == 2) { tmem_alloc2(tmem_slot, TMEM_COLS); tmem_relinquish2(); }
-  for (int i = threadIdx.x; i < 128; i += TC_THREADS) {
-    sparam[i] = ep.bias[i]; sparam[128 + i] = ep.ln_g[i]; sparam[256 + i] = ep.ln_b[i];
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                                        // the peer's barriers are initialised before anything signals them
-  tc_fence_after();
-  const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);
-  const int halo = hs.P + 1;
-
-  if (warp == 0) {
-    if (lane == 0) {                                         // ===== TMA producer (both CTAs) =====
-      int stage = 0; uint32_t phase = 0; uint32_t it = 0;
-      const int half_rows = hs.HR / 2;
-      for (int pt = pair; pt < n_pair_tiles; pt += npairs_grid, ++it) {
-        const long long q0 = ((long long)pt * 2 + rank) * BM;
-        for (int cb = 0; cb < 2; ++cb) {
-          mbar_wait(a_free + cb, (it & 1) ^ 1);
-          if (rank == 0) mbar_arrive_expect_tx(a_full + cb, 2 * hs.HR * 128);      // the bytes of both CTAs
-          uint8_t* sa = smem + cb * HALO_A_BYTES;
-          tma_load_2d_pair(sa, &mapA, a_full + cb, cb * 64, (int)(q0 - halo));
-          tma_load_2d_pair(sa + half_rows * 128, &mapA, a_full + cb, cb * 64, (int)(q0 - halo + half_rows));
-          for (int tap = 0; tap < 9; ++tap) {
-            mbar_wait(empty + stage, phase ^ 1);
-            if (rank == 0) mbar_arrive_expect_tx(full + stage, 2 * B2_BYTES);
-            tma_load_2d_pair(sB + stage * B2_BYTES, &mapB, full + stage, tap * 128 + cb * 64, (int)rank * 64);   // this CTA's 64 output channels
-            if (++stage == HB2_STAGES) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    if (rank == 0) {                                         // ===== MMA issuer (leader CTA, for the pair): converged warp, elected lane issues =====
-      constexpr uint32_t idesc = umma_idesc_bf16(256, BN);
-      int stage = 0; uint32_t phase = 0; uint32_t it = 0;
-      for (int pt = pair; pt < n_pair_tiles; pt += npairs_grid, ++it) {
-        const int as = it & 1; const uint32_t aphase = (it >> 1) & 1;
-        mbar_wait(tempty + as, aphase ^ 1);
-        tc_fence_after();
-        const uint32_t d0 = tmem_base + as * 256, d1 = d0 + 128;
-        for (int cb = 0; cb < 2; ++cb) {
-          mbar_wait(a_full + cb, it & 1);
-          tc_fence_after();
-          const uint32_t sa = smem_u32(smem + cb * HALO_A_BYTES);
-          for (int tap = 0; tap < 9; ++tap) {
-            const int r0 = halo + (tap / 3 - 1) * hs.P + (tap % 3 - 1);
-            mbar_wait(full + stage, phase);
-            tc_fence_after();
-            if (elect_one()) {
-              uint64_t da0 = umma_desc_k128_shift(sa, r0), da1 = umma_desc_k128_shift(sa, r0 + 128);
-              if (hs.use_base_offset) { da0 |= (uint64_t)(r0 & 7) << 49; da1 |= (uint64_t)((r0 + 128) & 7) << 49; }
-              const uint64_t db = umma_desc_k128(smem_u32(sB + stage * B2_BYTES));
-#pragma unroll
-              for (int k = 0; k < 4; ++k) {
-                const uint32_t acc = (cb | tap | k) ? 1u : 0u;
-                tc_mma_bf16_pair(d0, da0 + 2 * k, db + 2 * k, idesc, acc);
-                tc_mma_bf16_pair(d1, da1 + 2 * k, db + 2 * k, idesc, acc);
-              }
-              tc_commit_pair(empty + stage);
-              if (tap == 8) {
-                tc_commit_pair(a_free + cb);
-                if (cb == 1) tc_commit_pair(tfull + as);
-              }
-            }
-            __syncwarp();
-            if (++stage == HB2_STAGES) { stage = 0; phase ^= 1; }
-          }
-        }
-      }
-    }
-  } else if (warp >= 4) {                                    // ===== epilogue (both CTAs, own tile) =====
-    const int lg = warp & 3;
-    const int e = (warp - 4) >> 2;
-    EpiCtx cx;
-    cx.bias = sparam; cx.ln_g = sparam + 128; cx.ln_b = sparam + 256; cx.gb = nullptr; cx.n_first = 0; cx.params_smem = true;
-    const long long tile_stride = (long long)npairs_grid * 2 * BM;
-    if (hs.res_tma) {
-      cx.res_map = &mapR; cx.res_buf = sres + (warp - 4) * 8192; cx.res_bar = res_full + (warp - 4) * 2;
-      if (lane == 0 && pair < n_pair_tiles) {
-        const int r0 = (int)(((long long)pair * 2 + rank) * BM + e * 128 + lg * 32);
-        for (int c = 0; c < 2; ++c) {
-          mbar_arrive_expect_tx(cx.res_bar + c, 4096);
-          tma_load_2d(cx.res_buf + c * 4096, &mapR, cx.res_bar + c, c * 32, r0);
-        }
-      }
-    }
-    uint32_t it = 0;
-    for (int pt = pair; pt < n_pair_tiles; pt += npairs_grid, ++it) {
-      const long long row = ((long long)pt * 2 + rank) * BM + e * 128 + lg * 32 + lane;
-      const bool ok = row < hs.M;
-      const int as = it & 1; const uint32_t aphase = (it >> 1) & 1;
-      if (hs.res_tma) {
-        cx.res_g0 = it * 4; cx.res_row0 = row - lane;
-        cx.res_next_row0 = (pt + npairs_grid < n_pair_tiles) ? cx.res_row0 + tile_stride : -1;
-      } else {
-        epi_conv_ln_prefetch<bf16>(ep, row, ok);
-      }
-      mbar_wait(tfull + as, aphase);
-      tc_fence_after();
-      TmemLoader ld{tmem_base + as * 256 + e * 128 + ((uint32_t)(lg * 32) << 16)};
-      run_epilogue<TRAIN ? EPI_CONV_LN_TRAIN : EPI_CONV_LN, bf16>(ep, cx, row, ok, 0, ld);
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive_leader(tempty + as);
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                                        // the peer may still read this CTA's shared memory / signal its barriers
-  if (warp == 2) { tc_fence_after(); tmem_dealloc2(tmem_base, TMEM_COLS); }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -748,16 +547,10 @@ int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const Ep
   const int train = mode_k == 1;
   const int HR = ((BM + 2 * (P + 1)) + 15) / 16 * 16;
   if (HR > HALO_MAX_ROWS) return -1;
-  static int mode = -1;
-  if (mode < 0) { const char* e = getenv("VG_CONV_HALO"); mode = (e && e[0] == '0') ? 0 : 1;
-                  const char* b = getenv("VG_HALO_BASEOFF"); if (b) g_halo_base_offset = (b[0] != '0'); }
-  if (!mode) return -1;
-  static int res_tma_mode = -1;
-  if (res_tma_mode < 0) { const char* e = getenv("VG_CONV_RES_TMA"); res_tma_mode = (e && e[0] == '0') ? 0 : 1; }
   CUtensorMap ma, mb, mr;
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) return set_error("cuTensorMapEncodeTiled entry point unavailable");
-  const bool res_tma = mode_k != 2 && res_tma_mode && ep.res && ep.res_f32 && ep.ldres == 128 && (reinterpret_cast<uintptr_t>(ep.res) & 15) == 0;
+  const bool res_tma = mode_k != 2 && ep.res && ep.res_f32 && ep.ldres == 128 && (reinterpret_cast<uintptr_t>(ep.res) & 15) == 0;
   if (res_tma) {
     int rc = make_map_2d(&mr, true, ep.res, 128, M, 32);
     if (rc) return rc;
@@ -775,7 +568,7 @@ int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const Ep
   int rc = make_map_2d(&mb, false, Wt, 9 * 128, 128, BN);
   if (rc) return rc;
   HaloShape hs;
-  hs.M = M; hs.num_tiles = (int)((hs.M + BM - 1) / BM); hs.P = P; hs.HR = HR; hs.use_base_offset = g_halo_base_offset; hs.res_tma = res_tma ? 1 : 0;
+  hs.M = M; hs.num_tiles = (int)((hs.M + BM - 1) / BM); hs.P = P; hs.HR = HR; hs.res_tma = res_tma ? 1 : 0;
   hs.flip = flip;
   // fp32 copy through TMA stores (needs the residual buffers: residual launches only); VG_CONV_OUT2_TMA=0 restores the per-thread stores
   const char* o2e = getenv("VG_CONV_OUT2_TMA");             // read per call so one process can compare the two
@@ -798,36 +591,6 @@ int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const Ep
   }
   const int grid = hs.num_tiles < num_sms() ? hs.num_tiles : num_sms();
   if (!res_tma) mr = ma;                                     // unused by the kernel
-  // VG_CONV_PAIR=1 selects the CTA-pair kernel (cta_group::2); read per call so a process can compare the two.  Off by
-  // default: on B200 it measures 1.28 ms against 1.18 ms -- the single-CTA kernel already runs at 0.81 of the sustained
-  // (power-capped) bf16 peak, so halving the weight-tile traffic buys nothing (profiles/r01_summary.md).
-  const char* pe = getenv("VG_CONV_PAIR");
-  const bool pair_mode = pe && pe[0] == '1' && mode_k != 2;
-  if (pair_mode && num_sms() >= 2) {
-    CUtensorMap mb2;
-    rc = make_map_2d(&mb2, false, Wt, 9 * 128, 128, 64);     // half of the output channels per CTA
-    if (rc) return rc;
-    static PerDeviceFlag attr2_pd;
-    bool& attr2 = attr2_pd.cur();
-    if (!attr2) {
-      cudaError_t e = cudaFuncSetAttribute(conv_halo2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, HALO2_SMEM_BYTES);
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_halo2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, HALO2_SMEM_BYTES);
-      if (e != cudaSuccess) return set_error("cudaFuncSetAttribute(conv_halo2): %s", cudaGetErrorString(e));
-      attr2 = true;
-    }
-    const int n_pair_tiles = (hs.num_tiles + 1) / 2;
-    const int max_pairs = num_sms() / 2;
-    const int pairs = n_pair_tiles < max_pairs ? n_pair_tiles : max_pairs;
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(2 * pairs)); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = HALO2_SMEM_BYTES; cfg.stream = st;
-    cudaLaunchAttribute at[1];
-    at[0].id = cudaLaunchAttributeClusterDimension; at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-    cfg.attrs = at; cfg.numAttrs = 1;
-    cudaError_t le = train ? cudaLaunchKernelEx(&cfg, conv_halo2_kernel<true>, ma, mb2, mr, hs, ep)
-                           : cudaLaunchKernelEx(&cfg, conv_halo2_kernel<false>, ma, mb2, mr, hs, ep);
-    if (le != cudaSuccess) return set_error("conv_halo2 launch: %s", cudaGetErrorString(le));
-    return check_launch("conv_halo2_kernel");
-  }
   if (mode_k == 2) conv_halo_kernel<2><<<grid, TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);
   else if (train) conv_halo_kernel<1><<<grid, TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);
   else conv_halo_kernel<0><<<grid, TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);

@@ -108,11 +108,7 @@ int attn_gather_run(int dtype, const void* x, const float* reg, int reg_per_fiel
 int attn_core_run(int dtype, const void* qkv, const float* qgamma, const float* kgamma, const float* bias_table,
                   const AttnGeom& g, int heads, int dh, void* out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
 
-int attn_fused_run(const float* x, float* x_out, const float* reg_in, int reg_per_field, float* reg_out,
-                   const float* film, const void* wqkv_h, const float* wout_h, const float* head_tab, const AttnGeom& g, int heads, int dh, float ln_eps,
-                   unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
-
-// second-generation fused attention (vg_attn_fused2.cu): in place on the residual stream, partition through TMA tensor maps
+// fused attention (vg_attn_fused2.cu): in place on the residual stream, partition through TMA tensor maps
 int attn_fused2_run(float* xio, const float* reg_in, int reg_per_field, float* reg_out, const float* film, const void* wqkv_h,
                     const float* wout_h, const float* head_tab, const AttnGeom& g, int heads, int dh, float ln_eps, unsigned seed,
                     unsigned salt, int drop_thresh, float logit_bound, cudaStream_t st);

@@ -35,7 +35,6 @@ struct WgradShape {
   int ksplit;
   long long rows_per_split;    // multiple of KT
   int stages;
-  int swap_lbo_sbo;            // debugging switch for the descriptor convention
 };
 
 // MN-major 128-byte-swizzled operand: 128-byte column groups `lbo` bytes apart, K row groups `sbo` bytes apart.
@@ -119,8 +118,7 @@ wgrad_tc_kernel(const __grid_constant__ CUtensorMap mapY, const __grid_constant_
       constexpr int KSTEP_ROWS = TF32 ? 8 : 16;                // rows consumed per MMA
       constexpr uint32_t KGROUP_BYTES = TF32 ? 512u : 1024u;   // 4 rows (tf32) / 8 rows (bf16) of 128 bytes
       constexpr uint32_t LAYOUT = TF32 ? 1u : 2u;
-      const uint32_t lbo = ws.swap_lbo_sbo ? KGROUP_BYTES : (uint32_t)BOX_BYTES;
-      const uint32_t sbo = ws.swap_lbo_sbo ? (uint32_t)BOX_BYTES : KGROUP_BYTES;
+      constexpr uint32_t lbo = (uint32_t)BOX_BYTES, sbo = KGROUP_BYTES;
       int stage = 0; uint32_t phase = 0;
       for (int kb = 0; kb < k_steps; ++kb) {
         mbar_wait(full + stage, phase);
@@ -304,9 +302,6 @@ static int wgrad_plan(WgradShape& ws, int dtype, long long M, int Ntot, int Ca, 
   rps = (rps + kt - 1) / kt * kt;
   ws.rows_per_split = rps;
   ws.ksplit = (int)((M + rps - 1) / rps);
-  static int swap = -1;
-  if (swap < 0) { const char* e = getenv("VG_WGRAD_SWAP"); swap = (e && e[0] == '1') ? 1 : 0; }
-  ws.swap_lbo_sbo = swap;
   return 0;
 }
 

@@ -165,7 +165,6 @@ class MaxViT(nn.Module):
         if cond_dim is None:
             raise NotImplementedError("MaxViT needs cond_dim: the reference's forward asserts cond.shape == (b, cond_dim) (maxvit.py:290)")
         self.set_precision("bf16")
-        self.fused_attention = True      # one-kernel attention (tf32 mode, dim 128, dim_head 32, <=64 tokens/window)
         self._packed = None
         self._packed_key = None
         self._capture = None
@@ -249,11 +248,17 @@ class MaxViT(nn.Module):
         return layers
 
     # ------------------------------------------------------------------ forward
+    def fused_attn_applies(self, C):
+        """whether an attention layer of width C runs as the one-kernel ops.attn_fused (inference and training); every
+        other shape / precision takes the un-fused path (gather -> QKV GEMM -> attn_core -> attn_out)"""
+        return (self.tf32 and C == 128 and self.dim_head == 32 and self.vit_window_size == 7 and self.num_register_tokens == 4
+                and self.heads >= 4 and self.heads % 2 == 0)
+
     def _attention(self, x, film, P, reg_in, grid_mode, want_reg_out):
         """x: CL (N,H,W,C).  returns (x + attn(x), reg_out)"""
         N, H, W, C = x.shape
         w, R = self.vit_window_size, self.num_register_tokens
-        if self.fused_attention and self.tf32 and C == 128 and self.dim_head == 32 and w == 7 and R == 4 and self.heads >= 4:
+        if self.fused_attn_applies(C):
             # x is a temporary of forward_cl (MBConv output / the previous attention's result): updated in place
             return ops.attn_fused(x, reg_in, film, P["wqkv_h"], P["wout_h"], P["head_tab"], w, R, grid_mode, want_reg_out,
                                   self.heads, self.dim_head, inplace=True, logit_bound=P.get("logit_bound", 0.0))

@@ -8,10 +8,7 @@ import torch
 
 from . import _lib
 
-import os
-
 DT_CODE = {torch.bfloat16: 0, torch.float32: 1, torch.float16: 3}
-_ATTN_V1 = os.environ.get("VG_ATTN_V1", "0") == "1"
 
 
 def _p(t):
@@ -358,19 +355,13 @@ def attn_fused(x, reg_in, film, wqkv_h, wout_h, head_tab, win, R, grid_mode, wan
     drop = (seed, salt, T): training dropout with probability T/256 on the probabilities and the to_out output.
     The kernel works in place on the residual stream (its TMA reduce-store performs the residual add): inplace=True lets it
     overwrite x (inference: x is a temporary), otherwise x is copied first (training keeps the input for backward).
-    VG_ATTN_V1=1 selects the first-generation kernel (A/B comparisons)."""
+    Needs heads even (the kernel's two compute groups alternate heads)."""
     N, Hl, Wl, C = x.shape
     assert x.dtype == torch.float32 and x.is_contiguous()
     nwin = (Hl // win) * (Wl // win)
     reg_out = torch.empty(N * nwin, R, C, dtype=torch.float32, device=x.device) if want_reg_out else None
     if wqkv_h.dtype != torch.float16:                       # the kernel's QKV operand format (the modules pack it once)
         wqkv_h = wqkv_h.half()
-    if _ATTN_V1 or heads % 2:
-        x_out = torch.empty_like(x)
-        _lib.call("vg_attn_fused_fwd", x.data_ptr(), x_out.data_ptr(), reg_in.data_ptr(), int(reg_in.dim() == 3), _p(reg_out),
-                  film.data_ptr(), wqkv_h.data_ptr(), wout_h.data_ptr(), head_tab.data_ptr(), N, Hl, Wl, C, win, R, int(grid_mode), heads, dh, float(eps),
-                  int(drop[0]), int(drop[1]), int(drop[2]), _st())
-        return x_out, reg_out
     xio = x if inplace else x.clone()
     _lib.call("vg_attn_fused2_fwd", xio.data_ptr(), reg_in.data_ptr(), int(reg_in.dim() == 3), _p(reg_out), film.data_ptr(),
               wqkv_h.data_ptr(), wout_h.data_ptr(), head_tab.data_ptr(), N, Hl, Wl, C, win, R, int(grid_mode), heads, dh, float(eps),

@@ -3,7 +3,6 @@ PyTorch supplies device memory and streams; every computation is a libvitgrid ke
 from __future__ import annotations
 
 import ctypes
-import os
 
 import torch
 
@@ -258,9 +257,9 @@ def attn_core_bwd(qkv, datt, q_gamma, k_gamma, bias_table, N, Hl, Wl, win, R, he
     """-> dqkv (, att = softmax(.) V re-materialised by the tensor-core kernel when want_att)"""
     dqkv = torch.empty_like(qkv)
     att = torch.empty(qkv.shape[0], heads * dh, dtype=qkv.dtype, device=qkv.device) if want_att else None
-    # tensor-core variants: 2 = bf16 mma + ldmatrix (default), 1 = tf32 mma (VG_ATTN_BWD=tf32); 0 = exact-fp32 SIMT;
+    # 2 = bf16 mma + ldmatrix on fp32 tensors; 0 = exact-fp32 SIMT;
     # 3 = the bf16 kernel on bf16 tensors (qkv, datt -> dqkv, att), selected by the dtype of qkv
-    mode = 0 if not tf32 else (1 if os.environ.get("VG_ATTN_BWD", "bf16") == "tf32" else 2)
+    mode = 2 if tf32 else 0
     if qkv.dtype == torch.bfloat16:
         assert datt.dtype == torch.bfloat16
         mode = 3

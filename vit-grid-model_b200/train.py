@@ -147,17 +147,13 @@ def _unpack_wgrad3x3(dWt, co, ci_pad, ci):
 
 
 # ------------------------------------------------------------------------------------------------ MaxViT block
-def _fused_ok(vit, C):
-    return (vit.fused_attention and vit.tf32 and C == 128 and vit.dim_head == 32 and vit.vit_window_size == 7
-            and vit.num_register_tokens == 4 and vit.heads >= 4)
-
-
 def _attention_train_fwd(vit, x, film, P, reg_in, grid_mode, want_reg_out, drop=(0, 0, 0)):
-    """mixed precision: the fused one-kernel attention, nothing but its inputs is kept (backward re-materialises
-    tokens / qkv / att on the tensor cores); fp32 mode: unfused path, intermediates saved."""
+    """shapes vit.fused_attn_applies accepts (mixed precision): the fused one-kernel attention, nothing but its inputs is
+    kept (backward re-materialises tokens / qkv / att on the tensor cores); fp32 mode and every other shape: un-fused path,
+    intermediates saved (attention dropout there is not built for the tf32 mode)."""
     N, H, W, C = x.shape
     w, R = vit.vit_window_size, vit.num_register_tokens
-    if _fused_ok(vit, C):
+    if vit.fused_attn_applies(C):
         x_out, reg_out = ops.attn_fused(x, reg_in, film, P["wqkv_h"], P["wout_h"], P["head_tab"], w, R, grid_mode, want_reg_out,
                                         vit.heads, vit.dim_head, drop=drop)
         return x_out, reg_out, dict(x=x, film=film, reg_in=reg_in, grid_mode=grid_mode, drop=drop)
