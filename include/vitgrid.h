@@ -158,9 +158,6 @@ VG_API int vg_pool2_fwd(int dtype, int out_f32, const void* in, void* out, int N
 VG_API int vg_dw3x3_bnact_fwd(int dtype, const void* in, const float* w9, const float* scale, const float* shift,
                        void* out, float* psum, int N, int H, int W, int C, void* stream);
 
-/* maxvit.py:38-48 -- squeeze-excite gate from the row sums: gate (N,C) fp32 */
-VG_API int vg_se_gate_fwd(const float* psum, int N, int H, int W, const float* W1, const float* W2, int C, int se,
-                   float* gate, void* stream);
 /* x *= gate (in place), CL (N,HW,C) */
 VG_API int vg_se_scale_fwd(int dtype, void* x, const float* gate, int N, long long HW, int C, void* stream);
 

@@ -253,11 +253,6 @@ int vg_dw3x3_bnact_fwd(int dtype, const void* in, const float* w9, const float* 
   return dwconv_run(dtype, in, w9, scale, shift, out, psum, N, H, W, C, (cudaStream_t)stream);
 }
 
-int vg_se_gate_fwd(const float* psum, int N, int H, int W, const float* W1, const float* W2, int C, int se, float* gate,
-                   void* stream) {
-  return se_gate_run(psum, N, H, H * W, W1, W2, C, se, gate, (cudaStream_t)stream);
-}
-
 int vg_se_scale_fwd(int dtype, void* x, const float* gate, int N, long long HW, int C, void* stream) {
   return se_scale_run(dtype, x, gate, N, HW, C, (cudaStream_t)stream);
 }

@@ -25,9 +25,6 @@
 // 32 head dims, one of the four raw matrices each), warp 16 TMA, warp 17 MMA issuer.  Compute order per tile:
 // softmax(t) -> staging(t+1) -> epilogue(t), so the four output products of tile t run under staging(t+1) and S / dP of
 // tile t+1 under epilogue(t).
-#include <stdio.h>
-#include <stdlib.h>
-
 #include "vg_common.cuh"
 #include "vg_host.h"
 #include "vg_rng.cuh"
@@ -68,7 +65,6 @@ struct AttnBwdTcParams {
   AttnGeom g;
   int heads;
   DropCfg drop;
-  long long* dbg;                                // optional clock64 stamps of CTA 0, warp 0: [64 tiles][8] (VG_ABTC_DBG)
 };
 
 namespace {
@@ -270,7 +266,6 @@ attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid
     auto stage = [&](uint32_t Tn, int tt_n) {
       const uint32_t st = Tn & 1, buf = Tn & 1;
       mbar_wait_tag(raw_full + st, (Tn >> 1) & 1, 404);
-      if (p.dbg && blockIdx.x == 0 && lane == 0 && Tn >= 1 && Tn <= 64) p.dbg[((Tn - 1) * 16 + warp) * 8 + 6] = clock64();
       const bool valid = i < S && (2 * tt_n + half) < nwin;
       const int sx = (i >> 1) & 3;                           // TMA SWIZZLE_64B rows: 16-byte chunk c of row i sits at chunk c ^ ((i >> 1) & 3)
       auto stage_matrix = [&](int mi) {                      // mi: 0 q, 1 k, 2 v, 3 dO
@@ -313,7 +308,6 @@ attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid
       if (cq == 0) stage_matrix(0);
       else if (cq == 1) stage_matrix(2);
       else if (cq == 3) { stage_matrix(1); stage_matrix(3); }
-      if (p.dbg && blockIdx.x == 0 && lane == 0 && Tn >= 1 && Tn <= 64) p.dbg[((Tn - 1) * 16 + warp) * 8 + 7] = clock64();
       fence_proxy_async_smem();
       tc_fence_before();
       __syncwarp();
@@ -352,13 +346,10 @@ attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid
         const uint32_t buf = T & 1;
         const int wdx_i = n * nwin + 2 * tt + half;
         const bool row_ok = i < S && (2 * tt + half) < nwin;
-        long long* dm = (p.dbg && blockIdx.x == 0 && lane == 0 && T < 64) ? p.dbg + (T * 16 + warp) * 8 : nullptr;
-        if (dm) dm[0] = clock64();
         // ---------------- softmax + dS ----------------
         {
           mbar_wait_tag(sdp_done, T & 1, 405);
           tc_fence_after();
-          if (dm) dm[1] = clock64();
           float s[16], dp[16];
           tmld16(lane_addr + T_S + half * 64 + cq * 16, s);
           tmld16(lane_addr + T_DP + half * 64 + cq * 16, dp);
@@ -431,16 +422,13 @@ attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid
           tc_fence_before();
           __syncwarp();
           if (lane == 0) mbar_arrive(pds_ready);
-          if (dm) dm[2] = clock64();
         }
         // ---------------- operands of the next tile (the four output products of this one run meanwhile) ----------------
         if (tt + 1 < ntile) stage(T + 1, tt + 1);
-        if (dm) dm[3] = clock64();
         // ---------------- epilogue: thread (row, cq) owns the whole 32-dim row of output cq (dV, dQ^, dK^, att) ----------------
         {
           mbar_wait_tag(out_done + cq, T & 1, 406);
           tc_fence_after();
-          if (dm) dm[4] = clock64();
           const long long rg = (long long)wdx_i * S + i;
           const uint32_t tacc = lane_addr + T_OUT + cq * 32;
           if (cq == 1 || cq == 2) {
@@ -507,7 +495,6 @@ attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid
               else if (p.att_out) { bf16* dst = p.att_out + rg * inner + hd * DH; st16_256(dst, acc); st16_256(dst + 16, acc + 16); }
             }
           }
-          if (dm) dm[5] = clock64();
         }
       }
       // ---------------- item flush: bias and gamma gradients, no shared-memory atomics (fp32 ones are CAS loops) ----------------
@@ -647,30 +634,6 @@ int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma,
   p.drop.seed = seed; p.drop.salt = salt; p.drop.thresh = drop_thresh; p.drop.scale = 256.0f / (256.0f - (float)drop_thresh);
   const int items = g.N * heads;
   const int grid = items < sms ? items : sms;
-  p.dbg = nullptr;
-  const char* de = getenv("VG_ABTC_DBG");
-  if (de && de[0] == '1') {                                  // clock stamps of CTA 0 (tools/ab_attn_bwd.py)
-    static long long* dbuf = nullptr;
-    const size_t nd = 64 * 16 * 8;
-    if (!dbuf) cudaMalloc(&dbuf, nd * sizeof(long long));
-    cudaMemsetAsync(dbuf, 0, nd * sizeof(long long), st);
-    p.dbg = dbuf;
-    attn_core_bwd_tc_kernel<<<grid, ab::THREADS, ab::SMEM_BYTES, st>>>(mq, md, p);
-    cudaStreamSynchronize(st);
-    static long long h[64 * 16 * 8];
-    cudaMemcpy(h, dbuf, sizeof(h), cudaMemcpyDeviceToHost);
-    // per warp (lg = warp & 3, cq = warp >> 2), cycles relative to warp 0's loop top of tile 8: loop top, S ready, softmax end, raw ready,
-    // staged, (stage end), out ready, epilogue end
-    for (int t = 8; t < 12; ++t) {
-      const long long t0 = h[(8 * 16) * 8];
-      for (int w = 0; w < 16; ++w) {
-        const long long* r = h + (t * 16 + w) * 8;
-        printf("tile %2d warp %2d (lg %d cq %d): top %6lld  S %6lld  sm_end %6lld  raw %6lld  stored %6lld  st_end %6lld  out %6lld  epi_end %6lld\n", t, w, w & 3, w >> 2,
-               r[0] - t0, r[1] - t0, r[2] - t0, r[6] - t0, r[7] - t0, r[3] - t0, r[4] - t0, r[5] - t0);
-      }
-    }
-    return check_launch("attn_core_bwd_tc_kernel");
-  }
   attn_core_bwd_tc_kernel<<<grid, ab::THREADS, ab::SMEM_BYTES, st>>>(mq, md, p);
   return check_launch("attn_core_bwd_tc_kernel");
 }

@@ -28,8 +28,6 @@
 // goes through an mbarrier; each issuer runs converged with an elected lane issuing; warps 2..9 = compute group 0 (even
 // heads; builds the X tile of the next tile), warps 10..17 = compute group 1 (odd heads; runs the tile epilogue).  Two threads
 // per token row (= TMEM lane) in each group.
-#include <stdlib.h>
-
 #include "vg_common.cuh"
 #include "vg_host.h"
 #include "vg_rng.cuh"
@@ -76,7 +74,6 @@ struct Fused2Params {
   float ln_eps;
   long long n_windows;
   DropCfg drop;
-  long long* dbg;                      // optional clock64 stamps of CTA 0: [3 roles][128 heads][8] (VG_ATTN2_DBG)
 };
 
 namespace {
@@ -229,12 +226,12 @@ __device__ __forceinline__ WinPos win_pos(const Fused2Params& p, long long tile,
 
 }  // namespace
 
-// DROP: training instantiation with the dropout code; DBG: clock-stamp instrumentation (tools/run_attn_fused2.py) -- both
-// compiled out of the production instantiation, whose cold paths share an instruction cache with five hot role loops
+// DROP: training instantiation with the dropout code -- compiled out of the inference instantiations, whose cold paths share
+// an instruction cache with five hot role loops
 // NOMAX: the caller proved |logit + bias| <= 115 in the exp2 domain (unit q-hat / k-hat: |logit| <= log2e * dh * max|gamma_q gamma_k|), so
 // neither exp2 (>= 2^-115, a normal number) nor the row sum of 53 of them (< 2^121) can leave the fp32 range and the softmax skips the
 // running maximum: 32 FMNMX + 16 packed subtractions per thread and head, and two exp2 of the pair exchange
-template <bool DROP, bool DBG, bool NOMAX>
+template <bool DROP, bool NOMAX>
 __global__ void __launch_bounds__(fb::THREADS, 1)
 attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_constant__ CUtensorMap mapWo,
                    const __grid_constant__ CUtensorMap mapX, const Fused2Params p) {
@@ -350,12 +347,11 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
     // ============================== QKV issuer: QKV(j+1) as soon as staging(j) holds the accumulator in registers ==============================
     constexpr uint32_t id_qkv = umma_idesc_f16(128, 96);
     const uint32_t sWQ = smem_u32(smem + WQ_OFF);
-    auto issue_qkv = [&](int j, int h, int tl, long long* dm) {   // QKV(j): needs X of its tile, WQ(j), and the accumulator released by staging(j-1)
+    auto issue_qkv = [&](int j, int h, int tl) {   // QKV(j): needs X of its tile, WQ(j), and the accumulator released by staging(j-1)
         const uint32_t b = (uint32_t)(j & 1);
         wait3(lane, h == 0 ? x_ready : nullptr, (uint32_t)(tl & 1), j > 0 ? qkv_free : nullptr, (uint32_t)((j - 1) & 1),
               wq_full + b, (uint32_t)((j >> 1) & 1), 311);
         tc_fence_after();
-        if (dm) dm[6] = clock64();
         if (elect_one()) {
           const uint64_t db = umma_desc_k128(sWQ + b * WQ_BYTES);
 #pragma unroll
@@ -369,13 +365,10 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
         }
         __syncwarp();
     };
-    if (total > 0) issue_qkv(0, 0, 0, nullptr);
+    if (total > 0) issue_qkv(0, 0, 0);
     int hq = 1 % heads, tlq = heads == 1 ? 1 : 0;            // (head, tile) of j + 1
     for (int j = 0; j + 1 < total; ++j) {
-      long long* dm = (DBG && p.dbg && blockIdx.x == 0 && j < 128 && lane == 0) ? p.dbg + (2 * 128 + j) * 8 : nullptr;
-      if (dm) dm[0] = clock64();
-      issue_qkv(j + 1, hq, tlq, dm);
-      if (dm) dm[1] = clock64();
+      issue_qkv(j + 1, hq, tlq);
       if (++hq == heads) { hq = 0; ++tlq; }
     }
   } else if (warp == 19) {
@@ -383,14 +376,12 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
     constexpr uint32_t id_s = umma_idesc_f16(128, 128);
     const uint32_t sQK = smem_u32(smem + QK_OFF);
     for (int j = 0; j < total; ++j) {
-      long long* dm = (DBG && p.dbg && blockIdx.x == 0 && j < 128 && lane == 0) ? p.dbg + (2 * 128 + j) * 8 : nullptr;
       const uint32_t b = (uint32_t)(j & 1);
       // s_free(j-1) first (the other group took S(j-1) long ago); the operands of head j arrive over a hardware named
       // barrier: an mbarrier poll by a whole warp costs ~190 cycles, and this hand-over is in front of every softmax
       if (j > 0) mbar_wait_tag(s_free, (uint32_t)((j - 1) & 1), 315);
       asm volatile("bar.sync %0, 288;" ::"r"(12 + (int)b) : "memory");
       tc_fence_after();
-      if (dm) dm[7] = clock64();
       if (elect_one()) {
         const uint64_t da = umma_desc_k128(sQK + b * 16384);
 #pragma unroll
@@ -398,7 +389,6 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
         tc_commit(s_done + b);
       }
       __syncwarp();
-      if (dm) dm[2] = clock64();
     }
   } else if (warp == 18) {
     // ============================== back-end MMA issuer: PV(k), out(k) ==============================
@@ -408,13 +398,11 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
     int h = 0, tl = 0;
     if (lane == 0) { mbar_arrive(qkv_done + 0); mbar_arrive(qkv_done + 1); }      // heads 0 and 1 have no PV(j-2) to wait for
     for (int k = 0; k < total; ++k) {
-      long long* dm = (DBG && p.dbg && blockIdx.x == 0 && k < 128 && lane == 0) ? p.dbg + (2 * 128 + k) * 8 : nullptr;
       const uint32_t b = (uint32_t)(k & 1);
       mbar_wait_tag(wo_full + b, (uint32_t)((k >> 1) & 1), 316);
       if (h == 0 && tl > 0) mbar_wait_tag(out_free, (uint32_t)((tl - 1) & 1), 317);
       asm volatile("bar.sync %0, 288;" ::"r"(14 + (int)b) : "memory");      // P(k) stored by the 8 warps of group b
       tc_fence_after();
-      if (dm) dm[3] = clock64();
       if (elect_one()) {
         // MN-major SWIZZLE_128B operand: 16 key rows (2048 B) per K step, 8-row groups 1024 B apart; this head's 64 bytes
         // start at byte b*64 of every row
@@ -428,7 +416,6 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
       // a TMEM A operand is not ordered behind the MMA that writes it: wait for PV(k) to retire before out(k)
       wait3(lane, pv_done + b, (uint32_t)((k >> 1) & 1), nullptr, 0, nullptr, 0, 319);
       tc_fence_after();
-      if (dm) dm[4] = clock64();
       if (elect_one()) {
         const uint64_t dwo = umma_desc_k128(sWO + b * 16384);
 #pragma unroll
@@ -437,7 +424,6 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
         if (h == heads - 1) tc_commit(tile_done);
       }
       __syncwarp();
-      if (dm) dm[5] = clock64();
       if (++h == heads) { h = 0; ++tl; }
     }
   } else {
@@ -610,13 +596,10 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
     for (int j = grp; j < total; j += 2) {
       const uint32_t u = (uint32_t)(j >> 1);                  // sequence number inside this group
 
-      long long* dg = (DBG && p.dbg && blockIdx.x == 0 && j < 128 && lane == 0 && (warp == 2 || warp == 10)) ? p.dbg + (grp * 128 + j) * 8 : nullptr;
-      if (dg) dg[0] = clock64();
       // ---------------- staging: q^ | K" (fp16) and V^T (bf16) of head j ----------------
       // one barrier: the table of this head has landed, PV(j-2) has read this group's V bytes, QKV(j) has retired
       mbar_wait_a(a_stage, u & 1, 341);
       tc_fence_after();
-      if (dg) dg[1] = clock64();
       {
         float a[32], vv[16];
         tmem_ld32(lane_addr + T_QKV + ch * 32, a);                       // ch 0: q, ch 1: k
@@ -664,13 +647,10 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
       }
       fence_proxy_async_smem();
       asm volatile("bar.arrive %0, 288;" ::"r"(12 + grp) : "memory");      // q^ | K" staged: the S issuer (warp 19) syncs on this barrier
-      if (dg) dg[2] = clock64();
-      if (DBG && p.dbg && blockIdx.x == 0 && j < 128 && lane == 0) p.dbg[3 * 128 * 8 + ((warp - 2) * 128 + j) * 2] = clock64();
 
       // ---------------- softmax of head j ----------------
       mbar_wait_a(a_s_done, u & 1, 344);
       tc_fence_after();
-      if (dg) dg[3] = clock64();
       {
         float2 sc2[16];
         float* sc = reinterpret_cast<float*>(sc2);
@@ -716,7 +696,6 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
         // the P buffer is single: PV(j-1) (the other group's head) must have retired before this head's P is stored.  Polled
         // here, where the thread has independent work in flight; a completed poll costs ~190 cycles at the hand-over otherwise
         const bool p_free = j > 0 ? mbar_try_a(a_pv_other, (uint32_t)(((j - 1) >> 1) & 1)) : true;
-        if (dg) dg[4] = clock64();
         const float2 nm = make_float2(-m, -m);
         float2 acc0 = make_float2(0.f, 0.f), acc1 = make_float2(0.f, 0.f);
         if (ch == 0) {
@@ -771,10 +750,8 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
         }
         // P (bf16 pairs, one 32-bit TMEM column per two keys): own 32 keys -> columns [half*32 + ch*16, +16); the same keys of
         // the other window are zero.  The P buffer is single: PV(j-1) (the other group's head) must have retired.
-        if (dg) dg[5] = clock64();
         if (!p_free) mbar_wait_a(a_pv_other, (uint32_t)(((j - 1) >> 1) & 1), 345);
         tc_fence_after();
-        if (dg) dg[6] = clock64();
         uint32_t pk[16];
 #pragma unroll
         for (int c = 0; c < 16; ++c) pk[c] = pk_bf16(sc[2 * c], sc[2 * c + 1]);
@@ -783,8 +760,6 @@ attn_fused2_kernel(const __grid_constant__ CUtensorMap mapWq, const __grid_const
       }
       tc_fence_before();
       asm volatile("bar.arrive %0, 288;" ::"r"(14 + grp) : "memory");      // P(j) is in TMEM: the back-end issuer (warp 18) syncs on this barrier
-      if (dg) dg[7] = clock64();
-      if (DBG && p.dbg && blockIdx.x == 0 && j < 128 && lane == 0) p.dbg[3 * 128 * 8 + ((warp - 2) * 128 + j) * 2 + 1] = clock64();
 
       // ---------------- tile boundary work after this group's last head of the tile ----------------
       if (h == heads - 2 + grp) {
@@ -881,17 +856,14 @@ int attn_fused2_run(float* xio, const float* reg_in, int reg_per_field, float* r
   p.xio = xio; p.reg_in = reg_in; p.reg_per_field = reg_per_field; p.reg_out = reg_out; p.film = film;
   p.head_tab = head_tab; p.g = g; p.heads = heads; p.ln_eps = ln_eps; p.n_windows = (long long)g.N * g.nwin();
   p.drop.seed = seed; p.drop.salt = salt; p.drop.thresh = drop_thresh; p.drop.scale = 256.0f / (256.0f - (float)drop_thresh);
-  p.dbg = nullptr;
-  if (const char* e = getenv("VG_ATTN2_DBG")) p.dbg = reinterpret_cast<long long*>(strtoull(e, nullptr, 0));
   int dev = 0, sms = 148;
   cudaGetDevice(&dev);
   static bool attr[64] = {};
   if (dev < 0 || dev >= 64) return set_error("attn_fused2: device ordinal %d out of range", dev);
   if (!attr[dev]) {
-    cudaError_t e = cudaFuncSetAttribute(attn_fused2_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fused2_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fused2_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fused2_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(attn_fused2_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fused2_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_fused2_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, fb::SMEM_BYTES);
     if (e != cudaSuccess) return set_error("attn_fused2 smem attr: %s", cudaGetErrorString(e));
     attr[dev] = true;
   }
@@ -900,10 +872,9 @@ int attn_fused2_run(float* xio, const float* reg_in, int reg_per_field, float* r
   const int grid = (int)(n_tiles < sms ? n_tiles : sms);
   // logit_bound: the caller's bound of |logit + bias| in the exp2 domain (0 = none given: keep the running maximum)
   const bool nomax = logit_bound > 0.f && logit_bound <= 115.f;
-  if (drop_thresh) attn_fused2_kernel<true, false, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
-  else if (p.dbg) attn_fused2_kernel<false, true, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
-  else if (nomax) attn_fused2_kernel<false, false, true><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
-  else attn_fused2_kernel<false, false, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
+  if (drop_thresh) attn_fused2_kernel<true, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
+  else if (nomax) attn_fused2_kernel<false, true><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
+  else attn_fused2_kernel<false, false><<<grid, fb::THREADS, fb::SMEM_BYTES, st>>>(mq, mo, mx, p);
   return check_launch("attn_fused2_kernel");
 }
 

@@ -86,7 +86,6 @@ int conv_ln_rows_run(int dtype, const float* acc, int C, const float* bias, cons
 int maxpool2_run(int dtype, int out_f32, const void* in, void* out, int N, int HP, int WP, int C, cudaStream_t st);
 int dwconv_run(int dtype, const void* in, const float* w9, const float* scale, const float* shift, void* out, float* psum,
                int N, int H, int W, int C, cudaStream_t st);
-int se_gate_run(const float* psum, int N, int H, int HW, const float* W1, const float* W2, int C, int se, float* gate, cudaStream_t st);
 int se_scale_run(int dtype, void* x, const float* gate, int N, long long HW, int C, cudaStream_t st);
 int reg_mean_run(const float* in, float* out, int N, int nwin, int RC, cudaStream_t st);
 int head_run(int dtype, const void* h, const float* w, float bias, float stdv, float mean, int N, int HP, int WP, int C,

@@ -536,35 +536,6 @@ __global__ void __launch_bounds__(256) dwconv3x3_kernel(const T* __restrict__ in
   }
 }
 
-// SE gate (maxvit.py:38-44): mean -> Linear(C,se) -> ReLU -> Linear(se,C) -> Sigmoid.  One block per field.
-__global__ void __launch_bounds__(256) se_gate_kernel(const float* __restrict__ psum, int H, float inv_count,
-                                                      const float* __restrict__ W1, const float* __restrict__ W2,
-                                                      int C, int se, float* __restrict__ gate) {
-  extern __shared__ float sh[];            // mean[C] + hid[se]
-  float* mean = sh; float* hid = sh + C;
-  const int n = blockIdx.x;
-  for (int c = threadIdx.x; c < C; c += blockDim.x) {
-    float s = 0.f;
-    for (int h = 0; h < H; ++h) s += psum[((long long)n * H + h) * C + c];
-    mean[c] = s * inv_count;
-  }
-  __syncthreads();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
-  for (int j = warp; j < se; j += nw) {
-    float a = 0.f;
-    for (int c = lane; c < C; c += 32) a += W1[(long long)j * C + c] * mean[c];
-    a = warp_sum(a);
-    if (lane == 0) hid[j] = fmaxf(a, 0.f);
-  }
-  __syncthreads();
-  for (int c = warp; c < C; c += nw) {
-    float a = 0.f;
-    for (int j = lane; j < se; j += 32) a += W2[(long long)c * se + j] * hid[j];
-    a = warp_sum(a);
-    if (lane == 0) gate[(long long)n * C + c] = 1.0f / (1.0f + expf(-a));
-  }
-}
-
 // x[n][p][c] *= gate[n][c]   (in place)
 template <typename T>
 __global__ void __launch_bounds__(256) se_scale_kernel(T* __restrict__ x, const float* __restrict__ gate, long long HW, int C, long long total_vec) {
@@ -951,11 +922,6 @@ int dwconv_run(int dtype, const void* in, const float* w9, const float* scale, c
   if (dtype == 0) dwconv3x3_kernel<bf16><<<N * H, threads, smem, st>>>(reinterpret_cast<const bf16*>(in), w9, scale, shift, reinterpret_cast<bf16*>(out), psum, H, W, C);
   else dwconv3x3_kernel<float><<<N * H, threads, smem, st>>>(reinterpret_cast<const float*>(in), w9, scale, shift, reinterpret_cast<float*>(out), psum, H, W, C);
   return check_launch("dwconv3x3_kernel");
-}
-
-int se_gate_run(const float* psum, int N, int H, int HW, const float* W1, const float* W2, int C, int se, float* gate, cudaStream_t st) {
-  se_gate_kernel<<<N, 256, (C + se) * sizeof(float), st>>>(psum, H, 1.0f / (float)HW, W1, W2, C, se, gate);
-  return check_launch("se_gate_kernel");
 }
 
 int se_scale_run(int dtype, void* x, const float* gate, int N, long long HW, int C, cudaStream_t st) {

@@ -263,9 +263,7 @@ class MaxViT(nn.Module):
             return ops.attn_fused(x, reg_in, film, P["wqkv_h"], P["wout_h"], P["head_tab"], w, R, grid_mode, want_reg_out,
                                   self.heads, self.dim_head, inplace=True, logit_bound=P.get("logit_bound", 0.0))
         tokens = ops.attn_gather(x, reg_in, film, w, R, grid_mode)
-        # qkv_exact: the QKV projection alone in exact fp32 -- its rounding error is multiplied by the un-scaled logits
-        # (+-32 gamma_q gamma_k, maxvit.py:26-30,203) before the softmax; every other contraction of the block stays tf32
-        qkv = ops.gemm(tokens, P["w_qkv"], tf32=self.tf32 and not getattr(self, "qkv_exact", False), x3=self.fp32_x3, Wt_x3=P.get("w_qkv_x3"))
+        qkv = ops.gemm(tokens, P["w_qkv"], tf32=self.tf32, x3=self.fp32_x3, Wt_x3=P.get("w_qkv_x3"))
         del tokens
         split = self.fp32_x3 and qkv.dtype == torch.float32 and w * w + R <= 64 and self.dim_head in (32, 64)
         att = ops.attn_core(qkv, P["q_gamma"], P["k_gamma"], P["bias_table"], N, H, W, w, R, self.heads, self.dim_head, x3=self.fp32_x3, tf32=self.tf32,
