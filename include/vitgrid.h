@@ -380,9 +380,10 @@ VG_API int vg_attn_out_bwd_gather(const float* dx_out, const float* dreg, float 
 VG_API int vg_dropout_mask_debug(long long drop_seed, int drop_salt, int drop_thresh, long long n_windows, int heads, int C,
                           void* prob_mask, void* out_mask, void* stream);
 /* per-(field, head) core backward: dqkv written; dq_gamma, dk_gamma, dbias_table accumulated.  use_tf32 = 2 / 3: tensor-core
- * kernel (2: bf16 mma + ldmatrix on fp32 tensors; 3: qkv, datt, dqkv and att_out as bf16 tensors; fp32 accumulate), which can
- * also re-materialise the forward output att = softmax(.) V [rows][inner] (att_out, or NULL) for the to_out weight gradient
- * when the forward pass was the fused kernel; 0: exact-fp32 SIMT kernel.  Any other mode is an error.
+ * kernel (2: bf16 mma + ldmatrix on fp32 tensors; 3: the tcgen05 kernel on bf16 tensors qkv, datt, dqkv and att_out, which
+ * must be 16-byte aligned, S <= 64; fp32 accumulate), which can also re-materialise the forward output
+ * att = softmax(.) V [rows][inner] (att_out, or NULL) for the to_out weight gradient when the forward pass was the fused
+ * kernel; 0: exact-fp32 SIMT kernel.  Any other mode is an error.
  * drop_thresh > 0: the forward pass applied dropout to the probabilities with these parameters. */
 VG_API int vg_attn_core_bwd(const void* qkv, const void* datt, const float* q_gamma, const float* k_gamma,
                      const float* bias_table, int N, int Hl, int Wl, int win, int R, int heads, int dh, void* dqkv,

@@ -68,21 +68,16 @@ def test_library_exports_every_declared_symbol():
     assert lib.vg_pg_pixels(2, 84, 70) == (2 * 85 + 1) * 71
 
 
-def test_environment_switches_are_the_documented_ab_switches():
-    """The library reads exactly the environment variables INTEGRATION.md §5 lists: the A/B switches that let the GPU tests
-    reach a reference path.  Anything else read from the environment would be an undocumented switch in a library call."""
+def test_library_reads_no_environment_variable():
+    """Every code path of a library call is selected by its arguments or by what the library observes (the device, the
+    shapes), never by an environment variable: the CUDA sources call no getenv, and INTEGRATION.md documents no switch."""
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     csrc = os.path.join(root, "vit-grid-model_b200", "csrc")
-    calls, names = 0, set()
     for fn in os.listdir(csrc):
         src = open(os.path.join(csrc, fn)).read()
-        calls += len(re.findall(r"\bgetenv\s*\(", src))
-        names |= set(re.findall(r"\bgetenv\s*\(\s*\"(\w+)\"\s*\)", src))
-    assert names == {"VG_ATTN_BWD_TC", "VG_CONV_OUT2_TMA"}
-    assert calls == len(names)                                  # every call names its variable literally, once
+        assert not re.search(r"getenv\s*\(", src), fn
     doc = open(os.path.join(root, "INTEGRATION.md")).read()
-    section = doc.split("\n## 5.", 1)[1].split("\n## ", 1)[0]
-    assert set(re.findall(r"^\| `(VG_\w+)=", section, flags=re.M)) == names
+    assert not re.search(r"^\| `VG_\w+=", doc, flags=re.M)
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")

@@ -204,17 +204,15 @@ def _head_ref(y64, hw, hb, HP, WP, pads, std, mean):
     return (z + hb) * std + mean
 
 
-def _run_conv_block(code, geom, epi, monkeypatch, C=128):
+def _run_conv_block(code, geom, epi, C=128):
     """one conv block call for epilogue `epi`; returns the measured ratios (each must be <= 1)"""
     o = O()
     (N, HP, WP, pads), (x, w, b, g, be, film, res), h64 = _conv_case(code, geom, C)
     adt = BF16 if code == 0 else F32
     use_film = epi == "film"
-    res_f32 = code == 0 and epi in ("res32_copy_tma1", "res32_copy_tma0", "head_only", "head_out")
-    use_res = epi != "film"
-    want_copy = epi.startswith("res32_copy")
-    if want_copy:
-        monkeypatch.setenv("VG_CONV_OUT2_TMA", epi[-1])
+    res_f32 = code == 0 and epi in ("res32_copy_tma1", "head_only", "head_out")
+    use_res = epi not in ("film", "copy_thread_stores")
+    want_copy = "copy" in epi
     resq = None
     if use_res:
         resq = res if (res_f32 or code != 0) else res.to(BF16).float()
@@ -248,7 +246,7 @@ def _run_conv_block(code, geom, epi, monkeypatch, C=128):
         r["copy"], r["copy_rel"] = f32_ratio(pg_frame(copy, N, HP, WP), yref)
         assert_pads_zero(copy, N, HP, WP)
         if out is not None:
-            assert torch.equal(out.float(), copy.to(BF16).float()), "bf16 output != rounded fp32 copy"
+            assert torch.equal(out.float(), copy.to(adt).float()), "output != (rounded) fp32 copy"
     if pred is not None:
         pref = _head_ref(y64, hw, hb, HP, WP, pads, std, mean)
         # the head sums 128 block outputs: allow 2e-5 of sum |w||y| per pixel (times std) on the block's own allowance
@@ -260,14 +258,16 @@ def _run_conv_block(code, geom, epi, monkeypatch, C=128):
 
 @pytest.mark.parametrize("geom", list(CONV_GEOMS))
 @pytest.mark.parametrize("code", list(CONV_DTYPES), ids=list(CONV_DTYPES.values()))
-@pytest.mark.parametrize("epi", ["film", "res", "res32_copy_tma1", "res32_copy_tma0", "head_only", "head_out"])
-def test_conv3x3_ln(code, geom, epi, monkeypatch):
+@pytest.mark.parametrize("epi", ["film", "res", "res32_copy_tma1", "copy_thread_stores", "head_only", "head_out"])
+def test_conv3x3_ln(code, geom, epi):
     """metnet3.py:110-126 Block (+ the ResnetBlock residual, + the fused 1x1 head) in the three conv dtypes: 0 = bf16 operands
     (halo kernel up to WP = 78, generic tcgen05 above), 1 = exact fp32 (SIMT), 2 = fp32 storage with tf32 tcgen05 (here on
-    tf32-representable operands: the bound is the fp32 one; test_conv3x3_ln_tf32_plain_operands covers rounding)"""
+    tf32-representable operands: the bound is the fp32 one; test_conv3x3_ln_tf32_plain_operands covers rounding).  The fp32
+    copy of the output leaves through TMA tensor stores with an fp32 residual (res32_copy_tma1, halo kernel), and through
+    per-thread stores without a residual (copy_thread_stores)."""
     if epi.startswith("res32_copy") and code != 0:
-        pytest.skip("the fp32 residual and the fp32 copy are the bf16 block's skip connection")
-    r = _run_conv_block(code, geom, epi, monkeypatch)
+        pytest.skip("the fp32 residual is the bf16 block's skip connection")
+    r = _run_conv_block(code, geom, epi)
     note(**r)
     for k, v in r.items():
         if not k.endswith("_rel"):
@@ -305,23 +305,24 @@ def test_conv3x3_ln_tf32_plain_operands():
     assert ratio_trunc <= 1.0 and rel > 5 * FP32_TOL, (ratio_trunc, rel)
 
 
-@pytest.mark.parametrize("out2_tma", ["1", "0"], ids=["copy_tma", "copy_thread_stores"])
-def test_conv3x3_ln_headline_batch(out2_tma, monkeypatch):
-    """bench.py's size: 768 fields at 84x70, bf16 with the fp32 residual and the fp32 copy (stored by TMA, and by the
-    threads under VG_CONV_OUT2_TMA=0), then the fused head.  The fp32 buffers are 4,634,951 x 128 x 4 B = 2.37 GB; a field
-    spans 85 x 71 rows of 512 B, so field 694 straddles 2^31 bytes and fields 695 and up lie past it.  Fields 0, 1, 383, 694,
-    695, 766 and 767 against float64; over the whole buffers every pad is 0.0 and nothing is NaN."""
-    monkeypatch.setenv("VG_CONV_OUT2_TMA", out2_tma)
+@pytest.mark.parametrize("with_res", [True, False], ids=["copy_tma", "copy_thread_stores"])
+def test_conv3x3_ln_headline_batch(with_res):
+    """bench.py's size: 768 fields at 84x70, bf16 with the fp32 copy, then the fused head: with the fp32 residual (the copy
+    is stored by TMA) and without a residual (the copy is stored by the threads).  The fp32 buffers are 4,634,951 x 128 x 4 B =
+    2.37 GB; a field spans 85 x 71 rows of 512 B, so field 694 straddles 2^31 bytes and fields 695 and up lie past it.
+    Fields 0, 1, 383, 694, 695, 766 and 767 against float64; over the whole buffers every pad is 0.0 and nothing is NaN."""
     o = O()
     N, HP, WP, C = 768, 84, 70, 128
     pads = synth.CFG_12HR.pads
     pl, pr, pt, pb = pads
     H, W = HP - pt - pb, WP - pl - pr
     xp = torch.zeros(o.pg_pixels(N, HP, WP), C, dtype=BF16, device=DEV)
-    rp = torch.zeros(o.pg_pixels(N, HP, WP), C, device=DEV)
     g_ = torch.Generator(device=DEV).manual_seed(51)
     pg_frame(xp, N, HP, WP).copy_(torch.randn(N, HP, WP, C, device=DEV, generator=g_).to(BF16))
-    pg_frame(rp, N, HP, WP).copy_(torch.randn(N, HP, WP, C, device=DEV, generator=g_))
+    rp = None
+    if with_res:
+        rp = torch.zeros(o.pg_pixels(N, HP, WP), C, device=DEV)
+        pg_frame(rp, N, HP, WP).copy_(torch.randn(N, HP, WP, C, device=DEV, generator=g_))
     w = rnd(C, C, 3, 3, seed=52, scale=1 / math.sqrt(9 * C)).to(BF16).float()
     b, be = rnd(C, seed=53, scale=0.1), rnd(C, seed=54, scale=0.1)
     g = 1.0 + 0.5 * torch.rand(C, device=DEV, generator=torch.Generator(device=DEV).manual_seed(55))
@@ -340,7 +341,7 @@ def test_conv3x3_ln_headline_batch(out2_tma, monkeypatch):
     worst = {}
     for n in (0, 1, 383, 694, 695, 766, 767):
         xn = pg_field(xp, n, HP, WP).permute(2, 0, 1)[None].to(F64)
-        rn = pg_field(rp, n, HP, WP).permute(2, 0, 1)[None].to(F64)
+        rn = pg_field(rp, n, HP, WP).permute(2, 0, 1)[None].to(F64) if with_res else None
         y64, _ = _block_ref(F.conv2d(xn, w.to(F64), b.to(F64), padding=1), g, be, None, rn)
         yref = y64.permute(0, 2, 3, 1)
         rc, relc = f32_ratio(pg_field(copy, n, HP, WP)[None], yref)
@@ -359,12 +360,12 @@ def test_conv3x3_ln_headline_batch(out2_tma, monkeypatch):
 @pytest.mark.parametrize("C", [256, 384, 512])
 @pytest.mark.parametrize("code", list(CONV_DTYPES), ids=list(CONV_DTYPES.values()))
 @pytest.mark.parametrize("epi", ["film", "res", "res32_copy_tma1", "head_only", "head_out"])
-def test_conv3x3_ln_wide(C, code, epi, monkeypatch):
+def test_conv3x3_ln_wide(C, code, epi):
     """vg_conv3x3_ln_wide_fwd (n_start_channels 256 / 384 / 512, BASELINE configs[4]): shifted-row GEMM + row-wise LayerNorm /
     FiLM / ReLU / residual / copy / head, at 2 fields of 28x35"""
     if epi.startswith("res32_copy") and code != 0:
         pytest.skip("the fp32 residual and the fp32 copy are the bf16 block's skip connection")
-    r = _run_conv_block(code, (2, 28, 35, (1, 2, 3, 0)), epi, monkeypatch, C=C)
+    r = _run_conv_block(code, (2, 28, 35, (1, 2, 3, 0)), epi, C=C)
     note(**r)
     for k, v in r.items():
         if not k.endswith("_rel"):

@@ -1,4 +1,5 @@
-"""Run the attention core backward (tf32 mma.sync kernel) alone (for ncu / timing)."""
+"""Run the attention core backward alone (for timing): the tcgen05 kernel on bf16 tensors (mode 3), the mma.sync kernel on
+fp32 tensors (mode 2) and the exact-fp32 SIMT kernel (mode 0)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -14,11 +15,12 @@ datt = torch.randn(rows, heads * dh, generator=g).cuda()
 qg, kg = torch.ones(heads * dh).cuda(), torch.ones(heads * dh).cuda()
 tab = torch.randn(170, heads, generator=g).cuda()
 dq, dk, dt = torch.zeros_like(qg), torch.zeros_like(kg), torch.zeros_like(tab)
-for tf32 in (True, False):
+for name, q, d, tf32 in (("tcgen05 bf16", qkv.bfloat16(), datt.bfloat16(), True), ("mma.sync fp32", qkv, datt, True),
+                         ("SIMT fp32", qkv, datt, False)):
     for _ in range(iters):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
-        ot.attn_core_bwd(qkv, datt, qg, kg, tab, N, H, W, w, R, heads, dh, dq, dk, dt, tf32=tf32, want_att=tf32)
+        ot.attn_core_bwd(q, d, qg, kg, tab, N, H, W, w, R, heads, dh, dq, dk, dt, tf32=tf32, want_att=tf32)
         e1.record()
         torch.cuda.synchronize()
-    print(f"N={N} windows={N * 30} tf32={tf32}: {e0.elapsed_time(e1):.3f} ms")
+    print(f"N={N} windows={N * 30} {name}: {e0.elapsed_time(e1):.3f} ms")

@@ -1,4 +1,4 @@
-"""The residual + fp32-copy variant of the conv kernel alone at bench shape (VG_CONV_OUT2_TMA=0/1 for A/B; for ncu)."""
+"""The residual + fp32-copy variant of the conv kernel alone at bench shape (for timing)."""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -16,4 +16,4 @@ for _ in range(5):
     e0.record()
     ops.conv3x3_ln(x, w, b, ga, be, 1e-5, None, res, out, N, HP, WP, out_copy=out2)
     e1.record(); torch.cuda.synchronize()
-print(f"res+copy N={N}: {e0.elapsed_time(e1):.3f} ms  (VG_CONV_OUT2_TMA={os.environ.get('VG_CONV_OUT2_TMA', '1')})")
+print(f"res+copy N={N}: {e0.elapsed_time(e1):.3f} ms")

@@ -601,16 +601,17 @@ static int rows_map(CUtensorMap* m, const void* base, long long cols, long long 
   return 0;
 }
 
-// returns -1 when the shape is outside what the kernel is built for (the caller falls back to the mma.sync kernel)
 int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                          const AttnGeom& g, int heads, void* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                          void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
   const int S = g.S(), nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
-  if (S > 64 || nb > 256 || S < 1) return -1;
+  if (S < 1 || S > 64) return set_error("attn_core_bwd_tc: sequence %d outside [1, 64]", S);
+  if (nb > 256) return set_error("attn_core_bwd_tc: %d bias-table rows > 256 (window %d)", nb, g.win);
   const long long rows = (long long)g.N * g.nwin() * S;
-  if (rows * 3 * heads * ab::DH >= (1ll << 40) || rows >= (1ll << 31)) return -1;
+  if (rows >= (1ll << 31)) return set_error("attn_core_bwd_tc: %lld rows >= 2^31", rows);
+  if (rows * 3 * heads * ab::DH >= (1ll << 40)) return set_error("attn_core_bwd_tc: qkv of %lld elements >= 2^40", rows * 3 * heads * ab::DH);
   if ((reinterpret_cast<uintptr_t>(qkv) | reinterpret_cast<uintptr_t>(datt) | reinterpret_cast<uintptr_t>(dqkv) |
-       reinterpret_cast<uintptr_t>(att_out)) & 15) return -1;
+       reinterpret_cast<uintptr_t>(att_out)) & 15) return set_error("attn_core_bwd_tc: qkv, datt, dqkv and att_out must be 16-byte aligned");
   CUtensorMap mq, md;
   int rc = rows_map(&mq, qkv, 3ll * heads * ab::DH, rows, S);
   if (rc) return rc;

@@ -565,7 +565,7 @@ __global__ void __launch_bounds__(256) attn_out_bwd_gather_kernel(const float* _
 // relative-position-bias and q/k-gamma gradients accumulate in shared memory / registers and reach global memory
 // once per block.  fp32, DH = 32, S <= 64.
 struct AttnCoreBwdParams {
-  const float* qkv;        // [rows][3*inner]   (bf16 when the IO16 instantiation of the bf16 kernel runs)
+  const float* qkv;        // [rows][3*inner]
   const float* datt;       // [rows][inner]
   const float* qgamma; const float* kgamma;   // [heads*DH]
   const float* bias_table; // [nb][heads]
@@ -725,8 +725,8 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
 }
 
 // ------------------------------------------------------------------------------------------------
-// Tensor-core version of the core backward for the mixed-precision path: bf16 mma.sync m16n8k16 (fp32 accumulate) with
-// ldmatrix operand fetch (transposed operands come for free from ldmatrix.trans).
+// Tensor-core version of the core backward on fp32 tensors (mode 2, the un-fused mixed-precision path): bf16 mma.sync
+// m16n8k16 (fp32 accumulate) with ldmatrix operand fetch (transposed operands come for free from ldmatrix.trans).
 // Block = (field, head), 4 warps, looping over the field's windows (3 blocks per SM hide each other's load latency);
 // each warp owns 16 rows of the window:
 //   phase 1  load q,k,v,dO rows, RMSNorm -> Qh, Kh, V, dO in shared memory (row stride 80 B: conflict-free ldmatrix)
@@ -782,15 +782,6 @@ __device__ __forceinline__ uint32_t pack2bf(float a, float b) {
   return *reinterpret_cast<uint32_t*>(&h);
 }
 
-// IO16: qkv, datt, dqkv and att_out are bf16 tensors (the mixed-precision training step keeps the whole attention backward
-// chain -- tokens, qkv, datt, dqkv, att -- in 16-bit storage: half the HBM bytes of this kernel and of the GEMMs around it)
-template <bool IO16>
-__device__ __forceinline__ void st2_io(float* base, long long off, float a, float b) {
-  if constexpr (IO16) *reinterpret_cast<__nv_bfloat162*>(reinterpret_cast<bf16*>(base) + off) = __floats2bfloat162_rn(a, b);
-  else *reinterpret_cast<float2*>(base + off) = make_float2(a, b);
-}
-
-template <bool IO16>
 __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCoreBwdParams p, float* __restrict__ att_out, const DropCfg drop) {
   using namespace cbh;
   extern __shared__ __align__(16) uint8_t smraw[];
@@ -798,17 +789,12 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
   const int S = g_.S(), nwin = g_.nwin(), W2 = 2 * g_.win - 1, nb = W2 * W2 + 1, R = g_.R, win = g_.win;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int g = lane >> 2, t = lane & 3;
-  // (IO16: V and dO live in the cp.async stages; their static tiles are not allocated -- three blocks per SM must fit)
-  bf16* sQ = reinterpret_cast<bf16*>(smraw); bf16* sK = sQ + SM * LDQ; bf16* sV = sK + SM * LDQ; bf16* sdO = sV + (IO16 ? 0 : SM * LDQ);
-  bf16* sP = sdO + (IO16 ? 0 : SM * LDQ); bf16* sDS = sP + SM * LDP;
+  bf16* sQ = reinterpret_cast<bf16*>(smraw); bf16* sK = sQ + SM * LDQ; bf16* sV = sK + SM * LDQ; bf16* sdO = sV + SM * LDQ;
+  bf16* sP = sdO + SM * LDQ; bf16* sDS = sP + SM * LDP;
   float* inq = reinterpret_cast<float*>(sDS + SM * LDP); float* ink = inq + SM;
   float* sbias = ink + SM; float* dbias = sbias + nb; float* gred = dbias + nb;
   float* sgam = gred + 2 * DH;             // [4][DH]: rs*gq, 1/(rs*gq), rs*gk, 1/(rs*gk)   (1/. = 0 where gamma = 0)
-  // IO16: two stages of raw bf16 rows [q | k | v | dO][64][LDQ], filled with cp.async one window ahead; V and dO are used
-  // by the MMAs in place (their bytes ARE the operands), q and k are normalised from the stage into sQ / sK
-  bf16* stage0 = reinterpret_cast<bf16*>(sgam + 4 * DH);
-  const uint32_t aQ = smem_u32(sQ), aK = smem_u32(sK), aP = smem_u32(sP), aDS = smem_u32(sDS);
-  uint32_t aV = smem_u32(sV), adO = smem_u32(sdO);
+  const uint32_t aQ = smem_u32(sQ), aK = smem_u32(sK), aV = smem_u32(sV), adO = smem_u32(sdO), aP = smem_u32(sP), aDS = smem_u32(sDS);
   const int n = blockIdx.x / p.heads, hd = blockIdx.x - n * p.heads;
   const int inner = p.heads * DH;
   const float rs = sqrtf((float)DH);
@@ -830,30 +816,7 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
   if (ib >= R && ib < S) { const int ti = ib - R, a = ti / win, b = ti - a * win; base_b = (a + win - 1) * W2 + (b + win - 1); }
   float bsa[16], bsb[16];                 // bias of this thread's 32 fixed (query, key) pairs (head-specific, window-independent)
   float dba[16], dbb[16];                 // and its gradient, summed over the windows
-  auto prefetch = [&](int wi, int st) {     // IO16: rows r0..r0+15 of window wi -> stage st (pad rows stay zero)
-    const long long rw0 = ((long long)n * nwin + wi) * S;
-    bf16* sb = stage0 + st * (4 * SM * LDQ);
-#pragma unroll
-    for (int ps = 0; ps < 2; ++ps) {
-      const int i = r0 + ps * 8 + prow;
-      if (i < S) {
-        const bf16* src = reinterpret_cast<const bf16*>(p.qkv) + (rw0 + i) * 3 * inner + hd * DH + pd0;
-        const bf16* sdo = reinterpret_cast<const bf16*>(p.datt) + (rw0 + i) * inner + hd * DH + pd0;
-#pragma unroll
-        for (int m = 0; m < 4; ++m) {
-          const uint32_t dst = smem_u32(sb + m * SM * LDQ + i * LDQ + pd0);
-          const bf16* g = m < 3 ? src + m * inner : sdo;
-          asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(g) : "memory");
-        }
-      }
-    }
-    asm volatile("cp.async.commit_group;" ::: "memory");
-  };
-  if constexpr (IO16) {
-    for (int i = threadIdx.x; i < 2 * 4 * SM * LDQ / 8; i += 128) reinterpret_cast<uint4*>(stage0)[i] = make_uint4(0u, 0u, 0u, 0u);
-  }
   __syncthreads();
-  if constexpr (IO16) prefetch(0, 0);
 #pragma unroll
   for (int k = 0; k < 16; ++k) {
     const int j = (k >> 1) * 8 + 2 * t + (k & 1);
@@ -866,38 +829,24 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
 
   for (int wi = 0; wi < nwin; ++wi) {
     const long long row0 = ((long long)n * nwin + wi) * S;
-    const bf16* stg = stage0 + (wi & 1) * (4 * SM * LDQ);
-    if constexpr (IO16) {
-      // the next window's rows stream into the other stage while this window computes (the global-load latency was 14 % of
-      // the kernel's samples when every window started with its own loads)
-      if (wi + 1 < nwin) { prefetch(wi + 1, (wi + 1) & 1); asm volatile("cp.async.wait_group 1;" ::: "memory"); }
-      else asm volatile("cp.async.wait_group 0;" ::: "memory");
-      __syncthreads();
-      aV = smem_u32(stg + 2 * SM * LDQ); adO = smem_u32(stg + 3 * SM * LDQ);
-    }
     // ---------------- phase 1: rows r0..r0+15; 4 lanes per row, 16-byte loads, all issued before the first use
     {
-      float4 ld[2][4][IO16 ? 1 : 2];                        // [pass][q,k,v,dO][half]  (IO16: one 16-byte load = 8 bf16)
+      float4 ld[2][4][2];                                   // [pass][q,k,v,dO][half]
 #pragma unroll
       for (int ps = 0; ps < 2; ++ps) {
         const int i = r0 + ps * 8 + prow;
 #pragma unroll
-        for (int m = 0; m < 4; ++m) { ld[ps][m][0] = make_float4(0.f, 0.f, 0.f, 0.f); if (!IO16) ld[ps][m][IO16 ? 0 : 1] = ld[ps][m][0]; }
+        for (int m = 0; m < 4; ++m) { ld[ps][m][0] = make_float4(0.f, 0.f, 0.f, 0.f); ld[ps][m][1] = ld[ps][m][0]; }
         if (i < S) {
-          if constexpr (IO16) {
+          const float* src = p.qkv + (row0 + i) * 3 * inner + hd * DH + pd0;
+          const float* sdo = p.datt + (row0 + i) * inner + hd * DH + pd0;
 #pragma unroll
-            for (int m = 0; m < 2; ++m) ld[ps][m][0] = *reinterpret_cast<const float4*>(stg + m * SM * LDQ + i * LDQ + pd0);
-          } else {
-            const float* src = p.qkv + (row0 + i) * 3 * inner + hd * DH + pd0;
-            const float* sdo = p.datt + (row0 + i) * inner + hd * DH + pd0;
-#pragma unroll
-            for (int m = 0; m < 3; ++m) {
-              ld[ps][m][0] = __ldg(reinterpret_cast<const float4*>(src + m * inner));
-              ld[ps][m][IO16 ? 0 : 1] = __ldg(reinterpret_cast<const float4*>(src + m * inner + 4));
-            }
-            ld[ps][3][0] = __ldg(reinterpret_cast<const float4*>(sdo));
-            ld[ps][3][IO16 ? 0 : 1] = __ldg(reinterpret_cast<const float4*>(sdo + 4));
+          for (int m = 0; m < 3; ++m) {
+            ld[ps][m][0] = __ldg(reinterpret_cast<const float4*>(src + m * inner));
+            ld[ps][m][1] = __ldg(reinterpret_cast<const float4*>(src + m * inner + 4));
           }
+          ld[ps][3][0] = __ldg(reinterpret_cast<const float4*>(sdo));
+          ld[ps][3][1] = __ldg(reinterpret_cast<const float4*>(sdo + 4));
         }
       }
 #pragma unroll
@@ -906,14 +855,8 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
         float x[4][8];
 #pragma unroll
         for (int m = 0; m < 4; ++m) {
-          if constexpr (IO16) {
-            const __nv_bfloat162* h2 = reinterpret_cast<const __nv_bfloat162*>(&ld[ps][m][0]);
-#pragma unroll
-            for (int e = 0; e < 4; ++e) { const float2 f = __bfloat1622float2(h2[e]); x[m][2 * e] = f.x; x[m][2 * e + 1] = f.y; }
-          } else {
-            x[m][0] = ld[ps][m][0].x; x[m][1] = ld[ps][m][0].y; x[m][2] = ld[ps][m][0].z; x[m][3] = ld[ps][m][0].w;
-            x[m][4] = ld[ps][m][IO16 ? 0 : 1].x; x[m][5] = ld[ps][m][IO16 ? 0 : 1].y; x[m][6] = ld[ps][m][IO16 ? 0 : 1].z; x[m][7] = ld[ps][m][IO16 ? 0 : 1].w;
-          }
+          x[m][0] = ld[ps][m][0].x; x[m][1] = ld[ps][m][0].y; x[m][2] = ld[ps][m][0].z; x[m][3] = ld[ps][m][0].w;
+          x[m][4] = ld[ps][m][1].x; x[m][5] = ld[ps][m][1].y; x[m][6] = ld[ps][m][1].z; x[m][7] = ld[ps][m][1].w;
         }
         float nq = 0.f, nk = 0.f;
 #pragma unroll
@@ -934,7 +877,7 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
         uv.x = pack2bf(x[2][0], x[2][1]); uv.y = pack2bf(x[2][2], x[2][3]); uv.z = pack2bf(x[2][4], x[2][5]); uv.w = pack2bf(x[2][6], x[2][7]);
         ud.x = pack2bf(x[3][0], x[3][1]); ud.y = pack2bf(x[3][2], x[3][3]); ud.z = pack2bf(x[3][4], x[3][5]); ud.w = pack2bf(x[3][6], x[3][7]);
         *reinterpret_cast<uint4*>(sQ + i * LDQ + pd0) = uq; *reinterpret_cast<uint4*>(sK + i * LDQ + pd0) = uk;
-        if constexpr (!IO16) { *reinterpret_cast<uint4*>(sV + i * LDQ + pd0) = uv; *reinterpret_cast<uint4*>(sdO + i * LDQ + pd0) = ud; }
+        *reinterpret_cast<uint4*>(sV + i * LDQ + pd0) = uv; *reinterpret_cast<uint4*>(sdO + i * LDQ + pd0) = ud;
         if ((lane & 3) == 0) { inq[i] = iq; ink[i] = ik; }
       }
     }
@@ -995,8 +938,8 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
         warp_mma_bf16<4, SM, false, true>(av, aP, LDP, r0, aV, LDQ, lane);
 #pragma unroll
         for (int nt = 0; nt < 4; ++nt) {
-          if (ia < S) st2_io<IO16>(att_out, (row0 + ia) * inner + hd * DH + nt * 8 + 2 * t, av[nt][0], av[nt][1]);
-          if (ib < S) st2_io<IO16>(att_out, (row0 + ib) * inner + hd * DH + nt * 8 + 2 * t, av[nt][2], av[nt][3]);
+          if (ia < S) *reinterpret_cast<float2*>(att_out + ((row0 + ia) * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(av[nt][0], av[nt][1]);
+          if (ib < S) *reinterpret_cast<float2*>(att_out + ((row0 + ib) * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(av[nt][2], av[nt][3]);
         }
       }
       float dp[8][4];
@@ -1033,8 +976,8 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
       warp_mma_bf16<4, SM, true, true>(acc, aP, LDP, r0, adO, LDQ, lane);                 // dV[j][d] = sum_i P[i][j] dO[i][d]
 #pragma unroll
       for (int nt = 0; nt < 4; ++nt) {
-        if (ia < S) st2_io<IO16>(p.dqkv, (row0 + ia) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t, acc[nt][0], acc[nt][1]);
-        if (ib < S) st2_io<IO16>(p.dqkv, (row0 + ib) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t, acc[nt][2], acc[nt][3]);
+        if (ia < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ia) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(acc[nt][0], acc[nt][1]);
+        if (ib < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ib) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(acc[nt][2], acc[nt][3]);
       }
 #pragma unroll
       for (int which = 0; which < 2; ++which) {
@@ -1067,10 +1010,10 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
 #pragma unroll
         for (int nt = 0; nt < 4; ++nt) {
           const int d = nt * 8 + 2 * t;
-          if (ia < S) st2_io<IO16>(p.dqkv, (row0 + ia) * 3 * inner + which * inner + hd * DH + d,
-                                   inva * (ga[2 * nt] - ua[2 * nt] * dota), inva * (ga[2 * nt + 1] - ua[2 * nt + 1] * dota));
-          if (ib < S) st2_io<IO16>(p.dqkv, (row0 + ib) * 3 * inner + which * inner + hd * DH + d,
-                                   invb * (gb[2 * nt] - ub[2 * nt] * dotb), invb * (gb[2 * nt + 1] - ub[2 * nt + 1] * dotb));
+          if (ia < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ia) * 3 * inner + which * inner + hd * DH + d)) =
+                            make_float2(inva * (ga[2 * nt] - ua[2 * nt] * dota), inva * (ga[2 * nt + 1] - ua[2 * nt + 1] * dota));
+          if (ib < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ib) * 3 * inner + which * inner + hd * DH + d)) =
+                            make_float2(invb * (gb[2 * nt] - ub[2 * nt] * dotb), invb * (gb[2 * nt + 1] - ub[2 * nt + 1] * dotb));
         }
       }
     }
@@ -1377,7 +1320,7 @@ int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma,
                          void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
 
 // use_tf32: 0 exact-fp32 SIMT, 2 bf16 mma.sync on fp32 tensors, 3 bf16 tensors (qkv, datt, dqkv, att_out): the
-// tcgen05 kernel (vg_attn_bwd_tc.cu); VG_ATTN_BWD_TC=0 or a shape outside it selects the bf16 mma.sync kernel
+// tcgen05 kernel (vg_attn_bwd_tc.cu)
 int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                       const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                       int use_tf32, float* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
@@ -1386,31 +1329,22 @@ int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, 
   if (use_tf32 != 0 && use_tf32 != 2 && use_tf32 != 3) return set_error("attn_core_bwd: mode %d (0 exact fp32, 2 bf16 mma on fp32 tensors, 3 bf16 tensors)", use_tf32);
   if (g.S() > 64) return set_error("attn_core_bwd: sequence %d > 64", g.S());
   const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
-  if (use_tf32 == 3) {
-    const char* e = getenv("VG_ATTN_BWD_TC");                // read per call so one process can compare the two kernels
-    if (!(e && e[0] == '0')) {
-      const int rc = attn_core_bwd_tc_run(qkv, datt, qgamma, kgamma, bias_table, g, heads, dqkv, dqgamma, dkgamma, dbias_table, att_out,
-                                          seed, salt, drop_thresh, st);
-      if (rc >= 0) return rc;
-    }
-  }
-  if (use_tf32 == 2 || use_tf32 == 3) {
-    // mode 3: two cp.async stages of [q | k | v | dO] rows instead of the static V / dO tiles
-    const size_t smem3 = (size_t)cbh::BYTES + (size_t)(2 * nb + 6 * cbh::DH) * sizeof(float) +
-                         (use_tf32 == 3 ? (size_t)(2 * 4 - 2) * cbh::SM * cbh::LDQ * 2 : 0);
+  if (use_tf32 == 3)
+    return attn_core_bwd_tc_run(qkv, datt, qgamma, kgamma, bias_table, g, heads, dqkv, dqgamma, dkgamma, dbias_table, att_out, seed, salt,
+                                drop_thresh, st);
+  if (use_tf32 == 2) {
+    const size_t smem3 = (size_t)cbh::BYTES + (size_t)(2 * nb + 6 * cbh::DH) * sizeof(float);
     static PerDeviceSize attr3_pd;                  // depends on the window size: raise the limit when it grows
     size_t& attr3 = attr3_pd.cur();
     if (smem3 > attr3) {
-      cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_bf16_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
-      if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_core_bwd_bf16_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
+      cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
       if (e != cudaSuccess) return set_error("attn_core_bwd_bf16 smem attr: %s", cudaGetErrorString(e));
       attr3 = smem3;
     }
     AttnCoreBwdParams q;
     q.qkv = qkv; q.datt = datt; q.qgamma = qgamma; q.kgamma = kgamma; q.bias_table = bias_table; q.dqkv = dqkv;
     q.dqgamma = dqgamma; q.dkgamma = dkgamma; q.dbias_table = dbias_table; q.g = g; q.heads = heads;
-    if (use_tf32 == 3) attn_core_bwd_bf16_kernel<true><<<g.N * heads, 128, smem3, st>>>(q, att_out, make_drop(seed, salt, drop_thresh));
-    else attn_core_bwd_bf16_kernel<false><<<g.N * heads, 128, smem3, st>>>(q, att_out, make_drop(seed, salt, drop_thresh));
+    attn_core_bwd_bf16_kernel<<<g.N * heads, 128, smem3, st>>>(q, att_out, make_drop(seed, salt, drop_thresh));
     return check_launch("attn_core_bwd_bf16_kernel");
   }
   if (att_out) return set_error("attn_core_bwd: att_out is only produced by the tensor-core kernels (modes 2, 3)");

@@ -570,12 +570,10 @@ int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const Ep
   HaloShape hs;
   hs.M = M; hs.num_tiles = (int)((hs.M + BM - 1) / BM); hs.P = P; hs.HR = HR; hs.res_tma = res_tma ? 1 : 0;
   hs.flip = flip;
-  // fp32 copy through TMA stores (needs the residual buffers: residual launches only); VG_CONV_OUT2_TMA=0 restores the per-thread stores
-  const char* o2e = getenv("VG_CONV_OUT2_TMA");             // read per call so one process can compare the two
-  const int o2_mode = (o2e && o2e[0] == '0') ? 0 : 1;
+  // fp32 copy through TMA stores (needs the residual buffers: fp32-residual launches only; the others store it per thread)
   CUtensorMap mo = ma;
   hs.out2_tma = 0;
-  if (o2_mode && res_tma && ep.out2 && ep.ldo == 128 && (reinterpret_cast<uintptr_t>(ep.out2) & 15) == 0) {
+  if (res_tma && ep.out2 && ep.ldo == 128 && (reinterpret_cast<uintptr_t>(ep.out2) & 15) == 0) {
     int rc2 = make_map_2d(&mo, true, ep.out2, 128, M, 32);
     if (rc2) return rc2;
     hs.out2_tma = 1;

@@ -258,7 +258,7 @@ def attn_core_bwd(qkv, datt, q_gamma, k_gamma, bias_table, N, Hl, Wl, win, R, he
     dqkv = torch.empty_like(qkv)
     att = torch.empty(qkv.shape[0], heads * dh, dtype=qkv.dtype, device=qkv.device) if want_att else None
     # 2 = bf16 mma + ldmatrix on fp32 tensors; 0 = exact-fp32 SIMT;
-    # 3 = the bf16 kernel on bf16 tensors (qkv, datt -> dqkv, att), selected by the dtype of qkv
+    # 3 = the tcgen05 kernel on bf16 tensors (qkv, datt -> dqkv, att), selected by the dtype of qkv
     mode = 2 if tf32 else 0
     if qkv.dtype == torch.bfloat16:
         assert datt.dtype == torch.bfloat16
