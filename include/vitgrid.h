@@ -291,7 +291,8 @@ VG_API int vg_conv_ln_param_grads(const float* sumA, const float* sumB, const fl
 /* Weight gradient of a shifted-row GEMM / 3x3 conv / linear layer:
  *   dW[n][tap*Ca + c] = beta*dW + sum_m dY[m][n] * A[m + tap_shift[tap]][c],   dW fp32 [Ntot][ntaps*Ca]
  * dtype 0: bf16 operands (tcgen05, MN-major operands straight from the row-major activations), 1: fp32 SIMT,
- * 2: fp32 operands as tf32 (tcgen05).  work: fp32 workspace of vg_wgrad_workspace() floats (split-K partials). */
+ * 2: fp32 operands as tf32 (tcgen05).  work: fp32 workspace of vg_wgrad_workspace() floats (split-K partials).
+ * M = 0 sums no rows: dW = beta*dW (zeros for beta = 0), with no workspace; M < 0 is an error. */
 VG_API long long vg_wgrad_workspace(int dtype, long long M, int Ntot, int Ca, int ntaps);
 VG_API int vg_wgrad(int dtype, const void* dY, const void* A, long long rowsA, long long M, int Ntot, int Ca, int ntaps,
              const int* tap_shift, float* dW, float beta, float* work, long long work_elems, void* stream);

@@ -306,6 +306,7 @@ static int wgrad_plan(WgradShape& ws, int dtype, long long M, int Ntot, int Ca, 
 }
 
 long long wgrad_workspace_elems(int dtype, long long M, int Ntot, int Ca, int ntaps) {
+  if (M <= 0) return 0;                                        // an empty reduction needs no slices (wgrad_plan divides by M)
   WgradShape ws;
   int shifts[9] = {0};
   wgrad_plan(ws, dtype, M, Ntot, Ca, ntaps, shifts);
@@ -316,8 +317,13 @@ long long wgrad_workspace_elems(int dtype, long long M, int Ntot, int Ca, int nt
 int wgrad_run(int dtype, const void* dY, const void* A, long long rowsA, long long M, int Ntot, int Ca, int ntaps,
               const int* tap_shift, float* dW, float beta, float* work, long long work_elems, cudaStream_t st) {
   if (ntaps < 1 || ntaps > 9) return set_error("wgrad: bad tap count %d", ntaps);
-  if (M <= 0) return 0;
+  if (M < 0) return set_error("wgrad: negative row count %lld", M);
   if (dtype != 1 && (Ca % 128 || Ntot % 64)) return set_error("wgrad: tensor-core path needs Ca %% 128 == 0 and Ntot %% 64 == 0 (got %d, %d)", Ca, Ntot);
+  if (M == 0) {                                                // the sum over no rows is zero: dW = beta * dW, as for any M
+    const long long n = (long long)Ntot * ntaps * Ca;
+    wgrad_reduce_kernel<<<(unsigned)((n / 4 + 256) / 256), 256, 0, st>>>(work, 0, n, beta, dW);
+    return check_launch("wgrad_reduce_kernel");
+  }
   WgradShape ws;
   wgrad_plan(ws, dtype, M, Ntot, Ca, ntaps, tap_shift);
   const long long need = (long long)ws.ksplit * Ntot * ws.Ktot;
