@@ -61,6 +61,14 @@ VG_API int vg_prepare_fwd(int dtype, const float* x, const long long* xstride, i
                    int pad_top, int pad_left, int HP, int WP, int Cpad, float pm_mean, float pm_std, void* out,
                    void* stream);
 
+/* Adjoint of vg_prepare_fwd (the gradient with respect to the input grids): g is the fp32 PG gradient [q][Cpad] of the B
+ * sample frames (the stem's data gradient, summed over the lead times); dx is a fresh contiguous fp32 (B,T,C,H,W) tensor,
+ * every element written.  Pad rows / columns and channels >= T*C are dropped; the PM2.5 channels {4,10,16,22} of every
+ * time step, and extra_channel (-1 = none; 24 for MetNet3_with_stn_imgs, metnet3.py:701), are divided by pm_std.
+ * HBM-bound: channel rows are read and (H,W) planes written coalesced through a shared-memory transpose. */
+VG_API int vg_prepare_bwd(const float* g, int B, int T, int C, int H, int W, int pad_top, int pad_left, int HP, int WP, int Cpad,
+                   float pm_std, int extra_channel, float* dx, void* stream);
+
 /* metnet3.py:701 (MetNet3_with_stn_imgs) -- x[:, :, channel] = (x[:, :, channel] - pm_mean) / pm_std IN PLACE on the caller's
  * fp32 (B,T,C,H,W) tensor with element strides xstride[5] (HOST array): the reference normalises the station-image variable
  * through a view before it clones the input, so the caller's tensor changes; kept. */
@@ -344,6 +352,14 @@ VG_API int vg_bn_bwd(const float* dOut, const float* raw, const float* scale, co
               const float* rstd, const float* gamma, int act, const float* fgate, const float* fadd,
               long long rows_per_field, long long M, int C, float* dgamma, float* dbeta, float* draw, float* work,
               long long work_elems, void* stream);
+/* BatchNorm with its running statistics (eval mode, frozen) (+ activation) backward, same upstream form as vg_bn_bwd
+ * (g = dOut*fgate[n] + fadd[n]) and the same C limits: running_mean, running_rstd = 1/sqrt(running_var + eps), scale / shift
+ * the affine folded from them.  draw = g*act'*scale written; dgamma += sum g*act'*(raw - running_mean)*running_rstd and
+ * dbeta += sum g*act' accumulated (deterministic partial sums).  There are no batch-mean terms.  work: vg_bn_workspace() floats */
+VG_API int vg_bn_bwd_frozen(const float* dOut, const float* raw, const float* scale, const float* shift, const float* running_mean,
+                     const float* running_rstd, int act, const float* fgate, const float* fadd, long long rows_per_field,
+                     long long M, int C, float* dgamma, float* dbeta, float* draw, float* work, long long work_elems,
+                     void* stream);
 /* out[c] += sum_m x[m][c] (bias gradients) */
 VG_API int vg_colsum(const float* x, long long M, int C, float* out, void* stream);
 /* depthwise 3x3 (marching stencil): out = act(conv(in, w9)*scale + shift); psum (or NULL): (N, vg_dw_strips(W), C)

@@ -93,6 +93,11 @@ int vg_prepare_packed_fwd(int dtype, const void* x_bf16, const long long* xstrid
                      (cudaStream_t)stream);
 }
 
+int vg_prepare_bwd(const float* g, int B, int T, int C, int H, int W, int pad_top, int pad_left, int HP, int WP, int Cpad,
+                   float pm_std, int extra_channel, float* dx, void* stream) {
+  return prepare_bwd_run(g, B, T, C, H, W, pad_top, pad_left, HP, WP, Cpad, pm_std, extra_channel, dx, (cudaStream_t)stream);
+}
+
 int vg_standardise_channel(float* x, const long long* xstride, int B, int T, int C, int H, int W, int channel, float pm_mean,
                            float pm_std, void* stream) {
   return standardise_channel_run(x, xstride, B, T, C, H, W, channel, pm_mean, pm_std, (cudaStream_t)stream);
@@ -447,6 +452,13 @@ int vg_bn_bwd(const float* dOut, const float* raw, const float* scale, const flo
               long long work_elems, void* stream) {
   return bn_bwd_run(dOut, raw, scale, shift, mean, rstd, gamma, act, fgate, fadd, rows_per_field, M, C, dgamma, dbeta, draw,
                     work, work_elems, (cudaStream_t)stream);
+}
+
+int vg_bn_bwd_frozen(const float* dOut, const float* raw, const float* scale, const float* shift, const float* running_mean,
+                     const float* running_rstd, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M,
+                     int C, float* dgamma, float* dbeta, float* draw, float* work, long long work_elems, void* stream) {
+  return bn_bwd_frozen_run(dOut, raw, scale, shift, running_mean, running_rstd, act, fgate, fadd, rows_per_field, M, C, dgamma, dbeta,
+                           draw, work, work_elems, (cudaStream_t)stream);
 }
 
 int vg_colsum(const float* x, long long M, int C, float* out, void* stream) { return colsum_run(x, M, C, out, (cudaStream_t)stream); }

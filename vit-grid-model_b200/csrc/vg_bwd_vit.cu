@@ -169,7 +169,20 @@ __global__ void bn_bwd_finalize_kernel(const float* __restrict__ part, int npart
   sum_parts2(part, nparts, C, c, s1, s2);
   if (c >= C || threadIdx.x >= 32) return;
   dbeta[c] += (float)s1; dgamma[c] += (float)s2;
-  k1[c] = (float)(s1 / (double)M); k2[c] = (float)(s2 / (double)M);
+  if (k1) { k1[c] = (float)(s1 / (double)M); k2[c] = (float)(s2 / (double)M); }
+}
+
+// BatchNorm with running statistics (eval mode, frozen): no batch-mean terms, draw = dpre * scale
+__global__ void __launch_bounds__(256) bn_bwd_frozen_apply_kernel(const BnBwdParams p, float* __restrict__ draw) {
+  const int quads = p.C / 4;
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= p.M * quads) return;
+  const long long r = i / quads;
+  const int c = (int)(i - r * quads) * 4;
+  const float4 rawv = *reinterpret_cast<const float4*>(p.raw + r * p.C + c);
+  const float4 d = bn_dpre4(p, r, c, rawv);
+  const float4 sc = *reinterpret_cast<const float4*>(p.scale + c);
+  *reinterpret_cast<float4*>(draw + r * p.C + c) = make_float4(d.x * sc.x, d.y * sc.y, d.z * sc.z, d.w * sc.w);
 }
 
 __global__ void __launch_bounds__(256) bn_bwd_apply_kernel(const BnBwdParams p, const float* __restrict__ k1, const float* __restrict__ k2,
@@ -1174,6 +1187,27 @@ int bn_bwd_run(const float* dOut, const float* raw, const float* scale, const fl
   if (rc) return rc;
   bn_bwd_apply_kernel<<<nblk(M * (C / 4), 256), 256, 0, st>>>(p, k1, k2, draw);
   return check_launch("bn_bwd_apply_kernel");
+}
+
+// mean / rstd: the running mean and 1/sqrt(running_var + eps); scale / shift: the affine folded from them
+int bn_bwd_frozen_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
+                      int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C, float* dgamma,
+                      float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st) {
+  const int nparts = (int)((M + STAT_ROWS - 1) / STAT_ROWS);
+  if (C % 4 || C / 4 > 256 || 256 % (C / 4)) return set_error("bn_bwd_frozen: C=%d must be 4*k with k | 256", C);
+  if (work_elems < (long long)nparts * 2 * C) return set_error("bn_bwd_frozen: workspace too small");
+  if (M <= 0) return 0;
+  BnBwdParams p;
+  p.dOut = dOut; p.raw = raw; p.scale = scale; p.shift = shift; p.mean = mean; p.rstd = rstd; p.gamma = nullptr;
+  p.fgate = fgate; p.fadd = fadd; p.rows_per_field = rows_per_field > 0 ? rows_per_field : 1; p.act = act; p.C = C; p.M = M;
+  bn_bwd_reduce_kernel<<<nparts, 256, 0, st>>>(p, work);
+  int rc = check_launch("bn_bwd_reduce_kernel");
+  if (rc) return rc;
+  bn_bwd_finalize_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, M, C, dgamma, dbeta, nullptr, nullptr);
+  rc = check_launch("bn_bwd_finalize_kernel");
+  if (rc) return rc;
+  bn_bwd_frozen_apply_kernel<<<nblk(M * (C / 4), 256), 256, 0, st>>>(p, draw);
+  return check_launch("bn_bwd_frozen_apply_kernel");
 }
 
 int colsum_run(const float* X, long long M, int C, float* out, cudaStream_t st) {

@@ -71,6 +71,8 @@ struct StemParams {
 
 int prepare_run(int dtype, const void* x, int x_bf16, int prestd, const long long* xs, int B, int T, int C, int H, int W, int pad_top,
                 int pad_left, int HP, int WP, int Cpad, float mean, float stdv, void* out, cudaStream_t st);
+int prepare_bwd_run(const float* g, int B, int T, int C, int H, int W, int pad_top, int pad_left, int HP, int WP, int Cpad,
+                    float stdv, int extra, float* dx, cudaStream_t st);
 int time_terms_run(const TimeParams& p, cudaStream_t st);
 int standardise_channel_run(float* x, const long long* xs, int B, int T, int C, int H, int W, int ch, float mean, float stdv, cudaStream_t st);
 int dense_rows_run(const float* in, int N, int cd, int pre_relu, const float* W, const float* b, int od, int act, float* out,
@@ -149,6 +151,9 @@ int bn_act_run(const float* raw, const float* scale, const float* shift, int act
 int bn_bwd_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
                const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
                float* dgamma, float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st);
+int bn_bwd_frozen_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
+                      int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C, float* dgamma,
+                      float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st);
 int colsum_run(const float* X, long long M, int C, float* out, cudaStream_t st);
 int dwconv_march_run(int dtype, const void* in, const float* w9, const float* scale, const float* shift, int act, void* out,
                      float* psum, int N, int H, int W, int C, cudaStream_t st);

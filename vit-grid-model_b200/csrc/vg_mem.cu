@@ -147,6 +147,58 @@ __global__ void __launch_bounds__(256) prepare_flat_kernel(const PrepParams p, T
   }
 }
 
+// adjoint of prepare (the input gradient): g fp32 PG [q][Cpad] over B frames -> dx fp32 (B, T*C, H*W) contiguous, every element
+// written.  Pad rows / columns and channels >= T*C are dropped; the PM2.5 channels (and `extra`, the station image of
+// MetNet3_with_stn_imgs, metnet3.py:701) are divided by std, the derivative of their standardisation.  The tiling of
+// prepare_flat_kernel in reverse: 64 channels x 128 pixels per block, read as 256-byte channel rows, written as 128-byte
+// plane rows through a shared-memory transpose.
+__global__ void __launch_bounds__(256) prepare_bwd_kernel(const float* __restrict__ g, int TC, int C, int HW, int W, int pad_top,
+                                                          int pad_left, int Cpad, PGeom pg, float stdv, int extra,
+                                                          float* __restrict__ dx) {
+  constexpr int PT = 4;                                            // 32-pixel tiles per block
+  __shared__ float tile[PT][64][33];
+  __shared__ long long s_row[PT * 32];                             // PG row of pixel px0 + i, -1 = outside the field
+  __shared__ int s_pm[64];
+  const int px0 = blockIdx.x * 32 * PT;
+  const int cblocks = (TC + 63) / 64;
+  const int b = blockIdx.y / cblocks, ch0 = (blockIdx.y - b * cblocks) * 64;
+  if (threadIdx.x < 64) {
+    const int c = (ch0 + threadIdx.x) % C;
+    s_pm[threadIdx.x] = c == 4 || c == 10 || c == 16 || c == 22 || c == extra;
+  } else if (threadIdx.x < 64 + PT * 32) {
+    const int i = threadIdx.x - 64, px = px0 + i;
+    long long q = -1;
+    if (px < HW) { const int h = px / W, w = px - h * W; q = pg.q(b, h + pad_top, w + pad_left); }
+    s_row[i] = q;
+  }
+  __syncthreads();
+  const int wl = threadIdx.x >> 3, c8 = (threadIdx.x & 7) * 8;
+#pragma unroll
+  for (int u = 0; u < PT; ++u) {
+    const long long q = s_row[u * 32 + wl];
+    float v[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+    if (q >= 0) ld8(g + q * Cpad + ch0 + c8, v);
+#pragma unroll
+    for (int j = 0; j < 8; ++j) tile[u][c8 + j][wl] = v[j];
+  }
+  __syncthreads();
+  const int pl = threadIdx.x & 31, cl0 = threadIdx.x >> 5;         // lane = pixel (coalesced plane rows), warp = channel
+#pragma unroll
+  for (int k = 0; k < 8; ++k) {
+    const int cl = cl0 + 8 * k, ch = ch0 + cl;
+    if (ch >= TC) break;                                           // warp-uniform
+    float* o = dx + ((long long)b * TC + ch) * HW + px0 + pl;
+    const bool pm = s_pm[cl];
+#pragma unroll
+    for (int u = 0; u < PT; ++u) {
+      if (px0 + u * 32 + pl < HW) {
+        const float v = tile[u][cl][pl];
+        o[u * 32] = pm ? v / stdv : v;
+      }
+    }
+  }
+}
+
 // MetNet3_with_stn_imgs (metnet3.py:701): x[:, :, ch] = (x[:, :, ch] - mean) / std, written back into the CALLER's tensor
 // (the reference normalises the view before its clone).  x (B,T,C,H,W) fp32 with arbitrary element strides.
 __global__ void __launch_bounds__(256) standardise_channel_kernel(float* __restrict__ x, long long sB, long long sT, long long sC, long long sH,
@@ -821,6 +873,18 @@ int prepare_run(int dtype, const void* x, int x_bf16, int prestd, const long lon
   else { if (x_bf16) VG_PREP(float, bf16); else VG_PREP(float, float); }
 #undef VG_PREP
   return check_launch(flat ? "prepare_flat_kernel" : "prepare_kernel");
+}
+
+int prepare_bwd_run(const float* g, int B, int T, int C, int H, int W, int pad_top, int pad_left, int HP, int WP, int Cpad,
+                    float stdv, int extra, float* dx, cudaStream_t st) {
+  if (Cpad % 64 || Cpad < T * C) return set_error("prepare_bwd: Cpad=%d must be a multiple of 64 and >= T*C=%d", Cpad, T * C);
+  if (extra < -1 || extra >= C) return set_error("prepare_bwd: extra channel %d outside [-1, %d)", extra, C);
+  if (pad_top < 0 || pad_left < 0 || H + pad_top > HP || W + pad_left > WP)
+    return set_error("prepare_bwd: the %dx%d field at (%d, %d) does not fit the %dx%d frame", H, W, pad_top, pad_left, HP, WP);
+  if (B <= 0 || T * C <= 0 || H * W <= 0) return 0;
+  dim3 grid((unsigned)((H * W + 127) / 128), (unsigned)(B * ((T * C + 63) / 64)));
+  prepare_bwd_kernel<<<grid, 256, 0, st>>>(g, T * C, C, H * W, W, pad_top, pad_left, Cpad, make_pgeom(B, HP, WP), stdv, extra, dx);
+  return check_launch("prepare_bwd_kernel");
 }
 
 int standardise_channel_run(float* x, const long long* xs, int B, int T, int C, int H, int W, int ch, float mean, float stdv, cudaStream_t st) {

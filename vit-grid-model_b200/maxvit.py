@@ -333,17 +333,20 @@ class MaxViT(nn.Module):
     def forward(self, x: torch.Tensor, cond: torch.Tensor) -> torch.Tensor:
         """reference signature (maxvit.py:289): x (N,dim,H,W) -> (N,dim_out,H,W), same dtype as x.  In train() mode the module
         runs the training kernels (batch-statistic BatchNorm, dropout) and is differentiable with respect to x, cond and its
-        parameters (train.MaxViTTrainFn), like the reference module under autograd."""
+        parameters (train.MaxViTTrainFn), like the reference module under autograd.  In eval() mode the same holds when x
+        requires grad and grad mode is on (BatchNorm from its running statistics, no dropout); every other eval() call is
+        the inference path."""
         assert cond.shape == (x.shape[0], self.cond_dim)
         if not x.is_cuda:
             raise _lib.VitGridError("vit_grid_model_b200 runs on a CUDA (sm_100a) device only; there is no CPU fallback")
         with torch.cuda.device(x.device):
             x_cl = x.permute(0, 2, 3, 1).to(self.compute_dtype).contiguous()
-            if self.training:
+            frozen = not self.training and torch.is_grad_enabled() and x.requires_grad
+            if self.training or frozen:
                 from .train import MaxViTTrainFn
                 if self.compute_dtype != torch.float32:
-                    raise NotImplementedError("MaxViT training supports set_precision('bf16') (mixed) and 'fp32'")
-                y = MaxViTTrainFn.apply(self, x_cl, cond.float().contiguous(), *self.parameters())
+                    raise NotImplementedError("MaxViT training and input gradients support set_precision('bf16') (mixed) and 'fp32'")
+                y = MaxViTTrainFn.apply(self, x_cl, cond.float().contiguous(), frozen, *self.parameters())
             else:
                 y = self.forward_cl(x_cl, cond)
             return y.permute(0, 3, 1, 2).to(x.dtype).contiguous()

@@ -81,6 +81,9 @@ def _check_timestamps(ts):
 
 
 class MetNet3(nn.Module):
+    # variable standardised with the PM2.5 statistics next to {4,10,16,22} (-1: none; 24 in MetNet3_with_stn_imgs)
+    standardised_extra_channel = -1
+
     def __init__(
         self,
         input_size_sample: tuple,      # window_size, n_variables, height, width
@@ -339,16 +342,18 @@ class MetNet3(nn.Module):
             self._grad_buffer = GradBuffer(self)
         return self._grad_buffer
 
-    def _forward_train(self, x, ts):
-        """train() mode: batch-statistic BatchNorm, activations saved, hand-written backward (train.py)"""
+    def _forward_train(self, x, ts, frozen=False):
+        """train() mode: batch-statistic BatchNorm, activations saved, hand-written backward (train.py).
+        frozen (eval() mode with an input that requires grad): the same graph with BatchNorm from its running statistics and
+        no dropout, so that x.grad and the parameter gradients are those of the reference module in eval() mode"""
         from .train import MetNet3TrainFn
+        what = "input gradients in eval() mode" if frozen else "training"
         if self.n_start_channels != 128:
-            raise NotImplementedError("the training kernels are built for n_start_channels=128; wider networks run inference only")
-        if self.precision == "bf16_all":
-            raise NotImplementedError("training supports set_precision('bf16') (mixed) and 'fp32'")
+            raise NotImplementedError(f"the training kernels are built for n_start_channels=128; wider networks run inference only "
+                                      f"({what} is not built)")
         if self.precision not in ("bf16", "fp32"):
-            raise NotImplementedError("training supports set_precision('bf16') (mixed) and 'fp32'")
-        return MetNet3TrainFn.apply(self, x, ts, *self.parameters())
+            raise NotImplementedError(f"{what} supports set_precision('bf16') (mixed) and 'fp32'")
+        return MetNet3TrainFn.apply(self, x, ts, frozen, *self.parameters())
 
     def next_dropout_seed(self) -> int:
         """32-bit seed of this step's dropout masks: derived from torch's seed at the first training step (so that
@@ -401,6 +406,10 @@ class MetNet3(nn.Module):
         ts = timestamps.to(device=x.device, dtype=torch.float32)
         if self.training:
             return self._forward_train(x, ts)
+        if not packed and torch.is_grad_enabled() and x.requires_grad:
+            # eval() mode under autograd with an input that requires grad (attribution, inverse problems): the frozen-BatchNorm
+            # graph.  Every other eval() call -- parameters require grad by default -- stays on the inference path below.
+            return self._forward_train(x, ts, frozen=True)
         P = self.packed(dtype)
         L = self.end_lead_time
         s0 = P["resnet1"][0]
@@ -421,7 +430,11 @@ class MetNet3_with_stn_imgs(MetNet3):
 
     Reference behaviour kept on purpose: the standardisation of variable 24 is written back into the CALLER's tensor
     (line 701 runs before the ``x.clone()`` of line 702), so calling ``forward`` twice on the same tensor normalises it
-    twice.  ``tests/golden/metnet3_stn_small128.pt`` records that side effect."""
+    twice.  ``tests/golden/metnet3_stn_small128.pt`` records that side effect.  Under autograd the write is the reference's
+    in-place op: on a leaf that requires grad it raises as torch does, and the gradient of a non-leaf input carries the 1/std
+    of the standardisation on variable 24."""
+
+    standardised_extra_channel = 24
 
     def __init__(self, *args, **kwargs):
         super().__init__(*args, **kwargs)
@@ -436,6 +449,10 @@ class MetNet3_with_stn_imgs(MetNet3):
         if self.normalization_method == "Standard":
             if x.dtype != torch.float32:
                 raise _lib.VitGridError("MetNet3_with_stn_imgs takes the reference's fp32 input tensor")
+            if torch.is_grad_enabled() and x.requires_grad:
+                if x.is_leaf:
+                    raise RuntimeError("a leaf Variable that requires grad is being used in an in-place operation.")
+                torch.autograd.graph.increment_version(x)       # what the reference's in-place write does to x's version
             with torch.cuda.device(x.device):                   # the caller's tensor is updated, as in the reference (:701)
                 ops.standardise_channel_(x, 24, self.pm25_mean, self.pm25_std)
         return super().forward(x, labels_pm25, region_targets_pm25, labels_pm10, region_targets_pm10, timestamps, prev_vals)

@@ -173,6 +173,37 @@ def bn_bwd(dOut, raw, st, gamma, act, dgamma, dbeta, fgate=None, fadd=None, rows
     return draw
 
 
+def bn_frozen_stats(bn):
+    """-> (mean, rstd, scale, shift) of an eval-mode BatchNorm: its running statistics, nothing updated"""
+    st = torch.empty(4, bn.num_features, dtype=torch.float32, device=bn.running_mean.device)
+    st[0] = bn.running_mean
+    torch.rsqrt(bn.running_var.float() + bn.eps, out=st[1])
+    torch.mul(bn.weight.detach(), st[1], out=st[2])
+    torch.sub(bn.bias.detach(), st[0] * st[2], out=st[3])
+    return st
+
+
+def bn_bwd_frozen(dOut, raw, st, act, dgamma, dbeta, fgate=None, fadd=None, rows_per_field=0, out=None):
+    """backward of bn_act with the running statistics of bn_frozen_stats: no batch-mean terms"""
+    M, C = raw.shape
+    draw = torch.empty_like(raw) if out is None else out
+    work = _f32(_lib.load().vg_bn_workspace(M, C), raw.device)
+    _lib.call("vg_bn_bwd_frozen", dOut.data_ptr(), raw.data_ptr(), st[2].data_ptr(), st[3].data_ptr(), st[0].data_ptr(),
+              st[1].data_ptr(), int(act), _p(fgate), _p(fadd), int(rows_per_field), M, C, dgamma.data_ptr(), dbeta.data_ptr(),
+              draw.data_ptr(), work.data_ptr(), work.numel(), _st())
+    return draw
+
+
+def prepare_bwd(g, B, T, C, H, W, pads, HP, WP, std, extra_channel=-1):
+    """adjoint of ops.prepare: g fp32 PG [q][Cpad] over B frames -> dx (B,T,C,H,W) fp32, every element written"""
+    assert g.dtype == torch.float32 and g.is_contiguous()
+    dx = torch.empty(B, T, C, H, W, dtype=torch.float32, device=g.device)
+    pl, _, pt, _ = pads
+    _lib.call("vg_prepare_bwd", g.data_ptr(), B, T, C, H, W, pt, pl, HP, WP, g.shape[1], float(std), int(extra_channel),
+              dx.data_ptr(), _st())
+    return dx
+
+
 def colsum(x2d, out):
     M, C = x2d.shape
     _lib.call("vg_colsum", x2d.data_ptr(), M, C, out.data_ptr(), _st())

@@ -207,8 +207,21 @@ def dropout_threshold(p: float) -> int:
     return max(0, min(255, int(round(p * 256))))
 
 
-def maxvit_train_forward(vit, x, cond, seed=0):
-    """x CL (N,H,W,C) fp32, cond (N,cd) -> (y, saved).  seed: dropout seed of this step (ignored when dropout is 0)"""
+def _bn_stats(bn, raw, frozen):
+    if frozen:
+        return ot.bn_frozen_stats(bn)
+    return ot.bn_stats(raw, bn.weight, bn.bias, bn.eps, bn.momentum, bn.running_mean, bn.running_var)
+
+
+def _bn_bwd(dOut, raw, st, bn, act, dgamma, dbeta, frozen, **kw):
+    if frozen:
+        return ot.bn_bwd_frozen(dOut, raw, st, act, dgamma, dbeta, **kw)
+    return ot.bn_bwd(dOut, raw, st, bn.weight, act, dgamma, dbeta, **kw)
+
+
+def maxvit_train_forward(vit, x, cond, seed=0, frozen=False):
+    """x CL (N,H,W,C) fp32, cond (N,cd) -> (y, saved).  seed: dropout seed of this step (ignored when dropout is 0).
+    frozen: the eval-mode graph -- BatchNorm from its running statistics (nothing updated), no dropout"""
     N, H, W, C = x.shape
     w = vit.vit_window_size
     nwin = (H // w) * (W // w)
@@ -221,22 +234,24 @@ def maxvit_train_forward(vit, x, cond, seed=0):
         bn1, bn2, bn3 = seq[1], seq[4], seq[8]
         h0 = ops.gemm(x2d, P["w_exp"], bias=P["b_exp"], tf32=tf32)
         hid = h0.shape[1]
-        st1 = ot.bn_stats(h0, bn1.weight, bn1.bias, bn1.eps, bn1.momentum, bn1.running_mean, bn1.running_var)
+        st1 = _bn_stats(bn1, h0, frozen)
         h1 = ot.bn_act(h0, st1, 1)
         h2, _ = ot.dw3x3(h1.view(N, H, W, hid), P["w_dw"], P["ones_hid"], P["b_dw"], 0)
-        st2 = ot.bn_stats(h2.view(M, hid), bn2.weight, bn2.bias, bn2.eps, bn2.momentum, bn2.running_mean, bn2.running_var)
+        st2 = _bn_stats(bn2, h2.view(M, hid), frozen)
         h3 = ot.bn_act(h2.view(M, hid), st2, 1).view(N, H, W, hid)
         gate, mean, hidv = ot.se_gate_train(ot.field_sum(h3), H * W, P["se_w1"], P["se_w2"])
         h4 = ot.se_scale_oop(h3, gate)
         y0 = ops.gemm(h4.view(M, hid), P["w_proj"], bias=P["b_proj"], tf32=tf32)
-        st3 = ot.bn_stats(y0, bn3.weight, bn3.bias, bn3.eps, bn3.momentum, bn3.running_mean, bn3.running_var)
+        st3 = _bn_stats(bn3, y0, frozen)
         y = ot.bn_act(y0, st3, 0, res=x2d if P["residual"] else None).view(N, H, W, C)
-        for bn in (bn1, bn2, bn3):
-            bn.num_batches_tracked += 1
-        sv = dict(x=x, h0=h0, st1=st1, h1=h1, h2=h2, st2=st2, h3=h3, gate=gate, mean=mean, hidv=hidv, h4=h4, y0=y0, st3=st3)
+        if not frozen:
+            for bn in (bn1, bn2, bn3):
+                bn.num_batches_tracked += 1
+        sv = dict(x=x, h0=h0, st1=st1, h1=h1, h2=h2, st2=st2, h3=h3, gate=gate, mean=mean, hidv=hidv, h4=h4, y0=y0, st3=st3,
+                  frozen=frozen)
         fb = P["block"]
         film_b = ops.cond_mlp(cond, fb["film_w0"], fb["film_b0"], fb["film_w1"], fb["film_b1"])
-        T = dropout_threshold(battn.dropout_p)
+        T = 0 if frozen else dropout_threshold(battn.dropout_p)
         xb, reg_out, sv["battn"] = _attention_train_fwd(vit, y, film_b, fb, P["reg"], False, True, drop=(seed, 2 * li, T))
         reg = ops.reg_mean(reg_out, N, nwin)
         fg = P["grid"]
@@ -270,21 +285,22 @@ def maxvit_train_backward(vit, saved, cond, dcond, dx, G, prefix):
         # ---- MBConv
         dy = dx.view(M, C)
         bn1, bn2, bn3 = seq[1], seq[4], seq[8]
-        dy0 = ot.bn_bwd(dy, sv["y0"], sv["st3"], bn3.weight, 0, G[pm + "8.weight"], G[pm + "8.bias"])
+        fz = sv["frozen"]
+        dy0 = _bn_bwd(dy, sv["y0"], sv["st3"], bn3, 0, G[pm + "8.weight"], G[pm + "8.bias"], fz)
         ot.colsum(dy0, G[pm + "7.bias"])
         ot.wgrad(dy0, sv["h4"].view(M, hid), G[pm + "7.weight"], tf32=tf32)
         dh4 = ops.gemm(dy0, seq[7].weight.detach().flatten(1).t().contiguous(), tf32=tf32)
         del dy0
         dmean = ot.se_bwd(dh4, sv["h3"], sv["gate"], sv["mean"], sv["hidv"], P["se_w1"], P["se_w2"], G[pm + "6.gate.1.weight"],
                           G[pm + "6.gate.3.weight"])
-        dh2 = ot.bn_bwd(dh4, sv["h2"].view(M, hid), sv["st2"], bn2.weight, 1, G[pm + "4.weight"], G[pm + "4.bias"],
-                        fgate=sv["gate"], fadd=dmean, rows_per_field=H * W, out=dh4)
+        dh2 = _bn_bwd(dh4, sv["h2"].view(M, hid), sv["st2"], bn2, 1, G[pm + "4.weight"], G[pm + "4.bias"], fz,
+                      fgate=sv["gate"], fadd=dmean, rows_per_field=H * W, out=dh4)
         dw9 = torch.zeros(9, hid, dtype=torch.float32, device=dx.device)
         ot.dw3x3_wgrad(sv["h1"].view(N, H, W, hid), dh2.view(N, H, W, hid), dw9, G[pm + "3.bias"])
         G[pm + "3.weight"].view(hid, 9).add_(dw9.t())
         dh1, _ = ot.dw3x3(dh2.view(N, H, W, hid), P["w_dw_flip"], P["ones_hid"], P["zeros_hid"], 0)
         del dh2, dh4
-        dh0 = ot.bn_bwd(dh1.view(M, hid), sv["h0"], sv["st1"], bn1.weight, 1, G[pm + "1.weight"], G[pm + "1.bias"], out=dh1.view(M, hid))
+        dh0 = _bn_bwd(dh1.view(M, hid), sv["h0"], sv["st1"], bn1, 1, G[pm + "1.weight"], G[pm + "1.bias"], fz, out=dh1.view(M, hid))
         ot.colsum(dh0, G[pm + "0.bias"])
         ot.wgrad(dh0, x.view(M, C), G[pm + "0.weight"], tf32=tf32)
         dx = ops.gemm(dh0, seq[0].weight.detach().flatten(1).t().contiguous(), res=dy if P["residual"] else None,
@@ -295,11 +311,12 @@ def maxvit_train_backward(vit, saved, cond, dcond, dx, G, prefix):
 
 class MaxViTTrainFn(torch.autograd.Function):
     """autograd node of a stand-alone ``MaxViT`` in train() mode (maxvit.py:289-341 under autograd): x CL (N,H,W,C) fp32,
-    cond (N,cond_dim) -> y CL; backward returns the gradients of x, cond and every parameter."""
+    cond (N,cond_dim) -> y CL; backward returns the gradients of x, cond and every parameter.  frozen: the eval-mode graph
+    (running-statistic BatchNorm, no dropout, the dropout seed not advanced)."""
 
     @staticmethod
-    def forward(ctx, vit, x, cond, *params):
-        y, saved = maxvit_train_forward(vit, x, cond, seed=vit.next_dropout_seed())
+    def forward(ctx, vit, x, cond, frozen, *params):
+        y, saved = maxvit_train_forward(vit, x, cond, seed=0 if frozen else vit.next_dropout_seed(), frozen=frozen)
         ctx.vit, ctx.saved, ctx.cond = vit, saved, cond
         return y
 
@@ -314,7 +331,7 @@ class MaxViTTrainFn(torch.autograd.Function):
         with torch.cuda.device(dy.device):
             dx = maxvit_train_backward(vit, ctx.saved, ctx.cond, dcond, dy.float().contiguous(), G, "")
         ctx.saved = None
-        return (None, dx, dcond, *[G[n] for n, _ in named])
+        return (None, dx, dcond, None, *[G[n] for n, _ in named])
 
 
 # ------------------------------------------------------------------------------------------------ MetNet3
@@ -356,8 +373,9 @@ def _resblock_train_bwd(dOut, sv, blk, d, G, pre, cond, dcond, N, HP, WP, dtype,
     return dx
 
 
-def metnet3_train_forward(model, x, ts):
-    """-> (pred (B,L,H,W) fp32, saved)"""
+def metnet3_train_forward(model, x, ts, frozen=False):
+    """-> (pred (B,L,H,W) fp32, saved).  frozen: the eval-mode graph (MaxViT BatchNorm from its running statistics, nothing
+    updated, no dropout, the dropout seed not advanced)"""
     B = x.shape[0]
     L, C = model.end_lead_time, model.n_start_channels
     N = B * L
@@ -395,7 +413,7 @@ def metnet3_train_forward(model, x, ts):
     S["enc"], S["h_enc"] = enc, h
     # ---- MaxViT at half resolution
     low = ops.pool2(h, N, HP, WP, out_dtype=model.vit.compute_dtype)
-    low, S["vit"] = maxvit_train_forward(model.vit, low, cond, seed=model.next_dropout_seed())
+    low, S["vit"] = maxvit_train_forward(model.vit, low, cond, seed=0 if frozen else model.next_dropout_seed(), frozen=frozen)
     S["low_out"] = low
     # ---- decoder
     up = torch.zeros(ops.pg_pixels(N, HP, WP), C, dtype=dtype, device=dev)
@@ -413,8 +431,9 @@ def metnet3_train_forward(model, x, ts):
     return pred, S
 
 
-def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None = None):
-    """dpred (B,L,H,W) fp32 -> fills G (parameter gradients, accumulated into the zeroed flat buffer)"""
+def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None = None, want_dx=False):
+    """dpred (B,L,H,W) fp32 -> fills G (parameter gradients, accumulated into the zeroed flat buffer); want_dx: also returns
+    the gradient with respect to the input grids x (B,T,C,H,W) fp32 (else None)"""
     B, N, HP, WP = S["B"], S["N"], S["HP"], S["WP"]
     L, C = model.end_lead_time, model.n_start_channels
     dtype = model.compute_dtype
@@ -477,10 +496,27 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
     ot.wgrad(draw3, st["xin"], dWt, ntaps=9, tap_shift=shifts, beta=0.0)
     gw3 = G[pre + "block1.proj.weight"]
     gw3[:, :c_data].add_(_unpack_wgrad3x3(dWt, C, c_pad, c_data))
-    del draw3, dWt
+    del dWt
+    if want_dx:
+        # data gradient of the per-sample stem: 3x3 conv^T over the data channels (negated tap shifts), c_pad outputs
+        w3t = torch.zeros(c_pad, 9 * C, dtype=dtype, device=dev)
+        w3t[:c_data] = _pack_dgrad3x3(blk0.block1.proj.weight.detach()[:, :c_data], dtype)
+        dxin = ops.gemm(draw3, w3t, ntaps=9, tap_shift=nshifts, out_f32=True)
+        del w3t
+    del draw3
     dres = ot.lead_sum(dH, B, L, HP, WP, dtype)
     dWr = torch.empty(C, c_pad, dtype=torch.float32, device=dev)
     ot.wgrad(dres, st["xin"], dWr, beta=0.0)
+    dx = None
+    if want_dx:
+        # + res_conv^T, accumulated in the GEMM epilogue (each element is read and written by the same thread)
+        wrt = torch.zeros(c_pad, C, dtype=dtype, device=dev)
+        wrt[:c_data] = blk0.res_conv.weight.detach()[:, :c_data, 0, 0].t()
+        ops.gemm(dres, wrt, res=dxin, out=dxin, out_f32=True)
+        del wrt
+        dx = ot.prepare_bwd(dxin, B, model.window_size, model.n_variables, model.input_height, model.input_width, pads, HP, WP,
+                            model.pm25_std, model.standardised_extra_channel)
+        del dxin
     gw1 = G[pre + "res_conv.weight"]
     gw1.view(C, -1)[:, :c_data].add_(dWr[:, :c_data])
     tres_sum = ot.pg_field_sum(dH, N, HP, WP)
@@ -494,6 +530,7 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
     done(5)
     if sync is not None:
         sync.finish()
+    return dx
 
 
 class MetNet3TrainFn(torch.autograd.Function):
@@ -505,8 +542,8 @@ class MetNet3TrainFn(torch.autograd.Function):
     snapshot keeps GradBuffer's layout: ``FlatAdamW`` consumes ``p.grad`` in place when it is still such a view."""
 
     @staticmethod
-    def forward(ctx, model, x, ts, *params):
-        pred, S = metnet3_train_forward(model, x, ts)
+    def forward(ctx, model, x, ts, frozen, *params):
+        pred, S = metnet3_train_forward(model, x, ts, frozen=frozen)
         ctx.model, ctx.S = model, S
         return pred
 
@@ -519,7 +556,7 @@ class MetNet3TrainFn(torch.autograd.Function):
         G = model.grad_buffer()
         G.zero_()
         with torch.cuda.device(dpred.device):
-            metnet3_train_backward(model, ctx.S, dpred.float(), G, model._grad_sync)
+            dx = metnet3_train_backward(model, ctx.S, dpred.float(), G, model._grad_sync, want_dx=ctx.needs_input_grad[1])
         ctx.S = None
         snap = G.snapshot()
-        return (None, None, None, *[snap[n] for n in G.names])
+        return (None, dx, None, None, *[snap[n] for n in G.names])
