@@ -347,7 +347,7 @@ VG_API int vg_bn_act(const float* raw, const float* scale, const float* shift, i
               long long M, int C, void* stream);
 /* BatchNorm (+ activation) backward; the upstream gradient is dOut*fgate[n] + fadd[n] (per-field vectors (N,C) or NULL,
  * n = row / rows_per_field: the squeeze-excite scale and mean paths).  dgamma, dbeta accumulated, draw [M][C] written.
- * work: vg_bn_workspace() + 2*C floats */
+ * C = 4*k with k | 256, or a multiple of 128 up to 2048.  work: vg_bn_workspace() + 2*C floats */
 VG_API int vg_bn_bwd(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean,
               const float* rstd, const float* gamma, int act, const float* fgate, const float* fadd,
               long long rows_per_field, long long M, int C, float* dgamma, float* dbeta, float* draw, float* work,
@@ -363,11 +363,12 @@ VG_API int vg_bn_bwd_frozen(const float* dOut, const float* raw, const float* sc
 /* out[c] += sum_m x[m][c] (bias gradients) */
 VG_API int vg_colsum(const float* x, long long M, int C, float* out, void* stream);
 /* depthwise 3x3 (marching stencil): out = act(conv(in, w9)*scale + shift); psum (or NULL): (N, vg_dw_strips(W), C)
- * partial channel sums of the outputs.  Training forward: scale = 1, shift = bias, act = 0; dgrad: flipped taps. */
+ * partial channel sums of the outputs.  Training forward: scale = 1, shift = bias, act = 0; dgrad: flipped taps.
+ * C = 4*k with k | 128, or (fp32 only) a multiple of 512 */
 VG_API int vg_dw_strips(int W);
 VG_API int vg_dw3x3_fwd(int dtype, const void* in, const float* w9, const float* scale, const float* shift, int act, void* out,
                  float* psum, int N, int H, int W, int C, void* stream);
-/* depthwise weight / bias gradient (accumulated): dw9 [9][C], dbias [C]; work: (N*strips + 1)*10*C floats */
+/* depthwise weight / bias gradient (accumulated): dw9 [9][C], dbias [C]; C as vg_dw3x3_fwd; work: (N*strips + 1)*10*C floats */
 VG_API int vg_dw3x3_wgrad(const float* x, const float* dY, int N, int H, int W, int C, float* dw9, float* dbias, float* work,
                    long long work_elems, void* stream);
 /* squeeze-excite (maxvit.py:33-48) with saved intermediates, out-of-place scale, and backward (dW1, dW2 accumulated,
@@ -396,7 +397,8 @@ VG_API int vg_attn_out_bwd_gather(const float* dx_out, const float* dreg, float 
  * key slot), out_mask [n_windows][64][C] */
 VG_API int vg_dropout_mask_debug(long long drop_seed, int drop_salt, int drop_thresh, long long n_windows, int heads, int C,
                           void* prob_mask, void* out_mask, void* stream);
-/* per-(field, head) core backward: dqkv written; dq_gamma, dk_gamma, dbias_table accumulated.  use_tf32 = 2 / 3: tensor-core
+/* per-(field, head) core backward: dqkv written; dq_gamma, dk_gamma, dbias_table accumulated.  dim_head 32 or 64 (mode 3: 32
+ * only), S <= 64.  use_tf32 = 2 / 3: tensor-core
  * kernel (2: bf16 mma + ldmatrix on fp32 tensors; 3: the tcgen05 kernel on bf16 tensors qkv, datt, dqkv and att_out, which
  * must be 16-byte aligned, S <= 64; fp32 accumulate), which can also re-materialise the forward output
  * att = softmax(.) V [rows][inner] (att_out, or NULL) for the to_out weight gradient when the forward pass was the fused
@@ -406,7 +408,8 @@ VG_API int vg_attn_core_bwd(const void* qkv, const void* datt, const float* q_ga
                      const float* bias_table, int N, int Hl, int Wl, int win, int R, int heads, int dh, void* dqkv,
                      float* dq_gamma, float* dk_gamma, float* dbias_table, int use_tf32, void* att_out, long long drop_seed,
                      int drop_salt, int drop_thresh, void* stream);
-/* LayerNorm + FiLM backward with the inverse partition; dx_in written (= dx + dx_out), dreg_in and dfilm accumulated */
+/* LayerNorm + FiLM backward with the inverse partition; dx_in written (= dx + dx_out), dreg_in and dfilm accumulated.
+ * C = 128, 256, 384 or 512 */
 VG_API int vg_attn_gather_bwd(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
                        const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in,
                        float* dfilm, int N, int Hl, int Wl, int C, int win, int R, int grid_mode, float ln_eps,

@@ -130,8 +130,30 @@ __device__ __forceinline__ float4 bn_dpre4(const BnBwdParams& p, long long r, in
   return g;
 }
 
-// block = 256 threads = (C/4 channel quads) x (256 / (C/4) row lanes) over STAT_ROWS rows; partial (S1, S2) per block
+// block = 256 threads = (C/4 channel quads) x (256 / (C/4) row lanes) over STAT_ROWS rows; partial (S1, S2) per block.
+// WIDE (C > 1024, more quads than threads): a thread per quad of the block's 1024-channel slice blockIdx.y, over all STAT_ROWS rows.
+template <bool WIDE>
 __global__ void __launch_bounds__(256) bn_bwd_reduce_kernel(const BnBwdParams p, float* __restrict__ part) {
+  if constexpr (WIDE) {
+    const int c = (blockIdx.y * 256 + threadIdx.x) * 4;
+    if (c >= p.C) return;
+    const long long r0 = (long long)blockIdx.x * STAT_ROWS;
+    long long r1 = r0 + STAT_ROWS;
+    if (r1 > p.M) r1 = p.M;
+    float4 s1 = make_float4(0.f, 0.f, 0.f, 0.f), s2 = s1;
+    const float4 m = *reinterpret_cast<const float4*>(p.mean + c), rs = *reinterpret_cast<const float4*>(p.rstd + c);
+#pragma unroll 2
+    for (long long r = r0; r < r1; ++r) {
+      const float4 rawv = *reinterpret_cast<const float4*>(p.raw + r * p.C + c);
+      const float4 d = bn_dpre4(p, r, c, rawv);
+      s1.x += d.x; s1.y += d.y; s1.z += d.z; s1.w += d.w;
+      s2.x = fmaf(d.x, (rawv.x - m.x) * rs.x, s2.x); s2.y = fmaf(d.y, (rawv.y - m.y) * rs.y, s2.y);
+      s2.z = fmaf(d.z, (rawv.z - m.z) * rs.z, s2.z); s2.w = fmaf(d.w, (rawv.w - m.w) * rs.w, s2.w);
+    }
+    *reinterpret_cast<float4*>(part + ((long long)blockIdx.x * 2) * p.C + c) = s1;
+    *reinterpret_cast<float4*>(part + ((long long)blockIdx.x * 2 + 1) * p.C + c) = s2;
+    return;
+  }
   __shared__ float4 red[2][256];
   const int quads = p.C / 4, nrl = 256 / quads;
   const int q = threadIdx.x % quads, rl = threadIdx.x / quads, c = q * 4;
@@ -286,16 +308,23 @@ template <> struct Ld4<__half> {
 struct F22 { float2 lo, hi; };
 __device__ __forceinline__ F22 f22(float4 v) { F22 r; r.lo = make_float2(v.x, v.y); r.hi = make_float2(v.z, v.w); return r; }
 
-template <typename T>
-__global__ void __launch_bounds__(128, 3) dwconv_march_kernel(const T* __restrict__ in, const float* __restrict__ w9,
+// SLICED (C a multiple of 512 above 512, fp32: the training forward and data gradient): a block covers one strip of the 512-channel
+// slice blockIdx.y.  At three blocks per SM its register cap spilled; two keep everything in registers.
+template <typename T, bool SLICED = false>
+__global__ void __launch_bounds__(128, SLICED ? 2 : 3) dwconv_march_kernel(const T* __restrict__ in, const float* __restrict__ w9,
                                                            const float* __restrict__ scale, const float* __restrict__ shift, int act,
                                                            T* __restrict__ out, float* __restrict__ psum, int H, int W, int C, int strips) {
-  const int quads = C / 4;
-  const int spb = 128 / quads > 0 ? 128 / quads : 1;             // strips per block
-  const int quad = threadIdx.x % quads, sub = threadIdx.x / quads;
+  const int quads = SLICED ? 128 : C / 4;
+  const int spb = SLICED ? 1 : (128 / quads > 0 ? 128 / quads : 1);             // strips per block
+  const int quad = SLICED ? threadIdx.x : threadIdx.x % quads, sub = SLICED ? 0 : threadIdx.x / quads;
   const int sblocks = (strips + spb - 1) / spb;
   const int n = blockIdx.x / sblocks, strip = (blockIdx.x - n * sblocks) * spb + sub;
   if (sub >= spb || strip >= strips) return;
+  if constexpr (SLICED) {                                          // the slice's channels: offset every channel-indexed pointer once
+    const int cs = blockIdx.y * 512;
+    in += cs; w9 += cs; scale += cs; shift += cs; out += cs;
+    if (psum) psum += cs;
+  }
   const int c0 = quad * 4, w0 = strip * DW_SW;
   F22 wk[9];
 #pragma unroll
@@ -352,14 +381,17 @@ __global__ void __launch_bounds__(128, 3) dwconv_march_kernel(const T* __restric
 
 // depthwise weight gradient: part[(n,strip)][k][c] = sum_{h, w in strip} dY[n,h,w,c] * X[n,h+dy,w+dx,c]  (k = 3*(dy+1)+dx+1),
 // k = 9: sum dY (bias gradient).  fp32 only.
+// SLICED as in dwconv_march_kernel
+template <bool SLICED = false>
 __global__ void __launch_bounds__(128) dw_wgrad_kernel(const float* __restrict__ X, const float* __restrict__ dY, float* __restrict__ part,
                                                        int H, int W, int C, int strips) {
-  const int quads = C / 4;
-  const int spb = 128 / quads > 0 ? 128 / quads : 1;
-  const int quad = threadIdx.x % quads, sub = threadIdx.x / quads;
+  const int quads = SLICED ? 128 : C / 4;
+  const int spb = SLICED ? 1 : (128 / quads > 0 ? 128 / quads : 1);
+  const int quad = SLICED ? threadIdx.x : threadIdx.x % quads, sub = SLICED ? 0 : threadIdx.x / quads;
   const int sblocks = (strips + spb - 1) / spb;
   const int n = blockIdx.x / sblocks, strip = (blockIdx.x - n * sblocks) * spb + sub;
   if (sub >= spb || strip >= strips) return;
+  if constexpr (SLICED) { const int cs = blockIdx.y * 512; X += cs; dY += cs; part += cs; }
   const int c0 = quad * 4, w0 = strip * DW_SW;
   const float* xb = X + (long long)n * H * W * C + c0;
   const float* gb = dY + (long long)n * H * W * C + c0;
@@ -576,7 +608,7 @@ __global__ void __launch_bounds__(256) attn_out_bwd_gather_kernel(const float* _
 
 // Core backward (maxvit.py:195-215), one block per (field, head), looping over the field's windows so that the
 // relative-position-bias and q/k-gamma gradients accumulate in shared memory / registers and reach global memory
-// once per block.  fp32, DH = 32, S <= 64.
+// once per block.  fp32, DH = 32 or 64, S <= 64.
 struct AttnCoreBwdParams {
   const float* qkv;        // [rows][3*inner]
   const float* datt;       // [rows][inner]
@@ -588,8 +620,18 @@ struct AttnCoreBwdParams {
   int heads;
 };
 
+// sum_k a[k] b[k] of one lane's values
+template <int K>
+__device__ __forceinline__ float lane_dot(const float (&a)[K], const float (&b)[K]) {
+  float r = a[0] * b[0];
+#pragma unroll
+  for (int k = 1; k < K; ++k) r = fmaf(a[k], b[k], r);
+  return r;
+}
+
+template <int DH>
 __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdParams p, const DropCfg drop) {
-  constexpr int DH = 32, LD = DH + 1, SM = 64;
+  constexpr int LD = DH + 1, SM = 64, DPL = DH / 32;        // DPL head dims per lane: d = lane + 32*k
   extern __shared__ float sm[];
   const AttnGeom g = p.g;
   const int S = g.S(), nwin = g.nwin(), W2 = 2 * g.win - 1, nb = W2 * W2 + 1;
@@ -613,8 +655,12 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
   const int inner = p.heads * DH;
   const float rs = sqrtf((float)DH);
   for (int i = threadIdx.x; i < nb; i += 256) { sbias[i] = p.bias_table[i * p.heads + hd]; dbias[i] = 0.f; }
-  const float gq = p.qgamma[hd * DH + lane], gk = p.kgamma[hd * DH + lane];
-  float dgq = 0.f, dgk = 0.f;
+  float gq[DPL], gk[DPL], dgq[DPL], dgk[DPL];
+#pragma unroll
+  for (int k = 0; k < DPL; ++k) {
+    gq[k] = p.qgamma[hd * DH + lane + 32 * k]; gk[k] = p.kgamma[hd * DH + lane + 32 * k];
+    dgq[k] = 0.f; dgk[k] = 0.f;
+  }
   __syncthreads();
 
   for (int wi = 0; wi < nwin; ++wi) {
@@ -622,13 +668,19 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
     // ---- load + normalise: warp per row, lane = d
     for (int i = warp; i < S; i += 8) {
       const float* src = p.qkv + (row0 + i) * 3 * inner + hd * DH + lane;
-      const float q = src[0], k = src[inner], v = src[2 * inner];
-      const float nq = fmaxf(sqrtf(warp_sum(q * q)), 1e-12f), nk = fmaxf(sqrtf(warp_sum(k * k)), 1e-12f);
-      const float uq = q / nq, uk = k / nk;
-      qu[i * LD + lane] = uq; ku[i * LD + lane] = uk;
-      qh[i * LD + lane] = uq * rs * gq; kh[i * LD + lane] = uk * rs * gk;
-      vv[i * LD + lane] = v;
-      dO[i * LD + lane] = p.datt[(row0 + i) * inner + hd * DH + lane];
+      float q[DPL], k[DPL], v[DPL];
+#pragma unroll
+      for (int j = 0; j < DPL; ++j) { q[j] = src[32 * j]; k[j] = src[inner + 32 * j]; v[j] = src[2 * inner + 32 * j]; }
+      const float nq = fmaxf(sqrtf(warp_sum(lane_dot<DPL>(q, q))), 1e-12f), nk = fmaxf(sqrtf(warp_sum(lane_dot<DPL>(k, k))), 1e-12f);
+#pragma unroll
+      for (int j = 0; j < DPL; ++j) {
+        const int d = lane + 32 * j;
+        const float uq = q[j] / nq, uk = k[j] / nk;
+        qu[i * LD + d] = uq; ku[i * LD + d] = uk;
+        qh[i * LD + d] = uq * rs * gq[j]; kh[i * LD + d] = uk * rs * gk[j];
+        vv[i * LD + d] = v[j];
+        dO[i * LD + d] = p.datt[(row0 + i) * inner + hd * DH + d];
+      }
       if (lane == 0) { inq[i] = 1.0f / nq; ink[i] = 1.0f / nk; }
     }
     __syncthreads();
@@ -668,10 +720,22 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
     __syncthreads();
     // ---- dV[j][d] = sum_i P'[i][j] dO[i][d] (P' = P * mask): warp per j, lane = d
     for (int j = warp; j < S; j += 8) {
-      float a = 0.f;
-      if (drop.thresh) { for (int i = 0; i < S; ++i) a = fmaf(P[i * (SM + 1) + j] * MK[i * (SM + 1) + j], dO[i * LD + lane], a); }
-      else for (int i = 0; i < S; ++i) a = fmaf(P[i * (SM + 1) + j], dO[i * LD + lane], a);
-      p.dqkv[(row0 + j) * 3 * inner + 2 * inner + hd * DH + lane] = a;
+      float a[DPL];
+#pragma unroll
+      for (int k = 0; k < DPL; ++k) a[k] = 0.f;
+      if (drop.thresh) {
+        for (int i = 0; i < S; ++i) {
+          const float pm = P[i * (SM + 1) + j] * MK[i * (SM + 1) + j];
+#pragma unroll
+          for (int k = 0; k < DPL; ++k) a[k] = fmaf(pm, dO[i * LD + lane + 32 * k], a[k]);
+        }
+      } else {
+        for (int i = 0; i < S; ++i)
+#pragma unroll
+          for (int k = 0; k < DPL; ++k) a[k] = fmaf(P[i * (SM + 1) + j], dO[i * LD + lane + 32 * k], a[k]);
+      }
+#pragma unroll
+      for (int k = 0; k < DPL; ++k) p.dqkv[(row0 + j) * 3 * inner + 2 * inner + hd * DH + lane + 32 * k] = a[k];
     }
     __syncthreads();
     // ---- dS = P * (dP - sum_j P dP), dP[i][j] = dO[i] . v[j]; overwrite P with dS; bias-table gradient
@@ -705,28 +769,42 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
     __syncthreads();
     // ---- dqh[i][d] = sum_j dS[i][j] kh[j][d];  dkh[j][d] = sum_i dS[i][j] qh[i][d]
     for (int i = warp; i < S; i += 8) {
-      float a = 0.f, b = 0.f;
+      float a[DPL], b[DPL];
+#pragma unroll
+      for (int k = 0; k < DPL; ++k) a[k] = b[k] = 0.f;
       for (int j = 0; j < S; ++j) {
-        a = fmaf(P[i * (SM + 1) + j], kh[j * LD + lane], a);
-        b = fmaf(P[j * (SM + 1) + i], qh[j * LD + lane], b);
+#pragma unroll
+        for (int k = 0; k < DPL; ++k) {
+          a[k] = fmaf(P[i * (SM + 1) + j], kh[j * LD + lane + 32 * k], a[k]);
+          b[k] = fmaf(P[j * (SM + 1) + i], qh[j * LD + lane + 32 * k], b[k]);
+        }
       }
-      dqh[i * LD + lane] = a; dkh[i * LD + lane] = b;
+#pragma unroll
+      for (int k = 0; k < DPL; ++k) { dqh[i * LD + lane + 32 * k] = a[k]; dkh[i * LD + lane + 32 * k] = b[k]; }
     }
     __syncthreads();
     // ---- RMSNorm backward (maxvit.py:30): xh = u * rs * gamma, u = x/|x|
     for (int i = warp; i < S; i += 8) {
-      const float aq = dqh[i * LD + lane], ak = dkh[i * LD + lane];
-      const float uq = qu[i * LD + lane], uk = ku[i * LD + lane];
-      dgq = fmaf(aq, uq * rs, dgq); dgk = fmaf(ak, uk * rs, dgk);
-      const float g1 = aq * rs * gq, g2 = ak * rs * gk;
-      const float d1 = warp_sum(g1 * uq), d2 = warp_sum(g2 * uk);
+      float uq[DPL], uk[DPL], g1[DPL], g2[DPL];
+#pragma unroll
+      for (int k = 0; k < DPL; ++k) {
+        const float aq = dqh[i * LD + lane + 32 * k], ak = dkh[i * LD + lane + 32 * k];
+        uq[k] = qu[i * LD + lane + 32 * k]; uk[k] = ku[i * LD + lane + 32 * k];
+        dgq[k] = fmaf(aq, uq[k] * rs, dgq[k]); dgk[k] = fmaf(ak, uk[k] * rs, dgk[k]);
+        g1[k] = aq * rs * gq[k]; g2[k] = ak * rs * gk[k];
+      }
+      const float d1 = warp_sum(lane_dot<DPL>(g1, uq)), d2 = warp_sum(lane_dot<DPL>(g2, uk));
       float* dst = p.dqkv + (row0 + i) * 3 * inner + hd * DH + lane;
-      dst[0] = inq[i] * (g1 - uq * d1);
-      dst[inner] = ink[i] * (g2 - uk * d2);
+#pragma unroll
+      for (int k = 0; k < DPL; ++k) {
+        dst[32 * k] = inq[i] * (g1[k] - uq[k] * d1);
+        dst[inner + 32 * k] = ink[i] * (g2[k] - uk[k] * d2);
+      }
     }
     __syncthreads();
   }
-  gred[(warp * 2) * DH + lane] = dgq; gred[(warp * 2 + 1) * DH + lane] = dgk;
+#pragma unroll
+  for (int k = 0; k < DPL; ++k) { gred[(warp * 2) * DH + lane + 32 * k] = dgq[k]; gred[(warp * 2 + 1) * DH + lane + 32 * k] = dgk[k]; }
   __syncthreads();
   if (threadIdx.x < 2 * DH) {
     const int which = threadIdx.x / DH, d = threadIdx.x % DH;
@@ -750,12 +828,15 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
 // The 53 valid tokens are padded to 64 with zero rows; padded keys are masked to -inf before the softmax.  The
 // relative-position-bias gradient of a thread's 32 fixed (query, key) pairs is accumulated in registers over the field's windows.
 // ------------------------------------------------------------------------------------------------
-namespace cbh {
-constexpr int DH = 32, SM = 64;
-constexpr int LDQ = 40;      // bf16 elements per Q/K/V/dO row (80 B: ldmatrix rows hit distinct banks)
-constexpr int LDP = 72;      // bf16 elements per P/dS row (144 B)
-constexpr int BYTES = 4 * SM * LDQ * 2 + 2 * SM * LDP * 2 + 2 * SM * 4;
-}  // namespace cbh
+template <int DH_>
+struct cbh {
+  static constexpr int DH = DH_, SM = 64;
+  static constexpr int LDQ = DH + 8;   // bf16 elements per Q/K/V/dO row (80 / 144 B: ldmatrix rows hit distinct banks)
+  static constexpr int LDP = 72;       // bf16 elements per P/dS row (144 B)
+  static constexpr int BYTES = 4 * SM * LDQ * 2 + 2 * SM * LDP * 2 + 2 * SM * 4;
+  static constexpr int LPR = DH / 8;   // phase 1: lanes per row (8 consecutive head dims each), rows per pass 32 / LPR
+  static constexpr int PASSES = 16 / (32 / LPR);
+};
 
 __device__ __forceinline__ void ldsm4(uint32_t addr, uint32_t* r) {
   asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];" : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]) : "r"(addr));
@@ -795,8 +876,11 @@ __device__ __forceinline__ uint32_t pack2bf(float a, float b) {
   return *reinterpret_cast<uint32_t*>(&h);
 }
 
-__global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCoreBwdParams p, float* __restrict__ att_out, const DropCfg drop) {
-  using namespace cbh;
+// DH 64: two blocks per SM (the 64-wide accumulators do not fit the three-block register cap; at 255 registers 20 bytes still spill)
+template <int DH_>
+__global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_kernel(const AttnCoreBwdParams p, float* __restrict__ att_out, const DropCfg drop) {
+  using K = cbh<DH_>;
+  constexpr int DH = K::DH, SM = K::SM, LDQ = K::LDQ, LDP = K::LDP, LPR = K::LPR, PASSES = K::PASSES;
   extern __shared__ __align__(16) uint8_t smraw[];
   const AttnGeom g_ = p.g;
   const int S = g_.S(), nwin = g_.nwin(), W2 = 2 * g_.win - 1, nb = W2 * W2 + 1, R = g_.R, win = g_.win;
@@ -818,9 +902,11 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
     sgam[threadIdx.x] = a; sgam[DH + threadIdx.x] = a != 0.f ? 1.0f / a : 0.f;
     sgam[2 * DH + threadIdx.x] = b; sgam[3 * DH + threadIdx.x] = b != 0.f ? 1.0f / b : 0.f;
   }
-  // phase-1 mapping: 4 lanes per row (8 rows per pass), each lane 8 consecutive head dims
-  const int prow = lane >> 2, pd0 = (lane & 3) * 8;
-  float dgq[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f}, dgk[8] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
+  // phase-1 mapping: LPR lanes per row (32 / LPR rows per pass), each lane 8 consecutive head dims
+  const int prow = lane / LPR, pd0 = (lane % LPR) * 8;
+  float dgq[DH / 4], dgk[DH / 4];         // DH 32 only (DH 64 sums them in gred once per window)
+#pragma unroll
+  for (int k = 0; k < DH / 4; ++k) dgq[k] = dgk[k] = 0.f;
   const int r0 = warp * 16;
   const int ia = r0 + g, ib = r0 + g + 8;
   // relative-position-bias index of (query i, key j) = base(i) - off(j); nb-1 when either token is a register token
@@ -842,12 +928,13 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
 
   for (int wi = 0; wi < nwin; ++wi) {
     const long long row0 = ((long long)n * nwin + wi) * S;
-    // ---------------- phase 1: rows r0..r0+15; 4 lanes per row, 16-byte loads, all issued before the first use
-    {
+    // ---------------- phase 1: rows r0..r0+15; LPR lanes per row, 16-byte loads, two passes' loads issued before the first use
+#pragma unroll
+    for (int pg = 0; pg < PASSES; pg += 2) {
       float4 ld[2][4][2];                                   // [pass][q,k,v,dO][half]
 #pragma unroll
       for (int ps = 0; ps < 2; ++ps) {
-        const int i = r0 + ps * 8 + prow;
+        const int i = r0 + (pg + ps) * (32 / LPR) + prow;
 #pragma unroll
         for (int m = 0; m < 4; ++m) { ld[ps][m][0] = make_float4(0.f, 0.f, 0.f, 0.f); ld[ps][m][1] = ld[ps][m][0]; }
         if (i < S) {
@@ -864,7 +951,7 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
       }
 #pragma unroll
       for (int ps = 0; ps < 2; ++ps) {
-        const int i = r0 + ps * 8 + prow;
+        const int i = r0 + (pg + ps) * (32 / LPR) + prow;
         float x[4][8];
 #pragma unroll
         for (int m = 0; m < 4; ++m) {
@@ -874,8 +961,10 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
         float nq = 0.f, nk = 0.f;
 #pragma unroll
         for (int d = 0; d < 8; ++d) { nq = fmaf(x[0][d], x[0][d], nq); nk = fmaf(x[1][d], x[1][d], nk); }
-        nq += __shfl_xor_sync(0xffffffffu, nq, 1); nq += __shfl_xor_sync(0xffffffffu, nq, 2);
-        nk += __shfl_xor_sync(0xffffffffu, nk, 1); nk += __shfl_xor_sync(0xffffffffu, nk, 2);
+#pragma unroll
+        for (int o = 1; o < LPR; o <<= 1) nq += __shfl_xor_sync(0xffffffffu, nq, o);
+#pragma unroll
+        for (int o = 1; o < LPR; o <<= 1) nk += __shfl_xor_sync(0xffffffffu, nk, o);
         const float iq = 1.0f / fmaxf(sqrtf(nq), 1e-12f), ik = 1.0f / fmaxf(sqrtf(nk), 1e-12f);    // F.normalize eps (maxvit.py:30)
         float gq8[8], gk8[8];
         *reinterpret_cast<float4*>(gq8) = *reinterpret_cast<const float4*>(sgam + pd0);
@@ -891,7 +980,7 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
         ud.x = pack2bf(x[3][0], x[3][1]); ud.y = pack2bf(x[3][2], x[3][3]); ud.z = pack2bf(x[3][4], x[3][5]); ud.w = pack2bf(x[3][6], x[3][7]);
         *reinterpret_cast<uint4*>(sQ + i * LDQ + pd0) = uq; *reinterpret_cast<uint4*>(sK + i * LDQ + pd0) = uk;
         *reinterpret_cast<uint4*>(sV + i * LDQ + pd0) = uv; *reinterpret_cast<uint4*>(sdO + i * LDQ + pd0) = ud;
-        if ((lane & 3) == 0) { inq[i] = iq; ink[i] = ik; }
+        if (lane % LPR == 0) { inq[i] = iq; ink[i] = ik; }
       }
     }
     __syncthreads();
@@ -945,12 +1034,12 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
       }
       __syncwarp();
       if (att_out) {                                                // att = P V (re-materialised forward output)
-        float av[4][4];
+        float av[DH / 8][4];
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) av[nt][0] = av[nt][1] = av[nt][2] = av[nt][3] = 0.f;
-        warp_mma_bf16<4, SM, false, true>(av, aP, LDP, r0, aV, LDQ, lane);
+        for (int nt = 0; nt < DH / 8; ++nt) av[nt][0] = av[nt][1] = av[nt][2] = av[nt][3] = 0.f;
+        warp_mma_bf16<DH / 8, SM, false, true>(av, aP, LDP, r0, aV, LDQ, lane);
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
+        for (int nt = 0; nt < DH / 8; ++nt) {
           if (ia < S) *reinterpret_cast<float2*>(att_out + ((row0 + ia) * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(av[nt][0], av[nt][1]);
           if (ib < S) *reinterpret_cast<float2*>(att_out + ((row0 + ib) * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(av[nt][2], av[nt][3]);
         }
@@ -983,36 +1072,43 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
     __syncthreads();
     // ---------------- phase 3: rows r0..r0+15 as keys (dV, dKh) and as queries (dQh)
     {
-      float acc[4][4];
+      float acc[DH / 8][4];
 #pragma unroll
-      for (int nt = 0; nt < 4; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
-      warp_mma_bf16<4, SM, true, true>(acc, aP, LDP, r0, adO, LDQ, lane);                 // dV[j][d] = sum_i P[i][j] dO[i][d]
+      for (int nt = 0; nt < DH / 8; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+      warp_mma_bf16<DH / 8, SM, true, true>(acc, aP, LDP, r0, adO, LDQ, lane);                 // dV[j][d] = sum_i P[i][j] dO[i][d]
 #pragma unroll
-      for (int nt = 0; nt < 4; ++nt) {
+      for (int nt = 0; nt < DH / 8; ++nt) {
         if (ia < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ia) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(acc[nt][0], acc[nt][1]);
         if (ib < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ib) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(acc[nt][2], acc[nt][3]);
       }
 #pragma unroll
       for (int which = 0; which < 2; ++which) {
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
-        if (which == 0) warp_mma_bf16<4, SM, false, true>(acc, aDS, LDP, r0, aK, LDQ, lane);   // dQh = dS Kh
-        else warp_mma_bf16<4, SM, true, true>(acc, aDS, LDP, r0, aQ, LDQ, lane);               // dKh = dS^T Qh
+        for (int nt = 0; nt < DH / 8; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+        if (which == 0) warp_mma_bf16<DH / 8, SM, false, true>(acc, aDS, LDP, r0, aK, LDQ, lane);   // dQh = dS Kh
+        else warp_mma_bf16<DH / 8, SM, true, true>(acc, aDS, LDP, r0, aQ, LDQ, lane);               // dKh = dS^T Qh
         const float* inv = which == 0 ? inq : ink;
         const bf16* sX = which == 0 ? sQ : sK;               // xh = u * rs * gamma (bf16): u = xh / (rs * gamma)
         const float* gtab = sgam + which * 2 * DH;
         float* dg = which == 0 ? dgq : dgk;
-        float ua[8], ub[8], ga[8], gb[8], dota = 0.f, dotb = 0.f;
+        float ua[DH / 4], ub[DH / 4], ga[DH / 4], gb[DH / 4], dota = 0.f, dotb = 0.f;
         const float inva = inv[ia], invb = inv[ib];
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
+        for (int nt = 0; nt < DH / 8; ++nt) {
           const int d = nt * 8 + 2 * t;
           const float2 xa = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(sX + ia * LDQ + d));
           const float2 xb = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(sX + ib * LDQ + d));
           const float2 gg = *reinterpret_cast<const float2*>(gtab + d), ig = *reinterpret_cast<const float2*>(gtab + DH + d);
           ua[2 * nt] = xa.x * ig.x; ua[2 * nt + 1] = xa.y * ig.y; ub[2 * nt] = xb.x * ig.x; ub[2 * nt + 1] = xb.y * ig.y;
-          dg[2 * nt] += (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs;
-          dg[2 * nt + 1] += (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
+          if constexpr (DH == 32) {
+            dg[2 * nt] += (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs;
+            dg[2 * nt + 1] += (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
+          } else {                                         // DH 64: the window's gamma partials go to shared memory (register cap)
+            float a0 = (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs, a1 = (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
+#pragma unroll
+            for (int o = 4; o < 32; o <<= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
+            if (g == 0) { atomicAdd(&gred[which * DH + d], a0); atomicAdd(&gred[which * DH + d + 1], a1); }
+          }
           ga[2 * nt] = acc[nt][0] * gg.x; ga[2 * nt + 1] = acc[nt][1] * gg.y;
           gb[2 * nt] = acc[nt][2] * gg.x; gb[2 * nt + 1] = acc[nt][3] * gg.y;
           dota += ga[2 * nt] * ua[2 * nt] + ga[2 * nt + 1] * ua[2 * nt + 1];
@@ -1021,7 +1117,7 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
         dota += __shfl_xor_sync(0xffffffffu, dota, 1); dota += __shfl_xor_sync(0xffffffffu, dota, 2);
         dotb += __shfl_xor_sync(0xffffffffu, dotb, 1); dotb += __shfl_xor_sync(0xffffffffu, dotb, 2);
 #pragma unroll
-        for (int nt = 0; nt < 4; ++nt) {
+        for (int nt = 0; nt < DH / 8; ++nt) {
           const int d = nt * 8 + 2 * t;
           if (ia < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ia) * 3 * inner + which * inner + hd * DH + d)) =
                             make_float2(inva * (ga[2 * nt] - ua[2 * nt] * dota), inva * (ga[2 * nt + 1] - ua[2 * nt + 1] * dota));
@@ -1044,7 +1140,7 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
     }
   }
 #pragma unroll
-  for (int k = 0; k < 8; ++k) {
+  for (int k = 0; k < (DH == 32 ? DH / 4 : 0); ++k) {
     float a = dgq[k], b = dgk[k];
     a += __shfl_xor_sync(0xffffffffu, a, 4); a += __shfl_xor_sync(0xffffffffu, a, 8); a += __shfl_xor_sync(0xffffffffu, a, 16);
     b += __shfl_xor_sync(0xffffffffu, b, 4); b += __shfl_xor_sync(0xffffffffu, b, 8); b += __shfl_xor_sync(0xffffffffu, b, 16);
@@ -1061,11 +1157,11 @@ __global__ void __launch_bounds__(128, 3) attn_core_bwd_bf16_kernel(const AttnCo
   for (int i = threadIdx.x; i < nb; i += 128) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
 }
 
-// LayerNorm (no affine) + FiLM backward with the inverse partition (maxvit.py:176-187, 298-308, 322-332), C = 128.
+// LayerNorm (no affine) + FiLM backward with the inverse partition (maxvit.py:176-187, 298-308, 322-332), C = 128 .. 512.
 //   tok = xhat*gamma[n] + beta[n];  dgamma[n][c] += dtok*xhat;  dbeta[n][c] += dtok;  dxhat = dtok*gamma
 //   dx = rstd*(dxhat - mean(dxhat) - xhat*mean(dxhat*xhat)) + dres   (dres = gradient of the residual path)
 // window rows write dx_in[pix] = dx + dx_out[pix]; register rows accumulate into dreg_in ([R][C] or [N][R][C]) with
-// the residual gradient dreg_res (N,R,C)*reg_scale (or none).
+// the residual gradient dreg_res (N,R,C)*reg_scale (or none).  A warp per row; lane owns channels [lane*4 + 128*k, +4).
 struct AttnGatherBwdParams {
   const float* x; const float* reg; int reg_per_field; const float* film;
   const float* dtok; const float* dx_out; const float* dreg_res; float reg_scale;
@@ -1073,17 +1169,26 @@ struct AttnGatherBwdParams {
   AttnGeom g; float eps;
 };
 
+template <int C>
 __global__ void __launch_bounds__(256) attn_gather_bwd_kernel(const AttnGatherBwdParams p, long long rows) {
-  constexpr int C = 128, RPW = 16;
+  constexpr int RPW = 16, NV = C / 128, NE = 4 * NV;
   const AttnGeom g = p.g;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c0 = lane * 4;
   const int S = g.S(), nwin = g.nwin();
-  float ag[4] = {0.f, 0.f, 0.f, 0.f}, ab[4] = {0.f, 0.f, 0.f, 0.f};
+  float ag[NE], ab[NE];
+#pragma unroll
+  for (int i = 0; i < NE; ++i) ag[i] = ab[i] = 0.f;
   int n_cur = -1;
   auto flush = [&]() {
     if (n_cur < 0) return;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) { atomicAdd(p.dfilm + (long long)n_cur * 2 * C + c0 + i, ag[i]); atomicAdd(p.dfilm + (long long)n_cur * 2 * C + C + c0 + i, ab[i]); ag[i] = ab[i] = 0.f; }
+    for (int k = 0; k < NV; ++k)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        atomicAdd(p.dfilm + (long long)n_cur * 2 * C + 128 * k + c0 + i, ag[4 * k + i]);
+        atomicAdd(p.dfilm + (long long)n_cur * 2 * C + C + 128 * k + c0 + i, ab[4 * k + i]);
+        ag[4 * k + i] = ab[4 * k + i] = 0.f;
+      }
   };
   const long long r0 = ((long long)blockIdx.x * 8 + warp) * RPW;
   // (window, token) of the warp's first row by division, then incrementally: four 64- / 32-bit divisions per row were most of the
@@ -1104,34 +1209,52 @@ __global__ void __launch_bounds__(256) attn_gather_bwd_kernel(const AttnGatherBw
       pix = (long long)n * g.Hl * g.Wl + (long long)ph * g.Wl + pw;
       src = p.x + pix * C;
     }
-    const float4 xv = *reinterpret_cast<const float4*>(src + c0);
-    float v[4] = {xv.x, xv.y, xv.z, xv.w};
-    const float mean = warp_sum(v[0] + v[1] + v[2] + v[3]) * (1.0f / C);
+    float v[NE];
+#pragma unroll
+    for (int j = 0; j < NV; ++j) {
+      const float4 xv = *reinterpret_cast<const float4*>(src + 128 * j + c0);
+      v[4 * j] = xv.x; v[4 * j + 1] = xv.y; v[4 * j + 2] = xv.z; v[4 * j + 3] = xv.w;
+    }
+    float sum = v[0] + v[1] + v[2] + v[3];
+#pragma unroll
+    for (int j = 1; j < NV; ++j) sum += v[4 * j] + v[4 * j + 1] + v[4 * j + 2] + v[4 * j + 3];
+    const float mean = warp_sum(sum) * (1.0f / C);
     float ss = 0.f;
 #pragma unroll
-    for (int i = 0; i < 4; ++i) { v[i] -= mean; ss += v[i] * v[i]; }
+    for (int i = 0; i < NE; ++i) { v[i] -= mean; ss += v[i] * v[i]; }
     const float rstd = rsqrtf(warp_sum(ss) * (1.0f / C) + p.eps);
-    const float4 gm = *reinterpret_cast<const float4*>(p.film + (long long)n * 2 * C + c0);
-    const float4 dt = *reinterpret_cast<const float4*>(p.dtok + r * C + c0);
-    const float gmv[4] = {gm.x, gm.y, gm.z, gm.w}, dtv[4] = {dt.x, dt.y, dt.z, dt.w};
-    float dx[4], s1 = 0.f, s2 = 0.f;
+    float gmv[NE], dtv[NE];
 #pragma unroll
-    for (int i = 0; i < 4; ++i) {
+    for (int j = 0; j < NV; ++j) {
+      const float4 gm = *reinterpret_cast<const float4*>(p.film + (long long)n * 2 * C + 128 * j + c0);
+      const float4 dt = *reinterpret_cast<const float4*>(p.dtok + r * C + 128 * j + c0);
+      gmv[4 * j] = gm.x; gmv[4 * j + 1] = gm.y; gmv[4 * j + 2] = gm.z; gmv[4 * j + 3] = gm.w;
+      dtv[4 * j] = dt.x; dtv[4 * j + 1] = dt.y; dtv[4 * j + 2] = dt.z; dtv[4 * j + 3] = dt.w;
+    }
+    float dx[NE], s1 = 0.f, s2 = 0.f;
+#pragma unroll
+    for (int i = 0; i < NE; ++i) {
       v[i] *= rstd;                                            // xhat
       ag[i] = fmaf(dtv[i], v[i], ag[i]); ab[i] += dtv[i];
       dx[i] = dtv[i] * gmv[i]; s1 += dx[i]; s2 = fmaf(dx[i], v[i], s2);
     }
     s1 = warp_sum(s1) * (1.0f / C); s2 = warp_sum(s2) * (1.0f / C);
 #pragma unroll
-    for (int i = 0; i < 4; ++i) dx[i] = rstd * (dx[i] - s1 - v[i] * s2);
+    for (int i = 0; i < NE; ++i) dx[i] = rstd * (dx[i] - s1 - v[i] * s2);
     if (tok < g.R) {
       float* d = p.dreg_in + (p.reg_per_field ? (long long)n * g.R * C : 0) + (long long)tok * C + c0;
       const float* rr = p.dreg_res ? p.dreg_res + ((long long)n * g.R + tok) * C + c0 : nullptr;
 #pragma unroll
-      for (int i = 0; i < 4; ++i) atomicAdd(d + i, dx[i] + (rr ? rr[i] * p.reg_scale : 0.f));
+      for (int j = 0; j < NV; ++j)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) atomicAdd(d + 128 * j + i, dx[4 * j + i] + (rr ? rr[128 * j + i] * p.reg_scale : 0.f));
     } else {
-      const float4 ro = *reinterpret_cast<const float4*>(p.dx_out + pix * C + c0);
-      *reinterpret_cast<float4*>(p.dx_in + pix * C + c0) = make_float4(dx[0] + ro.x, dx[1] + ro.y, dx[2] + ro.z, dx[3] + ro.w);
+#pragma unroll
+      for (int j = 0; j < NV; ++j) {
+        const float4 ro = *reinterpret_cast<const float4*>(p.dx_out + pix * C + 128 * j + c0);
+        *reinterpret_cast<float4*>(p.dx_in + pix * C + 128 * j + c0) =
+            make_float4(dx[4 * j] + ro.x, dx[4 * j + 1] + ro.y, dx[4 * j + 2] + ro.z, dx[4 * j + 3] + ro.w);
+      }
     }
     // next row
     if (tok >= g.R) { if (++tb == g.win) { tb = 0; ++ta; } }
@@ -1169,18 +1292,26 @@ int bn_act_run(const float* raw, const float* scale, const float* shift, int act
   return check_launch("bn_act_kernel");
 }
 
+static bool bn_bwd_width_ok(int C) { return C > 0 && ((C % 4 == 0 && 256 % (C / 4) == 0) || (C % 128 == 0 && C <= 2048)); }
+
+// partial (S1, S2) per STAT_ROWS rows into work[nparts][2][C]
+static int bn_bwd_reduce_launch(const BnBwdParams& p, int nparts, float* work, cudaStream_t st) {
+  if (p.C <= 1024) bn_bwd_reduce_kernel<false><<<nparts, 256, 0, st>>>(p, work);
+  else bn_bwd_reduce_kernel<true><<<dim3(nparts, (p.C + 1023) / 1024), 256, 0, st>>>(p, work);
+  return check_launch("bn_bwd_reduce_kernel");
+}
+
 int bn_bwd_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
                const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
                float* dgamma, float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st) {
   const int nparts = (int)((M + STAT_ROWS - 1) / STAT_ROWS);
-  if (C % 4 || C / 4 > 256 || 256 % (C / 4)) return set_error("bn_bwd: C=%d must be 4*k with k | 256", C);
+  if (!bn_bwd_width_ok(C)) return set_error("bn_bwd: C=%d must be 4*k with k | 256, or a multiple of 128 up to 2048", C);
   if (work_elems < (long long)nparts * 2 * C + 2 * C) return set_error("bn_bwd: workspace too small");
   BnBwdParams p;
   p.dOut = dOut; p.raw = raw; p.scale = scale; p.shift = shift; p.mean = mean; p.rstd = rstd; p.gamma = gamma;
   p.fgate = fgate; p.fadd = fadd; p.rows_per_field = rows_per_field > 0 ? rows_per_field : 1; p.act = act; p.C = C; p.M = M;
   float* k1 = work + (long long)nparts * 2 * C; float* k2 = k1 + C;
-  bn_bwd_reduce_kernel<<<nparts, 256, 0, st>>>(p, work);
-  int rc = check_launch("bn_bwd_reduce_kernel");
+  int rc = bn_bwd_reduce_launch(p, nparts, work, st);
   if (rc) return rc;
   bn_bwd_finalize_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, M, C, dgamma, dbeta, k1, k2);
   rc = check_launch("bn_bwd_finalize_kernel");
@@ -1194,14 +1325,13 @@ int bn_bwd_frozen_run(const float* dOut, const float* raw, const float* scale, c
                       int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C, float* dgamma,
                       float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st) {
   const int nparts = (int)((M + STAT_ROWS - 1) / STAT_ROWS);
-  if (C % 4 || C / 4 > 256 || 256 % (C / 4)) return set_error("bn_bwd_frozen: C=%d must be 4*k with k | 256", C);
+  if (!bn_bwd_width_ok(C)) return set_error("bn_bwd_frozen: C=%d must be 4*k with k | 256, or a multiple of 128 up to 2048", C);
   if (work_elems < (long long)nparts * 2 * C) return set_error("bn_bwd_frozen: workspace too small");
   if (M <= 0) return 0;
   BnBwdParams p;
   p.dOut = dOut; p.raw = raw; p.scale = scale; p.shift = shift; p.mean = mean; p.rstd = rstd; p.gamma = nullptr;
   p.fgate = fgate; p.fadd = fadd; p.rows_per_field = rows_per_field > 0 ? rows_per_field : 1; p.act = act; p.C = C; p.M = M;
-  bn_bwd_reduce_kernel<<<nparts, 256, 0, st>>>(p, work);
-  int rc = check_launch("bn_bwd_reduce_kernel");
+  int rc = bn_bwd_reduce_launch(p, nparts, work, st);
   if (rc) return rc;
   bn_bwd_finalize_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, M, C, dgamma, dbeta, nullptr, nullptr);
   rc = check_launch("bn_bwd_finalize_kernel");
@@ -1217,8 +1347,15 @@ int colsum_run(const float* X, long long M, int C, float* out, cudaStream_t st) 
 
 int dwconv_march_run(int dtype, const void* in, const float* w9, const float* scale, const float* shift, int act, void* out,
                      float* psum, int N, int H, int W, int C, cudaStream_t st) {
-  if (C % 4 || C / 4 > 128 || (128 % (C / 4))) return set_error("dwconv: C=%d must be 4*k with k | 128", C);
+  const bool sliced = C > 512 && C % 512 == 0;
+  if (!sliced && (C % 4 || C / 4 > 128 || (128 % (C / 4)))) return set_error("dwconv: C=%d must be 4*k with k | 128, or a multiple of 512", C);
   const int strips = (W + DW_SW - 1) / DW_SW;
+  if (sliced) {
+    if (dtype != 1) return set_error("dwconv: C=%d > 512 is built for fp32 only", C);
+    dwconv_march_kernel<float, true><<<dim3(N * strips, C / 512), 128, 0, st>>>(reinterpret_cast<const float*>(in), w9, scale, shift, act,
+                                                                               reinterpret_cast<float*>(out), psum, H, W, C, strips);
+    return check_launch("dwconv_march_kernel");
+  }
   const int spb = 128 / (C / 4);
   const int sblocks = (strips + spb - 1) / spb;
   if (dtype == 0) dwconv_march_kernel<bf16><<<N * sblocks, 128, 0, st>>>(reinterpret_cast<const bf16*>(in), w9, scale, shift, act, reinterpret_cast<bf16*>(out), psum, H, W, C, strips);
@@ -1230,13 +1367,18 @@ int dwconv_strips(int W) { return (W + DW_SW - 1) / DW_SW; }
 
 int dw_wgrad_run(const float* X, const float* dY, int N, int H, int W, int C, float* dw9, float* dbias, float* work,
                  long long work_elems, cudaStream_t st) {
-  if (C % 4 || C / 4 > 128 || (128 % (C / 4))) return set_error("dw_wgrad: C=%d must be 4*k with k | 128", C);
+  const bool sliced = C > 512 && C % 512 == 0;
+  if (!sliced && (C % 4 || C / 4 > 128 || (128 % (C / 4)))) return set_error("dw_wgrad: C=%d must be 4*k with k | 128, or a multiple of 512", C);
   const int strips = (W + DW_SW - 1) / DW_SW;
   const long long nparts = (long long)N * strips;
   if (work_elems < nparts * 10 * C + 10 * C) return set_error("dw_wgrad: workspace too small");
-  const int spb = 128 / (C / 4);
-  const int sblocks = (strips + spb - 1) / spb;
-  dw_wgrad_kernel<<<N * sblocks, 128, 0, st>>>(X, dY, work, H, W, C, strips);
+  if (sliced) {
+    dw_wgrad_kernel<true><<<dim3(N * strips, C / 512), 128, 0, st>>>(X, dY, work, H, W, C, strips);
+  } else {
+    const int spb = 128 / (C / 4);
+    const int sblocks = (strips + spb - 1) / spb;
+    dw_wgrad_kernel<<<N * sblocks, 128, 0, st>>>(X, dY, work, H, W, C, strips);
+  }
   int rc = check_launch("dw_wgrad_kernel");
   if (rc) return rc;
   float* tot = work + nparts * 10 * C;
@@ -1353,59 +1495,79 @@ int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma,
                          const AttnGeom& g, int heads, void* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                          void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
 
+// exact-fp32 SIMT core backward: 8 [64][DH+1] row tiles, P (and the dropout mask) [64][65], bias-table rows, 1/|q|, 1/|k| and the
+// per-warp gamma partials (DH 64 with dropout: 172 KB)
+template <int DH>
+static int core_bwd_simt_launch(const AttnCoreBwdParams& p, int nb, const DropCfg& drop, cudaStream_t st) {
+  const size_t smem = (size_t)(8 * 64 * (DH + 1) + 64 * 65 + 2 * nb + 128 + 8 * 2 * DH + (drop.thresh ? 64 * 65 : 0)) * sizeof(float);
+  static PerDeviceSize attr_pd;                  // depends on the window size: raise the limit when it grows
+  size_t& attr = attr_pd.cur();
+  if (smem > attr) {
+    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_kernel<DH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return set_error("attn_core_bwd smem attr: %s", cudaGetErrorString(e));
+    attr = smem;
+  }
+  attn_core_bwd_kernel<DH><<<p.g.N * p.heads, 256, smem, st>>>(p, drop);
+  return check_launch("attn_core_bwd_kernel");
+}
+
+template <int DH>
+static int core_bwd_bf16_launch(const AttnCoreBwdParams& q, int nb, float* att_out, const DropCfg& drop, cudaStream_t st) {
+  const size_t smem3 = (size_t)cbh<DH>::BYTES + (size_t)(2 * nb + 6 * DH) * sizeof(float);
+  static PerDeviceSize attr3_pd;                  // depends on the window size: raise the limit when it grows
+  size_t& attr3 = attr3_pd.cur();
+  if (smem3 > attr3) {
+    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_bf16_kernel<DH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
+    if (e != cudaSuccess) return set_error("attn_core_bwd_bf16 smem attr: %s", cudaGetErrorString(e));
+    attr3 = smem3;
+  }
+  attn_core_bwd_bf16_kernel<DH><<<q.g.N * q.heads, 128, smem3, st>>>(q, att_out, drop);
+  return check_launch("attn_core_bwd_bf16_kernel");
+}
+
 // use_tf32: 0 exact-fp32 SIMT, 2 bf16 mma.sync on fp32 tensors, 3 bf16 tensors (qkv, datt, dqkv, att_out): the
 // tcgen05 kernel (vg_attn_bwd_tc.cu)
 int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                       const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                       int use_tf32, float* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
-  if (dh != 32) return set_error("attn_core_bwd: dim_head must be 32 (got %d)", dh);
   if (drop_thresh < 0 || drop_thresh > 255) return set_error("attn_core_bwd: dropout threshold %d outside [0, 255]", drop_thresh);
   if (use_tf32 != 0 && use_tf32 != 2 && use_tf32 != 3) return set_error("attn_core_bwd: mode %d (0 exact fp32, 2 bf16 mma on fp32 tensors, 3 bf16 tensors)", use_tf32);
+  if ((use_tf32 == 3 && dh != 32) || (dh != 32 && dh != 64)) return set_error("attn_core_bwd: dim_head must be 32 (got %d)", dh);
   if (g.S() > 64) return set_error("attn_core_bwd: sequence %d > 64", g.S());
   const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
   if (use_tf32 == 3)
     return attn_core_bwd_tc_run(qkv, datt, qgamma, kgamma, bias_table, g, heads, dqkv, dqgamma, dkgamma, dbias_table, att_out, seed, salt,
                                 drop_thresh, st);
   if (use_tf32 == 2) {
-    const size_t smem3 = (size_t)cbh::BYTES + (size_t)(2 * nb + 6 * cbh::DH) * sizeof(float);
-    static PerDeviceSize attr3_pd;                  // depends on the window size: raise the limit when it grows
-    size_t& attr3 = attr3_pd.cur();
-    if (smem3 > attr3) {
-      cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_bf16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem3);
-      if (e != cudaSuccess) return set_error("attn_core_bwd_bf16 smem attr: %s", cudaGetErrorString(e));
-      attr3 = smem3;
-    }
     AttnCoreBwdParams q;
     q.qkv = qkv; q.datt = datt; q.qgamma = qgamma; q.kgamma = kgamma; q.bias_table = bias_table; q.dqkv = dqkv;
     q.dqgamma = dqgamma; q.dkgamma = dkgamma; q.dbias_table = dbias_table; q.g = g; q.heads = heads;
-    attn_core_bwd_bf16_kernel<<<g.N * heads, 128, smem3, st>>>(q, att_out, make_drop(seed, salt, drop_thresh));
-    return check_launch("attn_core_bwd_bf16_kernel");
+    return dh == 32 ? core_bwd_bf16_launch<32>(q, nb, att_out, make_drop(seed, salt, drop_thresh), st)
+                    : core_bwd_bf16_launch<64>(q, nb, att_out, make_drop(seed, salt, drop_thresh), st);
   }
   if (att_out) return set_error("attn_core_bwd: att_out is only produced by the tensor-core kernels (modes 2, 3)");
-  const size_t smem = (size_t)(8 * 64 * 33 + 64 * 65 + 2 * nb + 128 + 8 * 2 * 32 + (drop_thresh ? 64 * 65 : 0)) * sizeof(float);
-  static PerDeviceSize attr_pd;                  // depends on the window size: raise the limit when it grows
-  size_t& attr = attr_pd.cur();
-  if (smem > attr) {
-    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return set_error("attn_core_bwd smem attr: %s", cudaGetErrorString(e));
-    attr = smem;
-  }
   AttnCoreBwdParams p;
   p.qkv = qkv; p.datt = datt; p.qgamma = qgamma; p.kgamma = kgamma; p.bias_table = bias_table; p.dqkv = dqkv;
   p.dqgamma = dqgamma; p.dkgamma = dkgamma; p.dbias_table = dbias_table; p.g = g; p.heads = heads;
-  attn_core_bwd_kernel<<<g.N * heads, 256, smem, st>>>(p, make_drop(seed, salt, drop_thresh));
-  return check_launch("attn_core_bwd_kernel");
+  return dh == 32 ? core_bwd_simt_launch<32>(p, nb, make_drop(seed, salt, drop_thresh), st)
+                  : core_bwd_simt_launch<64>(p, nb, make_drop(seed, salt, drop_thresh), st);
 }
 
 int attn_gather_bwd_run(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
                         const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in, float* dfilm,
                         const AttnGeom& g, float eps, cudaStream_t st) {
-  if (g.C != 128) return set_error("attn_gather_bwd: C must be 128");
+  if (g.C != 128 && g.C != 256 && g.C != 384 && g.C != 512) return set_error("attn_gather_bwd: C=%d must be 128, 256, 384 or 512", g.C);
   AttnGatherBwdParams p;
   p.x = x; p.reg = reg; p.reg_per_field = reg_per_field; p.film = film; p.dtok = dtok; p.dx_out = dx_out; p.dreg_res = dreg_res;
   p.reg_scale = reg_scale; p.dx_in = dx_in; p.dreg_in = dreg_in; p.dfilm = dfilm; p.g = g; p.eps = eps;
   const long long rows = (long long)g.N * g.nwin() * g.S();
-  attn_gather_bwd_kernel<<<nblk(rows, 8 * 16), 256, 0, st>>>(p, rows);
+  const unsigned grid = nblk(rows, 8 * 16);
+  switch (g.C) {
+    case 128: attn_gather_bwd_kernel<128><<<grid, 256, 0, st>>>(p, rows); break;
+    case 256: attn_gather_bwd_kernel<256><<<grid, 256, 0, st>>>(p, rows); break;
+    case 384: attn_gather_bwd_kernel<384><<<grid, 256, 0, st>>>(p, rows); break;
+    default: attn_gather_bwd_kernel<512><<<grid, 256, 0, st>>>(p, rows); break;
+  }
   return check_launch("attn_gather_bwd_kernel");
 }
 

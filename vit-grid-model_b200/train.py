@@ -150,15 +150,13 @@ def _unpack_wgrad3x3(dWt, co, ci_pad, ci):
 def _attention_train_fwd(vit, x, film, P, reg_in, grid_mode, want_reg_out, drop=(0, 0, 0)):
     """shapes vit.fused_attn_applies accepts (mixed precision): the fused one-kernel attention, nothing but its inputs is
     kept (backward re-materialises tokens / qkv / att on the tensor cores); fp32 mode and every other shape: un-fused path,
-    intermediates saved (attention dropout there is not built for the tf32 mode)."""
+    intermediates saved (its core applies the same dropout masks as the fused kernel)."""
     N, H, W, C = x.shape
     w, R = vit.vit_window_size, vit.num_register_tokens
     if vit.fused_attn_applies(C):
         x_out, reg_out = ops.attn_fused(x, reg_in, film, P["wqkv_h"], P["wout_h"], P["head_tab"], w, R, grid_mode, want_reg_out,
                                         vit.heads, vit.dim_head, drop=drop)
         return x_out, reg_out, dict(x=x, film=film, reg_in=reg_in, grid_mode=grid_mode, drop=drop)
-    if drop[2] and vit.tf32:
-        raise NotImplementedError("attention dropout on the un-fused tf32 path (shapes the fused kernel does not cover) is not built")
     tokens = ops.attn_gather(x, reg_in, film, w, R, grid_mode)
     qkv = ops.gemm(tokens, P["w_qkv"], tf32=vit.tf32)
     att = ops.attn_core(qkv, P["q_gamma"], P["k_gamma"], P["bias_table"], N, H, W, w, R, vit.heads, vit.dim_head, drop=drop)
@@ -221,8 +219,9 @@ def _bn_bwd(dOut, raw, st, bn, act, dgamma, dbeta, frozen, **kw):
 
 def maxvit_train_forward(vit, x, cond, seed=0, frozen=False):
     """x CL (N,H,W,C) fp32, cond (N,cd) -> (y, saved).  seed: dropout seed of this step (ignored when dropout is 0).
-    frozen: the eval-mode graph -- BatchNorm from its running statistics (nothing updated), no dropout"""
-    N, H, W, C = x.shape
+    frozen: the eval-mode graph -- BatchNorm from its running statistics (nothing updated), no dropout.  The first layer of a
+    stage of a tuple-depth MaxViT widens the map: its MBConv maps C_in -> C_out and everything after it runs at C_out."""
+    N, H, W, _ = x.shape
     w = vit.vit_window_size
     nwin = (H // w) * (W // w)
     M = N * H * W
@@ -230,7 +229,7 @@ def maxvit_train_forward(vit, x, cond, seed=0, frozen=False):
     saved = []
     for li, (P, (conv, battn, gattn)) in enumerate(zip(vit.packed(x.dtype), vit.layers)):
         seq = conv.fn if isinstance(conv, MBConvResidual) else conv
-        x2d = x.view(M, C)
+        x2d = x.view(M, x.shape[3])
         bn1, bn2, bn3 = seq[1], seq[4], seq[8]
         h0 = ops.gemm(x2d, P["w_exp"], bias=P["b_exp"], tf32=tf32)
         hid = h0.shape[1]
@@ -243,7 +242,7 @@ def maxvit_train_forward(vit, x, cond, seed=0, frozen=False):
         h4 = ot.se_scale_oop(h3, gate)
         y0 = ops.gemm(h4.view(M, hid), P["w_proj"], bias=P["b_proj"], tf32=tf32)
         st3 = _bn_stats(bn3, y0, frozen)
-        y = ot.bn_act(y0, st3, 0, res=x2d if P["residual"] else None).view(N, H, W, C)
+        y = ot.bn_act(y0, st3, 0, res=x2d if P["residual"] else None).view(N, H, W, y0.shape[1])
         if not frozen:
             for bn in (bn1, bn2, bn3):
                 bn.num_batches_tracked += 1
@@ -272,18 +271,19 @@ def maxvit_train_backward(vit, saved, cond, dcond, dx, G, prefix):
         seq = conv.fn if isinstance(conv, MBConvResidual) else conv
         pm = f"{prefix}layers.{li}.0." + ("fn." if isinstance(conv, MBConvResidual) else "")
         x = sv["x"]
-        N, H, W, C = x.shape
+        N, H, W, C = x.shape                              # MBConv input width; the attention runs at the output width C_out
+        C_out = dx.shape[3]
         nwin = (H // w) * (W // w)
         M = N * H * W
         hid = sv["h0"].shape[1]
         # ---- grid attention, then block attention (register tokens link the two, maxvit.py:326)
-        dreg_mean = torch.zeros(N, R, C, dtype=torch.float32, device=dx.device)
+        dreg_mean = torch.zeros(N, R, C_out, dtype=torch.float32, device=dx.device)
         dx = _attention_train_bwd(vit, sv["gattn"], P["grid"], gattn, f"{prefix}layers.{li}.2.", G, cond, dcond, dx, None, 0.0,
                                   dreg_mean)
         dx = _attention_train_bwd(vit, sv["battn"], P["block"], battn, f"{prefix}layers.{li}.1.", G, cond, dcond, dx, dreg_mean,
                                   1.0 / nwin, G[f"{prefix}register_tokens.{li}"])
         # ---- MBConv
-        dy = dx.view(M, C)
+        dy = dx.view(M, C_out)
         bn1, bn2, bn3 = seq[1], seq[4], seq[8]
         fz = sv["frozen"]
         dy0 = _bn_bwd(dy, sv["y0"], sv["st3"], bn3, 0, G[pm + "8.weight"], G[pm + "8.bias"], fz)
