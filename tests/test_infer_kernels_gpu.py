@@ -590,12 +590,14 @@ def test_mbconv_dw_fp16_se_chain(N):
 
 
 @pytest.mark.parametrize("dtype", [BF16, F32], ids=["bf16", "fp32"])
-@pytest.mark.parametrize("C", [1536, 2048])
-def test_dw3x3_bnact_wide_hidden(dtype, C):
-    """vg_dw3x3_bnact_fwd at hidden widths where 128 % (C / 4) != 0 (dims 384 and 512 x expansion 4), with its per-row
-    channel sums, and vg_se_scale_fwd in place"""
+@pytest.mark.parametrize("C,N,H,W", [(1536, 2, 14, 21), (2048, 2, 14, 21), (1024, 2, 14, 21), (1024, 48, 42, 35), (2048, 48, 42, 35)],
+                         ids=["1536", "2048", "1024", "1024_n48_42x35", "2048_n48_42x35"])
+def test_dw3x3_bnact_wide_hidden(dtype, C, N, H, W):
+    """vg_dw3x3_bnact_fwd at hidden widths where 128 % (C / 4) != 0 (dims 256, 384 and 512 x expansion 4), with its per-row
+    channel sums, and vg_se_scale_fwd in place.  C = 1024 is the one width where a block of 256 threads holds two pixel lanes
+    per row (C / 8 = 128 channel groups) whose partial sums the block adds up; at W = 35 the two lanes get 18 and 17 pixels.
+    48 fields of 42x35: the configs[4] chunk"""
     o = O()
-    N, H, W = 2, 14, 21
     x, w, s, t = _dw_operands(N, H, W, C, dtype, seed=110)
     out = nan_like((N, H, W, C), dtype)
     out, psum = o.dw3x3_bnact(x, w.reshape(C, 9).t().contiguous(), s, t, out=out)

@@ -322,13 +322,16 @@ def test_dw3x3_wide(C, W):
 
 
 # =========================================================================================== squeeze-excite
-@pytest.mark.parametrize("N,H,W", [(3, 14, 21), (1100, 7, 7)])
-def test_squeeze_excite_wide(N, H, W):
-    """maxvit.py:33-48 at C = 2048, se = 512: the gate with its saved intermediates on both branches of vg_se_gate_train_fwd
-    (N <= 1024: field means + two dense-row passes; N = 1100: one block per field) and the backward (dW1, dW2 accumulated, dmean
-    written), from partial sums and intermediates derived in float64"""
+@pytest.mark.parametrize("N,H,W,C", [(3, 14, 21, 2048), (1100, 7, 7, 2048), (48, 42, 35, 2048), (48, 42, 35, 1024),
+                                     (1100, 7, 7, 1024)],
+                         ids=["3-14-21", "1100-7-7", "48-42-35", "48-42-35-c1024", "1100-7-7-c1024"])
+def test_squeeze_excite_wide(N, H, W, C):
+    """maxvit.py:33-48 at C = 2048, se = 512 (512-channel networks) and C = 1024, se = 256 (256-channel networks): the gate
+    with its saved intermediates on both branches of vg_se_gate_train_fwd (N <= 1024: field means + two dense-row passes, here
+    also the 48-field fp32 inference chunk of BASELINE configs[4]; N = 1100: one block per field) and the backward (dW1, dW2
+    accumulated, dmean written), from partial sums and intermediates derived in float64"""
     from vit_grid_model_b200 import _lib
-    C, se = 2048, 512
+    se = C // 4
     HW = H * W
     parts = _lib.load().vg_field_parts(HW)
     h3 = rnd(N, H, W, C, seed=100) + 0.5 * rnd(C, seed=101)
