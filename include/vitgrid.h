@@ -284,6 +284,19 @@ VG_API int vg_stem_finish_train_fwd(int dtype, const float* raw3, const float* r
                              const float* tt, const float* tres, const float* ln_g, const float* ln_b, float ln_eps,
                              const float* film, int B, int L, int HP, int WP, void* h1, float* res, void* xhat, float* rstd,
                              void* relu_mask, void* stream);
+/* Training forward at C = 256 / 384 / 512 (also 128) in fp32 storage, the 'tf32_conv' precision: vg_conv3x3_ln_wide_fwd (no head)
+ * that also saves xhat (fp32 [q][C]), rstd (fp32 [q]) and relu_mask (C/32 words per pixel: bit c%32 of word c/32 set where the
+ * ReLU input > 0); pads of every output are zeros.  dtype 2: tf32 tensor cores, 1: exact-fp32 SIMT; bf16 is rejected.
+ * scratch: q*C floats (2*q*C for dtype 1). */
+VG_API int vg_conv3x3_ln_wide_train_fwd(int dtype, const void* x, int C, const void* Wt, const float* bias, const float* ln_g,
+                                 const float* ln_b, float ln_eps, const float* film, const void* res, int res_f32, float* out,
+                                 float* out_f32_copy, float* xhat, float* rstd, void* relu_mask, int N, int HP, int WP, float* scratch,
+                                 long long scratch_elems, void* stream);
+/* vg_stem_finish_wide_fwd with the same three saved tensors (fp32 storage: dtype 1 only) */
+VG_API int vg_stem_finish_wide_train_fwd(int dtype, const float* raw3, const float* rawres, const float* bias3, const float* bias1,
+                                  const float* tt, const float* tres, const float* ln_g, const float* ln_b, float ln_eps,
+                                  const float* film, int B, int L, int HP, int WP, int C, float* h1, float* res, float* xhat,
+                                  float* rstd, void* relu_mask, void* stream);
 
 /* Block backward (metnet3.py:110-126): dY fp32 PG -> dconv (odtype: 0 bf16, 1 fp32; zeros at pads) and per-field sums
  * sumA += dZ*xhat, sumB += dZ, sumD += dconv ((N,128) fp32, zeroed by the caller); border (or NULL): (N,8,128) sums of
@@ -295,6 +308,13 @@ VG_API int vg_conv_ln_bwd(int xdtype, int odtype, const float* dY, const void* x
 VG_API int vg_conv_ln_param_grads(const float* sumA, const float* sumB, const float* sumD, int N, const float* ln_g,
                            const float* ln_b, const float* film, float* dg, float* db, float* dbias, float* dfilm,
                            void* stream);
+/* The same two operators at C = 128 / 256 / 384 / 512 on the saved tensors of vg_conv3x3_ln_wide_train_fwd (fp32 xhat, C/32
+ * mask words per pixel): dconv fp32 (zeros at pads); sums (N,C); border (N,8,C) or NULL; dfilm (N,2C) written (or NULL). */
+VG_API int vg_conv_ln_bwd_wide(int C, const float* dY, const float* xhat, const float* rstd, const void* relu_mask, const float* ln_g,
+                        const float* film, float ln_eps, float* dconv, float* sumA, float* sumB, float* sumD, float* border, int N,
+                        int HP, int WP, void* stream);
+VG_API int vg_conv_ln_param_grads_wide(const float* sumA, const float* sumB, const float* sumD, int N, int C, const float* ln_g,
+                                const float* ln_b, const float* film, float* dg, float* db, float* dbias, float* dfilm, void* stream);
 
 /* Weight gradient of a shifted-row GEMM / 3x3 conv / linear layer:
  *   dW[n][tap*Ca + c] = beta*dW + sum_m dY[m][n] * A[m + tap_shift[tap]][c],   dW fp32 [Ntot][ntaps*Ca]
@@ -308,15 +328,20 @@ VG_API int vg_wgrad(int dtype, const void* dY, const void* A, long long rowsA, l
 /* metnet3.py:424-430 backward: dH fp32 PG (every position written), dw[C] and db[1] accumulated */
 VG_API int vg_head_bwd(int dtype, const float* dpred, const void* h, const float* w, float pm_std, int N, int HP, int WP, int H,
                 int W, int pad_top, int pad_left, float* dH, float* dw, float* db, void* stream);
+/* vg_head_bwd at C = 128 / 256 / 384 / 512 */
+VG_API int vg_head_bwd_wide(int dtype, const float* dpred, const void* h, const float* w, float pm_std, int N, int HP, int WP, int C,
+                     int H, int W, int pad_top, int pad_left, float* dH, float* dw, float* db, void* stream);
 /* MaxPool2d(2,2) backward: gradient to the first maximum of each window; dx fp32 PG, every position written */
 VG_API int vg_pool2_bwd(int dtype, const void* x, const float* dlow, float* dx, int N, int HP, int WP, int C, void* stream);
 /* ConvTranspose2d(k2,s2) backward gather: dUp fp32 PG (N,2Hl,2Wl,C) -> G [N*Hl*Wl][4C] (odtype 0 bf16 / 1 fp32),
- * dbias[C] accumulated; dgrad / wgrad are then plain GEMMs on G */
+ * dbias[C] accumulated; dgrad / wgrad are then plain GEMMs on G.  C = 128, 256, 384 or 512. */
 VG_API int vg_convT2_bwd_gather(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, void* stream);
 /* transpose of the lead-time replication (metnet3.py:383): out[b] = sum_l in[b*L+l], PG over B frames */
 VG_API int vg_lead_sum(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, void* stream);
-/* out[n][c] += sum over the frame pixels of an fp32 PG tensor (C = 128) */
+VG_API int vg_lead_sum_wide(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, int C, void* stream);
+/* out[n][c] += sum over the frame pixels of an fp32 PG tensor (C = 128; _wide: C = 128 / 256 / 384 / 512) */
 VG_API int vg_pg_field_sum(const float* in, float* out, int N, int HP, int WP, void* stream);
+VG_API int vg_pg_field_sum_wide(const float* in, float* out, int N, int HP, int WP, int C, void* stream);
 /* transpose of vg_time_terms_fwd: time-channel slices of the stem conv / res_conv weight gradients (accumulated into
  * the ORIGINAL-layout gradients dw3 (Cout,c_in,3,3), dw1 (Cout,c_in,1,1)), db1 (Cout) and dtemb (N, le+3te) written */
 VG_API int vg_time_terms_bwd(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,

@@ -249,6 +249,41 @@ int vg_stem_finish_wide_fwd(int dtype, const float* raw3, const float* rawres, c
   return stem_finish_wide_run(dtype, p, C, h1, res, (cudaStream_t)stream);
 }
 
+int vg_conv3x3_ln_wide_train_fwd(int dtype, const void* x, int C, const void* Wt, const float* bias, const float* ln_g,
+                                 const float* ln_b, float ln_eps, const float* film, const void* res, int res_f32, float* out,
+                                 float* out_f32_copy, float* xhat, float* rstd, void* relu_mask, int N, int HP, int WP, float* scratch,
+                                 long long scratch_elems, void* stream) {
+  PGeom pg = make_pgeom(N, HP, WP);
+  if (dtype != 1 && dtype != 2) return set_error("conv3x3_ln_wide_train: dtype %d (1 = fp32 SIMT, 2 = tf32 tensor cores)", dtype);
+  if (!out || !xhat || !rstd || !relu_mask) return set_error("conv3x3_ln_wide_train: out, xhat, rstd and relu_mask are required");
+  if (C % 128 || C < 128 || C > 512) return set_error("conv3x3_ln_wide_train: C=%d must be 128, 256, 384 or 512", C);
+  const long long need = pg.pixels() * (long long)C * (dtype == 1 ? 2 : 1);
+  if (scratch_elems < need) return set_error("conv3x3_ln_wide_train: scratch too small (%lld < %lld floats)", scratch_elems, need);
+  int shifts[9];
+  for (int ky = 0; ky < 3; ++ky)
+    for (int kx = 0; kx < 3; ++kx) shifts[ky * 3 + kx] = (ky - 1) * pg.P + (kx - 1);
+  EpiParams ep = epi_zero();
+  ep.out = scratch; ep.ldo = C; ep.out_f32 = 1; ep.n_total = C;
+  int rc = gemm_run(dtype, EPI_STORE, x, pg.pixels(), C, Wt, C, 9, shifts, pg.pixels(), 0, 0, ep, scratch + pg.pixels() * (long long)C,
+                    scratch_elems - pg.pixels() * (long long)C, (cudaStream_t)stream);
+  if (rc) return rc;
+  return conv_ln_rows_train_run(scratch, C, bias, ln_g, ln_b, ln_eps, film, res, res_f32, out, out_f32_copy, xhat, rstd,
+                                reinterpret_cast<unsigned*>(relu_mask), pg, (cudaStream_t)stream);
+}
+
+int vg_stem_finish_wide_train_fwd(int dtype, const float* raw3, const float* rawres, const float* bias3, const float* bias1,
+                                  const float* tt, const float* tres, const float* ln_g, const float* ln_b, float ln_eps,
+                                  const float* film, int B, int L, int HP, int WP, int C, float* h1, float* res, float* xhat,
+                                  float* rstd, void* relu_mask, void* stream) {
+  if (!xhat || !rstd || !relu_mask) return set_error("stem_finish_wide_train: xhat, rstd and relu_mask are required");
+  StemParams p;
+  p.raw3 = raw3; p.rawres = rawres; p.bias3 = bias3; p.bias1 = bias1; p.tt = tt; p.tres = tres;
+  p.ln_g = ln_g; p.ln_b = ln_b; p.eps = ln_eps; p.film = film; p.L = L;
+  p.xhat = xhat; p.rstd = rstd; p.mask = reinterpret_cast<unsigned*>(relu_mask);
+  p.pgB = make_pgeom(B, HP, WP); p.pgN = make_pgeom(B * L, HP, WP);
+  return stem_finish_wide_run(dtype, p, C, h1, res, (cudaStream_t)stream);
+}
+
 int vg_pool2_fwd(int dtype, int out_f32, const void* in, void* out, int N, int HP, int WP, int C, void* stream) {
   return maxpool2_run(dtype, out_f32, in, out, N, HP, WP, C, (cudaStream_t)stream);
 }
@@ -373,7 +408,19 @@ int vg_conv_ln_bwd(int xdtype, int odtype, const float* dY, const void* xhat, co
 int vg_conv_ln_param_grads(const float* sumA, const float* sumB, const float* sumD, int N, const float* ln_g,
                            const float* ln_b, const float* film, float* dg, float* db, float* dbias, float* dfilm,
                            void* stream) {
-  return conv_ln_param_grads_run(sumA, sumB, sumD, N, ln_g, ln_b, film, dg, db, dbias, dfilm, (cudaStream_t)stream);
+  return conv_ln_param_grads_run(sumA, sumB, sumD, N, ln_g, ln_b, film, dg, db, dbias, dfilm, 128, (cudaStream_t)stream);
+}
+
+int vg_conv_ln_bwd_wide(int C, const float* dY, const float* xhat, const float* rstd, const void* relu_mask, const float* ln_g,
+                        const float* film, float ln_eps, float* dconv, float* sumA, float* sumB, float* sumD, float* border, int N,
+                        int HP, int WP, void* stream) {
+  return conv_ln_bwd_wide_run(C, dY, xhat, rstd, reinterpret_cast<const unsigned*>(relu_mask), ln_g, film, ln_eps, dconv, sumA, sumB,
+                              sumD, border, N, HP, WP, (cudaStream_t)stream);
+}
+
+int vg_conv_ln_param_grads_wide(const float* sumA, const float* sumB, const float* sumD, int N, int C, const float* ln_g,
+                                const float* ln_b, const float* film, float* dg, float* db, float* dbias, float* dfilm, void* stream) {
+  return conv_ln_param_grads_run(sumA, sumB, sumD, N, ln_g, ln_b, film, dg, db, dbias, dfilm, C, (cudaStream_t)stream);
 }
 
 long long vg_wgrad_workspace(int dtype, long long M, int Ntot, int Ca, int ntaps) {
@@ -387,7 +434,12 @@ int vg_wgrad(int dtype, const void* dY, const void* A, long long rowsA, long lon
 
 int vg_head_bwd(int dtype, const float* dpred, const void* h, const float* w, float pm_std, int N, int HP, int WP, int H,
                 int W, int pad_top, int pad_left, float* dH, float* dw, float* db, void* stream) {
-  return head_bwd_run(dtype, dpred, h, w, pm_std, N, HP, WP, H, W, pad_top, pad_left, dH, dw, db, (cudaStream_t)stream);
+  return head_bwd_run(dtype, dpred, h, w, pm_std, N, HP, WP, H, W, pad_top, pad_left, dH, dw, db, 128, (cudaStream_t)stream);
+}
+
+int vg_head_bwd_wide(int dtype, const float* dpred, const void* h, const float* w, float pm_std, int N, int HP, int WP, int C, int H,
+                     int W, int pad_top, int pad_left, float* dH, float* dw, float* db, void* stream) {
+  return head_bwd_run(dtype, dpred, h, w, pm_std, N, HP, WP, H, W, pad_top, pad_left, dH, dw, db, C, (cudaStream_t)stream);
 }
 
 int vg_pool2_bwd(int dtype, const void* x, const float* dlow, float* dx, int N, int HP, int WP, int C, void* stream) {
@@ -399,11 +451,19 @@ int vg_convT2_bwd_gather(int odtype, const float* dUp, void* G, float* dbias, in
 }
 
 int vg_lead_sum(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, void* stream) {
-  return lead_sum_run(idtype, odtype, in, out, B, L, HP, WP, (cudaStream_t)stream);
+  return lead_sum_run(idtype, odtype, in, out, B, L, HP, WP, 128, (cudaStream_t)stream);
+}
+
+int vg_lead_sum_wide(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, int C, void* stream) {
+  return lead_sum_run(idtype, odtype, in, out, B, L, HP, WP, C, (cudaStream_t)stream);
 }
 
 int vg_pg_field_sum(const float* in, float* out, int N, int HP, int WP, void* stream) {
-  return pg_field_sum_run(in, out, N, HP, WP, (cudaStream_t)stream);
+  return pg_field_sum_run(in, out, N, HP, WP, 128, (cudaStream_t)stream);
+}
+
+int vg_pg_field_sum_wide(const float* in, float* out, int N, int HP, int WP, int C, void* stream) {
+  return pg_field_sum_run(in, out, N, HP, WP, C, (cudaStream_t)stream);
 }
 
 int vg_time_terms_bwd(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,

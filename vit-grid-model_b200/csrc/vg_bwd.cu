@@ -187,12 +187,141 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_kernel(const ConvLnBwdParams 
   }
 }
 
-// parameter gradients of one Block from the per-field sums (one thread per channel):
+// Block backward at C = 128 * NV (n_start_channels 256 / 384 / 512; tf32_conv training): the math of conv_ln_bwd_kernel on fp32
+// xhat / dconv.  One warp per pixel (lane owns channels v*128 + lane*4 .. +3, v < NV; ReLU mask word v*4 + lane/8 of the C/32
+// words of a pixel), 32 consecutive pixels per warp, 256 per block.  The per-field sums of the block's first field collect in
+// shared memory (most pixels of a block), the sums of any other field go to global atomics when the warp leaves the field.
+template <int NV>
+__global__ void __launch_bounds__(256) conv_ln_bwd_wide_kernel(const ConvLnBwdParams p) {
+  constexpr int C = 128 * NV, PPW = 32, MW = C / 32;
+  __shared__ float sacc[3][C];
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c0 = lane * 4;
+  const long long q_block = (long long)blockIdx.x * (8 * PPW);
+  for (int i = threadIdx.x; i < 3 * C; i += 256) (&sacc[0][0])[i] = 0.f;
+  int nf0, hh, ww;
+  p.pg.decode(q_block, nf0, hh, ww);
+  if (nf0 >= p.pg.N) nf0 = p.pg.N - 1;
+  __syncthreads();
+  const float* xh = reinterpret_cast<const float*>(p.xhat);
+  float* dc = reinterpret_cast<float*>(p.dconv);
+  float A[NV][4], B[NV][4], D[NV][4], gs[NV][4];
+#pragma unroll
+  for (int v = 0; v < NV; ++v)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) A[v][i] = B[v][i] = D[v][i] = gs[v][i] = 0.f;
+  int n_cur = -1;
+  auto flush = [&]() {
+    if (n_cur < 0) return;
+    const bool loc = n_cur == nf0;
+#pragma unroll
+    for (int v = 0; v < NV; ++v)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        const int c = v * 128 + c0 + i;
+        const long long g = (long long)n_cur * C + c;
+        atomicAdd(loc ? &sacc[0][c] : p.sumA + g, A[v][i]);
+        atomicAdd(loc ? &sacc[1][c] : p.sumB + g, B[v][i]);
+        atomicAdd(loc ? &sacc[2][c] : p.sumD + g, D[v][i]);
+        A[v][i] = B[v][i] = D[v][i] = 0.f;
+      }
+  };
+  const long long npix = p.pg.pixels();
+  long long q = q_block + warp * PPW;
+  const int Pp = p.pg.P, Rr = p.pg.R, Nn = p.pg.N, HPm = p.pg.HP - 1, WPm = p.pg.WP - 1;
+  int col, rr_, n;
+  {
+    const long long row = q / Pp;
+    col = (int)(q - row * Pp);
+    n = (int)(row / Rr);
+    rr_ = (int)(row - (long long)n * Rr);
+  }
+  for (int k = 0; k < PPW && q < npix; ++k) {
+    const bool valid = col >= 1 && rr_ >= 1 && n < Nn;          // warp-uniform: the whole warp works on pixel q
+    float o[NV][4];
+#pragma unroll
+    for (int v = 0; v < NV; ++v) o[v][0] = o[v][1] = o[v][2] = o[v][3] = 0.f;
+    if (valid) {
+      float dy[NV][4], x[NV][4];
+      unsigned bits[NV];
+#pragma unroll
+      for (int v = 0; v < NV; ++v) {
+        const float4 a = *reinterpret_cast<const float4*>(p.dY + q * C + v * 128 + c0);
+        const float4 b = *reinterpret_cast<const float4*>(xh + q * C + v * 128 + c0);
+        dy[v][0] = a.x; dy[v][1] = a.y; dy[v][2] = a.z; dy[v][3] = a.w;
+        x[v][0] = b.x; x[v][1] = b.y; x[v][2] = b.z; x[v][3] = b.w;
+        bits[v] = p.mask[q * MW + v * 4 + (lane >> 3)] >> ((lane & 7) * 4);
+      }
+      const float rstd = p.rstd[q];
+      if (n != n_cur) {
+        flush();
+        n_cur = n;
+#pragma unroll
+        for (int v = 0; v < NV; ++v)
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            const int c = v * 128 + c0 + i;
+            gs[v][i] = p.ln_g[c] * (p.film ? p.film[(long long)n * 2 * C + c] + 1.0f : 1.0f);
+          }
+      }
+      float dx[NV][4], s1 = 0.f, s2 = 0.f;
+#pragma unroll
+      for (int v = 0; v < NV; ++v)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          const float dz = (bits[v] & (1u << i)) ? dy[v][i] : 0.f;
+          dx[v][i] = dz * gs[v][i]; s1 += dx[v][i]; s2 = fmaf(dx[v][i], x[v][i], s2);
+          A[v][i] = fmaf(dz, x[v][i], A[v][i]); B[v][i] += dz;
+        }
+      s1 = warp_sum(s1) * (1.0f / C);
+      s2 = warp_sum(s2);
+      s2 = rstd >= p.rstd_clamp ? 0.f : s2 * (1.0f / C);          // var.clamp(min=eps): no gradient through a clamped variance
+#pragma unroll
+      for (int v = 0; v < NV; ++v)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) { o[v][i] = rstd * (dx[v][i] - s1 - x[v][i] * s2); D[v][i] += o[v][i]; }
+      if (p.border) {
+        const int h = rr_ - 1, w = col - 1;
+        const bool r0 = h == 0, rl = h == HPm, k0 = w == 0, kl = w == WPm;
+        if (r0 | rl | k0 | kl) {
+          float* bb = p.border + (long long)n * 8 * C + c0;
+#pragma unroll
+          for (int v = 0; v < NV; ++v)
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+              float* b1 = bb + v * 128 + i;
+              if (r0) atomicAdd(b1 + 0 * C, o[v][i]);
+              if (rl) atomicAdd(b1 + 1 * C, o[v][i]);
+              if (k0) atomicAdd(b1 + 2 * C, o[v][i]);
+              if (kl) atomicAdd(b1 + 3 * C, o[v][i]);
+              if (r0 && k0) atomicAdd(b1 + 4 * C, o[v][i]);
+              if (r0 && kl) atomicAdd(b1 + 5 * C, o[v][i]);
+              if (rl && k0) atomicAdd(b1 + 6 * C, o[v][i]);
+              if (rl && kl) atomicAdd(b1 + 7 * C, o[v][i]);
+            }
+        }
+      }
+    }
+#pragma unroll
+    for (int v = 0; v < NV; ++v)
+      *reinterpret_cast<float4*>(dc + q * C + v * 128 + c0) = make_float4(o[v][0], o[v][1], o[v][2], o[v][3]);
+    ++q;
+    if (++col == Pp) { col = 0; if (++rr_ == Rr) { rr_ = 0; ++n; } }
+  }
+  flush();
+  __syncthreads();
+  for (int c = threadIdx.x; c < C; c += 256) {
+    if (sacc[0][c] != 0.f) atomicAdd(p.sumA + (long long)nf0 * C + c, sacc[0][c]);
+    if (sacc[1][c] != 0.f) atomicAdd(p.sumB + (long long)nf0 * C + c, sacc[1][c]);
+    if (sacc[2][c] != 0.f) atomicAdd(p.sumD + (long long)nf0 * C + c, sacc[2][c]);
+  }
+}
+
+// parameter gradients of one Block from the per-field sums (one thread per channel; C / 32 blocks):
 //   dg += sum_n A (s+1);  db += sum_n B (s+1);  dbias += sum_n D;  dfilm[n] = (A g + B b | B)
+template <int C>
 __global__ void __launch_bounds__(256) conv_ln_param_grads_kernel(const float* __restrict__ sumA, const float* __restrict__ sumB, const float* __restrict__ sumD,
                                            int N, const float* __restrict__ g, const float* __restrict__ b, const float* __restrict__ film,
                                            float* __restrict__ dg, float* __restrict__ db, float* __restrict__ dbias, float* __restrict__ dfilm) {
-  constexpr int C = 128;
   __shared__ float red[3][8][32];
   const int l = threadIdx.x & 31, slice = threadIdx.x >> 5, c = blockIdx.x * 32 + l;     // 32 channels x 8 slices of the fields
   float ag = 0.f, ab = 0.f, ad = 0.f;
@@ -215,42 +344,56 @@ __global__ void __launch_bounds__(256) conv_ln_param_grads_kernel(const float* _
 // ================================================================================================
 // head backward (metnet3.py:424-430): pred = (sum_c h*w + b)*std + mean on the un-padded window
 //   dH[q][c] = dpred*std*w[c] inside the window, 0 elsewhere (incl. pads);  dw[c] += dpred*std*h;  db += dpred*std
+// C = 128 * NV: lane owns channels v*128 + lane*4 .. +3 (v < NV)
 // ================================================================================================
-template <typename T>
+template <int C, typename T>
 __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ dpred, const T* __restrict__ h, const float* __restrict__ w,
                                                        float stdv, PGeom pg, int H, int W, int pt, int pl, float* __restrict__ dH,
                                                        float* __restrict__ dw, float* __restrict__ db) {
-  constexpr int C = 128, PPW = 32;
+  constexpr int PPW = 32, NV = C / 128;
   __shared__ float sw_[C + 1];
   for (int i = threadIdx.x; i < C + 1; i += 256) sw_[i] = 0.f;
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c0 = lane * 4;
-  const float4 w4 = *reinterpret_cast<const float4*>(w + c0);
-  float aw[4] = {0.f, 0.f, 0.f, 0.f}, ab = 0.f;
+  float4 w4[NV];
+#pragma unroll
+  for (int v = 0; v < NV; ++v) w4[v] = *reinterpret_cast<const float4*>(w + v * 128 + c0);
+  float aw[NV][4] = {}, ab = 0.f;
   const long long q0 = ((long long)blockIdx.x * 8 + warp) * PPW;
+#pragma unroll 1
   for (int k = 0; k < PPW; ++k) {
     const long long q = q0 + k;
     if (q >= pg.pixels()) break;
     int n, y, x;
-    float4 o = make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 o[NV];
+#pragma unroll
+    for (int v = 0; v < NV; ++v) o[v] = make_float4(0.f, 0.f, 0.f, 0.f);
     if (pg.decode(q, n, y, x)) {
       const int hh = y - pt, ww = x - pl;
       if (hh >= 0 && hh < H && ww >= 0 && ww < W) {
         const float d = dpred[((long long)n * H + hh) * W + ww] * stdv;
-        o = make_float4(d * w4.x, d * w4.y, d * w4.z, d * w4.w);
 #pragma unroll
-        for (int i = 0; i < 4; ++i) aw[i] += d * Act<T>::ld(h + q * C + c0 + i);
+        for (int v = 0; v < NV; ++v) {
+          o[v] = make_float4(d * w4[v].x, d * w4[v].y, d * w4[v].z, d * w4[v].w);
+#pragma unroll
+          for (int i = 0; i < 4; ++i) aw[v][i] += d * Act<T>::ld(h + q * C + v * 128 + c0 + i);
+        }
         ab += d;
       }
     }
-    *reinterpret_cast<float4*>(dH + q * C + c0) = o;
+#pragma unroll
+    for (int v = 0; v < NV; ++v) *reinterpret_cast<float4*>(dH + q * C + v * 128 + c0) = o[v];
   }
 #pragma unroll
-  for (int i = 0; i < 4; ++i) atomicAdd(&sw_[c0 + i], aw[i]);
+  for (int v = 0; v < NV; ++v)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) atomicAdd(&sw_[v * 128 + c0 + i], aw[v][i]);
   if (lane == 0) atomicAdd(&sw_[C], ab);
   __syncthreads();
-  if (threadIdx.x < C) atomicAdd(dw + threadIdx.x, sw_[threadIdx.x]);
-  if (threadIdx.x == C) atomicAdd(db, sw_[C]);
+#pragma unroll
+  for (int k = 0; k < (C + 255) / 256; ++k)
+    if (k * 256 + threadIdx.x < C) atomicAdd(dw + k * 256 + threadIdx.x, sw_[k * 256 + threadIdx.x]);
+  if (threadIdx.x == C % 256) atomicAdd(db, sw_[C]);
 }
 
 // ================================================================================================
@@ -287,17 +430,21 @@ __global__ void __launch_bounds__(256) maxpool2_bwd_kernel(const T* __restrict__
 
 // ================================================================================================
 // ConvTranspose2d(k2,s2) backward gather (metnet3.py:88-89): dUp PG (N,2Hl,2Wl,C) fp32 -> G [N*Hl*Wl][4C] in the GEMM
-// dtype, column (di*2+dj)*C + co (the forward GEMM's column order), plus dbias[co] += sum.
+// dtype, column (di*2+dj)*C + co (the forward GEMM's column order), plus dbias[co] += sum.  C = 128 * NV.
 // ================================================================================================
-template <typename TO>
+template <int C, typename TO>
 __global__ void __launch_bounds__(256) convT_bwd_gather_kernel(const float* __restrict__ dUp, TO* __restrict__ G, float* __restrict__ dbias,
                                                                PGeom pg, int Hl, int Wl, long long M) {
-  constexpr int C = 128, PPW = 16;
+  constexpr int PPW = 16, NV = C / 128;
   __shared__ float sb[C];
-  if (threadIdx.x < C) sb[threadIdx.x] = 0.f;
+#pragma unroll
+  for (int k = 0; k < (C + 255) / 256; ++k)
+    if (k * 256 + threadIdx.x < C) sb[k * 256 + threadIdx.x] = 0.f;
   __syncthreads();
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c0 = lane * 4;
-  float acc[4] = {0.f, 0.f, 0.f, 0.f};
+  float acc[NV][4];
+#pragma unroll
+  for (int u = 0; u < NV; ++u) acc[u][0] = acc[u][1] = acc[u][2] = acc[u][3] = 0.f;
   const long long r0 = ((long long)blockIdx.x * 8 + warp) * PPW;
   for (int k = 0; k < PPW; ++k) {
     const long long r = r0 + k;
@@ -307,59 +454,84 @@ __global__ void __launch_bounds__(256) convT_bwd_gather_kernel(const float* __re
     const int i = pp / Wl, j = pp - i * Wl;
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
-      const float4 v = *reinterpret_cast<const float4*>(dUp + pg.q(n, 2 * i + (t >> 1), 2 * j + (t & 1)) * C + c0);
-      acc[0] += v.x; acc[1] += v.y; acc[2] += v.z; acc[3] += v.w;
-      TO* d = G + r * 4 * C + t * C + c0;
-      Act<TO>::st(d, v.x); Act<TO>::st(d + 1, v.y); Act<TO>::st(d + 2, v.z); Act<TO>::st(d + 3, v.w);
+#pragma unroll
+      for (int u = 0; u < NV; ++u) {
+        const float4 v = *reinterpret_cast<const float4*>(dUp + pg.q(n, 2 * i + (t >> 1), 2 * j + (t & 1)) * C + u * 128 + c0);
+        acc[u][0] += v.x; acc[u][1] += v.y; acc[u][2] += v.z; acc[u][3] += v.w;
+        TO* d = G + r * 4 * C + t * C + u * 128 + c0;
+        Act<TO>::st(d, v.x); Act<TO>::st(d + 1, v.y); Act<TO>::st(d + 2, v.z); Act<TO>::st(d + 3, v.w);
+      }
     }
   }
 #pragma unroll
-  for (int i = 0; i < 4; ++i) atomicAdd(&sb[c0 + i], acc[i]);
+  for (int u = 0; u < NV; ++u)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) atomicAdd(&sb[u * 128 + c0 + i], acc[u][i]);
   __syncthreads();
-  if (threadIdx.x < C) atomicAdd(dbias + threadIdx.x, sb[threadIdx.x]);
+#pragma unroll
+  for (int k = 0; k < (C + 255) / 256; ++k)
+    if (k * 256 + threadIdx.x < C) atomicAdd(dbias + k * 256 + threadIdx.x, sb[k * 256 + threadIdx.x]);
 }
 
 // ================================================================================================
 // stem: sum over the L lead times of a per-field tensor -> per-sample tensor (GEMM dtype), pads written as zeros:
 //   out[b][h][w][c] = sum_l in[b*L + l][h][w][c]        (the transpose of the lead-time replication, metnet3.py:383)
 // ================================================================================================
-template <typename TI, typename TO>
+template <int C, typename TI, typename TO>
 __global__ void __launch_bounds__(256) lead_sum_kernel(const TI* __restrict__ in, TO* __restrict__ out, PGeom pgN, PGeom pgB, int L) {
-  constexpr int C = 128;
+  constexpr int NV = C / 128;
   const long long qb = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (qb >= pgB.pixels()) return;
   const int lane = threadIdx.x & 31, c0 = lane * 4;
   int b, h, w;
-  float a[4] = {0.f, 0.f, 0.f, 0.f};
+  float a[NV][4];
+#pragma unroll
+  for (int v = 0; v < NV; ++v) a[v][0] = a[v][1] = a[v][2] = a[v][3] = 0.f;
   if (pgB.decode(qb, b, h, w)) {
     for (int l = 0; l < L; ++l) {
       const TI* s = in + pgN.q(b * L + l, h, w) * C + c0;
 #pragma unroll
-      for (int i = 0; i < 4; ++i) a[i] += Act<TI>::ld(s + i);
+      for (int v = 0; v < NV; ++v)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) a[v][i] += Act<TI>::ld(s + v * 128 + i);
     }
   }
 #pragma unroll
-  for (int i = 0; i < 4; ++i) Act<TO>::st(out + qb * C + c0 + i, a[i]);
+  for (int v = 0; v < NV; ++v)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) Act<TO>::st(out + qb * C + v * 128 + c0 + i, a[v][i]);
 }
 
-// per-field sums over the frame pixels of an fp32 PG tensor: out[n][c] = sum_{h,w} in[n][h][w][c].  grid (chunks, N)
+// per-field sums over the frame pixels of an fp32 PG tensor: out[n][c] = sum_{h,w} in[n][h][w][c].  grid (chunks, N); C = 128 * NV
+template <int C>
 __global__ void __launch_bounds__(256) pg_field_sum_kernel(const float* __restrict__ in, float* __restrict__ out, PGeom pg) {
-  constexpr int C = 128;
+  constexpr int NV = C / 128;
   __shared__ float sb[C];
-  if (threadIdx.x < C) sb[threadIdx.x] = 0.f;
+#pragma unroll
+  for (int k = 0; k < (C + 255) / 256; ++k)
+    if (k * 256 + threadIdx.x < C) sb[k * 256 + threadIdx.x] = 0.f;
   __syncthreads();
   const int n = blockIdx.y, warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c0 = lane * 4;
   const int npix = pg.HP * pg.WP;
-  float a[4] = {0.f, 0.f, 0.f, 0.f};
+  float a[NV][4];
+#pragma unroll
+  for (int u = 0; u < NV; ++u) a[u][0] = a[u][1] = a[u][2] = a[u][3] = 0.f;
   for (int i = blockIdx.x * 8 + warp; i < npix; i += gridDim.x * 8) {
     const int h = i / pg.WP, w = i - h * pg.WP;
-    const float4 v = *reinterpret_cast<const float4*>(in + pg.q(n, h, w) * C + c0);
-    a[0] += v.x; a[1] += v.y; a[2] += v.z; a[3] += v.w;
+#pragma unroll
+    for (int u = 0; u < NV; ++u) {
+      const float4 v = *reinterpret_cast<const float4*>(in + pg.q(n, h, w) * C + u * 128 + c0);
+      a[u][0] += v.x; a[u][1] += v.y; a[u][2] += v.z; a[u][3] += v.w;
+    }
   }
 #pragma unroll
-  for (int i = 0; i < 4; ++i) atomicAdd(&sb[c0 + i], a[i]);
+  for (int u = 0; u < NV; ++u)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) atomicAdd(&sb[u * 128 + c0 + i], a[u][i]);
   __syncthreads();
-  if (threadIdx.x < C) atomicAdd(out + (long long)n * C + threadIdx.x, sb[threadIdx.x]);
+#pragma unroll
+  for (int k = 0; k < (C + 255) / 256; ++k)
+    if (k * 256 + threadIdx.x < C) atomicAdd(out + (long long)n * C + k * 256 + threadIdx.x, sb[k * 256 + threadIdx.x]);
 }
 
 // ================================================================================================
@@ -601,18 +773,47 @@ int conv_ln_bwd_run(int xdtype, int odtype, const float* dY, const void* xhat, c
   return check_launch("conv_ln_bwd_kernel");
 }
 
+static int wide_c_check(const char* what, int C) {
+  if (C != 128 && C != 256 && C != 384 && C != 512) return set_error("%s: C=%d must be 128, 256, 384 or 512", what, C);
+  return 0;
+}
+
+// expands BODY with the compile-time width CW = C (128, 256, 384 or 512; checked by the caller)
+#define VG_WIDTH_SWITCH(C, BODY)                           \
+  switch (C) {                                             \
+    case 128: { constexpr int CW = 128; BODY; } break;     \
+    case 256: { constexpr int CW = 256; BODY; } break;     \
+    case 384: { constexpr int CW = 384; BODY; } break;     \
+    default:  { constexpr int CW = 512; BODY; } break;     \
+  }
+
+int conv_ln_bwd_wide_run(int C, const float* dY, const float* xhat, const float* rstd, const unsigned* mask, const float* ln_g,
+                         const float* film, float eps, float* dconv, float* sumA, float* sumB, float* sumD, float* border, int N,
+                         int HP, int WP, cudaStream_t st) {
+  if (wide_c_check("conv_ln_bwd_wide", C)) return 1;
+  ConvLnBwdParams p;
+  p.dY = dY; p.xhat = xhat; p.rstd = rstd; p.mask = mask; p.ln_g = ln_g; p.film = film; p.dconv = dconv;
+  p.sumA = sumA; p.sumB = sumB; p.sumD = sumD; p.border = border; p.rstd_clamp = 1.0f / sqrtf(eps) * (1.0f - 1e-6f);
+  p.pg = make_pgeom(N, HP, WP);
+  const unsigned g = nblk(p.pg.pixels(), 256);
+  VG_WIDTH_SWITCH(C, (conv_ln_bwd_wide_kernel<CW / 128><<<g, 256, 0, st>>>(p)));
+  return check_launch("conv_ln_bwd_wide_kernel");
+}
+
 int conv_ln_param_grads_run(const float* sumA, const float* sumB, const float* sumD, int N, const float* g, const float* b,
-                            const float* film, float* dg, float* db, float* dbias, float* dfilm, cudaStream_t st) {
-  conv_ln_param_grads_kernel<<<4, 256, 0, st>>>(sumA, sumB, sumD, N, g, b, film, dg, db, dbias, dfilm);
+                            const float* film, float* dg, float* db, float* dbias, float* dfilm, int C, cudaStream_t st) {
+  if (wide_c_check("conv_ln_param_grads", C)) return 1;
+  VG_WIDTH_SWITCH(C, (conv_ln_param_grads_kernel<CW><<<CW / 32, 256, 0, st>>>(sumA, sumB, sumD, N, g, b, film, dg, db, dbias, dfilm)));
   return check_launch("conv_ln_param_grads_kernel");
 }
 
 int head_bwd_run(int dtype, const float* dpred, const void* h, const float* w, float stdv, int N, int HP, int WP, int H, int W,
-                 int pt, int pl, float* dH, float* dw, float* db, cudaStream_t st) {
+                 int pt, int pl, float* dH, float* dw, float* db, int C, cudaStream_t st) {
+  if (wide_c_check("head_bwd", C)) return 1;
   PGeom pg = make_pgeom(N, HP, WP);
   const unsigned g = nblk(pg.pixels(), 256);
-  if (dtype == 0) head_bwd_kernel<bf16><<<g, 256, 0, st>>>(dpred, reinterpret_cast<const bf16*>(h), w, stdv, pg, H, W, pt, pl, dH, dw, db);
-  else head_bwd_kernel<float><<<g, 256, 0, st>>>(dpred, reinterpret_cast<const float*>(h), w, stdv, pg, H, W, pt, pl, dH, dw, db);
+  if (dtype == 0) VG_WIDTH_SWITCH(C, (head_bwd_kernel<CW, bf16><<<g, 256, 0, st>>>(dpred, reinterpret_cast<const bf16*>(h), w, stdv, pg, H, W, pt, pl, dH, dw, db)))
+  else VG_WIDTH_SWITCH(C, (head_bwd_kernel<CW, float><<<g, 256, 0, st>>>(dpred, reinterpret_cast<const float*>(h), w, stdv, pg, H, W, pt, pl, dH, dw, db)))
   return check_launch("head_bwd_kernel");
 }
 
@@ -626,30 +827,32 @@ int maxpool2_bwd_run(int dtype, const void* x, const float* dlow, float* dx, int
 }
 
 int convT_bwd_gather_run(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, cudaStream_t st) {
-  if (C != 128) return set_error("convT_bwd_gather: C must be 128");
+  if (wide_c_check("convT_bwd_gather", C)) return 1;
   PGeom pg = make_pgeom(N, 2 * Hl, 2 * Wl);
   const long long M = (long long)N * Hl * Wl;
   const unsigned g = nblk(M, 8 * 16);
-  if (odtype == 0) convT_bwd_gather_kernel<bf16><<<g, 256, 0, st>>>(dUp, reinterpret_cast<bf16*>(G), dbias, pg, Hl, Wl, M);
-  else convT_bwd_gather_kernel<float><<<g, 256, 0, st>>>(dUp, reinterpret_cast<float*>(G), dbias, pg, Hl, Wl, M);
+  if (odtype == 0) VG_WIDTH_SWITCH(C, (convT_bwd_gather_kernel<CW, bf16><<<g, 256, 0, st>>>(dUp, reinterpret_cast<bf16*>(G), dbias, pg, Hl, Wl, M)))
+  else VG_WIDTH_SWITCH(C, (convT_bwd_gather_kernel<CW, float><<<g, 256, 0, st>>>(dUp, reinterpret_cast<float*>(G), dbias, pg, Hl, Wl, M)))
   return check_launch("convT_bwd_gather_kernel");
 }
 
-int lead_sum_run(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, cudaStream_t st) {
+int lead_sum_run(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, int C, cudaStream_t st) {
+  if (wide_c_check("lead_sum", C)) return 1;
   PGeom pgN = make_pgeom(B * L, HP, WP), pgB = make_pgeom(B, HP, WP);
   const unsigned g = nblk(pgB.pixels(), 8);
-  if (idtype == 0 && odtype == 0) lead_sum_kernel<bf16, bf16><<<g, 256, 0, st>>>(reinterpret_cast<const bf16*>(in), reinterpret_cast<bf16*>(out), pgN, pgB, L);
-  else if (idtype == 1 && odtype == 0) lead_sum_kernel<float, bf16><<<g, 256, 0, st>>>(reinterpret_cast<const float*>(in), reinterpret_cast<bf16*>(out), pgN, pgB, L);
-  else if (idtype == 1 && odtype == 1) lead_sum_kernel<float, float><<<g, 256, 0, st>>>(reinterpret_cast<const float*>(in), reinterpret_cast<float*>(out), pgN, pgB, L);
+  if (idtype == 0 && odtype == 0) VG_WIDTH_SWITCH(C, (lead_sum_kernel<CW, bf16, bf16><<<g, 256, 0, st>>>(reinterpret_cast<const bf16*>(in), reinterpret_cast<bf16*>(out), pgN, pgB, L)))
+  else if (idtype == 1 && odtype == 0) VG_WIDTH_SWITCH(C, (lead_sum_kernel<CW, float, bf16><<<g, 256, 0, st>>>(reinterpret_cast<const float*>(in), reinterpret_cast<bf16*>(out), pgN, pgB, L)))
+  else if (idtype == 1 && odtype == 1) VG_WIDTH_SWITCH(C, (lead_sum_kernel<CW, float, float><<<g, 256, 0, st>>>(reinterpret_cast<const float*>(in), reinterpret_cast<float*>(out), pgN, pgB, L)))
   else return set_error("lead_sum: unsupported dtype combination (%d, %d)", idtype, odtype);
   return check_launch("lead_sum_kernel");
 }
 
-int pg_field_sum_run(const float* in, float* out, int N, int HP, int WP, cudaStream_t st) {
+int pg_field_sum_run(const float* in, float* out, int N, int HP, int WP, int C, cudaStream_t st) {
+  if (wide_c_check("pg_field_sum", C)) return 1;
   PGeom pg = make_pgeom(N, HP, WP);
   int chunks = (HP * WP + 255) / 256;
   if (chunks > 32) chunks = 32;
-  pg_field_sum_kernel<<<dim3(chunks, N), 256, 0, st>>>(in, out, pg);
+  VG_WIDTH_SWITCH(C, (pg_field_sum_kernel<CW><<<dim3(chunks, N), 256, 0, st>>>(in, out, pg)));
   return check_launch("pg_field_sum_kernel");
 }
 

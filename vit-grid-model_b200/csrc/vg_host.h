@@ -85,6 +85,10 @@ int conv_ln_rows_run(int dtype, const float* acc, int C, const float* bias, cons
                      const float* film, const void* res, int res_f32, void* out, float* out2, const PGeom& pg,
                      const float* head_w, float head_b, float head_std, float head_mean, int H, int W, int pad_top,
                      int pad_left, float* head_out, cudaStream_t st);
+// training instantiation of conv_ln_rows_kernel: also writes xhat (fp32 [q][C]), rstd ([q]) and the ReLU mask ([q][C/32])
+int conv_ln_rows_train_run(const float* acc, int C, const float* bias, const float* ln_g, const float* ln_b, float eps,
+                           const float* film, const void* res, int res_f32, float* out, float* out2, float* xhat, float* rstd,
+                           unsigned* mask, const PGeom& pg, cudaStream_t st);
 int maxpool2_run(int dtype, int out_f32, const void* in, void* out, int N, int HP, int WP, int C, cudaStream_t st);
 int dwconv_run(int dtype, const void* in, const float* w9, const float* scale, const float* shift, void* out, float* psum,
                int N, int H, int W, int C, cudaStream_t st);
@@ -122,14 +126,17 @@ int wgrad_run(int dtype, const void* dY, const void* A, long long rowsA, long lo
 int conv_ln_bwd_run(int xdtype, int odtype, const float* dY, const void* xhat, const float* rstd, const unsigned* mask,
                     const float* ln_g, const float* film, float eps, void* dconv, float* sumA, float* sumB, float* sumD,
                     float* border, int N, int HP, int WP, cudaStream_t st);
+int conv_ln_bwd_wide_run(int C, const float* dY, const float* xhat, const float* rstd, const unsigned* mask, const float* ln_g,
+                         const float* film, float eps, float* dconv, float* sumA, float* sumB, float* sumD, float* border, int N,
+                         int HP, int WP, cudaStream_t st);
 int conv_ln_param_grads_run(const float* sumA, const float* sumB, const float* sumD, int N, const float* g, const float* b,
-                            const float* film, float* dg, float* db, float* dbias, float* dfilm, cudaStream_t st);
+                            const float* film, float* dg, float* db, float* dbias, float* dfilm, int C, cudaStream_t st);
 int head_bwd_run(int dtype, const float* dpred, const void* h, const float* w, float stdv, int N, int HP, int WP, int H, int W,
-                 int pt, int pl, float* dH, float* dw, float* db, cudaStream_t st);
+                 int pt, int pl, float* dH, float* dw, float* db, int C, cudaStream_t st);
 int maxpool2_bwd_run(int dtype, const void* x, const float* dlow, float* dx, int N, int HP, int WP, int C, cudaStream_t st);
 int convT_bwd_gather_run(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, cudaStream_t st);
-int lead_sum_run(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, cudaStream_t st);
-int pg_field_sum_run(const float* in, float* out, int N, int HP, int WP, cudaStream_t st);
+int lead_sum_run(int idtype, int odtype, const void* in, void* out, int B, int L, int HP, int WP, int C, cudaStream_t st);
+int pg_field_sum_run(const float* in, float* out, int N, int HP, int WP, int C, cudaStream_t st);
 int time_terms_bwd_run(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,
                        const float* w1, int N, int ntc, int c_in, int c_data, int Cout, float* dw3, float* dw1, float* db1,
                        float* dtemb, cudaStream_t st);

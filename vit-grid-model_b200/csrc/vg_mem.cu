@@ -667,19 +667,32 @@ struct WideRowParams {
   const float* head_w; float* head_out; float head_b, head_std, head_mean; int head_H, head_W, head_pt, head_pl;
   int C;
   PGeom pg;
+  // training (TRAIN instantiation): xhat fp32 [q][C], rstd [q], ReLU mask [q][C/32] (bit c%32 of word c/32: input > 0); pads zeros
+  float* xhat; float* rstd; unsigned* mask;
 };
 
-template <typename T>
+// the C / 32 mask words of pixel q from the per-lane nibbles (lane owns channels v*128 + lane*4 .. +3): word v*4 + lane/8
+__device__ __forceinline__ void store_relu_mask(unsigned* mask, long long q, int C, int v, int lane, unsigned nib) {
+  unsigned wbits = nib << ((lane & 7) * 4);
+  wbits |= __shfl_xor_sync(0xffffffffu, wbits, 1);
+  wbits |= __shfl_xor_sync(0xffffffffu, wbits, 2);
+  wbits |= __shfl_xor_sync(0xffffffffu, wbits, 4);
+  if ((lane & 7) == 0) mask[q * (C >> 5) + v * 4 + (lane >> 3)] = wbits;
+}
+
+template <typename T, bool TRAIN>
 __global__ void __launch_bounds__(256) conv_ln_rows_kernel(const WideRowParams p) {
   const long long q = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (q >= p.pg.pixels()) return;
   const int lane = threadIdx.x & 31, C = p.C, nv = C >> 7;
   int n = 0, h = 0, w = 0;
   const bool valid = p.pg.decode(q, n, h, w);
-  float4 y[4];
+  float4 y[4], xs[4];
+  unsigned nib[4] = {0u, 0u, 0u, 0u};
+  float rstd = 0.f;
   float head = 0.f;
 #pragma unroll
-  for (int i = 0; i < 4; ++i) y[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int i = 0; i < 4; ++i) y[i] = xs[i] = make_float4(0.f, 0.f, 0.f, 0.f);
   if (valid) {
     float s = 0.f;
 #pragma unroll
@@ -698,19 +711,21 @@ __global__ void __launch_bounds__(256) conv_ln_rows_kernel(const WideRowParams p
         y[i].x -= mean; y[i].y -= mean; y[i].z -= mean; y[i].w -= mean;
         ss += y[i].x * y[i].x + y[i].y * y[i].y + y[i].z * y[i].z + y[i].w * y[i].w;
       }
-    const float rstd = rsqrtf(fmaxf(warp_sum(ss) / (float)C, p.eps));       // var.clamp(min=eps).rsqrt()  (metnet3.py:104)
+    rstd = rsqrtf(fmaxf(warp_sum(ss) / (float)C, p.eps));                   // var.clamp(min=eps).rsqrt()  (metnet3.py:104)
 #pragma unroll
     for (int i = 0; i < 4; ++i)
       if (i < nv) {
         const int c = i * 128 + lane * 4;
         const float4 g = *reinterpret_cast<const float4*>(p.ln_g + c), b = *reinterpret_cast<const float4*>(p.ln_b + c);
         float z[4] = {y[i].x * rstd * g.x + b.x, y[i].y * rstd * g.y + b.y, y[i].z * rstd * g.z + b.z, y[i].w * rstd * g.w + b.w};
+        if (TRAIN) xs[i] = make_float4(y[i].x * rstd, y[i].y * rstd, y[i].z * rstd, y[i].w * rstd);
         if (p.film) {
           const float4 sc = *reinterpret_cast<const float4*>(p.film + (long long)n * 2 * C + c);
           const float4 sh = *reinterpret_cast<const float4*>(p.film + (long long)n * 2 * C + C + c);
           z[0] = z[0] * (sc.x + 1.0f) + sh.x; z[1] = z[1] * (sc.y + 1.0f) + sh.y;
           z[2] = z[2] * (sc.z + 1.0f) + sh.z; z[3] = z[3] * (sc.w + 1.0f) + sh.w;
         }
+        if (TRAIN) nib[i] = (z[0] > 0.f ? 1u : 0u) | (z[1] > 0.f ? 2u : 0u) | (z[2] > 0.f ? 4u : 0u) | (z[3] > 0.f ? 8u : 0u);
 #pragma unroll
         for (int k = 0; k < 4; ++k) z[k] = fmaxf(z[k], 0.f);
         if (p.res) {
@@ -731,7 +746,12 @@ __global__ void __launch_bounds__(256) conv_ln_rows_kernel(const WideRowParams p
       const int c = i * 128 + lane * 4;
       if (p.out) Ld4<T>::st(reinterpret_cast<T*>(p.out) + q * C + c, y[i]);
       if (p.out2) *reinterpret_cast<float4*>(p.out2 + q * C + c) = y[i];
+      if (TRAIN) {
+        *reinterpret_cast<float4*>(p.xhat + q * C + c) = xs[i];
+        store_relu_mask(p.mask, q, C, i, lane, nib[i]);
+      }
     }
+  if (TRAIN && lane == 0) p.rstd[q] = rstd;
   if (p.head_w && valid) {
     head = warp_sum(head);
     const int hh = h - p.head_pt, ww = w - p.head_pl;
@@ -740,17 +760,19 @@ __global__ void __launch_bounds__(256) conv_ln_rows_kernel(const WideRowParams p
   }
 }
 
-// stem_finish_kernel for C = 128 * nv (inference only)
-template <typename T>
+// stem_finish_kernel for C = 128 * nv; TRAIN also writes xhat (T [q][C]), rstd and the ReLU mask ([q][C/32]) of conv_ln_rows_kernel
+template <typename T, bool TRAIN>
 __global__ void __launch_bounds__(256) stem_finish_wide_kernel(const StemParams p, int C, T* __restrict__ h1, float* __restrict__ res) {
   const long long q = (long long)blockIdx.x * 8 + (threadIdx.x >> 5);
   if (q >= p.pgN.pixels()) return;
   const int lane = threadIdx.x & 31, nv = C >> 7;
   int n = 0, h = 0, w = 0;
   const bool valid = p.pgN.decode(q, n, h, w);
-  float4 y[4], r[4];
+  float4 y[4], r[4], xs[4];
+  unsigned nib[4] = {0u, 0u, 0u, 0u};
+  float rstd = 0.f;
 #pragma unroll
-  for (int i = 0; i < 4; ++i) y[i] = r[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int i = 0; i < 4; ++i) y[i] = r[i] = xs[i] = make_float4(0.f, 0.f, 0.f, 0.f);
   if (valid) {
     const int b = n / p.L;
     const long long qb = p.pgB.q(b, h, w);
@@ -776,7 +798,7 @@ __global__ void __launch_bounds__(256) stem_finish_wide_kernel(const StemParams 
         y[i].x -= mean; y[i].y -= mean; y[i].z -= mean; y[i].w -= mean;
         ss += y[i].x * y[i].x + y[i].y * y[i].y + y[i].z * y[i].z + y[i].w * y[i].w;
       }
-    const float rstd = rsqrtf(fmaxf(warp_sum(ss) / (float)C, p.eps));
+    rstd = rsqrtf(fmaxf(warp_sum(ss) / (float)C, p.eps));
 #pragma unroll
     for (int i = 0; i < 4; ++i)
       if (i < nv) {
@@ -784,6 +806,12 @@ __global__ void __launch_bounds__(256) stem_finish_wide_kernel(const StemParams 
         const float4 g = *reinterpret_cast<const float4*>(p.ln_g + c), be = *reinterpret_cast<const float4*>(p.ln_b + c);
         const float4 sc = *reinterpret_cast<const float4*>(p.film + (long long)n * 2 * C + c);
         const float4 sh = *reinterpret_cast<const float4*>(p.film + (long long)n * 2 * C + C + c);
+        if (TRAIN) {
+          xs[i] = make_float4(y[i].x * rstd, y[i].y * rstd, y[i].z * rstd, y[i].w * rstd);
+          const float z[4] = {(y[i].x * rstd * g.x + be.x) * (sc.x + 1.0f) + sh.x, (y[i].y * rstd * g.y + be.y) * (sc.y + 1.0f) + sh.y,
+                              (y[i].z * rstd * g.z + be.z) * (sc.z + 1.0f) + sh.z, (y[i].w * rstd * g.w + be.w) * (sc.w + 1.0f) + sh.w};
+          nib[i] = (z[0] > 0.f ? 1u : 0u) | (z[1] > 0.f ? 2u : 0u) | (z[2] > 0.f ? 4u : 0u) | (z[3] > 0.f ? 8u : 0u);
+        }
         y[i].x = fmaxf((y[i].x * rstd * g.x + be.x) * (sc.x + 1.0f) + sh.x, 0.f);
         y[i].y = fmaxf((y[i].y * rstd * g.y + be.y) * (sc.y + 1.0f) + sh.y, 0.f);
         y[i].z = fmaxf((y[i].z * rstd * g.z + be.z) * (sc.z + 1.0f) + sh.z, 0.f);
@@ -796,7 +824,12 @@ __global__ void __launch_bounds__(256) stem_finish_wide_kernel(const StemParams 
       const int c = i * 128 + lane * 4;
       Ld4<T>::st(h1 + q * C + c, y[i]);
       *reinterpret_cast<float4*>(res + q * C + c) = r[i];
+      if (TRAIN) {
+        Ld4<T>::st(reinterpret_cast<T*>(p.xhat) + q * C + c, xs[i]);
+        store_relu_mask(p.mask, q, C, i, lane, nib[i]);
+      }
     }
+  if (TRAIN && lane == 0) p.rstd[q] = rstd;
 }
 
 // ================================================================================================
@@ -944,8 +977,11 @@ int stem_finish_run(int dtype, const StemParams& p, void* h1, float* res, cudaSt
 int stem_finish_wide_run(int dtype, const StemParams& p, int C, void* h1, float* res, cudaStream_t st) {
   if (C % 128 || C < 128 || C > 512) return set_error("stem_finish_wide: C=%d must be 128, 256, 384 or 512", C);
   const unsigned g = nblk(p.pgN.pixels(), 8);
-  if (dtype == 0) stem_finish_wide_kernel<bf16><<<g, 256, 0, st>>>(p, C, reinterpret_cast<bf16*>(h1), res);
-  else stem_finish_wide_kernel<float><<<g, 256, 0, st>>>(p, C, reinterpret_cast<float*>(h1), res);
+  if (p.xhat) {                                              // training: fp32 storage only (the tf32_conv precision)
+    if (dtype != 1) return set_error("stem_finish_wide_train: dtype %d (the training instantiation is fp32 only)", dtype);
+    stem_finish_wide_kernel<float, true><<<g, 256, 0, st>>>(p, C, reinterpret_cast<float*>(h1), res);
+  } else if (dtype == 0) stem_finish_wide_kernel<bf16, false><<<g, 256, 0, st>>>(p, C, reinterpret_cast<bf16*>(h1), res);
+  else stem_finish_wide_kernel<float, false><<<g, 256, 0, st>>>(p, C, reinterpret_cast<float*>(h1), res);
   return check_launch("stem_finish_wide_kernel");
 }
 
@@ -958,10 +994,24 @@ int conv_ln_rows_run(int dtype, const float* acc, int C, const float* bias, cons
   p.acc = acc; p.bias = bias; p.ln_g = ln_g; p.ln_b = ln_b; p.eps = eps; p.film = film; p.res = res; p.res_f32 = res_f32;
   p.out = out; p.out2 = out2; p.head_w = head_w; p.head_out = head_out; p.head_b = head_b; p.head_std = head_std;
   p.head_mean = head_mean; p.head_H = H; p.head_W = W; p.head_pt = pad_top; p.head_pl = pad_left; p.C = C; p.pg = pg;
+  p.xhat = nullptr; p.rstd = nullptr; p.mask = nullptr;
   const unsigned g = nblk(pg.pixels(), 8);
-  if (dtype == 0) conv_ln_rows_kernel<bf16><<<g, 256, 0, st>>>(p);
-  else conv_ln_rows_kernel<float><<<g, 256, 0, st>>>(p);
+  if (dtype == 0) conv_ln_rows_kernel<bf16, false><<<g, 256, 0, st>>>(p);
+  else conv_ln_rows_kernel<float, false><<<g, 256, 0, st>>>(p);
   return check_launch("conv_ln_rows_kernel");
+}
+
+int conv_ln_rows_train_run(const float* acc, int C, const float* bias, const float* ln_g, const float* ln_b, float eps,
+                           const float* film, const void* res, int res_f32, float* out, float* out2, float* xhat, float* rstd,
+                           unsigned* mask, const PGeom& pg, cudaStream_t st) {
+  if (C % 128 || C < 128 || C > 512) return set_error("conv_ln_rows_train: C=%d must be 128, 256, 384 or 512", C);
+  WideRowParams p;
+  p.acc = acc; p.bias = bias; p.ln_g = ln_g; p.ln_b = ln_b; p.eps = eps; p.film = film; p.res = res; p.res_f32 = res_f32;
+  p.out = out; p.out2 = out2; p.head_w = nullptr; p.head_out = nullptr; p.head_b = 0.f; p.head_std = 1.f; p.head_mean = 0.f;
+  p.head_H = p.head_W = p.head_pt = p.head_pl = 0; p.C = C; p.pg = pg;
+  p.xhat = xhat; p.rstd = rstd; p.mask = mask;
+  conv_ln_rows_kernel<float, true><<<nblk(pg.pixels(), 8), 256, 0, st>>>(p);
+  return check_launch("conv_ln_rows_train_kernel");
 }
 
 int maxpool2_run(int dtype, int out_f32, const void* in, void* out, int N, int HP, int WP, int C, cudaStream_t st) {

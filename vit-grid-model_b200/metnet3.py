@@ -348,11 +348,13 @@ class MetNet3(nn.Module):
         no dropout, so that x.grad and the parameter gradients are those of the reference module in eval() mode"""
         from .train import MetNet3TrainFn
         what = "input gradients in eval() mode" if frozen else "training"
-        if self.n_start_channels != 128:
-            raise NotImplementedError(f"the training kernels are built for n_start_channels=128; wider networks run inference only "
-                                      f"({what} is not built)")
-        if self.precision not in ("bf16", "fp32"):
-            raise NotImplementedError(f"{what} supports set_precision('bf16') (mixed) and 'fp32'")
+        C = self.n_start_channels
+        # 128 channels: the fused conv epilogues in every precision but bf16_all / tf32; wider networks: the shifted-row GEMM +
+        # row kernels in fp32 storage with tf32 convolutions and the exact-fp32 MaxViT training kernels
+        built = ("bf16", "fp32", "tf32_conv") if C == 128 else ("tf32_conv",)
+        if self.precision not in built:
+            raise NotImplementedError(f"{what} at n_start_channels={C} supports set_precision("
+                                      f"{' | '.join(repr(p) for p in built)}), not {self.precision!r}")
         return MetNet3TrainFn.apply(self, x, ts, frozen, *self.parameters())
 
     def next_dropout_seed(self) -> int:

@@ -14,17 +14,27 @@ def _f32(n, dev):
     return torch.empty(int(n), dtype=torch.float32, device=dev)
 
 
-def conv3x3_ln_train(x, Wt, bias, ln_g, ln_b, eps, film, res, out, N, HP, WP, out_copy=None):
-    """forward Block that also returns the saved tensors (xhat, rstd, relu_mask) for backward"""
+def conv3x3_ln_train(x, Wt, bias, ln_g, ln_b, eps, film, res, out, N, HP, WP, out_copy=None, tf32=False):
+    """forward Block that also returns the saved tensors (xhat, rstd, relu_mask) for backward.  tf32 (fp32 storage): the
+    convolution runs on tcgen05 kind::tf32.  C = out.shape[1]; widths other than 128 take the shifted-row GEMM + row kernel
+    (fp32 storage only; xhat fp32, C/32 mask words per pixel)."""
     dtype = x.dtype
     dev = x.device
-    Q = x.shape[0]
-    xhat = torch.empty(Q, 128, dtype=dtype, device=dev)
-    rstd = _f32(Q, dev)
-    mask = torch.empty(Q, 4, dtype=torch.int32, device=dev)
-    scratch = _f32(Q * 128, dev) if dtype == torch.float32 else None
+    Q, C = x.shape[0], out.shape[1]
+    code = 2 if (tf32 and dtype == torch.float32) else DT_CODE[dtype]
     res_f32 = int(res is not None and res.dtype == torch.float32 and dtype != torch.float32)
-    _lib.call("vg_conv3x3_ln_train_fwd", DT_CODE[dtype], x.data_ptr(), x.shape[1], Wt.data_ptr(), bias.data_ptr(),
+    rstd = _f32(Q, dev)
+    mask = torch.empty(Q, C // 32, dtype=torch.int32, device=dev)
+    if C != 128:
+        xhat = torch.empty(Q, C, dtype=torch.float32, device=dev)
+        scratch = _f32(Q * C * (1 if code == 2 else 2), dev)
+        _lib.call("vg_conv3x3_ln_wide_train_fwd", code, x.data_ptr(), C, Wt.data_ptr(), bias.data_ptr(), ln_g.data_ptr(),
+                  ln_b.data_ptr(), float(eps), _p(film), _p(res), res_f32, out.data_ptr(), _p(out_copy), xhat.data_ptr(),
+                  rstd.data_ptr(), mask.data_ptr(), N, HP, WP, scratch.data_ptr(), scratch.numel(), _st())
+        return out, (xhat, rstd, mask)
+    xhat = torch.empty(Q, 128, dtype=dtype, device=dev)
+    scratch = _f32(Q * 128, dev) if code == 1 else None
+    _lib.call("vg_conv3x3_ln_train_fwd", code, x.data_ptr(), x.shape[1], Wt.data_ptr(), bias.data_ptr(),
               ln_g.data_ptr(), ln_b.data_ptr(), float(eps), _p(film), _p(res), res_f32, out.data_ptr(), _p(out_copy),
               xhat.data_ptr(), rstd.data_ptr(), mask.data_ptr(), N, HP, WP, _p(scratch),
               scratch.numel() if scratch is not None else 0, _st())
@@ -32,11 +42,17 @@ def conv3x3_ln_train(x, Wt, bias, ln_g, ln_b, eps, film, res, out, N, HP, WP, ou
 
 
 def stem_finish_train(raw3, rawres, bias3, bias1, tt, tres, ln_g, ln_b, eps, film, B, L, HP, WP, h1, res):
-    Q = h1.shape[0]
+    Q, C = h1.shape
     dev = h1.device
-    xhat = torch.empty(Q, 128, dtype=h1.dtype, device=dev)
+    xhat = torch.empty(Q, C, dtype=h1.dtype, device=dev)
     rstd = _f32(Q, dev)
-    mask = torch.empty(Q, 4, dtype=torch.int32, device=dev)
+    mask = torch.empty(Q, C // 32, dtype=torch.int32, device=dev)
+    if C != 128:
+        _lib.call("vg_stem_finish_wide_train_fwd", DT_CODE[h1.dtype], raw3.data_ptr(), rawres.data_ptr(), bias3.data_ptr(),
+                  bias1.data_ptr(), tt.data_ptr(), tres.data_ptr(), ln_g.data_ptr(), ln_b.data_ptr(), float(eps),
+                  film.data_ptr(), B, L, HP, WP, C, h1.data_ptr(), res.data_ptr(), xhat.data_ptr(), rstd.data_ptr(),
+                  mask.data_ptr(), _st())
+        return xhat, rstd, mask
     _lib.call("vg_stem_finish_train_fwd", DT_CODE[h1.dtype], raw3.data_ptr(), rawres.data_ptr(), bias3.data_ptr(),
               bias1.data_ptr(), tt.data_ptr(), tres.data_ptr(), ln_g.data_ptr(), ln_b.data_ptr(), float(eps),
               film.data_ptr(), B, L, HP, WP, h1.data_ptr(), res.data_ptr(), xhat.data_ptr(), rstd.data_ptr(),
@@ -45,12 +61,19 @@ def stem_finish_train(raw3, rawres, bias3, bias1, tt, tres, ln_g, ln_b, eps, fil
 
 
 def conv_ln_bwd(dY, saved, ln_g, film, eps, N, HP, WP, out_dtype, want_border=False):
-    """-> dconv (out_dtype, PG, zeros at pads), (sumA, sumB, sumD) (N,128) each, border (N,8,128) or None"""
+    """-> dconv (out_dtype, PG, zeros at pads), (sumA, sumB, sumD) (N,C) each, border (N,8,C) or None"""
     xhat, rstd, mask = saved
     dev = dY.device
-    dconv = torch.empty(dY.shape[0], 128, dtype=out_dtype, device=dev)
-    sums = torch.zeros(3, N, 128, dtype=torch.float32, device=dev)
-    border = torch.zeros(N, 8, 128, dtype=torch.float32, device=dev) if want_border else None
+    C = dY.shape[1]
+    dconv = torch.empty(dY.shape[0], C, dtype=out_dtype, device=dev)
+    sums = torch.zeros(3, N, C, dtype=torch.float32, device=dev)
+    border = torch.zeros(N, 8, C, dtype=torch.float32, device=dev) if want_border else None
+    if C != 128:
+        assert xhat.dtype == torch.float32 and out_dtype == torch.float32, "wide Block backward is fp32 (tf32_conv)"
+        _lib.call("vg_conv_ln_bwd_wide", C, dY.data_ptr(), xhat.data_ptr(), rstd.data_ptr(), mask.data_ptr(), ln_g.data_ptr(),
+                  _p(film), float(eps), dconv.data_ptr(), sums[0].data_ptr(), sums[1].data_ptr(), sums[2].data_ptr(), _p(border),
+                  N, HP, WP, _st())
+        return dconv, sums, border
     _lib.call("vg_conv_ln_bwd", DT_CODE[xhat.dtype], DT_CODE[out_dtype], dY.data_ptr(), xhat.data_ptr(), rstd.data_ptr(),
               mask.data_ptr(), ln_g.data_ptr(), _p(film), float(eps), dconv.data_ptr(), sums[0].data_ptr(),
               sums[1].data_ptr(), sums[2].data_ptr(), _p(border), N, HP, WP, _st())
@@ -58,7 +81,12 @@ def conv_ln_bwd(dY, saved, ln_g, film, eps, N, HP, WP, out_dtype, want_border=Fa
 
 
 def conv_ln_param_grads(sums, N, ln_g, ln_b, film, dg, db, dbias, want_dfilm):
-    dfilm = torch.empty(N, 256, dtype=torch.float32, device=sums.device) if want_dfilm else None
+    C = sums.shape[2]
+    dfilm = torch.empty(N, 2 * C, dtype=torch.float32, device=sums.device) if want_dfilm else None
+    if C != 128:
+        _lib.call("vg_conv_ln_param_grads_wide", sums[0].data_ptr(), sums[1].data_ptr(), sums[2].data_ptr(), N, C, ln_g.data_ptr(),
+                  ln_b.data_ptr(), _p(film), dg.data_ptr(), db.data_ptr(), dbias.data_ptr(), _p(dfilm), _st())
+        return dfilm
     _lib.call("vg_conv_ln_param_grads", sums[0].data_ptr(), sums[1].data_ptr(), sums[2].data_ptr(), N, ln_g.data_ptr(),
               ln_b.data_ptr(), _p(film), dg.data_ptr(), db.data_ptr(), dbias.data_ptr(), _p(dfilm), _st())
     return dfilm
@@ -81,8 +109,13 @@ def wgrad(dY, A, dW, *, ntaps=1, tap_shift=(0,), M=None, beta=1.0, tf32=False):
 
 
 def head_bwd(dpred, h, w, std, N, HP, WP, H, W, pads, dw, db):
-    dH = torch.empty(pg_pixels(N, HP, WP), 128, dtype=torch.float32, device=h.device)
+    C = h.shape[1]
+    dH = torch.empty(pg_pixels(N, HP, WP), C, dtype=torch.float32, device=h.device)
     pl, _, pt, _ = pads
+    if C != 128:
+        _lib.call("vg_head_bwd_wide", DT_CODE[h.dtype], dpred.data_ptr(), h.data_ptr(), w.data_ptr(), float(std), N, HP, WP, C, H,
+                  W, pt, pl, dH.data_ptr(), dw.data_ptr(), db.data_ptr(), _st())
+        return dH
     _lib.call("vg_head_bwd", DT_CODE[h.dtype], dpred.data_ptr(), h.data_ptr(), w.data_ptr(), float(std), N, HP, WP, H, W,
               pt, pl, dH.data_ptr(), dw.data_ptr(), db.data_ptr(), _st())
     return dH
@@ -102,13 +135,21 @@ def convT2_bwd_gather(dUp, N, Hl, Wl, C, out_dtype, dbias):
 
 
 def lead_sum(x, B, L, HP, WP, out_dtype):
-    out = torch.empty(pg_pixels(B, HP, WP), 128, dtype=out_dtype, device=x.device)
+    C = x.shape[1]
+    out = torch.empty(pg_pixels(B, HP, WP), C, dtype=out_dtype, device=x.device)
+    if C != 128:
+        _lib.call("vg_lead_sum_wide", DT_CODE[x.dtype], DT_CODE[out_dtype], x.data_ptr(), out.data_ptr(), B, L, HP, WP, C, _st())
+        return out
     _lib.call("vg_lead_sum", DT_CODE[x.dtype], DT_CODE[out_dtype], x.data_ptr(), out.data_ptr(), B, L, HP, WP, _st())
     return out
 
 
 def pg_field_sum(x, N, HP, WP):
-    out = torch.zeros(N, 128, dtype=torch.float32, device=x.device)
+    C = x.shape[1]
+    out = torch.zeros(N, C, dtype=torch.float32, device=x.device)
+    if C != 128:
+        _lib.call("vg_pg_field_sum_wide", x.data_ptr(), out.data_ptr(), N, HP, WP, C, _st())
+        return out
     _lib.call("vg_pg_field_sum", x.data_ptr(), out.data_ptr(), N, HP, WP, _st())
     return out
 

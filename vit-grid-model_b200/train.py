@@ -335,39 +335,43 @@ class MaxViTTrainFn(torch.autograd.Function):
 
 
 # ------------------------------------------------------------------------------------------------ MetNet3
-def _resblock_train_fwd(x, skip, cond, d, N, HP, WP, mixed):
-    """128->128 ResnetBlock.  x: conv input (compute dtype); skip: the same tensor as the residual operand (fp32 copy in
-    mixed mode).  -> (out, out_fp32_copy or None, saved)"""
-    dtype, dev = x.dtype, x.device
+def _resblock_train_fwd(x, skip, cond, d, N, HP, WP, mixed, tf32=False):
+    """C->C ResnetBlock.  x: conv input (compute dtype); skip: the same tensor as the residual operand (fp32 copy in
+    mixed mode); tf32: fp32 storage, convolutions on tcgen05 kind::tf32.  -> (out, out_fp32_copy or None, saved)"""
+    dtype, dev, C = x.dtype, x.device, x.shape[1]
     film = ops.cond_mlp(cond, d["mlp_w"], d["mlp_b"], pre_relu=True)
-    t1 = ops.pg_empty(N, HP, WP, 128, dtype, dev)
-    _, sv1 = ot.conv3x3_ln_train(x, d["w1"], d["b1"], d["g1"], d["be1"], d["eps1"], film, None, t1, N, HP, WP)
-    out = ops.pg_empty(N, HP, WP, 128, dtype, dev)
-    copy = ops.pg_empty(N, HP, WP, 128, torch.float32, dev) if mixed else None
-    _, sv2 = ot.conv3x3_ln_train(t1, d["w2"], d["b2"], d["g2"], d["be2"], d["eps2"], None, skip, out, N, HP, WP, out_copy=copy)
+    t1 = ops.pg_empty(N, HP, WP, C, dtype, dev)
+    _, sv1 = ot.conv3x3_ln_train(x, d["w1"], d["b1"], d["g1"], d["be1"], d["eps1"], film, None, t1, N, HP, WP, tf32=tf32)
+    out = ops.pg_empty(N, HP, WP, C, dtype, dev)
+    copy = ops.pg_empty(N, HP, WP, C, torch.float32, dev) if mixed else None
+    _, sv2 = ot.conv3x3_ln_train(t1, d["w2"], d["b2"], d["g2"], d["be2"], d["eps2"], None, skip, out, N, HP, WP, out_copy=copy,
+                                 tf32=tf32)
     return out, copy, dict(x=x, t1=t1, sv1=sv1, sv2=sv2, film=film)
 
 
-def _block_bwd(dY, sv, conv_in, blk, d, which, film, G, pre, N, HP, WP, dtype, shifts, want_dfilm):
+def _block_bwd(dY, sv, conv_in, blk, d, which, film, G, pre, N, HP, WP, dtype, shifts, want_dfilm, tf32=False):
     """backward of one Block up to (and including) its weight gradient; returns dconv (GEMM dtype) and dfilm"""
     g, be, eps = d["g" + which], d["be" + which], d["eps" + which]
     dconv, sums, _ = ot.conv_ln_bwd(dY, sv, g, film, eps, N, HP, WP, dtype)
     name = pre + ("block1." if which == "1" else "block2.")
     dfilm = ot.conv_ln_param_grads(sums, N, g, be, film, G[name + "norm.g"].view(-1), G[name + "norm.b"].view(-1),
                                    G[name + "proj.bias"], want_dfilm)
-    dWt = torch.empty(128, 9 * 128, dtype=torch.float32, device=dY.device)
-    ot.wgrad(dconv, conv_in, dWt, ntaps=9, tap_shift=shifts, beta=0.0)
-    G[name + "proj.weight"].add_(_unpack_wgrad3x3(dWt, 128, 128, 128))
+    C = dY.shape[1]
+    dWt = torch.empty(C, 9 * C, dtype=torch.float32, device=dY.device)
+    ot.wgrad(dconv, conv_in, dWt, ntaps=9, tap_shift=shifts, beta=0.0, tf32=tf32)
+    G[name + "proj.weight"].add_(_unpack_wgrad3x3(dWt, C, C, C))
     return dconv, dfilm
 
 
-def _resblock_train_bwd(dOut, sv, blk, d, G, pre, cond, dcond, N, HP, WP, dtype, shifts, nshifts):
-    dconv2, _ = _block_bwd(dOut, sv["sv2"], sv["t1"], blk, d, "2", None, G, pre, N, HP, WP, dtype, shifts, False)
-    dt1 = ops.gemm(dconv2, _pack_dgrad3x3(blk.block2.proj.weight.detach(), dtype), ntaps=9, tap_shift=nshifts, out_f32=True)
+def _resblock_train_bwd(dOut, sv, blk, d, G, pre, cond, dcond, N, HP, WP, dtype, shifts, nshifts, tf32=False):
+    dconv2, _ = _block_bwd(dOut, sv["sv2"], sv["t1"], blk, d, "2", None, G, pre, N, HP, WP, dtype, shifts, False, tf32)
+    dt1 = ops.gemm(dconv2, _pack_dgrad3x3(blk.block2.proj.weight.detach(), dtype), ntaps=9, tap_shift=nshifts, out_f32=True,
+                   tf32=tf32)
     del dconv2
-    dconv1, dfilm = _block_bwd(dt1, sv["sv1"], sv["x"], blk, d, "1", sv["film"], G, pre, N, HP, WP, dtype, shifts, True)
+    dconv1, dfilm = _block_bwd(dt1, sv["sv1"], sv["x"], blk, d, "1", sv["film"], G, pre, N, HP, WP, dtype, shifts, True, tf32)
     del dt1
-    dx = ops.gemm(dconv1, _pack_dgrad3x3(blk.block1.proj.weight.detach(), dtype), ntaps=9, tap_shift=nshifts, res=dOut, out_f32=True)
+    dx = ops.gemm(dconv1, _pack_dgrad3x3(blk.block1.proj.weight.detach(), dtype), ntaps=9, tap_shift=nshifts, res=dOut, out_f32=True,
+                  tf32=tf32)
     ot.cond_mlp_bwd(cond, d["mlp_w"], None, None, dfilm, G[pre + "mlp.1.weight"], G[pre + "mlp.1.bias"], None, None, dcond,
                     pre_relu=True)
     return dx
@@ -385,6 +389,7 @@ def metnet3_train_forward(model, x, ts, frozen=False):
     dtype = model.compute_dtype
     dev = x.device
     mixed = dtype != torch.float32
+    tf32 = model.conv_tf32                       # 'tf32_conv': fp32 storage, every convolution on tcgen05 kind::tf32
     P = model.packed(dtype)
     et = P["emb_time"]
     s0 = P["resnet1"][0]
@@ -393,8 +398,8 @@ def metnet3_train_forward(model, x, ts, frozen=False):
     S = dict(B=B, N=N, HP=HP, WP=WP, ts=ts, temb=temb, cond=cond)
     # ---- stem, once per sample
     xin = ops.prepare(x, pads, HP, WP, P["c_pad"], model.pm25_mean, model.pm25_std, dtype)
-    raw3 = ops.gemm(xin, s0["w1"], ntaps=9, tap_shift=ops.conv_tap_shifts(WP), out_f32=True)
-    rawres = ops.gemm(xin, s0["wres"], out_f32=True)
+    raw3 = ops.gemm(xin, s0["w1"], ntaps=9, tap_shift=ops.conv_tap_shifts(WP), out_f32=True, tf32=tf32)
+    rawres = ops.gemm(xin, s0["wres"], out_f32=True, tf32=tf32)
     film0 = ops.cond_mlp(cond, s0["mlp_w"], s0["mlp_b"], pre_relu=True)
     h1 = ops.pg_empty(N, HP, WP, C, dtype, dev)
     skip0 = ops.pg_empty(N, HP, WP, C, torch.float32, dev)
@@ -403,12 +408,13 @@ def metnet3_train_forward(model, x, ts, frozen=False):
     del raw3, rawres
     h = ops.pg_empty(N, HP, WP, C, dtype, dev)
     hs = ops.pg_empty(N, HP, WP, C, torch.float32, dev) if mixed else None
-    _, sv_b2 = ot.conv3x3_ln_train(h1, s0["w2"], s0["b2"], s0["g2"], s0["be2"], s0["eps2"], None, skip0, h, N, HP, WP, out_copy=hs)
+    _, sv_b2 = ot.conv3x3_ln_train(h1, s0["w2"], s0["b2"], s0["g2"], s0["be2"], s0["eps2"], None, skip0, h, N, HP, WP, out_copy=hs,
+                                   tf32=tf32)
     del skip0
     S["stem"] = dict(xin=xin, film=film0, h1=h1, sv1=sv_stem, sv2=sv_b2)
     enc = []
     for d in P["resnet1"][1:]:
-        h, hs, sv = _resblock_train_fwd(h, hs if mixed else h, cond, d, N, HP, WP, mixed)
+        h, hs, sv = _resblock_train_fwd(h, hs if mixed else h, cond, d, N, HP, WP, mixed, tf32)
         enc.append(sv)
     S["enc"], S["h_enc"] = enc, h
     # ---- MaxViT at half resolution
@@ -418,11 +424,11 @@ def metnet3_train_forward(model, x, ts, frozen=False):
     # ---- decoder
     up = torch.zeros(ops.pg_pixels(N, HP, WP), C, dtype=dtype, device=dev)
     ups = ops.pg_empty(N, HP, WP, C, torch.float32, dev) if mixed else None
-    ops.convT2(low, P["w_up_vit"], P["b_up"], up, tf32=model.vit.tf32, out_copy=ups)
+    ops.convT2(low, P["w_up_vit"], P["b_up"], up, tf32=model.vit.tf32 or tf32, out_copy=ups)
     h, hs = up, ups
     dec = []
     for d in P["resnet2"]:
-        h, hs, sv = _resblock_train_fwd(h, hs if mixed else h, cond, d, N, HP, WP, mixed)
+        h, hs, sv = _resblock_train_fwd(h, hs if mixed else h, cond, d, N, HP, WP, mixed, tf32)
         dec.append(sv)
     S["dec"], S["h_last"] = dec, h
     pred = torch.empty(B, L, model.input_height, model.input_width, dtype=torch.float32, device=dev)
@@ -444,6 +450,7 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
     cond = S["cond"]
     shifts = ops.conv_tap_shifts(WP)
     nshifts = tuple(-s for s in shifts)
+    tf32 = model.conv_tf32
     dcond = torch.zeros_like(cond)
     done = (lambda i: sync.section_done(G.section(i))) if sync is not None else (lambda i: None)
 
@@ -455,17 +462,18 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
     # ---- decoder
     for k in reversed(range(len(model.resnet2.blocks))):
         dH = _resblock_train_bwd(dH, S["dec"][k], model.resnet2.blocks[k], P["resnet2"][k], G, f"resnet2.blocks.{k}.", cond, dcond,
-                                 N, HP, WP, dtype, shifts, nshifts)
+                                 N, HP, WP, dtype, shifts, nshifts, tf32)
     done(1)
     # ---- ConvTranspose (metnet3.py:88-89)
     Hl, Wl = HP // 2, WP // 2
     Gm = ot.convT2_bwd_gather(dH, N, Hl, Wl, C, vdt, G["up.bias"])
     del dH
     low_out = S["low_out"].view(N * Hl * Wl, C)
+    up_tf32 = model.vit.tf32 or tf32                                               # as the forward ConvTranspose
     dWt = torch.empty(4 * C, C, dtype=torch.float32, device=dev)
-    ot.wgrad(Gm, low_out, dWt, beta=0.0, tf32=model.vit.tf32)
+    ot.wgrad(Gm, low_out, dWt, beta=0.0, tf32=up_tf32)
     G["up.weight"].add_(dWt.view(2, 2, C, C).permute(3, 2, 0, 1))                 # [(di,dj,co)][ci] -> (ci, co, di, dj)
-    dlow = ops.gemm(Gm, model.up.weight.detach().permute(0, 2, 3, 1).reshape(C, 4 * C).to(vdt).contiguous(), tf32=model.vit.tf32)
+    dlow = ops.gemm(Gm, model.up.weight.detach().permute(0, 2, 3, 1).reshape(C, 4 * C).to(vdt).contiguous(), tf32=up_tf32)
     del Gm
     done(2)
     # ---- MaxViT
@@ -476,12 +484,13 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
     del dlow
     for k in reversed(range(1, len(model.resnet1.blocks))):
         dH = _resblock_train_bwd(dH, S["enc"][k - 1], model.resnet1.blocks[k], P["resnet1"][k], G, f"resnet1.blocks.{k}.", cond,
-                                 dcond, N, HP, WP, dtype, shifts, nshifts)
+                                 dcond, N, HP, WP, dtype, shifts, nshifts, tf32)
     # ---- stem block (lead-time dedup): block2 is an ordinary Block, block1 / res_conv run per sample
     st, s0, blk0 = S["stem"], P["resnet1"][0], model.resnet1.blocks[0]
     pre = "resnet1.blocks.0."
-    dconv2, _ = _block_bwd(dH, st["sv2"], st["h1"], blk0, s0, "2", None, G, pre, N, HP, WP, dtype, shifts, False)
-    dh1 = ops.gemm(dconv2, _pack_dgrad3x3(blk0.block2.proj.weight.detach(), dtype), ntaps=9, tap_shift=nshifts, out_f32=True)
+    dconv2, _ = _block_bwd(dH, st["sv2"], st["h1"], blk0, s0, "2", None, G, pre, N, HP, WP, dtype, shifts, False, tf32)
+    dh1 = ops.gemm(dconv2, _pack_dgrad3x3(blk0.block2.proj.weight.detach(), dtype), ntaps=9, tap_shift=nshifts, out_f32=True,
+                   tf32=tf32)
     del dconv2
     dconv1, sums, border = ot.conv_ln_bwd(dh1, st["sv1"], s0["g1"], st["film"], s0["eps1"], N, HP, WP, torch.float32, want_border=True)
     del dh1
@@ -490,10 +499,13 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
     ot.cond_mlp_bwd(cond, s0["mlp_w"], None, None, dfilm, G[pre + "mlp.1.weight"], G[pre + "mlp.1.bias"], None, None, dcond,
                     pre_relu=True)
     c_data, c_pad = model.n_input_channels, P["c_pad"]
+    # GEMMs over the stem input xin [q][c_pad]: the tf32 weight gradient needs c_pad % 128 == 0 (640 for the 12-hour model); a
+    # narrower stem (c_pad 64: two input time steps) runs them as exact-fp32 SIMT products instead
+    stem_tf32 = tf32 and c_pad % 128 == 0
     draw3 = ot.lead_sum(dconv1, B, L, HP, WP, dtype)
     del dconv1
     dWt = torch.empty(C, 9 * c_pad, dtype=torch.float32, device=dev)
-    ot.wgrad(draw3, st["xin"], dWt, ntaps=9, tap_shift=shifts, beta=0.0)
+    ot.wgrad(draw3, st["xin"], dWt, ntaps=9, tap_shift=shifts, beta=0.0, tf32=stem_tf32)
     gw3 = G[pre + "block1.proj.weight"]
     gw3[:, :c_data].add_(_unpack_wgrad3x3(dWt, C, c_pad, c_data))
     del dWt
@@ -501,18 +513,18 @@ def metnet3_train_backward(model, S, dpred, G: GradBuffer, sync: GradSync | None
         # data gradient of the per-sample stem: 3x3 conv^T over the data channels (negated tap shifts), c_pad outputs
         w3t = torch.zeros(c_pad, 9 * C, dtype=dtype, device=dev)
         w3t[:c_data] = _pack_dgrad3x3(blk0.block1.proj.weight.detach()[:, :c_data], dtype)
-        dxin = ops.gemm(draw3, w3t, ntaps=9, tap_shift=nshifts, out_f32=True)
+        dxin = ops.gemm(draw3, w3t, ntaps=9, tap_shift=nshifts, out_f32=True, tf32=stem_tf32)
         del w3t
     del draw3
     dres = ot.lead_sum(dH, B, L, HP, WP, dtype)
     dWr = torch.empty(C, c_pad, dtype=torch.float32, device=dev)
-    ot.wgrad(dres, st["xin"], dWr, beta=0.0)
+    ot.wgrad(dres, st["xin"], dWr, beta=0.0, tf32=stem_tf32)
     dx = None
     if want_dx:
         # + res_conv^T, accumulated in the GEMM epilogue (each element is read and written by the same thread)
         wrt = torch.zeros(c_pad, C, dtype=dtype, device=dev)
         wrt[:c_data] = blk0.res_conv.weight.detach()[:, :c_data, 0, 0].t()
-        ops.gemm(dres, wrt, res=dxin, out=dxin, out_f32=True)
+        ops.gemm(dres, wrt, res=dxin, out=dxin, out_f32=True, tf32=stem_tf32)
         del wrt
         dx = ot.prepare_bwd(dxin, B, model.window_size, model.n_variables, model.input_height, model.input_width, pads, HP, WP,
                             model.pm25_std, model.standardised_extra_channel)
