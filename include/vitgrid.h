@@ -186,7 +186,9 @@ VG_API int vg_attn_gather_fwd(int dtype, const void* x, const float* reg, int re
  * (table (2w-1)^2+1 x heads, fp32), softmax, PV.  qkv [(Nw*S)][3*heads*dh] -> out [(Nw*S)][heads*dh].
  * dtype 0: bf16 tensors (tf32 mma products, fp32 softmax); 1: fp32 tensors, exact-fp32 FMAs; 2: fp32 tensors, QK^T and PV as 3xTF32
  * split products on the tensor cores (mma.sync; fp32-grade: 24 accumulation steps per score); 4: fp32 tensors, single tf32 products (the
- * mixed-precision modes); 6: as 2, with out [(Nw*S)][3*heads*dh] written as the split operand [hi | hi | lo] of vg_split3_tf32 (pattern 0).  Dropout and S > 64 run the SIMT kernel. */
+ * mixed-precision modes); 6: as 2, with out [(Nw*S)][3*heads*dh] written as the split operand [hi | hi | lo] of vg_split3_tf32 (pattern 0).  Dropout and S > 64 run the SIMT kernel.
+ * S <= 128, with or without dropout (drop_thresh > 0: nn.Dropout on the probabilities; at S > 64 the masks use 128 slots per
+ * window and need heads <= 128, see vg_dropout_mask_debug).  S > 128 is an error. */
 VG_API int vg_attn_core_fwd(int dtype, const void* qkv, const float* q_gamma, const float* k_gamma,
                      const float* bias_table, int N, int Hl, int Wl, int win, int R, int heads, int dh, void* out,
                      long long drop_seed, int drop_salt, int drop_thresh, void* stream);
@@ -418,12 +420,14 @@ VG_API int vg_se_bwd(const float* dh4, const float* h3, const float* gate, const
 VG_API int vg_attn_out_bwd_gather(const float* dx_out, const float* dreg, float reg_scale, int N, int Hl, int Wl, int C, int win,
                            int R, int grid_mode, void* dproj, int dproj_bf16, long long drop_seed, int drop_salt, int drop_thresh,
                            void* stream);
-/* test hook: the dropout masks the kernels use, as bytes (1 = kept): prob_mask [n_windows][heads][64][64] (query slot,
- * key slot), out_mask [n_windows][64][C] */
+/* test hook: the dropout masks the kernels use, as bytes (1 = kept): prob_mask [n_windows][heads][slots][slots] (query slot,
+ * key slot), out_mask [n_windows][slots][C].  slots = 64: the masks of windows of up to 64 tokens; slots = 128: those of windows
+ * of 65 .. 128 tokens (un-fused path only; heads <= 128).  Any other slot count is an error. */
 VG_API int vg_dropout_mask_debug(long long drop_seed, int drop_salt, int drop_thresh, long long n_windows, int heads, int C,
-                          void* prob_mask, void* out_mask, void* stream);
+                          int slots, void* prob_mask, void* out_mask, void* stream);
 /* per-(field, head) core backward: dqkv written; dq_gamma, dk_gamma, dbias_table accumulated.  dim_head 32 or 64 (mode 3: 32
- * only), S <= 64.  use_tf32 = 2 / 3: tensor-core
+ * only), S <= 128 (mode 3 and att_out: S <= 64; dropout at S > 64: heads <= 128).  Windows of 65 .. 128 tokens run kernels of
+ * their own in modes 0 and 2.  use_tf32 = 2 / 3: tensor-core
  * kernel (2: bf16 mma + ldmatrix on fp32 tensors; 3: the tcgen05 kernel on bf16 tensors qkv, datt, dqkv and att_out, which
  * must be 16-byte aligned, S <= 64; fp32 accumulate), which can also re-materialise the forward output
  * att = softmax(.) V [rows][inner] (att_out, or NULL) for the to_out weight gradient when the forward pass was the fused

@@ -570,8 +570,8 @@ int vg_attn_out_bwd_gather(const float* dx_out, const float* dreg, float reg_sca
 }
 
 int vg_dropout_mask_debug(long long drop_seed, int drop_salt, int drop_thresh, long long n_windows, int heads, int C,
-                          void* prob_mask, void* out_mask, void* stream) {
-  return dropout_mask_debug_run((unsigned)drop_seed, (unsigned)drop_salt, drop_thresh, n_windows, heads, C,
+                          int slots, void* prob_mask, void* out_mask, void* stream) {
+  return dropout_mask_debug_run((unsigned)drop_seed, (unsigned)drop_salt, drop_thresh, n_windows, heads, C, slots,
                                 reinterpret_cast<unsigned char*>(prob_mask), reinterpret_cast<unsigned char*>(out_mask),
                                 (cudaStream_t)stream);
 }

@@ -160,9 +160,11 @@ __global__ void __launch_bounds__(128, DH == 64 ? 3 : 5) attn_core_kernel(const 
   for (int d = 0; d < DH; ++d) { q[d] *= inv * qgamma[hd * DH + d]; o[d] = 0.f; }
   const int ti = i - g.R, ai = ti / g.win, bi = ti - ai * g.win;
   float m = -INFINITY, l = 0.f;
+  const int slots = drop_slots(S);
   for (int j0 = 0; j0 < Sp; j0 += 4) {
-    // nn.Dropout on the probabilities (maxvit.py:146): the same counter-based mask as the fused kernels (vg_rng.cuh)
-    const uint32_t hsh = drop.thresh ? drop_hash(drop.seed, drop_row(wdx, i), drop_group_prob(drop.salt, hd, j0 >> 2)) : 0u;
+    // nn.Dropout on the probabilities (maxvit.py:146): the same counter-based mask as the fused kernels (vg_rng.cuh; 128 slots
+    // per window when S > 64)
+    const uint32_t hsh = drop.thresh ? drop_hash(drop.seed, drop_row(wdx, i, slots), drop_group_prob(drop.salt, hd, j0 >> 2, slots)) : 0u;
     float sc[4];
 #pragma unroll
     for (int u = 0; u < 4; ++u) {
@@ -467,7 +469,9 @@ int attn_core_run(int dtype, const void* qkv, const float* qgamma, const float* 
                   const AttnGeom& g, int heads, int dh, void* out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
   if (g.S() > 128) return set_error("attn_core: sequence %d too long", g.S());
   if (dtype != 0 && dtype != 1 && dtype != 2 && dtype != 4 && dtype != 6) return set_error("attn_core: dtype code %d (0 bf16, 1 fp32, 2 / 6 fp32 3xTF32, 4 fp32 tf32)", dtype);
-  if (drop_thresh < 0 || drop_thresh > 255 || (drop_thresh && g.S() > 64)) return set_error("attn_core: bad dropout threshold %d (or sequence > 64)", drop_thresh);
+  if (drop_thresh < 0 || drop_thresh > 255) return set_error("attn_core: dropout threshold %d outside [0, 255]", drop_thresh);
+  if (drop_thresh && g.S() > 64 && heads > DROP_MAX_HEADS_LONG)
+    return set_error("attn_core: dropout with %d heads at sequence %d > 64 (at most %d heads)", heads, g.S(), DROP_MAX_HEADS_LONG);
   DropCfg drop;
   drop.seed = seed; drop.salt = salt; drop.thresh = drop_thresh; drop.scale = 256.0f / (256.0f - (float)drop_thresh);
   // dtype 2 = fp32 storage with 3xTF32 tensor-core products (the 'tf32_conv' precision of wide networks); dtype 4 = fp32 storage and

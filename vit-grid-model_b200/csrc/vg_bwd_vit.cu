@@ -589,7 +589,7 @@ __global__ void __launch_bounds__(256) attn_out_bwd_gather_kernel(const float* _
       v = *reinterpret_cast<const float4*>(dx_out + ((long long)n * g.Hl * g.Wl + attn_token_pixel(g, wi, tok - g.R)) * C + c);
     }
     if (drop.thresh) {                                       // the to_out dropout mask of the forward pass (maxvit.py:151)
-      const uint32_t hsh = drop_hash(drop.seed, drop_row(wdx, tok), drop_group_out(drop.salt, c >> 2));
+      const uint32_t hsh = drop_hash(drop.seed, drop_row(wdx, tok, drop_slots(S)), drop_group_out(drop.salt, c >> 2));
       v.x *= (int)(hsh & 255u) >= drop.thresh ? drop.scale : 0.f;
       v.y *= (int)((hsh >> 8) & 255u) >= drop.thresh ? drop.scale : 0.f;
       v.z *= (int)((hsh >> 16) & 255u) >= drop.thresh ? drop.scale : 0.f;
@@ -1157,6 +1157,524 @@ __global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_ker
   for (int i = threadIdx.x; i < nb; i += 128) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Core backward for windows of 65 .. 128 tokens (the reference default, window 8 with four register tokens, has 68).
+// The kernels above keep every row tile of a window in shared memory; at 128 slots those tiles do not fit (mode 0: 266 KB of
+// [128][DH+1] tiles at DH 64), so these are kernels of their own, launched only when S > 64.  Their dropout masks use the
+// 128-slot ids of vg_rng.cuh.
+// ------------------------------------------------------------------------------------------------
+// Mode 0 (exact fp32, SIMT): K-hat, V and the key-side accumulators dK-hat, dV stay resident ([128][DH+1] each); the query rows
+// stream through in blocks of QB: per block Q-hat, the unit q, dO, P (overwritten by dS) and the dropout mask; dQ of a query row
+// is finished inside its block.  The key-side RMSNorm backward runs after the last block, with the unit k re-derived from k in
+// global memory.  Same arithmetic as attn_core_bwd_kernel per element; DH 64: 199 KB of shared memory (window 11).
+template <int DH>
+struct cbs_long {
+  static constexpr int SK = 128, QB = 32, LD = DH + 1, LP = SK + 1;
+  static size_t bytes(int nb) { return (size_t)(4 * SK * LD + 3 * QB * LD + 2 * QB * LP + 2 * nb + SK + QB + 8 * 2 * DH) * sizeof(float); }
+};
+
+template <int DH>
+__global__ void __launch_bounds__(256, 1) attn_core_bwd_long_kernel(const AttnCoreBwdParams p, const DropCfg drop) {
+  using L = cbs_long<DH>;
+  constexpr int SK = L::SK, QB = L::QB, LD = L::LD, LP = L::LP, DPL = DH / 32;
+  extern __shared__ float sm[];
+  const AttnGeom g = p.g;
+  const int S = g.S(), nwin = g.nwin(), W2 = 2 * g.win - 1, nb = W2 * W2 + 1;
+  float* kh = sm;                  // [SK][LD] normalised * gamma
+  float* vv = kh + SK * LD;
+  float* dkh = vv + SK * LD;       // accumulated over the query blocks of a window
+  float* dv = dkh + SK * LD;
+  float* qh = dv + SK * LD;        // [QB][LD]
+  float* qu = qh + QB * LD;        // unit vectors
+  float* dO = qu + QB * LD;
+  float* P = dO + QB * LD;         // [QB][LP]: P, then dS
+  float* MK = P + QB * LP;         // [QB][LP] dropout mask * scale
+  float* sbias = MK + QB * LP;     // [nb]
+  float* dbias = sbias + nb;       // [nb]
+  float* nrk = dbias + nb;         // [SK] |k|
+  float* inq = nrk + SK;           // [QB] 1/|q|
+  float* gred = inq + QB;          // [8][2][DH]
+  const int n = blockIdx.x / p.heads, hd = blockIdx.x - n * p.heads;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int inner = p.heads * DH;
+  const float rs = sqrtf((float)DH);
+  for (int i = threadIdx.x; i < nb; i += 256) { sbias[i] = p.bias_table[i * p.heads + hd]; dbias[i] = 0.f; }
+  float gq[DPL], gk[DPL], dgq[DPL], dgk[DPL];
+#pragma unroll
+  for (int k = 0; k < DPL; ++k) {
+    gq[k] = p.qgamma[hd * DH + lane + 32 * k]; gk[k] = p.kgamma[hd * DH + lane + 32 * k];
+    dgq[k] = 0.f; dgk[k] = 0.f;
+  }
+  __syncthreads();
+
+  for (int wi = 0; wi < nwin; ++wi) {
+    const long long wdx = (long long)n * nwin + wi, row0 = wdx * S;
+    // ---- keys: K-hat, V; dK-hat and dV start at zero.  Warp per row, lane = d
+    for (int j = warp; j < S; j += 8) {
+      const float* src = p.qkv + (row0 + j) * 3 * inner + hd * DH + lane;
+      float k[DPL], v[DPL];
+#pragma unroll
+      for (int c = 0; c < DPL; ++c) { k[c] = src[inner + 32 * c]; v[c] = src[2 * inner + 32 * c]; }
+      const float nk = fmaxf(sqrtf(warp_sum(lane_dot<DPL>(k, k))), 1e-12f);
+#pragma unroll
+      for (int c = 0; c < DPL; ++c) {
+        const int d = lane + 32 * c;
+        kh[j * LD + d] = k[c] / nk * rs * gk[c]; vv[j * LD + d] = v[c];
+        dkh[j * LD + d] = 0.f; dv[j * LD + d] = 0.f;
+      }
+      if (lane == 0) nrk[j] = nk;
+    }
+    for (int q0 = 0; q0 < S; q0 += QB) {
+      const int nq = min(QB, S - q0);
+      // ---- query rows q0 .. q0 + nq - 1
+      for (int r = warp; r < nq; r += 8) {
+        const float* src = p.qkv + (row0 + q0 + r) * 3 * inner + hd * DH + lane;
+        float q[DPL];
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) q[c] = src[32 * c];
+        const float nq_ = fmaxf(sqrtf(warp_sum(lane_dot<DPL>(q, q))), 1e-12f);
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) {
+          const int d = lane + 32 * c;
+          const float uq = q[c] / nq_;
+          qu[r * LD + d] = uq; qh[r * LD + d] = uq * rs * gq[c];
+          dO[r * LD + d] = p.datt[(row0 + q0 + r) * inner + hd * DH + d];
+        }
+        if (lane == 0) inq[r] = 1.0f / nq_;
+      }
+      __syncthreads();
+      // ---- P = softmax(qh kh^T + bias): warp per query row, lanes over keys j = lane + 32t
+      for (int r = warp; r < nq; r += 8) {
+        const int i = q0 + r;
+        const int ti = i - g.R, ai = ti / g.win, bi = ti - ai * g.win;
+        float s[4];
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const int j = lane + 32 * t;
+          float a = -INFINITY;
+          if (j < S) {
+            a = 0.f;
+#pragma unroll
+            for (int d = 0; d < DH; ++d) a = fmaf(qh[r * LD + d], kh[j * LD + d], a);
+            int bidx = nb - 1;
+            if (i >= g.R && j >= g.R) { const int tj = j - g.R, aj = tj / g.win, bj = tj - aj * g.win; bidx = (ai - aj + g.win - 1) * W2 + (bi - bj + g.win - 1); }
+            a += sbias[bidx];
+          }
+          s[t] = a;
+        }
+        const float m = warp_max(fmaxf(fmaxf(s[0], s[1]), fmaxf(s[2], s[3])));
+        float e[4];
+#pragma unroll
+        for (int t = 0; t < 4; ++t) e[t] = lane + 32 * t < S ? __expf(s[t] - m) : 0.f;
+        const float inv = 1.0f / warp_sum((e[0] + e[1]) + (e[2] + e[3]));
+#pragma unroll
+        for (int t = 0; t < 4; ++t) P[r * LP + lane + 32 * t] = e[t] * inv;
+        if (drop.thresh) {                                   // the forward pass's mask on the probabilities (maxvit.py:146)
+          const uint32_t rid = drop_row(wdx, i, SK);
+#pragma unroll
+          for (int t = 0; t < 4; ++t) {
+            const int j = lane + 32 * t;
+            const uint32_t hsh = drop_hash(drop.seed, rid, drop_group_prob(drop.salt, hd, j >> 2, SK));
+            MK[r * LP + j] = (int)((hsh >> (8 * (j & 3))) & 255u) >= drop.thresh ? drop.scale : 0.f;
+          }
+        }
+      }
+      __syncthreads();
+      // ---- dV[j][d] += sum_i P'[i][j] dO[i][d] (P' = P * mask): warp per key, lane = d
+      for (int j = warp; j < S; j += 8) {
+        float a[DPL];
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) a[c] = dv[j * LD + lane + 32 * c];
+        for (int r = 0; r < nq; ++r) {
+          const float pm = drop.thresh ? P[r * LP + j] * MK[r * LP + j] : P[r * LP + j];
+#pragma unroll
+          for (int c = 0; c < DPL; ++c) a[c] = fmaf(pm, dO[r * LD + lane + 32 * c], a[c]);
+        }
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) dv[j * LD + lane + 32 * c] = a[c];
+      }
+      __syncthreads();
+      // ---- dS = P * (dP - sum_j P dP), dP[i][j] = dO[i] . v[j] (* mask); overwrite P with dS; bias-table gradient
+      for (int r = warp; r < nq; r += 8) {
+        const int i = q0 + r;
+        const int ti = i - g.R, ai = ti / g.win, bi = ti - ai * g.win;
+        float dp[4], pr[4];
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const int j = lane + 32 * t;
+          float a = 0.f;
+          if (j < S) {
+#pragma unroll
+            for (int d = 0; d < DH; ++d) a = fmaf(dO[r * LD + d], vv[j * LD + d], a);
+            if (drop.thresh) a *= MK[r * LP + j];
+          }
+          dp[t] = a; pr[t] = j < S ? P[r * LP + j] : 0.f;
+        }
+        const float dot = warp_sum((pr[0] * dp[0] + pr[1] * dp[1]) + (pr[2] * dp[2] + pr[3] * dp[3]));
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+          const int j = lane + 32 * t;
+          if (j < S) {
+            const float ds = pr[t] * (dp[t] - dot);
+            P[r * LP + j] = ds;
+            int bidx = nb - 1;
+            if (i >= g.R && j >= g.R) { const int tj = j - g.R, aj = tj / g.win, bj = tj - aj * g.win; bidx = (ai - aj + g.win - 1) * W2 + (bi - bj + g.win - 1); }
+            atomicAdd(&dbias[bidx], ds);
+          }
+        }
+      }
+      __syncthreads();
+      // ---- dK-hat[j] += sum_i dS[i][j] qh[i] (warp per key); dQ-hat[i] = sum_j dS[i][j] kh[j] (warp per query row), then the
+      // RMSNorm backward of q (maxvit.py:30): qh = u * rs * gamma, u = q/|q|
+      for (int j = warp; j < S; j += 8) {
+        float b[DPL];
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) b[c] = dkh[j * LD + lane + 32 * c];
+        for (int r = 0; r < nq; ++r)
+#pragma unroll
+          for (int c = 0; c < DPL; ++c) b[c] = fmaf(P[r * LP + j], qh[r * LD + lane + 32 * c], b[c]);
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) dkh[j * LD + lane + 32 * c] = b[c];
+      }
+      for (int r = warp; r < nq; r += 8) {
+        float a[DPL], uq[DPL], g1[DPL];
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) a[c] = 0.f;
+        for (int j = 0; j < S; ++j)
+#pragma unroll
+          for (int c = 0; c < DPL; ++c) a[c] = fmaf(P[r * LP + j], kh[j * LD + lane + 32 * c], a[c]);
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) {
+          uq[c] = qu[r * LD + lane + 32 * c];
+          dgq[c] = fmaf(a[c], uq[c] * rs, dgq[c]);
+          g1[c] = a[c] * rs * gq[c];
+        }
+        const float d1 = warp_sum(lane_dot<DPL>(g1, uq));
+        float* dst = p.dqkv + (row0 + q0 + r) * 3 * inner + hd * DH + lane;
+#pragma unroll
+        for (int c = 0; c < DPL; ++c) dst[32 * c] = inq[r] * (g1[c] - uq[c] * d1);
+      }
+      __syncthreads();
+    }
+    // ---- keys: dV out, and the RMSNorm backward of k with u = k/|k| from global memory
+    for (int j = warp; j < S; j += 8) {
+      const float* src = p.qkv + (row0 + j) * 3 * inner + inner + hd * DH + lane;
+      const float nk = nrk[j];
+      float uk[DPL], g2[DPL];
+#pragma unroll
+      for (int c = 0; c < DPL; ++c) {
+        const float ak = dkh[j * LD + lane + 32 * c];
+        uk[c] = src[32 * c] / nk;
+        dgk[c] = fmaf(ak, uk[c] * rs, dgk[c]);
+        g2[c] = ak * rs * gk[c];
+      }
+      const float d2 = warp_sum(lane_dot<DPL>(g2, uk));
+      float* dst = p.dqkv + (row0 + j) * 3 * inner + hd * DH + lane;
+#pragma unroll
+      for (int c = 0; c < DPL; ++c) {
+        dst[inner + 32 * c] = (1.0f / nk) * (g2[c] - uk[c] * d2);
+        dst[2 * inner + 32 * c] = dv[j * LD + lane + 32 * c];
+      }
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int k = 0; k < DPL; ++k) { gred[(warp * 2) * DH + lane + 32 * k] = dgq[k]; gred[(warp * 2 + 1) * DH + lane + 32 * k] = dgk[k]; }
+  __syncthreads();
+  if (threadIdx.x < 2 * DH) {
+    const int which = threadIdx.x / DH, d = threadIdx.x % DH;
+    float s = 0.f;
+    for (int w = 0; w < 8; ++w) s += gred[(w * 2 + which) * DH + d];
+    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, s);
+  }
+  for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
+}
+
+// Mode 2 (bf16 mma.sync on fp32 tensors): the layout of attn_core_bwd_bf16_kernel at 128 slots, 8 warps of 16 query rows, one
+// block per SM (DH 64: 214 KB of shared memory at window 11).  Registers are the limit -- the 64-key kernel already needs 255 at
+// DH 64 -- so the score and dP fragments are taken in two 64-key halves: pass 1 finds the row max and the sum of exp over both
+// halves, pass 2 writes P' = P * mask and forms the row dot sum_j P dP', pass 3 recomputes the scores and dP' of each half for
+// dS.  The bias of a (query, key) pair is read from the table in shared memory, and the bias gradient sums dS per pair over the
+// field's windows in an fp32 [128][136] shared tile (the 64-key kernel keeps both in registers).  No att_out.
+template <int DH_>
+struct cbh_long {
+  static constexpr int DH = DH_, SM = 128;
+  static constexpr int LDQ = DH + 8;   // as cbh
+  static constexpr int LDP = SM + 8;   // bf16 elements per P/dS row (272 B: ldmatrix rows hit distinct banks)
+  static constexpr int LDS = SM + 8;   // floats per row of the dS sum (float2 stores of a warp hit distinct banks)
+  static constexpr int BYTES = 4 * SM * LDQ * 2 + 2 * SM * LDP * 2 + SM * LDS * 4 + 2 * SM * 4;
+  static constexpr int LPR = DH / 8;
+  static constexpr int PASSES = 16 / (32 / LPR);
+};
+
+template <int DH_>
+__global__ void __launch_bounds__(256, 1) attn_core_bwd_bf16_long_kernel(const AttnCoreBwdParams p, const DropCfg drop) {
+  using K = cbh_long<DH_>;
+  constexpr int DH = K::DH, SM = K::SM, LDQ = K::LDQ, LDP = K::LDP, LDS = K::LDS, LPR = K::LPR, PASSES = K::PASSES;
+  extern __shared__ __align__(16) uint8_t smraw[];
+  const AttnGeom g_ = p.g;
+  const int S = g_.S(), nwin = g_.nwin(), W2 = 2 * g_.win - 1, nb = W2 * W2 + 1, R = g_.R, win = g_.win;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int g = lane >> 2, t = lane & 3;
+  bf16* sQ = reinterpret_cast<bf16*>(smraw); bf16* sK = sQ + SM * LDQ; bf16* sV = sK + SM * LDQ; bf16* sdO = sV + SM * LDQ;
+  bf16* sP = sdO + SM * LDQ; bf16* sDS = sP + SM * LDP;
+  float* dsum = reinterpret_cast<float*>(sDS + SM * LDP);     // [SM][LDS] dS of each (query, key) pair summed over the windows
+  float* inq = dsum + SM * LDS; float* ink = inq + SM;
+  float* sbias = ink + SM; float* dbias = sbias + nb; float* gred = dbias + nb;
+  float* sgam = gred + 2 * DH;             // [4][DH]: rs*gq, 1/(rs*gq), rs*gk, 1/(rs*gk)   (1/. = 0 where gamma = 0)
+  const uint32_t aQ = smem_u32(sQ), aK = smem_u32(sK), aV = smem_u32(sV), adO = smem_u32(sdO), aP = smem_u32(sP), aDS = smem_u32(sDS);
+  const int n = blockIdx.x / p.heads, hd = blockIdx.x - n * p.heads;
+  const int inner = p.heads * DH;
+  const float rs = sqrtf((float)DH);
+  for (int i = threadIdx.x; i < nb; i += 256) { sbias[i] = p.bias_table[i * p.heads + hd]; dbias[i] = 0.f; }
+  for (int i = threadIdx.x; i < SM * LDS; i += 256) dsum[i] = 0.f;
+  if (threadIdx.x < 2 * DH) gred[threadIdx.x] = 0.f;
+  if (threadIdx.x < DH) {
+    const float a = rs * p.qgamma[hd * DH + threadIdx.x], b = rs * p.kgamma[hd * DH + threadIdx.x];
+    sgam[threadIdx.x] = a; sgam[DH + threadIdx.x] = a != 0.f ? 1.0f / a : 0.f;
+    sgam[2 * DH + threadIdx.x] = b; sgam[3 * DH + threadIdx.x] = b != 0.f ? 1.0f / b : 0.f;
+  }
+  const int prow = lane / LPR, pd0 = (lane % LPR) * 8;
+  const int r0 = warp * 16;
+  const int ia = r0 + g, ib = r0 + g + 8;
+  // relative-position-bias index of (query i, key j) = base(i) - off(j); nb-1 when either token is a register token
+  int base_a = -1, base_b = -1;
+  if (ia >= R && ia < S) { const int ti = ia - R, a = ti / win, b = ti - a * win; base_a = (a + win - 1) * W2 + (b + win - 1); }
+  if (ib >= R && ib < S) { const int ti = ib - R, a = ti / win, b = ti - a * win; base_b = (a + win - 1) * W2 + (b + win - 1); }
+  __syncthreads();
+
+  for (int wi = 0; wi < nwin; ++wi) {
+    const long long wdx = (long long)n * nwin + wi, row0 = wdx * S;
+    // ---------------- phase 1 (as attn_core_bwd_bf16_kernel): rows r0..r0+15, rows >= S zero
+#pragma unroll
+    for (int pg = 0; pg < PASSES; pg += 2) {
+      float4 ld[2][4][2];
+#pragma unroll
+      for (int ps = 0; ps < 2; ++ps) {
+        const int i = r0 + (pg + ps) * (32 / LPR) + prow;
+#pragma unroll
+        for (int m = 0; m < 4; ++m) { ld[ps][m][0] = make_float4(0.f, 0.f, 0.f, 0.f); ld[ps][m][1] = ld[ps][m][0]; }
+        if (i < S) {
+          const float* src = p.qkv + (row0 + i) * 3 * inner + hd * DH + pd0;
+          const float* sdo = p.datt + (row0 + i) * inner + hd * DH + pd0;
+#pragma unroll
+          for (int m = 0; m < 3; ++m) {
+            ld[ps][m][0] = __ldg(reinterpret_cast<const float4*>(src + m * inner));
+            ld[ps][m][1] = __ldg(reinterpret_cast<const float4*>(src + m * inner + 4));
+          }
+          ld[ps][3][0] = __ldg(reinterpret_cast<const float4*>(sdo));
+          ld[ps][3][1] = __ldg(reinterpret_cast<const float4*>(sdo + 4));
+        }
+      }
+#pragma unroll
+      for (int ps = 0; ps < 2; ++ps) {
+        const int i = r0 + (pg + ps) * (32 / LPR) + prow;
+        float x[4][8];
+#pragma unroll
+        for (int m = 0; m < 4; ++m) {
+          x[m][0] = ld[ps][m][0].x; x[m][1] = ld[ps][m][0].y; x[m][2] = ld[ps][m][0].z; x[m][3] = ld[ps][m][0].w;
+          x[m][4] = ld[ps][m][1].x; x[m][5] = ld[ps][m][1].y; x[m][6] = ld[ps][m][1].z; x[m][7] = ld[ps][m][1].w;
+        }
+        float nq = 0.f, nk = 0.f;
+#pragma unroll
+        for (int d = 0; d < 8; ++d) { nq = fmaf(x[0][d], x[0][d], nq); nk = fmaf(x[1][d], x[1][d], nk); }
+#pragma unroll
+        for (int o = 1; o < LPR; o <<= 1) nq += __shfl_xor_sync(0xffffffffu, nq, o);
+#pragma unroll
+        for (int o = 1; o < LPR; o <<= 1) nk += __shfl_xor_sync(0xffffffffu, nk, o);
+        const float iq = 1.0f / fmaxf(sqrtf(nq), 1e-12f), ik = 1.0f / fmaxf(sqrtf(nk), 1e-12f);    // F.normalize eps (maxvit.py:30)
+        float gq8[8], gk8[8];
+        *reinterpret_cast<float4*>(gq8) = *reinterpret_cast<const float4*>(sgam + pd0);
+        *reinterpret_cast<float4*>(gq8 + 4) = *reinterpret_cast<const float4*>(sgam + pd0 + 4);
+        *reinterpret_cast<float4*>(gk8) = *reinterpret_cast<const float4*>(sgam + 2 * DH + pd0);
+        *reinterpret_cast<float4*>(gk8 + 4) = *reinterpret_cast<const float4*>(sgam + 2 * DH + pd0 + 4);
+        uint4 uq, uk, uv, ud;
+        uq.x = pack2bf(x[0][0] * iq * gq8[0], x[0][1] * iq * gq8[1]); uq.y = pack2bf(x[0][2] * iq * gq8[2], x[0][3] * iq * gq8[3]);
+        uq.z = pack2bf(x[0][4] * iq * gq8[4], x[0][5] * iq * gq8[5]); uq.w = pack2bf(x[0][6] * iq * gq8[6], x[0][7] * iq * gq8[7]);
+        uk.x = pack2bf(x[1][0] * ik * gk8[0], x[1][1] * ik * gk8[1]); uk.y = pack2bf(x[1][2] * ik * gk8[2], x[1][3] * ik * gk8[3]);
+        uk.z = pack2bf(x[1][4] * ik * gk8[4], x[1][5] * ik * gk8[5]); uk.w = pack2bf(x[1][6] * ik * gk8[6], x[1][7] * ik * gk8[7]);
+        uv.x = pack2bf(x[2][0], x[2][1]); uv.y = pack2bf(x[2][2], x[2][3]); uv.z = pack2bf(x[2][4], x[2][5]); uv.w = pack2bf(x[2][6], x[2][7]);
+        ud.x = pack2bf(x[3][0], x[3][1]); ud.y = pack2bf(x[3][2], x[3][3]); ud.z = pack2bf(x[3][4], x[3][5]); ud.w = pack2bf(x[3][6], x[3][7]);
+        *reinterpret_cast<uint4*>(sQ + i * LDQ + pd0) = uq; *reinterpret_cast<uint4*>(sK + i * LDQ + pd0) = uk;
+        *reinterpret_cast<uint4*>(sV + i * LDQ + pd0) = uv; *reinterpret_cast<uint4*>(sdO + i * LDQ + pd0) = ud;
+        if (lane % LPR == 0) { inq[i] = iq; ink[i] = ik; }
+      }
+    }
+    __syncthreads();
+    // ---------------- phase 2: my 16 query rows x 128 keys, in two halves of 64 keys
+    {
+      // scores of half h (keys 64h + 8nt + 2t + e) with the relative-position bias; pad keys -inf
+      auto scores = [&](float (&pr)[8][4], int h) {
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) pr[nt][0] = pr[nt][1] = pr[nt][2] = pr[nt][3] = 0.f;
+        warp_mma_bf16<8, DH, false, false>(pr, aQ, LDQ, r0, aK + (uint32_t)(h * 64 * LDQ * 2), LDQ, lane);
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt)
+#pragma unroll
+          for (int e = 0; e < 2; ++e) {
+            const int j = h * 64 + nt * 8 + 2 * t + e;
+            if (j < S) {
+              int oj = -1;
+              if (j >= R) { const int tj = j - R, a = tj / win, b = tj - a * win; oj = a * W2 + b; }
+              pr[nt][e] += sbias[(oj >= 0 && base_a >= 0) ? base_a - oj : nb - 1];
+              pr[nt][2 + e] += sbias[(oj >= 0 && base_b >= 0) ? base_b - oj : nb - 1];
+            } else { pr[nt][e] = -INFINITY; pr[nt][2 + e] = -INFINITY; }
+          }
+      };
+      // dropout mask * scale of key tile nt of half h: (ia, 2t), (ia, 2t+1), (ib, 2t), (ib, 2t+1)
+      auto masks = [&](float (&mk)[4], int h, int nt) {
+        mk[0] = mk[1] = mk[2] = mk[3] = 1.0f;
+        if (drop.thresh) {
+          const int grp = h * 16 + nt * 2 + (t >> 1), sh = 16 * (t & 1);
+          const uint32_t ha = drop_hash(drop.seed, drop_row(wdx, ia, SM), drop_group_prob(drop.salt, hd, grp, SM)) >> sh;
+          const uint32_t hb = drop_hash(drop.seed, drop_row(wdx, ib, SM), drop_group_prob(drop.salt, hd, grp, SM)) >> sh;
+          mk[0] = (int)(ha & 255u) >= drop.thresh ? drop.scale : 0.f; mk[1] = (int)((ha >> 8) & 255u) >= drop.thresh ? drop.scale : 0.f;
+          mk[2] = (int)(hb & 255u) >= drop.thresh ? drop.scale : 0.f; mk[3] = (int)((hb >> 8) & 255u) >= drop.thresh ? drop.scale : 0.f;
+        }
+      };
+      // pass 1: row max and sum of exp (online over the halves; the first half is all valid keys since S > 64)
+      float ma = -INFINITY, mb = -INFINITY, la = 0.f, lb = 0.f;
+#pragma unroll 1
+      for (int h = 0; h < 2; ++h) {
+        float pr[8][4];
+        scores(pr, h);
+        float xa = -INFINITY, xb = -INFINITY;
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) { xa = fmaxf(xa, fmaxf(pr[nt][0], pr[nt][1])); xb = fmaxf(xb, fmaxf(pr[nt][2], pr[nt][3])); }
+        xa = fmaxf(xa, __shfl_xor_sync(0xffffffffu, xa, 1)); xa = fmaxf(xa, __shfl_xor_sync(0xffffffffu, xa, 2));
+        xb = fmaxf(xb, __shfl_xor_sync(0xffffffffu, xb, 1)); xb = fmaxf(xb, __shfl_xor_sync(0xffffffffu, xb, 2));
+        xa = fmaxf(ma, xa); xb = fmaxf(mb, xb);
+        float sa = 0.f, sb = 0.f;
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt)
+#pragma unroll
+          for (int e = 0; e < 2; ++e) { sa += __expf(pr[nt][e] - xa); sb += __expf(pr[nt][2 + e] - xb); }
+        sa += __shfl_xor_sync(0xffffffffu, sa, 1); sa += __shfl_xor_sync(0xffffffffu, sa, 2);
+        sb += __shfl_xor_sync(0xffffffffu, sb, 1); sb += __shfl_xor_sync(0xffffffffu, sb, 2);
+        la = la * __expf(ma - xa) + sa; lb = lb * __expf(mb - xb) + sb;
+        ma = xa; mb = xb;
+      }
+      const float ia_ = ia < S ? 1.0f / la : 0.f, ib_ = ib < S ? 1.0f / lb : 0.f;      // padded query rows: P = 0
+      // pass 2: P' = P * mask -> shared memory (att and dV use it), row dot sum_j P dP' with dP' = (dO V^T) * mask
+      float da = 0.f, db = 0.f;
+#pragma unroll 1
+      for (int h = 0; h < 2; ++h) {
+        float pr[8][4], dp[8][4];
+        scores(pr, h);
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) dp[nt][0] = dp[nt][1] = dp[nt][2] = dp[nt][3] = 0.f;
+        warp_mma_bf16<8, DH, false, false>(dp, adO, LDQ, r0, aV + (uint32_t)(h * 64 * LDQ * 2), LDQ, lane);
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) {
+          float mk[4];
+          masks(mk, h, nt);
+          const float p0 = __expf(pr[nt][0] - ma) * ia_, p1 = __expf(pr[nt][1] - ma) * ia_;
+          const float p2 = __expf(pr[nt][2] - mb) * ib_, p3 = __expf(pr[nt][3] - mb) * ib_;
+          da += p0 * (dp[nt][0] * mk[0]) + p1 * (dp[nt][1] * mk[1]); db += p2 * (dp[nt][2] * mk[2]) + p3 * (dp[nt][3] * mk[3]);
+          *reinterpret_cast<uint32_t*>(sP + ia * LDP + h * 64 + nt * 8 + 2 * t) = pack2bf(p0 * mk[0], p1 * mk[1]);
+          *reinterpret_cast<uint32_t*>(sP + ib * LDP + h * 64 + nt * 8 + 2 * t) = pack2bf(p2 * mk[2], p3 * mk[3]);
+        }
+      }
+      da += __shfl_xor_sync(0xffffffffu, da, 1); da += __shfl_xor_sync(0xffffffffu, da, 2);
+      db += __shfl_xor_sync(0xffffffffu, db, 1); db += __shfl_xor_sync(0xffffffffu, db, 2);
+      // pass 3: dS = P * (dP' - rowdot) -> shared memory (bf16) and the per-pair sum (fp32)
+#pragma unroll 1
+      for (int h = 0; h < 2; ++h) {
+        float pr[8][4], dp[8][4];
+        scores(pr, h);
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) dp[nt][0] = dp[nt][1] = dp[nt][2] = dp[nt][3] = 0.f;
+        warp_mma_bf16<8, DH, false, false>(dp, adO, LDQ, r0, aV + (uint32_t)(h * 64 * LDQ * 2), LDQ, lane);
+#pragma unroll
+        for (int nt = 0; nt < 8; ++nt) {
+          float mk[4];
+          masks(mk, h, nt);
+          const float p0 = __expf(pr[nt][0] - ma) * ia_, p1 = __expf(pr[nt][1] - ma) * ia_;
+          const float p2 = __expf(pr[nt][2] - mb) * ib_, p3 = __expf(pr[nt][3] - mb) * ib_;
+          const float s0 = p0 * (dp[nt][0] * mk[0] - da), s1 = p1 * (dp[nt][1] * mk[1] - da);
+          const float s2 = p2 * (dp[nt][2] * mk[2] - db), s3 = p3 * (dp[nt][3] * mk[3] - db);
+          const int j = h * 64 + nt * 8 + 2 * t;
+          *reinterpret_cast<uint32_t*>(sDS + ia * LDP + j) = pack2bf(s0, s1);
+          *reinterpret_cast<uint32_t*>(sDS + ib * LDP + j) = pack2bf(s2, s3);
+          float2* qa = reinterpret_cast<float2*>(dsum + ia * LDS + j);
+          float2* qb = reinterpret_cast<float2*>(dsum + ib * LDS + j);
+          const float2 va = *qa, vb = *qb;                     // zero for padded rows / keys (P = 0 there)
+          *qa = make_float2(va.x + s0, va.y + s1); *qb = make_float2(vb.x + s2, vb.y + s3);
+        }
+      }
+    }
+    __syncthreads();
+    // ---------------- phase 3: rows r0..r0+15 as keys (dV, dKh) and as queries (dQh), contractions over 128 slots
+    {
+      float acc[DH / 8][4];
+#pragma unroll
+      for (int nt = 0; nt < DH / 8; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+      warp_mma_bf16<DH / 8, SM, true, true>(acc, aP, LDP, r0, adO, LDQ, lane);                 // dV[j][d] = sum_i P'[i][j] dO[i][d]
+#pragma unroll
+      for (int nt = 0; nt < DH / 8; ++nt) {
+        if (ia < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ia) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(acc[nt][0], acc[nt][1]);
+        if (ib < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ib) * 3 * inner + 2 * inner + hd * DH + nt * 8 + 2 * t)) = make_float2(acc[nt][2], acc[nt][3]);
+      }
+#pragma unroll 1
+      for (int which = 0; which < 2; ++which) {
+#pragma unroll
+        for (int nt = 0; nt < DH / 8; ++nt) acc[nt][0] = acc[nt][1] = acc[nt][2] = acc[nt][3] = 0.f;
+        if (which == 0) warp_mma_bf16<DH / 8, SM, false, true>(acc, aDS, LDP, r0, aK, LDQ, lane);   // dQh = dS Kh
+        else warp_mma_bf16<DH / 8, SM, true, true>(acc, aDS, LDP, r0, aQ, LDQ, lane);               // dKh = dS^T Qh
+        const float* inv = which == 0 ? inq : ink;
+        const bf16* sX = which == 0 ? sQ : sK;               // xh = u * rs * gamma (bf16): u = xh / (rs * gamma)
+        const float* gtab = sgam + which * 2 * DH;
+        float ua[DH / 4], ub[DH / 4], ga[DH / 4], gb[DH / 4], dota = 0.f, dotb = 0.f;
+        const float inva = inv[ia], invb = inv[ib];
+#pragma unroll
+        for (int nt = 0; nt < DH / 8; ++nt) {
+          const int d = nt * 8 + 2 * t;
+          const float2 xa = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(sX + ia * LDQ + d));
+          const float2 xb = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(sX + ib * LDQ + d));
+          const float2 gg = *reinterpret_cast<const float2*>(gtab + d), ig = *reinterpret_cast<const float2*>(gtab + DH + d);
+          ua[2 * nt] = xa.x * ig.x; ua[2 * nt + 1] = xa.y * ig.y; ub[2 * nt] = xb.x * ig.x; ub[2 * nt + 1] = xb.y * ig.y;
+          float a0 = (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs, a1 = (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
+#pragma unroll
+          for (int o = 4; o < 32; o <<= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
+          if (g == 0) { atomicAdd(&gred[which * DH + d], a0); atomicAdd(&gred[which * DH + d + 1], a1); }
+          ga[2 * nt] = acc[nt][0] * gg.x; ga[2 * nt + 1] = acc[nt][1] * gg.y;
+          gb[2 * nt] = acc[nt][2] * gg.x; gb[2 * nt + 1] = acc[nt][3] * gg.y;
+          dota += ga[2 * nt] * ua[2 * nt] + ga[2 * nt + 1] * ua[2 * nt + 1];
+          dotb += gb[2 * nt] * ub[2 * nt] + gb[2 * nt + 1] * ub[2 * nt + 1];
+        }
+        dota += __shfl_xor_sync(0xffffffffu, dota, 1); dota += __shfl_xor_sync(0xffffffffu, dota, 2);
+        dotb += __shfl_xor_sync(0xffffffffu, dotb, 1); dotb += __shfl_xor_sync(0xffffffffu, dotb, 2);
+#pragma unroll
+        for (int nt = 0; nt < DH / 8; ++nt) {
+          const int d = nt * 8 + 2 * t;
+          if (ia < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ia) * 3 * inner + which * inner + hd * DH + d)) =
+                            make_float2(inva * (ga[2 * nt] - ua[2 * nt] * dota), inva * (ga[2 * nt + 1] - ua[2 * nt + 1] * dota));
+          if (ib < S) *reinterpret_cast<float2*>(p.dqkv + ((row0 + ib) * 3 * inner + which * inner + hd * DH + d)) =
+                            make_float2(invb * (gb[2 * nt] - ub[2 * nt] * dotb), invb * (gb[2 * nt + 1] - ub[2 * nt + 1] * dotb));
+        }
+      }
+    }
+    __syncthreads();
+  }
+  // relative-position-bias gradient: the per-pair sums into the table (shared atomics once per block), then one global atomic
+  // per entry
+  for (int e = threadIdx.x; e < S * S; e += 256) {
+    const int i = e / S, j = e - i * S;
+    int bidx = nb - 1;
+    if (i >= R && j >= R) {
+      const int ti = i - R, ai = ti / win, bi = ti - ai * win, tj = j - R, aj = tj / win, bj = tj - aj * win;
+      bidx = (ai - aj + win - 1) * W2 + (bi - bj + win - 1);
+    }
+    atomicAdd(&dbias[bidx], dsum[i * LDS + j]);
+  }
+  __syncthreads();
+  if (threadIdx.x < 2 * DH) {
+    const int which = threadIdx.x / DH, d = threadIdx.x % DH;
+    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, gred[threadIdx.x]);
+  }
+  for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
+}
+
 // LayerNorm (no affine) + FiLM backward with the inverse partition (maxvit.py:176-187, 298-308, 322-332), C = 128 .. 512.
 //   tok = xhat*gamma[n] + beta[n];  dgamma[n][c] += dtok*xhat;  dbeta[n][c] += dtok;  dxhat = dtok*gamma
 //   dx = rstd*(dxhat - mean(dxhat) - xhat*mean(dxhat*xhat)) + dres   (dres = gradient of the residual path)
@@ -1464,30 +1982,33 @@ int attn_out_bwd_gather_run(const float* dx_out, const float* dreg, float reg_sc
   return check_launch("attn_out_bwd_gather_kernel");
 }
 
-// test hook: the masks as bytes
-__global__ void dropout_mask_debug_kernel(DropCfg drop, long long n_windows, int heads, int C, unsigned char* __restrict__ prob_mask,
+// test hook: the masks as bytes, for windows of `slots` (64 or 128) token slots
+__global__ void dropout_mask_debug_kernel(DropCfg drop, long long n_windows, int heads, int C, int slots, unsigned char* __restrict__ prob_mask,
                                           unsigned char* __restrict__ out_mask) {
-  const long long total_p = n_windows * heads * 64 * 16, total_o = n_windows * 64 * (C / 4);
+  const int ng = slots / 4;
+  const long long total_p = n_windows * heads * slots * ng, total_o = n_windows * slots * (C / 4);
   for (long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x; idx < total_p + total_o; idx += (long long)gridDim.x * blockDim.x) {
     if (idx < total_p) {
-      const int g = (int)(idx % 16); long long r = idx / 16;
-      const int i = (int)(r % 64); r /= 64;
+      const int g = (int)(idx % ng); long long r = idx / ng;
+      const int i = (int)(r % slots); r /= slots;
       const int h = (int)(r % heads); const long long wdx = r / heads;
-      const uint32_t hsh = drop_hash(drop.seed, drop_row(wdx, i), drop_group_prob(drop.salt, h, g));
-      for (int k = 0; k < 4; ++k) prob_mask[((wdx * heads + h) * 64 + i) * 64 + g * 4 + k] = (int)((hsh >> (8 * k)) & 255u) >= drop.thresh;
+      const uint32_t hsh = drop_hash(drop.seed, drop_row(wdx, i, slots), drop_group_prob(drop.salt, h, g, slots));
+      for (int k = 0; k < 4; ++k) prob_mask[((wdx * heads + h) * slots + i) * slots + g * 4 + k] = (int)((hsh >> (8 * k)) & 255u) >= drop.thresh;
     } else {
       const long long j = idx - total_p;
       const int g = (int)(j % (C / 4)); long long r = j / (C / 4);
-      const int i = (int)(r % 64); const long long wdx = r / 64;
-      const uint32_t hsh = drop_hash(drop.seed, drop_row(wdx, i), drop_group_out(drop.salt, g));
-      for (int k = 0; k < 4; ++k) out_mask[(wdx * 64 + i) * C + g * 4 + k] = (int)((hsh >> (8 * k)) & 255u) >= drop.thresh;
+      const int i = (int)(r % slots); const long long wdx = r / slots;
+      const uint32_t hsh = drop_hash(drop.seed, drop_row(wdx, i, slots), drop_group_out(drop.salt, g));
+      for (int k = 0; k < 4; ++k) out_mask[(wdx * slots + i) * C + g * 4 + k] = (int)((hsh >> (8 * k)) & 255u) >= drop.thresh;
     }
   }
 }
 
-int dropout_mask_debug_run(unsigned seed, unsigned salt, int drop_thresh, long long n_windows, int heads, int C, unsigned char* prob_mask,
+int dropout_mask_debug_run(unsigned seed, unsigned salt, int drop_thresh, long long n_windows, int heads, int C, int slots, unsigned char* prob_mask,
                            unsigned char* out_mask, cudaStream_t st) {
-  dropout_mask_debug_kernel<<<1024, 256, 0, st>>>(make_drop(seed, salt, drop_thresh), n_windows, heads, C, prob_mask, out_mask);
+  if (slots != 64 && slots != 128) return set_error("dropout_mask_debug: %d slots (64 or 128)", slots);
+  if (slots == 128 && heads > DROP_MAX_HEADS_LONG) return set_error("dropout_mask_debug: %d heads with 128 slots (at most %d)", heads, DROP_MAX_HEADS_LONG);
+  dropout_mask_debug_kernel<<<1024, 256, 0, st>>>(make_drop(seed, salt, drop_thresh), n_windows, heads, C, slots, prob_mask, out_mask);
   return check_launch("dropout_mask_debug_kernel");
 }
 
@@ -1525,15 +2046,49 @@ static int core_bwd_bf16_launch(const AttnCoreBwdParams& q, int nb, float* att_o
   return check_launch("attn_core_bwd_bf16_kernel");
 }
 
+// windows of 65 .. 128 tokens: one block per (field, head) and SM
+template <int DH>
+static int core_bwd_simt_long_launch(const AttnCoreBwdParams& p, int nb, const DropCfg& drop, cudaStream_t st) {
+  const size_t smem = cbs_long<DH>::bytes(nb);
+  static PerDeviceSize attr_pd;                  // depends on the window size: raise the limit when it grows
+  size_t& attr = attr_pd.cur();
+  if (smem > attr) {
+    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_long_kernel<DH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return set_error("attn_core_bwd (S > 64) smem attr: %s", cudaGetErrorString(e));
+    attr = smem;
+  }
+  attn_core_bwd_long_kernel<DH><<<p.g.N * p.heads, 256, smem, st>>>(p, drop);
+  return check_launch("attn_core_bwd_long_kernel");
+}
+
+template <int DH>
+static int core_bwd_bf16_long_launch(const AttnCoreBwdParams& q, int nb, const DropCfg& drop, cudaStream_t st) {
+  const size_t smem = (size_t)cbh_long<DH>::BYTES + (size_t)(2 * nb + 6 * DH) * sizeof(float);
+  static PerDeviceSize attr_pd;                  // depends on the window size: raise the limit when it grows
+  size_t& attr = attr_pd.cur();
+  if (smem > attr) {
+    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_bf16_long_kernel<DH>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (e != cudaSuccess) return set_error("attn_core_bwd_bf16 (S > 64) smem attr: %s", cudaGetErrorString(e));
+    attr = smem;
+  }
+  attn_core_bwd_bf16_long_kernel<DH><<<q.g.N * q.heads, 256, smem, st>>>(q, drop);
+  return check_launch("attn_core_bwd_bf16_long_kernel");
+}
+
 // use_tf32: 0 exact-fp32 SIMT, 2 bf16 mma.sync on fp32 tensors, 3 bf16 tensors (qkv, datt, dqkv, att_out): the
-// tcgen05 kernel (vg_attn_bwd_tc.cu)
+// tcgen05 kernel (vg_attn_bwd_tc.cu).  S > 64 (modes 0 and 2 only) runs the long-window kernels.
 int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                       const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
                       int use_tf32, float* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
   if (drop_thresh < 0 || drop_thresh > 255) return set_error("attn_core_bwd: dropout threshold %d outside [0, 255]", drop_thresh);
   if (use_tf32 != 0 && use_tf32 != 2 && use_tf32 != 3) return set_error("attn_core_bwd: mode %d (0 exact fp32, 2 bf16 mma on fp32 tensors, 3 bf16 tensors)", use_tf32);
   if ((use_tf32 == 3 && dh != 32) || (dh != 32 && dh != 64)) return set_error("attn_core_bwd: dim_head must be 32 (got %d)", dh);
-  if (g.S() > 64) return set_error("attn_core_bwd: sequence %d > 64", g.S());
+  const int max_s = use_tf32 == 3 ? 64 : 128;
+  if (g.S() > max_s) return set_error("attn_core_bwd: sequence %d > %d", g.S(), max_s);
+  const bool long_win = g.S() > 64;
+  if (long_win && att_out) return set_error("attn_core_bwd: att_out needs S <= 64 (got %d)", g.S());
+  if (long_win && drop_thresh && heads > DROP_MAX_HEADS_LONG)
+    return set_error("attn_core_bwd: dropout with %d heads at sequence %d > 64 (at most %d heads)", heads, g.S(), DROP_MAX_HEADS_LONG);
   const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
   if (use_tf32 == 3)
     return attn_core_bwd_tc_run(qkv, datt, qgamma, kgamma, bias_table, g, heads, dqkv, dqgamma, dkgamma, dbias_table, att_out, seed, salt,
@@ -1542,6 +2097,9 @@ int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, 
     AttnCoreBwdParams q;
     q.qkv = qkv; q.datt = datt; q.qgamma = qgamma; q.kgamma = kgamma; q.bias_table = bias_table; q.dqkv = dqkv;
     q.dqgamma = dqgamma; q.dkgamma = dkgamma; q.dbias_table = dbias_table; q.g = g; q.heads = heads;
+    if (long_win)
+      return dh == 32 ? core_bwd_bf16_long_launch<32>(q, nb, make_drop(seed, salt, drop_thresh), st)
+                      : core_bwd_bf16_long_launch<64>(q, nb, make_drop(seed, salt, drop_thresh), st);
     return dh == 32 ? core_bwd_bf16_launch<32>(q, nb, att_out, make_drop(seed, salt, drop_thresh), st)
                     : core_bwd_bf16_launch<64>(q, nb, att_out, make_drop(seed, salt, drop_thresh), st);
   }
@@ -1549,6 +2107,9 @@ int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, 
   AttnCoreBwdParams p;
   p.qkv = qkv; p.datt = datt; p.qgamma = qgamma; p.kgamma = kgamma; p.bias_table = bias_table; p.dqkv = dqkv;
   p.dqgamma = dqgamma; p.dkgamma = dkgamma; p.dbias_table = dbias_table; p.g = g; p.heads = heads;
+  if (long_win)
+    return dh == 32 ? core_bwd_simt_long_launch<32>(p, nb, make_drop(seed, salt, drop_thresh), st)
+                    : core_bwd_simt_long_launch<64>(p, nb, make_drop(seed, salt, drop_thresh), st);
   return dh == 32 ? core_bwd_simt_launch<32>(p, nb, make_drop(seed, salt, drop_thresh), st)
                   : core_bwd_simt_launch<64>(p, nb, make_drop(seed, salt, drop_thresh), st);
 }

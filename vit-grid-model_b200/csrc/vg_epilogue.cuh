@@ -492,7 +492,7 @@ __device__ __forceinline__ void epi_attn_out(const EpiParams& ep, long long row,
     const int c0 = n0 + ch * 32;
     if (c0 >= C) continue;
     if (ep.drop_thresh && ok) {                              // nn.Dropout after to_out, before the residual (maxvit.py:151, 310)
-      const uint32_t rid = drop_row(wdx, tok);
+      const uint32_t rid = drop_row(wdx, tok, drop_slots(ep.S));       // 128 slots per window when S > 64 (vg_rng.cuh)
 #pragma unroll
       for (int j = 0; j < 32; j += 4) {
         const uint32_t hsh = drop_hash(ep.drop_seed, rid, drop_group_out(ep.drop_salt, (c0 + j) >> 2));

@@ -178,7 +178,7 @@ int se_bwd_run(const float* dh4, const float* h3, const float* gate, const float
                long long work_elems, cudaStream_t st);
 int attn_out_bwd_gather_run(const float* dx_out, const float* dreg, float reg_scale, const AttnGeom& g, void* dproj, int out_bf16,
                             unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
-int dropout_mask_debug_run(unsigned seed, unsigned salt, int drop_thresh, long long n_windows, int heads, int C, unsigned char* prob_mask,
+int dropout_mask_debug_run(unsigned seed, unsigned salt, int drop_thresh, long long n_windows, int heads, int C, int slots, unsigned char* prob_mask,
                            unsigned char* out_mask, cudaStream_t st);
 int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                       const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,

@@ -306,12 +306,14 @@ def se_bwd(dh4, h3, gate, mean, hid, W1, W2, dW1, dW2):
     return dmean
 
 
-def dropout_masks(drop, n_windows, heads, C):
-    """test hook: the (prob_mask [Nw][heads][64][64], out_mask [Nw][64][C]) uint8 masks the kernels derive from drop = (seed, salt, T)"""
+def dropout_masks(drop, n_windows, heads, C, slots=64):
+    """test hook: the (prob_mask [Nw][heads][slots][slots], out_mask [Nw][slots][C]) uint8 masks the kernels derive from
+    drop = (seed, salt, T); slots = 64 for windows of up to 64 tokens, 128 for windows of 65 .. 128 tokens"""
     dev = torch.device("cuda")
-    pm = torch.empty(n_windows, heads, 64, 64, dtype=torch.uint8, device=dev)
-    om = torch.empty(n_windows, 64, C, dtype=torch.uint8, device=dev)
-    _lib.call("vg_dropout_mask_debug", int(drop[0]), int(drop[1]), int(drop[2]), n_windows, heads, C, pm.data_ptr(), om.data_ptr(), _st())
+    pm = torch.empty(n_windows, heads, slots, slots, dtype=torch.uint8, device=dev)
+    om = torch.empty(n_windows, slots, C, dtype=torch.uint8, device=dev)
+    _lib.call("vg_dropout_mask_debug", int(drop[0]), int(drop[1]), int(drop[2]), n_windows, heads, C, int(slots), pm.data_ptr(),
+              om.data_ptr(), _st())
     return pm, om
 
 
