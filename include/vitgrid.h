@@ -444,6 +444,55 @@ VG_API int vg_attn_gather_bwd(const float* x, const float* reg, int reg_per_fiel
                        float* dfilm, int N, int Hl, int Wl, int C, int win, int R, int grid_mode, float ln_eps,
                        void* stream);
 
+/* Deterministic training backward (torch.use_deterministic_algorithms): the entry points above reduce with float atomics, whose
+ * order changes from run to run.  Each _det variant computes the same quantities (same arguments, same accumulate / write
+ * semantics) but stores per-warp or per-block partial sums into fixed slots of the caller's fp32 workspace `work` of
+ * work_elems floats (size from the _workspace query) and reduces the slots in a fixed order, so two calls on the same inputs
+ * and shapes give identical bits.  The result agrees with the atomic variant to fp32 reduction-order error. */
+VG_API long long vg_conv_ln_bwd_det_workspace(int C, int N, int HP, int WP);
+/* vg_conv_ln_bwd / vg_conv_ln_bwd_wide; border (or NULL) needs an fp32 dconv (odtype 1) */
+VG_API int vg_conv_ln_bwd_det(int xdtype, int odtype, const float* dY, const void* xhat, const float* rstd, const void* relu_mask,
+                       const float* ln_g, const float* film, float ln_eps, void* dconv, float* sumA, float* sumB, float* sumD,
+                       float* border, int N, int HP, int WP, float* work, long long work_elems, void* stream);
+VG_API int vg_conv_ln_bwd_wide_det(int C, const float* dY, const float* xhat, const float* rstd, const void* relu_mask,
+                            const float* ln_g, const float* film, float ln_eps, float* dconv, float* sumA, float* sumB,
+                            float* sumD, float* border, int N, int HP, int WP, float* work, long long work_elems, void* stream);
+VG_API long long vg_head_bwd_det_workspace(int N, int HP, int WP, int C);
+VG_API int vg_head_bwd_det(int dtype, const float* dpred, const void* h, const float* w, float pm_std, int N, int HP, int WP, int C,
+                    int H, int W, int pad_top, int pad_left, float* dH, float* dw, float* db, float* work, long long work_elems,
+                    void* stream);
+VG_API long long vg_convT2_bwd_gather_det_workspace(int N, int Hl, int Wl, int C);
+VG_API int vg_convT2_bwd_gather_det(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, float* work,
+                             long long work_elems, void* stream);
+VG_API long long vg_pg_field_sum_det_workspace(int N, int HP, int WP, int C);
+VG_API int vg_pg_field_sum_det(const float* in, float* out, int N, int HP, int WP, int C, float* work, long long work_elems,
+                        void* stream);
+VG_API long long vg_time_terms_bwd_det_workspace(int N, int Cout);
+VG_API int vg_time_terms_bwd_det(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,
+                          const float* w1, int N, int ntc, int c_in, int c_data, int Cout, float* dw3, float* dw1, float* db1,
+                          float* dtemb, float* work, long long work_elems, void* stream);
+/* one thread per embedding-table element gathers its contributions in field order: no workspace (the query returns 0) */
+VG_API long long vg_time_embed_bwd_det_workspace(int B, int L, int le, int te);
+VG_API int vg_time_embed_bwd_det(const float* dtemb, const float* dcond, const float* ts, long long ts_sB, long long ts_sT,
+                          long long ts_sF, int B, int L, int le, int te, float* d_lead, float* d_month, float* d_day,
+                          float* d_hour, float* work, long long work_elems, void* stream);
+VG_API long long vg_colsum_det_workspace(long long M, int C);
+VG_API int vg_colsum_det(const float* x, long long M, int C, float* out, float* work, long long work_elems, void* stream);
+/* vg_attn_core_bwd in every mode and window it accepts (modes 0, 2 and 3; S <= 128, mode 3 S <= 64): the bias-table gradient of a
+ * block is gathered from dS (or its per-pair sums over the windows) in a fixed order, the gamma partials of its warps are summed
+ * in warp order, and each (field, head) block / tcgen05 item stores its bias-table and gamma gradients into [field][...] slots
+ * that are reduced over the fields in a fixed order. */
+VG_API long long vg_attn_core_bwd_det_workspace(int N, int Hl, int Wl, int win, int R, int heads, int dh);
+VG_API int vg_attn_core_bwd_det(const void* qkv, const void* datt, const float* q_gamma, const float* k_gamma,
+                         const float* bias_table, int N, int Hl, int Wl, int win, int R, int heads, int dh, void* dqkv,
+                         float* dq_gamma, float* dk_gamma, float* dbias_table, int use_tf32, void* att_out, long long drop_seed,
+                         int drop_salt, int drop_thresh, float* work, long long work_elems, void* stream);
+VG_API long long vg_attn_gather_bwd_det_workspace(int N, int Hl, int Wl, int C, int win, int R, int reg_per_field);
+VG_API int vg_attn_gather_bwd_det(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
+                           const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in,
+                           float* dfilm, int N, int Hl, int Wl, int C, int win, int R, int grid_mode, float ln_eps,
+                           float* work, long long work_elems, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -596,4 +596,103 @@ int vg_attn_gather_bwd(const float* x, const float* reg, int reg_per_field, cons
                              (cudaStream_t)stream);
 }
 
+// ------------------------------------------------------------------------------------------------ deterministic backward
+long long vg_conv_ln_bwd_det_workspace(int C, int N, int HP, int WP) { return conv_ln_bwd_det_workspace_elems(C, N, HP, WP); }
+
+int vg_conv_ln_bwd_det(int xdtype, int odtype, const float* dY, const void* xhat, const float* rstd, const void* relu_mask,
+                       const float* ln_g, const float* film, float ln_eps, void* dconv, float* sumA, float* sumB, float* sumD,
+                       float* border, int N, int HP, int WP, float* work, long long work_elems, void* stream) {
+  return conv_ln_bwd_det_run(128, xdtype, odtype, dY, xhat, rstd, reinterpret_cast<const unsigned*>(relu_mask), ln_g, film, ln_eps,
+                             dconv, sumA, sumB, sumD, border, N, HP, WP, work, work_elems, (cudaStream_t)stream);
+}
+
+int vg_conv_ln_bwd_wide_det(int C, const float* dY, const float* xhat, const float* rstd, const void* relu_mask,
+                            const float* ln_g, const float* film, float ln_eps, float* dconv, float* sumA, float* sumB,
+                            float* sumD, float* border, int N, int HP, int WP, float* work, long long work_elems, void* stream) {
+  if (C == 128) return set_error("conv_ln_bwd_wide_det: C=128 is vg_conv_ln_bwd_det");
+  return conv_ln_bwd_det_run(C, 1, 1, dY, xhat, rstd, reinterpret_cast<const unsigned*>(relu_mask), ln_g, film, ln_eps, dconv,
+                             sumA, sumB, sumD, border, N, HP, WP, work, work_elems, (cudaStream_t)stream);
+}
+
+long long vg_head_bwd_det_workspace(int N, int HP, int WP, int C) { return head_bwd_det_workspace_elems(N, HP, WP, C); }
+
+int vg_head_bwd_det(int dtype, const float* dpred, const void* h, const float* w, float pm_std, int N, int HP, int WP, int C,
+                    int H, int W, int pad_top, int pad_left, float* dH, float* dw, float* db, float* work, long long work_elems,
+                    void* stream) {
+  return head_bwd_det_run(dtype, dpred, h, w, pm_std, N, HP, WP, H, W, pad_top, pad_left, dH, dw, db, C, work, work_elems,
+                          (cudaStream_t)stream);
+}
+
+long long vg_convT2_bwd_gather_det_workspace(int N, int Hl, int Wl, int C) { return convT_bwd_gather_det_workspace_elems(N, Hl, Wl, C); }
+
+int vg_convT2_bwd_gather_det(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, float* work,
+                             long long work_elems, void* stream) {
+  return convT_bwd_gather_det_run(odtype, dUp, G, dbias, N, Hl, Wl, C, work, work_elems, (cudaStream_t)stream);
+}
+
+long long vg_pg_field_sum_det_workspace(int N, int HP, int WP, int C) { return pg_field_sum_det_workspace_elems(N, HP, WP, C); }
+
+int vg_pg_field_sum_det(const float* in, float* out, int N, int HP, int WP, int C, float* work, long long work_elems,
+                        void* stream) {
+  return pg_field_sum_det_run(in, out, N, HP, WP, C, work, work_elems, (cudaStream_t)stream);
+}
+
+long long vg_time_terms_bwd_det_workspace(int N, int Cout) { return time_terms_bwd_det_workspace_elems(N, Cout); }
+
+int vg_time_terms_bwd_det(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,
+                          const float* w1, int N, int ntc, int c_in, int c_data, int Cout, float* dw3, float* dw1, float* db1,
+                          float* dtemb, float* work, long long work_elems, void* stream) {
+  return time_terms_bwd_det_run(border, sumD, tres_sum, temb, w3, w1, N, ntc, c_in, c_data, Cout, dw3, dw1, db1, dtemb, work,
+                                work_elems, (cudaStream_t)stream);
+}
+
+long long vg_time_embed_bwd_det_workspace(int, int, int, int) { return 0; }
+
+int vg_time_embed_bwd_det(const float* dtemb, const float* dcond, const float* ts, long long ts_sB, long long ts_sT,
+                          long long ts_sF, int B, int L, int le, int te, float* d_lead, float* d_month, float* d_day,
+                          float* d_hour, float*, long long, void* stream) {
+  return time_embed_bwd_det_run(dtemb, dcond, ts, ts_sB, ts_sT, ts_sF, B, L, le, te, d_lead, d_month, d_day, d_hour,
+                                (cudaStream_t)stream);
+}
+
+long long vg_colsum_det_workspace(long long M, int C) { return colsum_det_workspace_elems(M, C); }
+
+int vg_colsum_det(const float* x, long long M, int C, float* out, float* work, long long work_elems, void* stream) {
+  return colsum_det_run(x, M, C, out, work, work_elems, (cudaStream_t)stream);
+}
+
+long long vg_attn_core_bwd_det_workspace(int N, int Hl, int Wl, int win, int R, int heads, int dh) {
+  AttnGeom g;
+  if (make_attn_geom(g, N, Hl, Wl, 0, win, R, 0)) return -1;
+  return attn_core_bwd_det_workspace_elems(g, heads, dh);
+}
+
+int vg_attn_core_bwd_det(const void* qkv, const void* datt, const float* q_gamma, const float* k_gamma,
+                         const float* bias_table, int N, int Hl, int Wl, int win, int R, int heads, int dh, void* dqkv,
+                         float* dq_gamma, float* dk_gamma, float* dbias_table, int use_tf32, void* att_out, long long drop_seed,
+                         int drop_salt, int drop_thresh, float* work, long long work_elems, void* stream) {
+  AttnGeom g;
+  if (make_attn_geom(g, N, Hl, Wl, 0, win, R, 0)) return 1;
+  return attn_core_bwd_det_run(reinterpret_cast<const float*>(qkv), reinterpret_cast<const float*>(datt), q_gamma, k_gamma,
+                               bias_table, g, heads, dh, reinterpret_cast<float*>(dqkv), dq_gamma, dk_gamma, dbias_table, use_tf32,
+                               reinterpret_cast<float*>(att_out), (unsigned)drop_seed, (unsigned)drop_salt, drop_thresh, work,
+                               work_elems, (cudaStream_t)stream);
+}
+
+long long vg_attn_gather_bwd_det_workspace(int N, int Hl, int Wl, int C, int win, int R, int reg_per_field) {
+  AttnGeom g;
+  if (make_attn_geom(g, N, Hl, Wl, C, win, R, 0)) return -1;
+  return attn_gather_bwd_det_workspace_elems(g, reg_per_field);
+}
+
+int vg_attn_gather_bwd_det(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
+                           const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in,
+                           float* dfilm, int N, int Hl, int Wl, int C, int win, int R, int grid_mode, float ln_eps,
+                           float* work, long long work_elems, void* stream) {
+  AttnGeom g;
+  if (make_attn_geom(g, N, Hl, Wl, C, win, R, grid_mode)) return 1;
+  return attn_gather_bwd_det_run(x, reg, reg_per_field, film, dtok, dx_out, dreg_res, reg_scale, dx_in, dreg_in, dfilm, g, ln_eps,
+                                 work, work_elems, (cudaStream_t)stream);
+}
+
 }  // extern "C"

@@ -117,8 +117,12 @@ __device__ __forceinline__ void bar_sync(int id, int n) { asm volatile("bar.sync
 
 }  // namespace
 
+// DET: the item flush stores the item's bias-table and gamma gradients into its [field][...] slots of det (det.bias [N][nb][heads],
+// det.gamma [N][2][heads*DH]) instead of global atomics; the launcher reduces the fields in a fixed order
+template <bool DET = false>
 __global__ void __launch_bounds__(ab::THREADS, 1)
-attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid_constant__ CUtensorMap mapD, const AttnBwdTcParams p) {
+attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid_constant__ CUtensorMap mapD, const AttnBwdTcParams p,
+                        const AttnDetSlots det) {
   using namespace ab;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -555,16 +559,23 @@ attn_core_bwd_tc_kernel(const __grid_constant__ CUtensorMap mapQKV, const __grid
               acc += v;
             }
           }
-        atomicAdd(p.dbias_table + ct * heads + hd, acc);
+        if constexpr (DET) det.bias[((long long)n * nb + ct) * heads + hd] = acc;
+        else atomicAdd(p.dbias_table + ct * heads + hd, acc);
       } else if (ct == nb - 1) {
         float acc = 0.f;
         for (int k = 0; k < 16; ++k) acc += wpart[k];
-        atomicAdd(p.dbias_table + ct * heads + hd, acc);
+        if constexpr (DET) det.bias[((long long)n * nb + ct) * heads + hd] = acc;
+        else atomicAdd(p.dbias_table + ct * heads + hd, acc);
       } else if (ct >= 256 && ct < 256 + DH) {
         const int d = ct - 256;
         const float dG = (gpart[d] + gpart[32 + d]) + (gpart[64 + d] + gpart[96 + d]);
-        atomicAdd(p.dqgamma + hd * DH + d, dG * rs * rs * p.kgamma[hd * DH + d]);
-        atomicAdd(p.dkgamma + hd * DH + d, dG * rs * rs * p.qgamma[hd * DH + d]);
+        if constexpr (DET) {
+          det.gamma[((long long)n * 2) * heads * DH + hd * DH + d] = dG * rs * rs * p.kgamma[hd * DH + d];
+          det.gamma[((long long)n * 2 + 1) * heads * DH + hd * DH + d] = dG * rs * rs * p.qgamma[hd * DH + d];
+        } else {
+          atomicAdd(p.dqgamma + hd * DH + d, dG * rs * rs * p.kgamma[hd * DH + d]);
+          atomicAdd(p.dkgamma + hd * DH + d, dG * rs * rs * p.qgamma[hd * DH + d]);
+        }
       }
     }
   }
@@ -603,7 +614,7 @@ static int rows_map(CUtensorMap* m, const void* base, long long cols, long long 
 
 int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                          const AttnGeom& g, int heads, void* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
-                         void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st) {
+                         void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st, const AttnDetSlots* det) {
   const int S = g.S(), nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
   if (S < 1 || S > 64) return set_error("attn_core_bwd_tc: sequence %d outside [1, 64]", S);
   if (nb > 256) return set_error("attn_core_bwd_tc: %d bias-table rows > 256 (window %d)", nb, g.win);
@@ -620,7 +631,8 @@ int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma,
   static PerDeviceFlag attr_pd;
   bool& attr = attr_pd.cur();
   if (!attr) {
-    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, ab::SMEM_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(attn_core_bwd_tc_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, ab::SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(attn_core_bwd_tc_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, ab::SMEM_BYTES);
     if (e != cudaSuccess) return set_error("attn_core_bwd_tc smem attr: %s", cudaGetErrorString(e));
     attr = true;
   }
@@ -635,7 +647,8 @@ int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma,
   p.drop.seed = seed; p.drop.salt = salt; p.drop.thresh = drop_thresh; p.drop.scale = 256.0f / (256.0f - (float)drop_thresh);
   const int items = g.N * heads;
   const int grid = items < sms ? items : sms;
-  attn_core_bwd_tc_kernel<<<grid, ab::THREADS, ab::SMEM_BYTES, st>>>(mq, md, p);
+  if (det) attn_core_bwd_tc_kernel<true><<<grid, ab::THREADS, ab::SMEM_BYTES, st>>>(mq, md, p, *det);
+  else attn_core_bwd_tc_kernel<false><<<grid, ab::THREADS, ab::SMEM_BYTES, st>>>(mq, md, p, AttnDetSlots{});
   return check_launch("attn_core_bwd_tc_kernel");
 }
 

@@ -30,7 +30,16 @@ struct ConvLnBwdParams {
   float* border;            // optional (N, 8, 128): sums of dconv over row 0, last row, col 0, last col, 4 corners
   float rstd_clamp;         // rsqrt(eps): rows whose variance was clamped have no variance gradient
   PGeom pg;
+  float* slots;             // DET: (3, N, K, C) per-(field, warp) partials of sumA / sumB / sumD (zeroed by the launcher)
+  int K;                    // DET: slots per field
 };
+
+// Fixed-order slot indices of the deterministic (DET) instantiations: the warps w that touch field n (whose PG rows are the
+// pixels [n*R*P, (n+1)*R*P)) are numbered j = w - first warp of n, so a field has at most ceil(R*P / PPW) + 1 of them.
+__host__ __device__ inline int det_field_slots(const PGeom& pg, int ppw) { return (int)(((long long)pg.R * pg.P + ppw - 1) / ppw) + 1; }
+__device__ __forceinline__ int det_field_slot(const PGeom& pg, int ppw, long long warp_global, int n) {
+  return (int)(warp_global - ((long long)n * pg.R * pg.P) / ppw);
+}
 
 // Half a warp per pixel (lane = 8 channels).  The kernel is a stream of ~1 KB rows with two 16-lane reductions each; what bounds it
 // is how many bytes a warp keeps in flight.  Every warp owns a three-stage ring in shared memory; one lane fills a stage with
@@ -47,7 +56,9 @@ __device__ __forceinline__ void bulk_g2s_b(void* dst, const void* src, uint32_t 
                ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
 }
 
-template <typename T, typename TO>
+// DET: no atomics -- each half-warp stores its partial sums of a field into slot (n, 2 * warp-of-field + half) and the launcher
+// reduces the slots in a fixed order; the border sums are left to border_sum_kernel (fp32 dconv).
+template <typename T, typename TO, bool DET = false>
 __global__ void __launch_bounds__(256) conv_ln_bwd_kernel(const ConvLnBwdParams p) {
   using namespace lnb;
   constexpr int XB = C * (int)sizeof(T), SB = stage_bytes<T>();
@@ -71,6 +82,15 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_kernel(const ConvLnBwdParams 
   int n_cur = -1;
   auto flush = [&]() {
     if (n_cur < 0) return;
+    if constexpr (DET) {
+      const int j = det_field_slot(p.pg, PPW, q_block / PPW + warp, n_cur);
+      const long long plane = (long long)p.pg.N * p.K * C;
+      float* s = p.slots + ((long long)n_cur * p.K + 2 * j + sub) * C + c0;
+      st8(s, A); st8(s + plane, B); st8(s + 2 * plane, D);
+#pragma unroll
+      for (int i = 0; i < 8; ++i) A[i] = B[i] = D[i] = 0.f;
+      return;
+    }
     float* dA = n_cur == nf0 ? &sacc[0][c0] : p.sumA + (long long)n_cur * C + c0;
     float* dB = n_cur == nf0 ? &sacc[1][c0] : p.sumB + (long long)n_cur * C + c0;
     float* dD = n_cur == nf0 ? &sacc[2][c0] : p.sumD + (long long)n_cur * C + c0;
@@ -154,7 +174,7 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_kernel(const ConvLnBwdParams 
       const float rv = valid ? rstd : 0.f;                         // pad positions: zeros
 #pragma unroll
       for (int i = 0; i < 8; ++i) { o[i] = rv * (dx[i] - s1 - x[i] * s2); D[i] += o[i]; }
-      if (p.border && valid) {
+      if (!DET && p.border && valid) {
         const bool r0 = h == 0, rl = h == HPm, k0 = w == 0, kl = w == WPm;
         if (r0 | rl | k0 | kl) {
           float* bb = p.border + (long long)n * 8 * C + c0;
@@ -178,6 +198,7 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_kernel(const ConvLnBwdParams 
     }
   }
   flush();
+  if constexpr (DET) return;
   __syncthreads();
   if (threadIdx.x < C) {
     const int c = threadIdx.x;
@@ -191,7 +212,8 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_kernel(const ConvLnBwdParams 
 // xhat / dconv.  One warp per pixel (lane owns channels v*128 + lane*4 .. +3, v < NV; ReLU mask word v*4 + lane/8 of the C/32
 // words of a pixel), 32 consecutive pixels per warp, 256 per block.  The per-field sums of the block's first field collect in
 // shared memory (most pixels of a block), the sums of any other field go to global atomics when the warp leaves the field.
-template <int NV>
+// DET: as conv_ln_bwd_kernel, one slot per (field, warp-of-field)
+template <int NV, bool DET = false>
 __global__ void __launch_bounds__(256) conv_ln_bwd_wide_kernel(const ConvLnBwdParams p) {
   constexpr int C = 128 * NV, PPW = 32, MW = C / 32;
   __shared__ float sacc[3][C];
@@ -212,6 +234,20 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_wide_kernel(const ConvLnBwdPa
   int n_cur = -1;
   auto flush = [&]() {
     if (n_cur < 0) return;
+    if constexpr (DET) {
+      const int j = det_field_slot(p.pg, PPW, q_block / PPW + warp, n_cur);
+      const long long plane = (long long)p.pg.N * p.K * C;
+      float* s = p.slots + ((long long)n_cur * p.K + j) * C + c0;
+#pragma unroll
+      for (int v = 0; v < NV; ++v) {
+        *reinterpret_cast<float4*>(s + v * 128) = make_float4(A[v][0], A[v][1], A[v][2], A[v][3]);
+        *reinterpret_cast<float4*>(s + plane + v * 128) = make_float4(B[v][0], B[v][1], B[v][2], B[v][3]);
+        *reinterpret_cast<float4*>(s + 2 * plane + v * 128) = make_float4(D[v][0], D[v][1], D[v][2], D[v][3]);
+#pragma unroll
+        for (int i = 0; i < 4; ++i) A[v][i] = B[v][i] = D[v][i] = 0.f;
+      }
+      return;
+    }
     const bool loc = n_cur == nf0;
 #pragma unroll
     for (int v = 0; v < NV; ++v)
@@ -279,7 +315,7 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_wide_kernel(const ConvLnBwdPa
       for (int v = 0; v < NV; ++v)
 #pragma unroll
         for (int i = 0; i < 4; ++i) { o[v][i] = rstd * (dx[v][i] - s1 - x[v][i] * s2); D[v][i] += o[v][i]; }
-      if (p.border) {
+      if (!DET && p.border) {
         const int h = rr_ - 1, w = col - 1;
         const bool r0 = h == 0, rl = h == HPm, k0 = w == 0, kl = w == WPm;
         if (r0 | rl | k0 | kl) {
@@ -308,6 +344,7 @@ __global__ void __launch_bounds__(256) conv_ln_bwd_wide_kernel(const ConvLnBwdPa
     if (++col == Pp) { col = 0; if (++rr_ == Rr) { rr_ = 0; ++n; } }
   }
   flush();
+  if constexpr (DET) return;
   __syncthreads();
   for (int c = threadIdx.x; c < C; c += 256) {
     if (sacc[0][c] != 0.f) atomicAdd(p.sumA + (long long)nf0 * C + c, sacc[0][c]);
@@ -346,7 +383,8 @@ __global__ void __launch_bounds__(256) conv_ln_param_grads_kernel(const float* _
 //   dH[q][c] = dpred*std*w[c] inside the window, 0 elsewhere (incl. pads);  dw[c] += dpred*std*h;  db += dpred*std
 // C = 128 * NV: lane owns channels v*128 + lane*4 .. +3 (v < NV)
 // ================================================================================================
-template <int C, typename T>
+// DET: each warp stores (dw, db) partials into slot (block * 8 + warp) of dw ([slots][C + 1]); db is unused
+template <int C, typename T, bool DET = false>
 __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__ dpred, const T* __restrict__ h, const float* __restrict__ w,
                                                        float stdv, PGeom pg, int H, int W, int pt, int pl, float* __restrict__ dH,
                                                        float* __restrict__ dw, float* __restrict__ db) {
@@ -384,16 +422,25 @@ __global__ void __launch_bounds__(256) head_bwd_kernel(const float* __restrict__
 #pragma unroll
     for (int v = 0; v < NV; ++v) *reinterpret_cast<float4*>(dH + q * C + v * 128 + c0) = o[v];
   }
+  if constexpr (DET) {
+    float* s = dw + ((long long)blockIdx.x * 8 + warp) * (C + 1);
 #pragma unroll
-  for (int v = 0; v < NV; ++v)
+    for (int v = 0; v < NV; ++v)
 #pragma unroll
-    for (int i = 0; i < 4; ++i) atomicAdd(&sw_[v * 128 + c0 + i], aw[v][i]);
-  if (lane == 0) atomicAdd(&sw_[C], ab);
-  __syncthreads();
+      for (int i = 0; i < 4; ++i) s[v * 128 + c0 + i] = aw[v][i];
+    if (lane == 0) s[C] = ab;
+  } else {
 #pragma unroll
-  for (int k = 0; k < (C + 255) / 256; ++k)
-    if (k * 256 + threadIdx.x < C) atomicAdd(dw + k * 256 + threadIdx.x, sw_[k * 256 + threadIdx.x]);
-  if (threadIdx.x == C % 256) atomicAdd(db, sw_[C]);
+    for (int v = 0; v < NV; ++v)
+#pragma unroll
+      for (int i = 0; i < 4; ++i) atomicAdd(&sw_[v * 128 + c0 + i], aw[v][i]);
+    if (lane == 0) atomicAdd(&sw_[C], ab);
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < (C + 255) / 256; ++k)
+      if (k * 256 + threadIdx.x < C) atomicAdd(dw + k * 256 + threadIdx.x, sw_[k * 256 + threadIdx.x]);
+    if (threadIdx.x == C % 256) atomicAdd(db, sw_[C]);
+  }
 }
 
 // ================================================================================================
@@ -432,7 +479,8 @@ __global__ void __launch_bounds__(256) maxpool2_bwd_kernel(const T* __restrict__
 // ConvTranspose2d(k2,s2) backward gather (metnet3.py:88-89): dUp PG (N,2Hl,2Wl,C) fp32 -> G [N*Hl*Wl][4C] in the GEMM
 // dtype, column (di*2+dj)*C + co (the forward GEMM's column order), plus dbias[co] += sum.  C = 128 * NV.
 // ================================================================================================
-template <int C, typename TO>
+// DET: each warp stores its dbias partial into slot (block * 8 + warp) of dbias ([slots][C])
+template <int C, typename TO, bool DET = false>
 __global__ void __launch_bounds__(256) convT_bwd_gather_kernel(const float* __restrict__ dUp, TO* __restrict__ G, float* __restrict__ dbias,
                                                                PGeom pg, int Hl, int Wl, long long M) {
   constexpr int PPW = 16, NV = C / 128;
@@ -463,14 +511,20 @@ __global__ void __launch_bounds__(256) convT_bwd_gather_kernel(const float* __re
       }
     }
   }
+  if constexpr (DET) {
 #pragma unroll
-  for (int u = 0; u < NV; ++u)
+    for (int u = 0; u < NV; ++u)
+      *reinterpret_cast<float4*>(dbias + ((long long)blockIdx.x * 8 + warp) * C + u * 128 + c0) = make_float4(acc[u][0], acc[u][1], acc[u][2], acc[u][3]);
+  } else {
 #pragma unroll
-    for (int i = 0; i < 4; ++i) atomicAdd(&sb[u * 128 + c0 + i], acc[u][i]);
-  __syncthreads();
+    for (int u = 0; u < NV; ++u)
 #pragma unroll
-  for (int k = 0; k < (C + 255) / 256; ++k)
-    if (k * 256 + threadIdx.x < C) atomicAdd(dbias + k * 256 + threadIdx.x, sb[k * 256 + threadIdx.x]);
+      for (int i = 0; i < 4; ++i) atomicAdd(&sb[u * 128 + c0 + i], acc[u][i]);
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < (C + 255) / 256; ++k)
+      if (k * 256 + threadIdx.x < C) atomicAdd(dbias + k * 256 + threadIdx.x, sb[k * 256 + threadIdx.x]);
+  }
 }
 
 // ================================================================================================
@@ -503,7 +557,8 @@ __global__ void __launch_bounds__(256) lead_sum_kernel(const TI* __restrict__ in
 }
 
 // per-field sums over the frame pixels of an fp32 PG tensor: out[n][c] = sum_{h,w} in[n][h][w][c].  grid (chunks, N); C = 128 * NV
-template <int C>
+// DET: each warp stores its partial into slot ((n * chunks + chunk) * 8 + warp) of out ([N][chunks * 8][C])
+template <int C, bool DET = false>
 __global__ void __launch_bounds__(256) pg_field_sum_kernel(const float* __restrict__ in, float* __restrict__ out, PGeom pg) {
   constexpr int NV = C / 128;
   __shared__ float sb[C];
@@ -524,14 +579,20 @@ __global__ void __launch_bounds__(256) pg_field_sum_kernel(const float* __restri
       a[u][0] += v.x; a[u][1] += v.y; a[u][2] += v.z; a[u][3] += v.w;
     }
   }
+  if constexpr (DET) {
 #pragma unroll
-  for (int u = 0; u < NV; ++u)
+    for (int u = 0; u < NV; ++u)
+      *reinterpret_cast<float4*>(out + (((long long)n * gridDim.x + blockIdx.x) * 8 + warp) * C + u * 128 + c0) = make_float4(a[u][0], a[u][1], a[u][2], a[u][3]);
+  } else {
 #pragma unroll
-    for (int i = 0; i < 4; ++i) atomicAdd(&sb[u * 128 + c0 + i], a[u][i]);
-  __syncthreads();
+    for (int u = 0; u < NV; ++u)
 #pragma unroll
-  for (int k = 0; k < (C + 255) / 256; ++k)
-    if (k * 256 + threadIdx.x < C) atomicAdd(out + (long long)n * C + k * 256 + threadIdx.x, sb[k * 256 + threadIdx.x]);
+      for (int i = 0; i < 4; ++i) atomicAdd(&sb[u * 128 + c0 + i], a[u][i]);
+    __syncthreads();
+#pragma unroll
+    for (int k = 0; k < (C + 255) / 256; ++k)
+      if (k * 256 + threadIdx.x < C) atomicAdd(out + (long long)n * C + k * 256 + threadIdx.x, sb[k * 256 + threadIdx.x]);
+  }
 }
 
 // ================================================================================================
@@ -583,7 +644,9 @@ __global__ void __launch_bounds__(128) time_w_bwd_kernel(const TimeBwdParams p) 
     else p.dw3[((long long)co * p.c_in + p.c_data + ct) * 9 + tap] += acc;
   }
 }
-// one block per field n: dtemb[n][ct]; thread 0.. also adds db1 (res_conv bias) = sum_n tres_sum
+// one block per field n: dtemb[n][ct]; thread 0.. also adds db1 (res_conv bias) = sum_n tres_sum (DET: left to a fixed-order
+// reduction of tres_sum over the fields)
+template <bool DET = false>
 __global__ void __launch_bounds__(128) time_emb_bwd_kernel(const TimeBwdParams p) {
   const int n = blockIdx.x;
   __shared__ float red[128];
@@ -600,7 +663,8 @@ __global__ void __launch_bounds__(128) time_emb_bwd_kernel(const TimeBwdParams p
     if (threadIdx.x == 0) p.dtemb[n * p.ntc + ct] = red[0];
     __syncthreads();
   }
-  for (int co = threadIdx.x; co < p.Cout; co += 128) atomicAdd(p.db1 + co, p.tres_sum[(long long)n * p.Cout + co]);
+  if constexpr (!DET)
+    for (int co = threadIdx.x; co < p.Cout; co += 128) atomicAdd(p.db1 + co, p.tres_sum[(long long)n * p.Cout + co]);
 }
 
 // embedding gradients (transpose of time_embed_kernel, metnet3.py:389-416): dtemb (N, le+3te) and dcond (N, le)
@@ -624,6 +688,116 @@ __global__ void time_embed_bwd_kernel(const float* __restrict__ dtemb, const flo
     const int rows = which == 0 ? 13 : (which == 1 ? 32 : 25);
     if (k < 0 || k >= rows) { if (err) atomicOr(err, VG_DEVERR_TIMESTAMP); return; }   // forward already poisoned this field
     atomicAdd(e + k * te + col, g);
+  }
+}
+
+// deterministic time_embed_bwd_kernel: one thread per output element sums its contributions in field order.
+//   lead rows l+1 (l < L): d_lead[l+1][c] += sum_b (dtemb[b*L+l][c] + dcond[b*L+l][c])
+//   table `which` (month / day / hour), row k, column col: every r = which*N + idx whose timestamp index is k contributes
+//   dtemb at flat offset f = r*te + col of the (N, 3te) model-time block (the dim-0 concat quirk of metnet3.py:395-401)
+__global__ void time_embed_bwd_det_kernel(const float* __restrict__ dtemb, const float* __restrict__ dcond, const float* __restrict__ ts,
+                                          long long ts_sB, long long ts_sT, long long ts_sF, int B, int L, int le, int te,
+                                          float* __restrict__ d_lead, float* __restrict__ d_m, float* __restrict__ d_d, float* __restrict__ d_h,
+                                          int* err) {
+  const int N = B * L, ntc = le + 3 * te, nlead = L * le;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  auto tindex = [&](int which, int idx) { return (int)ts[(long long)(idx / L) * ts_sB + 6 * ts_sT + (long long)(1 + which) * ts_sF]; };
+  if (i < nlead) {
+    const int l = i / le, c = i - l * le;
+    float acc = 0.f;
+    for (int b = 0; b < B; ++b) {
+      const int n = b * L + l;
+      acc += dtemb[n * ntc + c] + (dcond ? dcond[n * le + c] : 0.f);
+    }
+    d_lead[(l + 1) * le + c] += acc;
+    return;
+  }
+  int j = i - nlead;
+  const int nrows[3] = {13, 32, 25};
+  for (int which = 0; which < 3; ++which) {
+    if (j < nrows[which] * te) {
+      const int k = j / te, col = j - k * te;
+      float acc = 0.f;
+      for (int idx = 0; idx < N; ++idx) {
+        const int kk = tindex(which, idx);
+        if (kk < 0 || kk >= nrows[which]) { if (err && k == 0 && col == 0) atomicOr(err, VG_DEVERR_TIMESTAMP); continue; }
+        if (kk != k) continue;
+        const long long f = ((long long)which * N + idx) * te + col;
+        const int n = (int)(f / (3 * te)), c = le + (int)(f - (long long)n * 3 * te);
+        acc += dtemb[(long long)n * ntc + c];
+      }
+      float* e = which == 0 ? d_m : (which == 1 ? d_d : d_h);
+      e[k * te + col] += acc;
+      return;
+    }
+    j -= nrows[which] * te;
+  }
+}
+
+// ================================================================================================
+// Fixed-order reductions of the deterministic (_det) entry points: out[g][w] += sum_{s < S} in[g*S + s][w] (rows of ld floats).
+// A block sums the slots [z*ch, z*ch + ch) of 32 columns (eight slot lanes, then the eight lane sums in order); with more than
+// one chunk the chunk sums go to tmp and a second pass reduces them.  The order depends on S alone.
+// ================================================================================================
+__global__ void __launch_bounds__(256) slot_sum_kernel(const float* __restrict__ in, int S, int W, long long ld, int ch,
+                                                       float* __restrict__ out, long long out_ld, int accumulate) {
+  __shared__ float red[8][33];
+  const int l = threadIdx.x & 31, sl = threadIdx.x >> 5;
+  const int w = blockIdx.x * 32 + l, g = blockIdx.y, z = blockIdx.z;
+  const int s0 = z * ch, s1 = min(S, s0 + ch);
+  float a = 0.f;
+  if (w < W)
+    for (int s = s0 + sl; s < s1; s += 8) a += in[((long long)g * S + s) * ld + w];
+  red[sl][l] = a;
+  __syncthreads();
+  if (sl == 0 && w < W) {
+    float t = 0.f;
+#pragma unroll
+    for (int k = 0; k < 8; ++k) t += red[k][l];
+    float* o = out + ((long long)g * gridDim.z + z) * out_ld + w;
+    *o = accumulate ? *o + t : t;
+  }
+}
+
+static int det_chunk(long long S) { int c = 64; while ((long long)c * c < S) c *= 2; return c; }
+
+long long det_sum_tmp_elems(int G, long long S, int W) {
+  const int ch = det_chunk(S);
+  return S <= ch ? 0 : (long long)G * ((S + ch - 1) / ch) * W;
+}
+
+int det_sum_run(const float* in, int G, long long S, int W, long long ld, float* out, long long out_ld, float* tmp, cudaStream_t st) {
+  if (G <= 0 || W <= 0) return 0;
+  const int ch = det_chunk(S);
+  const unsigned gx = (unsigned)((W + 31) / 32);
+  if (S <= ch) {
+    slot_sum_kernel<<<dim3(gx, G, 1), 256, 0, st>>>(in, (int)S, W, ld, ch, out, out_ld, 1);
+    return check_launch("slot_sum_kernel");
+  }
+  const int nz = (int)((S + ch - 1) / ch);
+  slot_sum_kernel<<<dim3(gx, G, nz), 256, 0, st>>>(in, (int)S, W, ld, ch, tmp, W, 0);
+  int rc = check_launch("slot_sum_kernel");
+  if (rc) return rc;
+  slot_sum_kernel<<<dim3(gx, G, 1), 256, 0, st>>>(tmp, nz, W, W, ch, out, out_ld, 1);
+  return check_launch("slot_sum_kernel");
+}
+
+// border (N, 8, C) += the sums of an fp32 dconv PG tensor over row 0, the last row, column 0, the last column and the four corners
+// (what conv_ln_bwd_kernel accumulates with atomics), each a loop in pixel order; grid (N, 8)
+__global__ void __launch_bounds__(128) border_sum_kernel(const float* __restrict__ dconv, float* __restrict__ border, PGeom pg, int C) {
+  const int n = blockIdx.x, k = blockIdx.y;
+  for (int c = threadIdx.x; c < C; c += 128) {
+    float s = 0.f;
+    if (k < 2) {
+      const int h = k == 0 ? 0 : pg.HP - 1;
+      for (int w = 0; w < pg.WP; ++w) s += dconv[pg.q(n, h, w) * C + c];
+    } else if (k < 4) {
+      const int w = k == 2 ? 0 : pg.WP - 1;
+      for (int h = 0; h < pg.HP; ++h) s += dconv[pg.q(n, h, w) * C + c];
+    } else {
+      s = dconv[pg.q(n, (k - 4) & 2 ? pg.HP - 1 : 0, (k - 4) & 1 ? pg.WP - 1 : 0) * C + c];
+    }
+    border[((long long)n * 8 + k) * C + c] += s;
   }
 }
 
@@ -895,6 +1069,151 @@ int cond_mlp_bwd_run(const float* cond, int N, int cd, int pre_relu, const float
 int outer_sum_run(const float* G, const float* X, int N, int O, int I, float* dW, float* db, cudaStream_t st) {
   outer_sum_kernel<<<dim3((I + 31) / 32, (O + 31) / 32), 256, 0, st>>>(G, X, N, O, I, dW, db);
   return check_launch("outer_sum_kernel");
+}
+
+// ------------------------------------------------------------------------------------------------
+// deterministic variants: per-warp partials in fixed slots of the caller's workspace, then det_sum_run
+// ------------------------------------------------------------------------------------------------
+static int det_work_check(const char* what, long long need, float* work, long long work_elems) {
+  if (need > 0 && (!work || work_elems < need)) return set_error("%s: workspace too small (%lld < %lld floats)", what, work_elems, need);
+  return 0;
+}
+
+static int conv_ln_slots(int C, const PGeom& pg) { return C == 128 ? 2 * det_field_slots(pg, lnb::PPW) : det_field_slots(pg, 32); }
+
+long long conv_ln_bwd_det_workspace_elems(int C, int N, int HP, int WP) {
+  const PGeom pg = make_pgeom(N, HP, WP);
+  const int K = conv_ln_slots(C, pg);
+  return 3LL * N * K * C + det_sum_tmp_elems(N, K, C);
+}
+
+int conv_ln_bwd_det_run(int C, int xdtype, int odtype, const float* dY, const void* xhat, const float* rstd, const unsigned* mask,
+                        const float* ln_g, const float* film, float eps, void* dconv, float* sumA, float* sumB, float* sumD,
+                        float* border, int N, int HP, int WP, float* work, long long work_elems, cudaStream_t st) {
+  if (wide_c_check("conv_ln_bwd_det", C)) return 1;
+  if (border && odtype != 1) return set_error("conv_ln_bwd_det: the border sums need an fp32 dconv (odtype 1)");
+  ConvLnBwdParams p;
+  p.dY = dY; p.xhat = xhat; p.rstd = rstd; p.mask = mask; p.ln_g = ln_g; p.film = film; p.dconv = dconv;
+  p.sumA = sumA; p.sumB = sumB; p.sumD = sumD; p.border = nullptr; p.rstd_clamp = 1.0f / sqrtf(eps) * (1.0f - 1e-6f);
+  p.pg = make_pgeom(N, HP, WP);
+  p.K = conv_ln_slots(C, p.pg);
+  const long long nslots = 3LL * N * p.K * C;
+  if (det_work_check("conv_ln_bwd_det", conv_ln_bwd_det_workspace_elems(C, N, HP, WP), work, work_elems)) return 1;
+  p.slots = work;
+  float* tmp = work + nslots;
+  cudaError_t e = cudaMemsetAsync(p.slots, 0, (size_t)nslots * sizeof(float), st);
+  if (e != cudaSuccess) return set_error("conv_ln_bwd_det: %s", cudaGetErrorString(e));
+  if (C == 128) {
+    const unsigned g = nblk(p.pg.pixels(), 512);
+    if ((reinterpret_cast<uintptr_t>(dY) | reinterpret_cast<uintptr_t>(xhat) | reinterpret_cast<uintptr_t>(mask) | reinterpret_cast<uintptr_t>(rstd)) & 15)
+      return set_error("conv_ln_bwd_det: dY / xhat / mask / rstd must be 16-byte aligned");
+    const size_t sm16 = 8 * lnb::NST * lnb::stage_bytes<bf16>() + 128, sm32 = 8 * lnb::NST * lnb::stage_bytes<float>() + 128;
+    static PerDeviceFlag attr_pd;
+    bool& attr = attr_pd.cur();
+    if (!attr) {
+      cudaError_t e2 = cudaFuncSetAttribute(conv_ln_bwd_kernel<bf16, bf16, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm16);
+      if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(conv_ln_bwd_kernel<bf16, float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm16);
+      if (e2 == cudaSuccess) e2 = cudaFuncSetAttribute(conv_ln_bwd_kernel<float, float, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sm32);
+      if (e2 != cudaSuccess) return set_error("conv_ln_bwd_det smem attr: %s", cudaGetErrorString(e2));
+      attr = true;
+    }
+    if (xdtype == 0 && odtype == 0) conv_ln_bwd_kernel<bf16, bf16, true><<<g, 256, sm16, st>>>(p);
+    else if (xdtype == 0 && odtype == 1) conv_ln_bwd_kernel<bf16, float, true><<<g, 256, sm16, st>>>(p);
+    else if (xdtype == 1 && odtype == 1) conv_ln_bwd_kernel<float, float, true><<<g, 256, sm32, st>>>(p);
+    else return set_error("conv_ln_bwd_det: unsupported dtype combination (%d, %d)", xdtype, odtype);
+  } else {
+    const unsigned g = nblk(p.pg.pixels(), 256);
+    VG_WIDTH_SWITCH(C, (conv_ln_bwd_wide_kernel<CW / 128, true><<<g, 256, 0, st>>>(p)));
+  }
+  int rc = check_launch("conv_ln_bwd_kernel (det)");
+  float* outs[3] = {sumA, sumB, sumD};
+  for (int k = 0; k < 3 && !rc; ++k) rc = det_sum_run(p.slots + k * (nslots / 3), N, p.K, C, C, outs[k], C, tmp, st);
+  if (rc || !border) return rc;
+  border_sum_kernel<<<dim3(N, 8), 128, 0, st>>>(reinterpret_cast<const float*>(dconv), border, p.pg, C);
+  return check_launch("border_sum_kernel");
+}
+
+static long long head_warps(const PGeom& pg) { return (long long)nblk(pg.pixels(), 256) * 8; }
+
+long long head_bwd_det_workspace_elems(int N, int HP, int WP, int C) {
+  const long long S = head_warps(make_pgeom(N, HP, WP));
+  return S * (C + 1) + det_sum_tmp_elems(1, S, C);
+}
+
+int head_bwd_det_run(int dtype, const float* dpred, const void* h, const float* w, float stdv, int N, int HP, int WP, int H, int W,
+                     int pt, int pl, float* dH, float* dw, float* db, int C, float* work, long long work_elems, cudaStream_t st) {
+  if (wide_c_check("head_bwd_det", C)) return 1;
+  if (det_work_check("head_bwd_det", head_bwd_det_workspace_elems(N, HP, WP, C), work, work_elems)) return 1;
+  PGeom pg = make_pgeom(N, HP, WP);
+  const unsigned g = nblk(pg.pixels(), 256);
+  const long long S = head_warps(pg);
+  float* tmp = work + S * (C + 1);
+  if (dtype == 0) VG_WIDTH_SWITCH(C, (head_bwd_kernel<CW, bf16, true><<<g, 256, 0, st>>>(dpred, reinterpret_cast<const bf16*>(h), w, stdv, pg, H, W, pt, pl, dH, work, nullptr)))
+  else VG_WIDTH_SWITCH(C, (head_bwd_kernel<CW, float, true><<<g, 256, 0, st>>>(dpred, reinterpret_cast<const float*>(h), w, stdv, pg, H, W, pt, pl, dH, work, nullptr)))
+  int rc = check_launch("head_bwd_kernel (det)");
+  if (!rc) rc = det_sum_run(work, 1, S, C, C + 1, dw, C, tmp, st);
+  if (!rc) rc = det_sum_run(work + C, 1, S, 1, C + 1, db, 1, tmp, st);
+  return rc;
+}
+
+long long convT_bwd_gather_det_workspace_elems(int N, int Hl, int Wl, int C) {
+  const long long S = (long long)nblk((long long)N * Hl * Wl, 8 * 16) * 8;
+  return S * C + det_sum_tmp_elems(1, S, C);
+}
+
+int convT_bwd_gather_det_run(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, float* work,
+                             long long work_elems, cudaStream_t st) {
+  if (wide_c_check("convT_bwd_gather_det", C)) return 1;
+  if (det_work_check("convT_bwd_gather_det", convT_bwd_gather_det_workspace_elems(N, Hl, Wl, C), work, work_elems)) return 1;
+  PGeom pg = make_pgeom(N, 2 * Hl, 2 * Wl);
+  const long long M = (long long)N * Hl * Wl;
+  const unsigned g = nblk(M, 8 * 16);
+  const long long S = (long long)g * 8;
+  if (odtype == 0) VG_WIDTH_SWITCH(C, (convT_bwd_gather_kernel<CW, bf16, true><<<g, 256, 0, st>>>(dUp, reinterpret_cast<bf16*>(G), work, pg, Hl, Wl, M)))
+  else VG_WIDTH_SWITCH(C, (convT_bwd_gather_kernel<CW, float, true><<<g, 256, 0, st>>>(dUp, reinterpret_cast<float*>(G), work, pg, Hl, Wl, M)))
+  int rc = check_launch("convT_bwd_gather_kernel (det)");
+  return rc ? rc : det_sum_run(work, 1, S, C, C, dbias, C, work + S * C, st);
+}
+
+static int field_sum_chunks(int HP, int WP) { int c = (HP * WP + 255) / 256; return c > 32 ? 32 : c; }
+
+long long pg_field_sum_det_workspace_elems(int N, int HP, int WP, int C) {
+  const long long S = (long long)field_sum_chunks(HP, WP) * 8;
+  return (long long)N * S * C + det_sum_tmp_elems(N, S, C);
+}
+
+int pg_field_sum_det_run(const float* in, float* out, int N, int HP, int WP, int C, float* work, long long work_elems, cudaStream_t st) {
+  if (wide_c_check("pg_field_sum_det", C)) return 1;
+  if (det_work_check("pg_field_sum_det", pg_field_sum_det_workspace_elems(N, HP, WP, C), work, work_elems)) return 1;
+  PGeom pg = make_pgeom(N, HP, WP);
+  const int chunks = field_sum_chunks(HP, WP);
+  VG_WIDTH_SWITCH(C, (pg_field_sum_kernel<CW, true><<<dim3(chunks, N), 256, 0, st>>>(in, work, pg)));
+  int rc = check_launch("pg_field_sum_kernel (det)");
+  return rc ? rc : det_sum_run(work, N, chunks * 8, C, C, out, C, work + (long long)N * chunks * 8 * C, st);
+}
+
+long long time_terms_bwd_det_workspace_elems(int N, int Cout) { return det_sum_tmp_elems(1, N, Cout); }
+
+int time_terms_bwd_det_run(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,
+                           const float* w1, int N, int ntc, int c_in, int c_data, int Cout, float* dw3, float* dw1, float* db1,
+                           float* dtemb, float* work, long long work_elems, cudaStream_t st) {
+  if (det_work_check("time_terms_bwd_det", time_terms_bwd_det_workspace_elems(N, Cout), work, work_elems)) return 1;
+  TimeBwdParams p;
+  p.border = border; p.sumD = sumD; p.tres_sum = tres_sum; p.temb = temb; p.w3 = w3; p.w1 = w1;
+  p.dw3 = dw3; p.dw1 = dw1; p.dtemb = dtemb; p.db1 = db1; p.N = N; p.ntc = ntc; p.c_in = c_in; p.c_data = c_data; p.Cout = Cout;
+  time_w_bwd_kernel<<<Cout * 10, 128, (size_t)N * sizeof(float), st>>>(p);
+  int rc = check_launch("time_w_bwd_kernel");
+  if (rc) return rc;
+  time_emb_bwd_kernel<true><<<N, 128, 0, st>>>(p);
+  rc = check_launch("time_emb_bwd_kernel (det)");
+  return rc ? rc : det_sum_run(tres_sum, 1, N, Cout, Cout, db1, Cout, work, st);
+}
+
+int time_embed_bwd_det_run(const float* dtemb, const float* dcond, const float* ts, long long sB, long long sT, long long sF, int B,
+                           int L, int le, int te, float* d_lead, float* d_m, float* d_d, float* d_h, cudaStream_t st) {
+  const long long total = (long long)L * le + 70LL * te;
+  time_embed_bwd_det_kernel<<<nblk(total, 128), 128, 0, st>>>(dtemb, dcond, ts, sB, sT, sF, B, L, le, te, d_lead, d_m, d_d, d_h, device_error_ptr());
+  return check_launch("time_embed_bwd_det_kernel");
 }
 
 int adamw_run(float* p, const float* g, float* m, float* v, long long n, float lr, float b1, float b2, float eps, float wd,

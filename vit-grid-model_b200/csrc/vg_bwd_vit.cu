@@ -246,7 +246,8 @@ __global__ void __launch_bounds__(256) partial_sum_kernel(const float* __restric
   }
 }
 
-// column sums of X fp32 [M][C] accumulated into out[C] (bias gradients)
+// column sums of X fp32 [M][C] accumulated into out[C] (bias gradients); DET: block b stores its sums into row b of out
+template <bool DET = false>
 __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ X, long long M, int C, float* __restrict__ out) {
   const long long r0 = (long long)blockIdx.x * STAT_ROWS;
   long long r1 = r0 + STAT_ROWS;
@@ -254,7 +255,8 @@ __global__ void __launch_bounds__(256) colsum_kernel(const float* __restrict__ X
   for (int c = threadIdx.x; c < C; c += 256) {
     float s = 0.f;
     for (long long r = r0; r < r1; ++r) s += X[r * C + c];
-    atomicAdd(out + c, s);
+    if constexpr (DET) out[(long long)blockIdx.x * C + c] = s;
+    else atomicAdd(out + c, s);
   }
 }
 
@@ -620,6 +622,37 @@ struct AttnCoreBwdParams {
   int heads;
 };
 
+
+// Deterministic bias-table gradient of one window (the DET kernels): dbias[b] += sum of dS[i][j] over the (i, j) pairs of
+// relative-position index b, in (i, j) order.  Index b < nb-1 is the offset (ai - aj, bi - bj) of two window tokens; nb-1 is
+// every pair with a register token.  dS: [S][ld] in shared memory; thread tid of nthreads.
+// Query rows i0 .. i0+ni-1 only (dS row i - i0 holds query i): the long-window kernels hold dS one block of query rows at a time.
+__device__ __forceinline__ void dbias_gather(const float* dS, int ld, const AttnGeom& g, int nb, float* dbias, int tid, int nthreads,
+                                             int i0 = 0, int ni = 1 << 30) {
+  const int S = g.S(), w = g.win, W2 = 2 * w - 1, R = g.R, i1 = min(S, i0 + ni);
+  for (int b = tid; b < nb; b += nthreads) {
+    float acc = 0.f;
+    if (b < nb - 1) {
+      const int da = b / W2 - (w - 1), db = b % W2 - (w - 1);
+      for (int ai = max(0, da); ai < min(w, w + da); ++ai)
+        for (int bi = max(0, db); bi < min(w, w + db); ++bi) {
+          const int i = R + ai * w + bi;
+          if (i >= i0 && i < i1) acc += dS[(i - i0) * ld + R + (ai - da) * w + (bi - db)];
+        }
+    } else {
+      for (int i = i0; i < i1; ++i)
+        for (int j = 0; j < (i < R ? S : R); ++j) acc += dS[(i - i0) * ld + j];
+    }
+    dbias[b] += acc;
+  }
+}
+
+// the block's bias-table gradient into its field's slots (DET kernels)
+__device__ __forceinline__ void det_flush_bias(const AttnDetSlots& det, const float* dbias, int n, int nb, int heads, int hd, int tid,
+                                               int nthreads) {
+  for (int i = tid; i < nb; i += nthreads) det.bias[((long long)n * nb + i) * heads + hd] = dbias[i];
+}
+
 // sum_k a[k] b[k] of one lane's values
 template <int K>
 __device__ __forceinline__ float lane_dot(const float (&a)[K], const float (&b)[K]) {
@@ -629,8 +662,10 @@ __device__ __forceinline__ float lane_dot(const float (&a)[K], const float (&b)[
   return r;
 }
 
-template <int DH>
-__global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdParams p, const DropCfg drop) {
+// DET: the bias-table gradient of a window is gathered from dS in a fixed order (dbias_gather) and the block's gamma / bias
+// gradients go to its field's slots (det_gamma, det_bias) instead of global atomics
+template <int DH, bool DET = false>
+__global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdParams p, const DropCfg drop, const AttnDetSlots det) {
   constexpr int LD = DH + 1, SM = 64, DPL = DH / 32;        // DPL head dims per lane: d = lane + 32*k
   extern __shared__ float sm[];
   const AttnGeom g = p.g;
@@ -760,13 +795,16 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
         if (j < S) {
           const float ds = pr[t] * (dp[t] - dot);
           P[i * (SM + 1) + j] = ds;
-          int bidx = nb - 1;
-          if (i >= g.R && j >= g.R) { const int tj = j - g.R, aj = tj / g.win, bj = tj - aj * g.win; bidx = (ai - aj + g.win - 1) * W2 + (bi - bj + g.win - 1); }
-          atomicAdd(&dbias[bidx], ds);
+          if constexpr (!DET) {
+            int bidx = nb - 1;
+            if (i >= g.R && j >= g.R) { const int tj = j - g.R, aj = tj / g.win, bj = tj - aj * g.win; bidx = (ai - aj + g.win - 1) * W2 + (bi - bj + g.win - 1); }
+            atomicAdd(&dbias[bidx], ds);
+          }
         }
       }
     }
     __syncthreads();
+    if constexpr (DET) dbias_gather(P, SM + 1, g, nb, dbias, threadIdx.x, 256);
     // ---- dqh[i][d] = sum_j dS[i][j] kh[j][d];  dkh[j][d] = sum_i dS[i][j] qh[i][d]
     for (int i = warp; i < S; i += 8) {
       float a[DPL], b[DPL];
@@ -810,9 +848,14 @@ __global__ void __launch_bounds__(256) attn_core_bwd_kernel(const AttnCoreBwdPar
     const int which = threadIdx.x / DH, d = threadIdx.x % DH;
     float s = 0.f;
     for (int w = 0; w < 8; ++w) s += gred[(w * 2 + which) * DH + d];
-    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, s);
+    if constexpr (DET) det.gamma[((long long)n * 2 + which) * inner + hd * DH + d] = s;
+    else atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, s);
   }
-  for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
+  if constexpr (DET) {
+    for (int i = threadIdx.x; i < nb; i += 256) det.bias[((long long)n * nb + i) * p.heads + hd] = dbias[i];
+  } else {
+    for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -877,8 +920,11 @@ __device__ __forceinline__ uint32_t pack2bf(float a, float b) {
 }
 
 // DH 64: two blocks per SM (the 64-wide accumulators do not fit the three-block register cap; at 255 registers 20 bytes still spill)
-template <int DH_>
-__global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_kernel(const AttnCoreBwdParams p, float* __restrict__ att_out, const DropCfg drop) {
+// DET (dynamic shared memory grows by 8*DH + 64*65 floats after sgam): the four warps' gamma partials go to per-warp rows gw
+// summed in warp order, and each thread's per-pair bias gradients to a [64][65] pair table that dbias_gather reduces
+template <int DH_, bool DET = false>
+__global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_kernel(const AttnCoreBwdParams p, float* __restrict__ att_out, const DropCfg drop,
+                                                                                    const AttnDetSlots det) {
   using K = cbh<DH_>;
   constexpr int DH = K::DH, SM = K::SM, LDQ = K::LDQ, LDP = K::LDP, LPR = K::LPR, PASSES = K::PASSES;
   extern __shared__ __align__(16) uint8_t smraw[];
@@ -915,6 +961,9 @@ __global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_ker
   if (ib >= R && ib < S) { const int ti = ib - R, a = ti / win, b = ti - a * win; base_b = (a + win - 1) * W2 + (b + win - 1); }
   float bsa[16], bsb[16];                 // bias of this thread's 32 fixed (query, key) pairs (head-specific, window-independent)
   float dba[16], dbb[16];                 // and its gradient, summed over the windows
+  float* gw = sgam + 4 * DH;              // DET: [4 warps][2][DH]
+  if constexpr (DET)
+    for (int i = threadIdx.x; i < 8 * DH; i += 128) gw[i] = 0.f;
   __syncthreads();
 #pragma unroll
   for (int k = 0; k < 16; ++k) {
@@ -1107,7 +1156,10 @@ __global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_ker
             float a0 = (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs, a1 = (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
 #pragma unroll
             for (int o = 4; o < 32; o <<= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
-            if (g == 0) { atomicAdd(&gred[which * DH + d], a0); atomicAdd(&gred[which * DH + d + 1], a1); }
+            if (g == 0) {
+              if constexpr (DET) { gw[warp * 2 * DH + which * DH + d] += a0; gw[warp * 2 * DH + which * DH + d + 1] += a1; }
+              else { atomicAdd(&gred[which * DH + d], a0); atomicAdd(&gred[which * DH + d + 1], a1); }
+            }
           }
           ga[2 * nt] = acc[nt][0] * gg.x; ga[2 * nt + 1] = acc[nt][1] * gg.y;
           gb[2 * nt] = acc[nt][2] * gg.x; gb[2 * nt + 1] = acc[nt][3] * gg.y;
@@ -1129,14 +1181,20 @@ __global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_ker
     __syncthreads();
   }
   // relative-position-bias gradient: one shared-memory atomic per (thread, pair) per BLOCK, then one global atomic per entry
+  float* pairs = gw + 8 * DH;             // DET: [64][65] per-pair sums over the windows
 #pragma unroll
   for (int k = 0; k < 16; ++k) {
     const int j = (k >> 1) * 8 + 2 * t + (k & 1);
     if (j < S) {
-      int oj = -1;
-      if (j >= R) { const int tj = j - R, a = tj / win, b = tj - a * win; oj = a * W2 + b; }
-      if (ia < S) atomicAdd(&dbias[(oj >= 0 && base_a >= 0) ? base_a - oj : nb - 1], dba[k]);
-      if (ib < S) atomicAdd(&dbias[(oj >= 0 && base_b >= 0) ? base_b - oj : nb - 1], dbb[k]);
+      if constexpr (DET) {
+        if (ia < S) pairs[ia * 65 + j] = dba[k];
+        if (ib < S) pairs[ib * 65 + j] = dbb[k];
+      } else {
+        int oj = -1;
+        if (j >= R) { const int tj = j - R, a = tj / win, b = tj - a * win; oj = a * W2 + b; }
+        if (ia < S) atomicAdd(&dbias[(oj >= 0 && base_a >= 0) ? base_a - oj : nb - 1], dba[k]);
+        if (ib < S) atomicAdd(&dbias[(oj >= 0 && base_b >= 0) ? base_b - oj : nb - 1], dbb[k]);
+      }
     }
   }
 #pragma unroll
@@ -1146,15 +1204,26 @@ __global__ void __launch_bounds__(128, DH_ == 32 ? 3 : 2) attn_core_bwd_bf16_ker
     b += __shfl_xor_sync(0xffffffffu, b, 4); b += __shfl_xor_sync(0xffffffffu, b, 8); b += __shfl_xor_sync(0xffffffffu, b, 16);
     if (g == 0) {
       const int d = (k >> 1) * 8 + 2 * t + (k & 1);
-      atomicAdd(&gred[d], a); atomicAdd(&gred[DH + d], b);
+      if constexpr (DET) { gw[warp * 2 * DH + d] += a; gw[warp * 2 * DH + DH + d] += b; }
+      else { atomicAdd(&gred[d], a); atomicAdd(&gred[DH + d], b); }
     }
   }
   __syncthreads();
-  if (threadIdx.x < 2 * DH) {
-    const int which = threadIdx.x / DH, d = threadIdx.x % DH;
-    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, gred[threadIdx.x]);
+  if constexpr (DET) {
+    dbias_gather(pairs, 65, g_, nb, dbias, threadIdx.x, 128);
+    if (threadIdx.x < 2 * DH) {
+      const int which = threadIdx.x / DH, d = threadIdx.x % DH;
+      det.gamma[((long long)n * 2 + which) * inner + hd * DH + d] =
+          (gw[threadIdx.x] + gw[2 * DH + threadIdx.x]) + (gw[4 * DH + threadIdx.x] + gw[6 * DH + threadIdx.x]);
+    }
+    det_flush_bias(det, dbias, n, nb, p.heads, hd, threadIdx.x, 128);
+  } else {
+    if (threadIdx.x < 2 * DH) {
+      const int which = threadIdx.x / DH, d = threadIdx.x % DH;
+      atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, gred[threadIdx.x]);
+    }
+    for (int i = threadIdx.x; i < nb; i += 128) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
   }
-  for (int i = threadIdx.x; i < nb; i += 128) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -1173,8 +1242,9 @@ struct cbs_long {
   static size_t bytes(int nb) { return (size_t)(4 * SK * LD + 3 * QB * LD + 2 * QB * LP + 2 * nb + SK + QB + 8 * 2 * DH) * sizeof(float); }
 };
 
-template <int DH>
-__global__ void __launch_bounds__(256, 1) attn_core_bwd_long_kernel(const AttnCoreBwdParams p, const DropCfg drop) {
+// DET: as attn_core_bwd_kernel, the bias-table gradient gathered per block of query rows (dbias_gather over rows q0 ..)
+template <int DH, bool DET = false>
+__global__ void __launch_bounds__(256, 1) attn_core_bwd_long_kernel(const AttnCoreBwdParams p, const DropCfg drop, const AttnDetSlots det) {
   using L = cbs_long<DH>;
   constexpr int SK = L::SK, QB = L::QB, LD = L::LD, LP = L::LP, DPL = DH / 32;
   extern __shared__ float sm[];
@@ -1317,13 +1387,16 @@ __global__ void __launch_bounds__(256, 1) attn_core_bwd_long_kernel(const AttnCo
           if (j < S) {
             const float ds = pr[t] * (dp[t] - dot);
             P[r * LP + j] = ds;
-            int bidx = nb - 1;
-            if (i >= g.R && j >= g.R) { const int tj = j - g.R, aj = tj / g.win, bj = tj - aj * g.win; bidx = (ai - aj + g.win - 1) * W2 + (bi - bj + g.win - 1); }
-            atomicAdd(&dbias[bidx], ds);
+            if constexpr (!DET) {
+              int bidx = nb - 1;
+              if (i >= g.R && j >= g.R) { const int tj = j - g.R, aj = tj / g.win, bj = tj - aj * g.win; bidx = (ai - aj + g.win - 1) * W2 + (bi - bj + g.win - 1); }
+              atomicAdd(&dbias[bidx], ds);
+            }
           }
         }
       }
       __syncthreads();
+      if constexpr (DET) dbias_gather(P, LP, g, nb, dbias, threadIdx.x, 256, q0, nq);
       // ---- dK-hat[j] += sum_i dS[i][j] qh[i] (warp per key); dQ-hat[i] = sum_j dS[i][j] kh[j] (warp per query row), then the
       // RMSNorm backward of q (maxvit.py:30): qh = u * rs * gamma, u = q/|q|
       for (int j = warp; j < S; j += 8) {
@@ -1385,9 +1458,12 @@ __global__ void __launch_bounds__(256, 1) attn_core_bwd_long_kernel(const AttnCo
     const int which = threadIdx.x / DH, d = threadIdx.x % DH;
     float s = 0.f;
     for (int w = 0; w < 8; ++w) s += gred[(w * 2 + which) * DH + d];
-    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, s);
+    if constexpr (DET) det.gamma[((long long)n * 2 + which) * inner + hd * DH + d] = s;
+    else atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, s);
   }
-  for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
+  if constexpr (DET) det_flush_bias(det, dbias, n, nb, p.heads, hd, threadIdx.x, 256);
+  else
+    for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
 }
 
 // Mode 2 (bf16 mma.sync on fp32 tensors): the layout of attn_core_bwd_bf16_kernel at 128 slots, 8 warps of 16 query rows, one
@@ -1407,8 +1483,10 @@ struct cbh_long {
   static constexpr int PASSES = 16 / (32 / LPR);
 };
 
-template <int DH_>
-__global__ void __launch_bounds__(256, 1) attn_core_bwd_bf16_long_kernel(const AttnCoreBwdParams p, const DropCfg drop) {
+// DET (dynamic shared memory grows by 16*DH floats after sgam): per-warp gamma rows gw summed in warp order, the bias table
+// gathered from dsum by dbias_gather
+template <int DH_, bool DET = false>
+__global__ void __launch_bounds__(256, 1) attn_core_bwd_bf16_long_kernel(const AttnCoreBwdParams p, const DropCfg drop, const AttnDetSlots det) {
   using K = cbh_long<DH_>;
   constexpr int DH = K::DH, SM = K::SM, LDQ = K::LDQ, LDP = K::LDP, LDS = K::LDS, LPR = K::LPR, PASSES = K::PASSES;
   extern __shared__ __align__(16) uint8_t smraw[];
@@ -1441,6 +1519,9 @@ __global__ void __launch_bounds__(256, 1) attn_core_bwd_bf16_long_kernel(const A
   int base_a = -1, base_b = -1;
   if (ia >= R && ia < S) { const int ti = ia - R, a = ti / win, b = ti - a * win; base_a = (a + win - 1) * W2 + (b + win - 1); }
   if (ib >= R && ib < S) { const int ti = ib - R, a = ti / win, b = ti - a * win; base_b = (a + win - 1) * W2 + (b + win - 1); }
+  float* gw = sgam + 4 * DH;              // DET: [8 warps][2][DH]
+  if constexpr (DET)
+    for (int i = threadIdx.x; i < 16 * DH; i += 256) gw[i] = 0.f;
   __syncthreads();
 
   for (int wi = 0; wi < nwin; ++wi) {
@@ -1636,7 +1717,10 @@ __global__ void __launch_bounds__(256, 1) attn_core_bwd_bf16_long_kernel(const A
           float a0 = (acc[nt][0] * ua[2 * nt] + acc[nt][2] * ub[2 * nt]) * rs, a1 = (acc[nt][1] * ua[2 * nt + 1] + acc[nt][3] * ub[2 * nt + 1]) * rs;
 #pragma unroll
           for (int o = 4; o < 32; o <<= 1) { a0 += __shfl_xor_sync(0xffffffffu, a0, o); a1 += __shfl_xor_sync(0xffffffffu, a1, o); }
-          if (g == 0) { atomicAdd(&gred[which * DH + d], a0); atomicAdd(&gred[which * DH + d + 1], a1); }
+          if (g == 0) {
+            if constexpr (DET) { gw[warp * 2 * DH + which * DH + d] += a0; gw[warp * 2 * DH + which * DH + d + 1] += a1; }
+            else { atomicAdd(&gred[which * DH + d], a0); atomicAdd(&gred[which * DH + d + 1], a1); }
+          }
           ga[2 * nt] = acc[nt][0] * gg.x; ga[2 * nt + 1] = acc[nt][1] * gg.y;
           gb[2 * nt] = acc[nt][2] * gg.x; gb[2 * nt + 1] = acc[nt][3] * gg.y;
           dota += ga[2 * nt] * ua[2 * nt] + ga[2 * nt + 1] * ua[2 * nt + 1];
@@ -1658,21 +1742,32 @@ __global__ void __launch_bounds__(256, 1) attn_core_bwd_bf16_long_kernel(const A
   }
   // relative-position-bias gradient: the per-pair sums into the table (shared atomics once per block), then one global atomic
   // per entry
-  for (int e = threadIdx.x; e < S * S; e += 256) {
-    const int i = e / S, j = e - i * S;
-    int bidx = nb - 1;
-    if (i >= R && j >= R) {
-      const int ti = i - R, ai = ti / win, bi = ti - ai * win, tj = j - R, aj = tj / win, bj = tj - aj * win;
-      bidx = (ai - aj + win - 1) * W2 + (bi - bj + win - 1);
+  if constexpr (DET) {
+    dbias_gather(dsum, LDS, g_, nb, dbias, threadIdx.x, 256);
+    if (threadIdx.x < 2 * DH) {
+      const int which = threadIdx.x / DH, d = threadIdx.x % DH;
+      float s = 0.f;
+      for (int w = 0; w < 8; ++w) s += gw[w * 2 * DH + threadIdx.x];
+      det.gamma[((long long)n * 2 + which) * inner + hd * DH + d] = s;
     }
-    atomicAdd(&dbias[bidx], dsum[i * LDS + j]);
+    det_flush_bias(det, dbias, n, nb, p.heads, hd, threadIdx.x, 256);
+  } else {
+    for (int e = threadIdx.x; e < S * S; e += 256) {
+      const int i = e / S, j = e - i * S;
+      int bidx = nb - 1;
+      if (i >= R && j >= R) {
+        const int ti = i - R, ai = ti / win, bi = ti - ai * win, tj = j - R, aj = tj / win, bj = tj - aj * win;
+        bidx = (ai - aj + win - 1) * W2 + (bi - bj + win - 1);
+      }
+      atomicAdd(&dbias[bidx], dsum[i * LDS + j]);
+    }
+    __syncthreads();
+    if (threadIdx.x < 2 * DH) {
+      const int which = threadIdx.x / DH, d = threadIdx.x % DH;
+      atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, gred[threadIdx.x]);
+    }
+    for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
   }
-  __syncthreads();
-  if (threadIdx.x < 2 * DH) {
-    const int which = threadIdx.x / DH, d = threadIdx.x % DH;
-    atomicAdd((which ? p.dkgamma : p.dqgamma) + hd * DH + d, gred[threadIdx.x]);
-  }
-  for (int i = threadIdx.x; i < nb; i += 256) atomicAdd(p.dbias_table + i * p.heads + hd, dbias[i]);
 }
 
 // LayerNorm (no affine) + FiLM backward with the inverse partition (maxvit.py:176-187, 298-308, 322-332), C = 128 .. 512.
@@ -1687,8 +1782,9 @@ struct AttnGatherBwdParams {
   AttnGeom g; float eps;
 };
 
-template <int C>
-__global__ void __launch_bounds__(256) attn_gather_bwd_kernel(const AttnGatherBwdParams p, long long rows) {
+// DET: dfilm partials go to slot (n, warp - first warp of field n) of det_film, register rows to their window's row of det_reg
+template <int C, bool DET = false>
+__global__ void __launch_bounds__(256) attn_gather_bwd_kernel(const AttnGatherBwdParams p, long long rows, const AttnDetSlots det) {
   constexpr int RPW = 16, NV = C / 128, NE = 4 * NV;
   const AttnGeom g = p.g;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, c0 = lane * 4;
@@ -1699,14 +1795,27 @@ __global__ void __launch_bounds__(256) attn_gather_bwd_kernel(const AttnGatherBw
   int n_cur = -1;
   auto flush = [&]() {
     if (n_cur < 0) return;
+    if constexpr (DET) {
+      const long long rf = (long long)nwin * S;                        // rows per field
+      const int j = (int)(((long long)blockIdx.x * 8 + warp) - ((long long)n_cur * rf) / RPW);
+      float* d = det.film + ((long long)n_cur * det.K + j) * 2 * C + c0;
 #pragma unroll
-    for (int k = 0; k < NV; ++k)
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        atomicAdd(p.dfilm + (long long)n_cur * 2 * C + 128 * k + c0 + i, ag[4 * k + i]);
-        atomicAdd(p.dfilm + (long long)n_cur * 2 * C + C + 128 * k + c0 + i, ab[4 * k + i]);
-        ag[4 * k + i] = ab[4 * k + i] = 0.f;
+      for (int k = 0; k < NV; ++k) {
+        *reinterpret_cast<float4*>(d + 128 * k) = make_float4(ag[4 * k], ag[4 * k + 1], ag[4 * k + 2], ag[4 * k + 3]);
+        *reinterpret_cast<float4*>(d + C + 128 * k) = make_float4(ab[4 * k], ab[4 * k + 1], ab[4 * k + 2], ab[4 * k + 3]);
       }
+#pragma unroll
+      for (int i = 0; i < NE; ++i) ag[i] = ab[i] = 0.f;
+    } else {
+#pragma unroll
+      for (int k = 0; k < NV; ++k)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+          atomicAdd(p.dfilm + (long long)n_cur * 2 * C + 128 * k + c0 + i, ag[4 * k + i]);
+          atomicAdd(p.dfilm + (long long)n_cur * 2 * C + C + 128 * k + c0 + i, ab[4 * k + i]);
+          ag[4 * k + i] = ab[4 * k + i] = 0.f;
+        }
+    }
   };
   const long long r0 = ((long long)blockIdx.x * 8 + warp) * RPW;
   // (window, token) of the warp's first row by division, then incrementally: four 64- / 32-bit divisions per row were most of the
@@ -1759,7 +1868,14 @@ __global__ void __launch_bounds__(256) attn_gather_bwd_kernel(const AttnGatherBw
     s1 = warp_sum(s1) * (1.0f / C); s2 = warp_sum(s2) * (1.0f / C);
 #pragma unroll
     for (int i = 0; i < NE; ++i) dx[i] = rstd * (dx[i] - s1 - v[i] * s2);
-    if (tok < g.R) {
+    if (DET && tok < g.R) {
+      float* d = det.reg + (((long long)n * nwin + wi) * g.R + tok) * C + c0;
+      const float* rr = p.dreg_res ? p.dreg_res + ((long long)n * g.R + tok) * C + c0 : nullptr;
+#pragma unroll
+      for (int j = 0; j < NV; ++j)
+#pragma unroll
+        for (int i = 0; i < 4; ++i) d[128 * j + i] = dx[4 * j + i] + (rr ? rr[128 * j + i] * p.reg_scale : 0.f);
+    } else if (tok < g.R) {
       float* d = p.dreg_in + (p.reg_per_field ? (long long)n * g.R * C : 0) + (long long)tok * C + c0;
       const float* rr = p.dreg_res ? p.dreg_res + ((long long)n * g.R + tok) * C + c0 : nullptr;
 #pragma unroll
@@ -2014,7 +2130,7 @@ int dropout_mask_debug_run(unsigned seed, unsigned salt, int drop_thresh, long l
 
 int attn_core_bwd_tc_run(const void* qkv, const void* datt, const float* qgamma, const float* kgamma, const float* bias_table,
                          const AttnGeom& g, int heads, void* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
-                         void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st);
+                         void* att_out, unsigned seed, unsigned salt, int drop_thresh, cudaStream_t st, const AttnDetSlots* det);
 
 // exact-fp32 SIMT core backward: 8 [64][DH+1] row tiles, P (and the dropout mask) [64][65], bias-table rows, 1/|q|, 1/|k| and the
 // per-warp gamma partials (DH 64 with dropout: 172 KB)
@@ -2028,7 +2144,7 @@ static int core_bwd_simt_launch(const AttnCoreBwdParams& p, int nb, const DropCf
     if (e != cudaSuccess) return set_error("attn_core_bwd smem attr: %s", cudaGetErrorString(e));
     attr = smem;
   }
-  attn_core_bwd_kernel<DH><<<p.g.N * p.heads, 256, smem, st>>>(p, drop);
+  attn_core_bwd_kernel<DH><<<p.g.N * p.heads, 256, smem, st>>>(p, drop, AttnDetSlots{});
   return check_launch("attn_core_bwd_kernel");
 }
 
@@ -2042,7 +2158,7 @@ static int core_bwd_bf16_launch(const AttnCoreBwdParams& q, int nb, float* att_o
     if (e != cudaSuccess) return set_error("attn_core_bwd_bf16 smem attr: %s", cudaGetErrorString(e));
     attr3 = smem3;
   }
-  attn_core_bwd_bf16_kernel<DH><<<q.g.N * q.heads, 128, smem3, st>>>(q, att_out, drop);
+  attn_core_bwd_bf16_kernel<DH><<<q.g.N * q.heads, 128, smem3, st>>>(q, att_out, drop, AttnDetSlots{});
   return check_launch("attn_core_bwd_bf16_kernel");
 }
 
@@ -2057,7 +2173,7 @@ static int core_bwd_simt_long_launch(const AttnCoreBwdParams& p, int nb, const D
     if (e != cudaSuccess) return set_error("attn_core_bwd (S > 64) smem attr: %s", cudaGetErrorString(e));
     attr = smem;
   }
-  attn_core_bwd_long_kernel<DH><<<p.g.N * p.heads, 256, smem, st>>>(p, drop);
+  attn_core_bwd_long_kernel<DH><<<p.g.N * p.heads, 256, smem, st>>>(p, drop, AttnDetSlots{});
   return check_launch("attn_core_bwd_long_kernel");
 }
 
@@ -2071,7 +2187,7 @@ static int core_bwd_bf16_long_launch(const AttnCoreBwdParams& q, int nb, const D
     if (e != cudaSuccess) return set_error("attn_core_bwd_bf16 (S > 64) smem attr: %s", cudaGetErrorString(e));
     attr = smem;
   }
-  attn_core_bwd_bf16_long_kernel<DH><<<q.g.N * q.heads, 256, smem, st>>>(q, drop);
+  attn_core_bwd_bf16_long_kernel<DH><<<q.g.N * q.heads, 256, smem, st>>>(q, drop, AttnDetSlots{});
   return check_launch("attn_core_bwd_bf16_long_kernel");
 }
 
@@ -2092,7 +2208,7 @@ int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, 
   const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1;
   if (use_tf32 == 3)
     return attn_core_bwd_tc_run(qkv, datt, qgamma, kgamma, bias_table, g, heads, dqkv, dqgamma, dkgamma, dbias_table, att_out, seed, salt,
-                                drop_thresh, st);
+                                drop_thresh, st, nullptr);
   if (use_tf32 == 2) {
     AttnCoreBwdParams q;
     q.qkv = qkv; q.datt = datt; q.qgamma = qgamma; q.kgamma = kgamma; q.bias_table = bias_table; q.dqkv = dqkv;
@@ -2114,6 +2230,154 @@ int attn_core_bwd_run(const float* qkv, const float* datt, const float* qgamma, 
                   : core_bwd_simt_launch<64>(p, nb, make_drop(seed, salt, drop_thresh), st);
 }
 
+// ------------------------------------------------------------------------------------------------
+// deterministic variants (fixed-order slot reductions, det_sum_run in vg_bwd.cu)
+// ------------------------------------------------------------------------------------------------
+static int det_work_check(const char* what, long long need, float* work, long long work_elems) {
+  if (need > 0 && (!work || work_elems < need)) return set_error("%s: workspace too small (%lld < %lld floats)", what, work_elems, need);
+  return 0;
+}
+
+long long colsum_det_workspace_elems(long long M, int C) {
+  const long long S = (M + STAT_ROWS - 1) / STAT_ROWS;
+  return S * C + det_sum_tmp_elems(1, S, C);
+}
+
+int colsum_det_run(const float* X, long long M, int C, float* out, float* work, long long work_elems, cudaStream_t st) {
+  if (det_work_check("colsum_det", colsum_det_workspace_elems(M, C), work, work_elems)) return 1;
+  const long long S = (M + STAT_ROWS - 1) / STAT_ROWS;
+  if (S == 0) return 0;
+  colsum_kernel<true><<<(unsigned)S, 256, 0, st>>>(X, M, C, work);
+  int rc = check_launch("colsum_kernel (det)");
+  return rc ? rc : det_sum_run(work, 1, S, C, C, out, C, work + S * C, st);
+}
+
+long long attn_core_bwd_det_workspace_elems(const AttnGeom& g, int heads, int dh) {
+  const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1, inner = heads * dh;
+  const long long a = (long long)g.N * 2 * inner, b = (long long)g.N * nb * heads;
+  const long long t1 = det_sum_tmp_elems(1, g.N, inner), t2 = det_sum_tmp_elems(1, g.N, nb * heads);
+  return a + b + (t1 > t2 ? t1 : t2);
+}
+
+template <typename KernelFn>
+static int det_smem_attr(KernelFn fn, size_t smem, size_t& attr, const char* what) {
+  if (smem <= attr) return 0;
+  cudaError_t e = cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  if (e != cudaSuccess) return set_error("%s smem attr: %s", what, cudaGetErrorString(e));
+  attr = smem;
+  return 0;
+}
+
+// the DET instantiations of the five core-backward kernels (the modes and limits of attn_core_bwd_run)
+template <int DH>
+static int core_bwd_det_launch(const AttnCoreBwdParams& p, int nb, int mode, float* att_out, const DropCfg& drop, const AttnDetSlots& det,
+                               cudaStream_t st) {
+  const bool long_win = p.g.S() > 64;
+  const unsigned grid = (unsigned)(p.g.N * p.heads);
+  if (mode == 0 && !long_win) {
+    const size_t smem = (size_t)(8 * 64 * (DH + 1) + 64 * 65 + 2 * nb + 128 + 8 * 2 * DH + (drop.thresh ? 64 * 65 : 0)) * sizeof(float);
+    static PerDeviceSize a_pd;
+    if (det_smem_attr(attn_core_bwd_kernel<DH, true>, smem, a_pd.cur(), "attn_core_bwd_det")) return 1;
+    attn_core_bwd_kernel<DH, true><<<grid, 256, smem, st>>>(p, drop, det);
+  } else if (mode == 0) {
+    const size_t smem = cbs_long<DH>::bytes(nb);
+    static PerDeviceSize a_pd;
+    if (det_smem_attr(attn_core_bwd_long_kernel<DH, true>, smem, a_pd.cur(), "attn_core_bwd_det (S > 64)")) return 1;
+    attn_core_bwd_long_kernel<DH, true><<<grid, 256, smem, st>>>(p, drop, det);
+  } else if (!long_win) {
+    const size_t smem = (size_t)cbh<DH>::BYTES + (size_t)(2 * nb + 6 * DH + 8 * DH + 64 * 65) * sizeof(float);
+    static PerDeviceSize a_pd;
+    if (det_smem_attr(attn_core_bwd_bf16_kernel<DH, true>, smem, a_pd.cur(), "attn_core_bwd_bf16_det")) return 1;
+    attn_core_bwd_bf16_kernel<DH, true><<<grid, 128, smem, st>>>(p, att_out, drop, det);
+  } else {
+    const size_t smem = (size_t)cbh_long<DH>::BYTES + (size_t)(2 * nb + 6 * DH + 16 * DH) * sizeof(float);
+    static PerDeviceSize a_pd;
+    if (det_smem_attr(attn_core_bwd_bf16_long_kernel<DH, true>, smem, a_pd.cur(), "attn_core_bwd_bf16_det (S > 64)")) return 1;
+    attn_core_bwd_bf16_long_kernel<DH, true><<<grid, 256, smem, st>>>(p, drop, det);
+  }
+  return check_launch("attn_core_bwd (det)");
+}
+
+int attn_core_bwd_det_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
+                          const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
+                          int use_tf32, float* att_out, unsigned seed, unsigned salt, int drop_thresh, float* work,
+                          long long work_elems, cudaStream_t st) {
+  // the checks of attn_core_bwd_run: every mode and window it accepts has a deterministic kernel
+  if (drop_thresh < 0 || drop_thresh > 255) return set_error("attn_core_bwd_det: dropout threshold %d outside [0, 255]", drop_thresh);
+  if (use_tf32 != 0 && use_tf32 != 2 && use_tf32 != 3) return set_error("attn_core_bwd_det: mode %d (0 exact fp32, 2 bf16 mma on fp32 tensors, 3 bf16 tensors)", use_tf32);
+  if ((use_tf32 == 3 && dh != 32) || (dh != 32 && dh != 64)) return set_error("attn_core_bwd_det: dim_head must be 32 (got %d)", dh);
+  const int max_s = use_tf32 == 3 ? 64 : 128;
+  if (g.S() > max_s) return set_error("attn_core_bwd_det: sequence %d > %d", g.S(), max_s);
+  const bool long_win = g.S() > 64;
+  if (long_win && att_out) return set_error("attn_core_bwd_det: att_out needs S <= 64 (got %d)", g.S());
+  if (long_win && drop_thresh && heads > DROP_MAX_HEADS_LONG)
+    return set_error("attn_core_bwd_det: dropout with %d heads at sequence %d > 64 (at most %d heads)", heads, g.S(), DROP_MAX_HEADS_LONG);
+  if (use_tf32 == 0 && att_out) return set_error("attn_core_bwd_det: att_out is only produced by the tensor-core kernels (modes 2, 3)");
+  if (det_work_check("attn_core_bwd_det", attn_core_bwd_det_workspace_elems(g, heads, dh), work, work_elems)) return 1;
+  const int nb = (2 * g.win - 1) * (2 * g.win - 1) + 1, inner = heads * dh;
+  AttnDetSlots det{};
+  det.gamma = work; det.bias = work + (long long)g.N * 2 * inner;
+  float* tmp = det.bias + (long long)g.N * nb * heads;
+  int rc;
+  if (use_tf32 == 3) {
+    rc = attn_core_bwd_tc_run(qkv, datt, qgamma, kgamma, bias_table, g, heads, dqkv, dqgamma, dkgamma, dbias_table, att_out, seed, salt,
+                              drop_thresh, st, &det);
+  } else {
+    AttnCoreBwdParams p;
+    p.qkv = qkv; p.datt = datt; p.qgamma = qgamma; p.kgamma = kgamma; p.bias_table = bias_table; p.dqkv = dqkv;
+    p.dqgamma = dqgamma; p.dkgamma = dkgamma; p.dbias_table = dbias_table; p.g = g; p.heads = heads;
+    const DropCfg drop = make_drop(seed, salt, drop_thresh);
+    rc = dh == 32 ? core_bwd_det_launch<32>(p, nb, use_tf32, att_out, drop, det, st)
+                  : core_bwd_det_launch<64>(p, nb, use_tf32, att_out, drop, det, st);
+  }
+  if (!rc) rc = det_sum_run(det.gamma, 1, g.N, inner, 2LL * inner, dqgamma, inner, tmp, st);
+  if (!rc) rc = det_sum_run(det.gamma + inner, 1, g.N, inner, 2LL * inner, dkgamma, inner, tmp, st);
+  if (!rc) rc = det_sum_run(det.bias, 1, g.N, nb * heads, (long long)nb * heads, dbias_table, (long long)nb * heads, tmp, st);
+  return rc;
+}
+
+static int gather_bwd_slots(const AttnGeom& g) { return (int)(((long long)g.nwin() * g.S() + 15) / 16) + 1; }
+
+long long attn_gather_bwd_det_workspace_elems(const AttnGeom& g, int reg_per_field) {
+  const int K = gather_bwd_slots(g);
+  const long long film = (long long)g.N * K * 2 * g.C, reg = (long long)g.N * g.nwin() * g.R * g.C;
+  const long long t1 = det_sum_tmp_elems(g.N, K, 2 * g.C);
+  const long long t2 = reg_per_field ? det_sum_tmp_elems(g.N, g.nwin(), g.R * g.C) : det_sum_tmp_elems(1, (long long)g.N * g.nwin(), g.R * g.C);
+  return film + reg + (t1 > t2 ? t1 : t2);
+}
+
+int attn_gather_bwd_det_run(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
+                            const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in, float* dfilm,
+                            const AttnGeom& g, float eps, float* work, long long work_elems, cudaStream_t st) {
+  if (g.C != 128 && g.C != 256 && g.C != 384 && g.C != 512) return set_error("attn_gather_bwd_det: C=%d must be 128, 256, 384 or 512", g.C);
+  if (det_work_check("attn_gather_bwd_det", attn_gather_bwd_det_workspace_elems(g, reg_per_field), work, work_elems)) return 1;
+  AttnGatherBwdParams p;
+  p.x = x; p.reg = reg; p.reg_per_field = reg_per_field; p.film = film; p.dtok = dtok; p.dx_out = dx_out; p.dreg_res = dreg_res;
+  p.reg_scale = reg_scale; p.dx_in = dx_in; p.dreg_in = dreg_in; p.dfilm = dfilm; p.g = g; p.eps = eps;
+  AttnDetSlots det{};
+  det.K = gather_bwd_slots(g);
+  const long long nfilm = (long long)g.N * det.K * 2 * g.C, nwr = (long long)g.N * g.nwin();
+  det.film = work; det.reg = work + nfilm;
+  float* tmp = det.reg + nwr * g.R * g.C;
+  cudaError_t e = cudaMemsetAsync(det.film, 0, (size_t)nfilm * sizeof(float), st);
+  if (e != cudaSuccess) return set_error("attn_gather_bwd_det: %s", cudaGetErrorString(e));
+  const long long rows = nwr * g.S();
+  const unsigned grid = nblk(rows, 8 * 16);
+  switch (g.C) {
+    case 128: attn_gather_bwd_kernel<128, true><<<grid, 256, 0, st>>>(p, rows, det); break;
+    case 256: attn_gather_bwd_kernel<256, true><<<grid, 256, 0, st>>>(p, rows, det); break;
+    case 384: attn_gather_bwd_kernel<384, true><<<grid, 256, 0, st>>>(p, rows, det); break;
+    default: attn_gather_bwd_kernel<512, true><<<grid, 256, 0, st>>>(p, rows, det); break;
+  }
+  int rc = check_launch("attn_gather_bwd_kernel (det)");
+  if (!rc) rc = det_sum_run(det.film, g.N, det.K, 2 * g.C, 2LL * g.C, dfilm, 2LL * g.C, tmp, st);
+  if (!rc && g.R > 0) {
+    if (reg_per_field) rc = det_sum_run(det.reg, g.N, g.nwin(), g.R * g.C, (long long)g.R * g.C, dreg_in, (long long)g.R * g.C, tmp, st);
+    else rc = det_sum_run(det.reg, 1, nwr, g.R * g.C, (long long)g.R * g.C, dreg_in, (long long)g.R * g.C, tmp, st);
+  }
+  return rc;
+}
+
 int attn_gather_bwd_run(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
                         const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in, float* dfilm,
                         const AttnGeom& g, float eps, cudaStream_t st) {
@@ -2124,10 +2388,10 @@ int attn_gather_bwd_run(const float* x, const float* reg, int reg_per_field, con
   const long long rows = (long long)g.N * g.nwin() * g.S();
   const unsigned grid = nblk(rows, 8 * 16);
   switch (g.C) {
-    case 128: attn_gather_bwd_kernel<128><<<grid, 256, 0, st>>>(p, rows); break;
-    case 256: attn_gather_bwd_kernel<256><<<grid, 256, 0, st>>>(p, rows); break;
-    case 384: attn_gather_bwd_kernel<384><<<grid, 256, 0, st>>>(p, rows); break;
-    default: attn_gather_bwd_kernel<512><<<grid, 256, 0, st>>>(p, rows); break;
+    case 128: attn_gather_bwd_kernel<128><<<grid, 256, 0, st>>>(p, rows, AttnDetSlots{}); break;
+    case 256: attn_gather_bwd_kernel<256><<<grid, 256, 0, st>>>(p, rows, AttnDetSlots{}); break;
+    case 384: attn_gather_bwd_kernel<384><<<grid, 256, 0, st>>>(p, rows, AttnDetSlots{}); break;
+    default: attn_gather_bwd_kernel<512><<<grid, 256, 0, st>>>(p, rows, AttnDetSlots{}); break;
   }
   return check_launch("attn_gather_bwd_kernel");
 }

@@ -75,6 +75,16 @@ __host__ __device__ __forceinline__ long long attn_token_pixel(const AttnGeom& g
   return (long long)ph * g.Wl + pw;
 }
 
+// slots of the deterministic (DET) instantiations of the attention core and gather backward
+// kernels (vg_bwd_vit.cu, vg_attn_bwd_tc.cu): a kernel parameter of its own after
+// the others, so that the parameters of the atomic instantiations keep their offsets
+struct AttnDetSlots {
+  float* gamma;            // core: [N][2][heads*DH] per-field q / k gamma gradients
+  float* bias;             // core: [N][nb][heads] per-field bias-table gradients
+  float* film; int K;      // gather: [N][K][2C] per-(field, warp-of-field) dfilm partials (zeroed by the launcher)
+  float* reg;              // gather: [N*nwin][R][C] register-row gradients of every window
+};
+
 // ----------------------------------------------------------------------------------------------
 // dtype traits: activations are bf16 ("bf16 mode") or float ("fp32 mode")
 // ----------------------------------------------------------------------------------------------

@@ -187,4 +187,37 @@ int attn_gather_bwd_run(const float* x, const float* reg, int reg_per_field, con
                         const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in, float* dfilm,
                         const AttnGeom& g, float eps, cudaStream_t st);
 
+// ---- deterministic training-backward variants (fixed-order reductions over per-warp / per-block slots; vg_bwd.cu, vg_bwd_vit.cu)
+long long det_sum_tmp_elems(int G, long long S, int W);
+int det_sum_run(const float* in, int G, long long S, int W, long long ld, float* out, long long out_ld, float* tmp, cudaStream_t st);
+long long conv_ln_bwd_det_workspace_elems(int C, int N, int HP, int WP);
+int conv_ln_bwd_det_run(int C, int xdtype, int odtype, const float* dY, const void* xhat, const float* rstd, const unsigned* mask,
+                        const float* ln_g, const float* film, float eps, void* dconv, float* sumA, float* sumB, float* sumD,
+                        float* border, int N, int HP, int WP, float* work, long long work_elems, cudaStream_t st);
+long long head_bwd_det_workspace_elems(int N, int HP, int WP, int C);
+int head_bwd_det_run(int dtype, const float* dpred, const void* h, const float* w, float stdv, int N, int HP, int WP, int H, int W,
+                     int pt, int pl, float* dH, float* dw, float* db, int C, float* work, long long work_elems, cudaStream_t st);
+long long convT_bwd_gather_det_workspace_elems(int N, int Hl, int Wl, int C);
+int convT_bwd_gather_det_run(int odtype, const float* dUp, void* G, float* dbias, int N, int Hl, int Wl, int C, float* work,
+                             long long work_elems, cudaStream_t st);
+long long pg_field_sum_det_workspace_elems(int N, int HP, int WP, int C);
+int pg_field_sum_det_run(const float* in, float* out, int N, int HP, int WP, int C, float* work, long long work_elems, cudaStream_t st);
+long long time_terms_bwd_det_workspace_elems(int N, int Cout);
+int time_terms_bwd_det_run(const float* border, const float* sumD, const float* tres_sum, const float* temb, const float* w3,
+                           const float* w1, int N, int ntc, int c_in, int c_data, int Cout, float* dw3, float* dw1, float* db1,
+                           float* dtemb, float* work, long long work_elems, cudaStream_t st);
+int time_embed_bwd_det_run(const float* dtemb, const float* dcond, const float* ts, long long sB, long long sT, long long sF, int B,
+                           int L, int le, int te, float* d_lead, float* d_m, float* d_d, float* d_h, cudaStream_t st);
+long long colsum_det_workspace_elems(long long M, int C);
+int colsum_det_run(const float* X, long long M, int C, float* out, float* work, long long work_elems, cudaStream_t st);
+long long attn_core_bwd_det_workspace_elems(const AttnGeom& g, int heads, int dh);
+int attn_core_bwd_det_run(const float* qkv, const float* datt, const float* qgamma, const float* kgamma, const float* bias_table,
+                          const AttnGeom& g, int heads, int dh, float* dqkv, float* dqgamma, float* dkgamma, float* dbias_table,
+                          int use_tf32, float* att_out, unsigned seed, unsigned salt, int drop_thresh, float* work,
+                          long long work_elems, cudaStream_t st);
+long long attn_gather_bwd_det_workspace_elems(const AttnGeom& g, int reg_per_field);
+int attn_gather_bwd_det_run(const float* x, const float* reg, int reg_per_field, const float* film, const float* dtok,
+                            const float* dx_out, const float* dreg_res, float reg_scale, float* dx_in, float* dreg_in, float* dfilm,
+                            const AttnGeom& g, float eps, float* work, long long work_elems, cudaStream_t st);
+
 }  // namespace vg

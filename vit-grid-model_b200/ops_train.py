@@ -14,6 +14,16 @@ def _f32(n, dev):
     return torch.empty(int(n), dtype=torch.float32, device=dev)
 
 
+def _det():
+    """torch.use_deterministic_algorithms(True) (warn_only too) is in force: the reductions below take the vg_*_det entry
+    points, which sum per-warp partials in a fixed order instead of with float atomics (checked when the backward runs)"""
+    return torch.are_deterministic_algorithms_enabled()
+
+
+def _work(query, *args, dev):
+    return _f32(max(1, getattr(_lib.load(), query)(*args)), dev)
+
+
 def conv3x3_ln_train(x, Wt, bias, ln_g, ln_b, eps, film, res, out, N, HP, WP, out_copy=None, tf32=False):
     """forward Block that also returns the saved tensors (xhat, rstd, relu_mask) for backward.  tf32 (fp32 storage): the
     convolution runs on tcgen05 kind::tf32.  C = out.shape[1]; widths other than 128 take the shifted-row GEMM + row kernel
@@ -68,6 +78,17 @@ def conv_ln_bwd(dY, saved, ln_g, film, eps, N, HP, WP, out_dtype, want_border=Fa
     dconv = torch.empty(dY.shape[0], C, dtype=out_dtype, device=dev)
     sums = torch.zeros(3, N, C, dtype=torch.float32, device=dev)
     border = torch.zeros(N, 8, C, dtype=torch.float32, device=dev) if want_border else None
+    if _det():
+        work = _work("vg_conv_ln_bwd_det_workspace", C, N, HP, WP, dev=dev)
+        args = (dY.data_ptr(), xhat.data_ptr(), rstd.data_ptr(), mask.data_ptr(), ln_g.data_ptr(), _p(film), float(eps),
+                dconv.data_ptr(), sums[0].data_ptr(), sums[1].data_ptr(), sums[2].data_ptr(), _p(border), N, HP, WP,
+                work.data_ptr(), work.numel(), _st())
+        if C != 128:
+            assert xhat.dtype == torch.float32 and out_dtype == torch.float32, "wide Block backward is fp32 (tf32_conv)"
+            _lib.call("vg_conv_ln_bwd_wide_det", C, *args)
+        else:
+            _lib.call("vg_conv_ln_bwd_det", DT_CODE[xhat.dtype], DT_CODE[out_dtype], *args)
+        return dconv, sums, border
     if C != 128:
         assert xhat.dtype == torch.float32 and out_dtype == torch.float32, "wide Block backward is fp32 (tf32_conv)"
         _lib.call("vg_conv_ln_bwd_wide", C, dY.data_ptr(), xhat.data_ptr(), rstd.data_ptr(), mask.data_ptr(), ln_g.data_ptr(),
@@ -112,6 +133,11 @@ def head_bwd(dpred, h, w, std, N, HP, WP, H, W, pads, dw, db):
     C = h.shape[1]
     dH = torch.empty(pg_pixels(N, HP, WP), C, dtype=torch.float32, device=h.device)
     pl, _, pt, _ = pads
+    if _det():
+        work = _work("vg_head_bwd_det_workspace", N, HP, WP, C, dev=h.device)
+        _lib.call("vg_head_bwd_det", DT_CODE[h.dtype], dpred.data_ptr(), h.data_ptr(), w.data_ptr(), float(std), N, HP, WP, C, H,
+                  W, pt, pl, dH.data_ptr(), dw.data_ptr(), db.data_ptr(), work.data_ptr(), work.numel(), _st())
+        return dH
     if C != 128:
         _lib.call("vg_head_bwd_wide", DT_CODE[h.dtype], dpred.data_ptr(), h.data_ptr(), w.data_ptr(), float(std), N, HP, WP, C, H,
                   W, pt, pl, dH.data_ptr(), dw.data_ptr(), db.data_ptr(), _st())
@@ -130,6 +156,11 @@ def pool2_bwd(x, dlow, N, HP, WP):
 
 def convT2_bwd_gather(dUp, N, Hl, Wl, C, out_dtype, dbias):
     G = torch.empty(N * Hl * Wl, 4 * C, dtype=out_dtype, device=dUp.device)
+    if _det():
+        work = _work("vg_convT2_bwd_gather_det_workspace", N, Hl, Wl, C, dev=dUp.device)
+        _lib.call("vg_convT2_bwd_gather_det", DT_CODE[out_dtype], dUp.data_ptr(), G.data_ptr(), dbias.data_ptr(), N, Hl, Wl, C,
+                  work.data_ptr(), work.numel(), _st())
+        return G
     _lib.call("vg_convT2_bwd_gather", DT_CODE[out_dtype], dUp.data_ptr(), G.data_ptr(), dbias.data_ptr(), N, Hl, Wl, C, _st())
     return G
 
@@ -147,6 +178,10 @@ def lead_sum(x, B, L, HP, WP, out_dtype):
 def pg_field_sum(x, N, HP, WP):
     C = x.shape[1]
     out = torch.zeros(N, C, dtype=torch.float32, device=x.device)
+    if _det():
+        work = _work("vg_pg_field_sum_det_workspace", N, HP, WP, C, dev=x.device)
+        _lib.call("vg_pg_field_sum_det", x.data_ptr(), out.data_ptr(), N, HP, WP, C, work.data_ptr(), work.numel(), _st())
+        return out
     if C != 128:
         _lib.call("vg_pg_field_sum_wide", x.data_ptr(), out.data_ptr(), N, HP, WP, C, _st())
         return out
@@ -158,6 +193,12 @@ def time_terms_bwd(border, sumD, tres_sum, temb, w3, w1, c_data, dw3, dw1, db1):
     N, ntc = temb.shape
     Cout, c_in = w3.shape[0], w3.shape[1]
     dtemb = torch.empty(N, ntc, dtype=torch.float32, device=temb.device)
+    if _det():
+        work = _work("vg_time_terms_bwd_det_workspace", N, Cout, dev=temb.device)
+        _lib.call("vg_time_terms_bwd_det", border.data_ptr(), sumD.data_ptr(), tres_sum.data_ptr(), temb.data_ptr(),
+                  w3.data_ptr(), w1.data_ptr(), N, ntc, c_in, c_data, Cout, dw3.data_ptr(), dw1.data_ptr(), db1.data_ptr(),
+                  dtemb.data_ptr(), work.data_ptr(), work.numel(), _st())
+        return dtemb
     _lib.call("vg_time_terms_bwd", border.data_ptr(), sumD.data_ptr(), tres_sum.data_ptr(), temb.data_ptr(), w3.data_ptr(),
               w1.data_ptr(), N, ntc, c_in, c_data, Cout, dw3.data_ptr(), dw1.data_ptr(), db1.data_ptr(), dtemb.data_ptr(), _st())
     return dtemb
@@ -165,6 +206,10 @@ def time_terms_bwd(border, sumD, tres_sum, temb, w3, w1, c_data, dw3, dw1, db1):
 
 def time_embed_bwd(dtemb, dcond, ts, B, L, le, te, d_lead, d_m, d_d, d_h):
     sB, sT, sF = ts.stride()
+    if _det():
+        _lib.call("vg_time_embed_bwd_det", dtemb.data_ptr(), _p(dcond), ts.data_ptr(), sB, sT, sF, B, L, le, te,
+                  d_lead.data_ptr(), d_m.data_ptr(), d_d.data_ptr(), d_h.data_ptr(), None, 0, _st())
+        return
     _lib.call("vg_time_embed_bwd", dtemb.data_ptr(), _p(dcond), ts.data_ptr(), sB, sT, sF, B, L, le, te, d_lead.data_ptr(),
               d_m.data_ptr(), d_d.data_ptr(), d_h.data_ptr(), _st())
 
@@ -247,6 +292,10 @@ def prepare_bwd(g, B, T, C, H, W, pads, HP, WP, std, extra_channel=-1):
 
 def colsum(x2d, out):
     M, C = x2d.shape
+    if _det():
+        work = _work("vg_colsum_det_workspace", M, C, dev=x2d.device)
+        _lib.call("vg_colsum_det", x2d.data_ptr(), M, C, out.data_ptr(), work.data_ptr(), work.numel(), _st())
+        return
     _lib.call("vg_colsum", x2d.data_ptr(), M, C, out.data_ptr(), _st())
 
 
@@ -337,6 +386,13 @@ def attn_core_bwd(qkv, datt, q_gamma, k_gamma, bias_table, N, Hl, Wl, win, R, he
     if qkv.dtype == torch.bfloat16:
         assert datt.dtype == torch.bfloat16
         mode = 3
+    if _det():
+        work = _work("vg_attn_core_bwd_det_workspace", N, Hl, Wl, win, R, heads, dh, dev=qkv.device)
+        _lib.call("vg_attn_core_bwd_det", qkv.data_ptr(), datt.data_ptr(), q_gamma.data_ptr(), k_gamma.data_ptr(),
+                  bias_table.data_ptr(), N, Hl, Wl, win, R, heads, dh, dqkv.data_ptr(), dq_gamma.data_ptr(), dk_gamma.data_ptr(),
+                  dbias_table.data_ptr(), mode, _p(att), int(drop[0]), int(drop[1]), int(drop[2]), work.data_ptr(), work.numel(),
+                  _st())
+        return (dqkv, att) if want_att else dqkv
     _lib.call("vg_attn_core_bwd", qkv.data_ptr(), datt.data_ptr(), q_gamma.data_ptr(), k_gamma.data_ptr(),
               bias_table.data_ptr(), N, Hl, Wl, win, R, heads, dh, dqkv.data_ptr(), dq_gamma.data_ptr(), dk_gamma.data_ptr(),
               dbias_table.data_ptr(), mode, _p(att), int(drop[0]), int(drop[1]), int(drop[2]), _st())
@@ -346,6 +402,12 @@ def attn_core_bwd(qkv, datt, q_gamma, k_gamma, bias_table, N, Hl, Wl, win, R, he
 def attn_gather_bwd(x, reg, film, dtok, dx_out, dreg_res, reg_scale, dreg_in, dfilm, win, R, grid_mode, eps=1e-5):
     N, Hl, Wl, C = x.shape
     dx_in = torch.empty_like(x)
+    if _det():
+        work = _work("vg_attn_gather_bwd_det_workspace", N, Hl, Wl, C, win, R, int(reg.dim() == 3), dev=x.device)
+        _lib.call("vg_attn_gather_bwd_det", x.data_ptr(), reg.data_ptr(), int(reg.dim() == 3), film.data_ptr(), dtok.data_ptr(),
+                  dx_out.data_ptr(), _p(dreg_res), float(reg_scale), dx_in.data_ptr(), dreg_in.data_ptr(), dfilm.data_ptr(),
+                  N, Hl, Wl, C, win, R, int(grid_mode), float(eps), work.data_ptr(), work.numel(), _st())
+        return dx_in
     _lib.call("vg_attn_gather_bwd", x.data_ptr(), reg.data_ptr(), int(reg.dim() == 3), film.data_ptr(), dtok.data_ptr(),
               dx_out.data_ptr(), _p(dreg_res), float(reg_scale), dx_in.data_ptr(), dreg_in.data_ptr(), dfilm.data_ptr(),
               N, Hl, Wl, C, win, R, int(grid_mode), float(eps), _st())
