@@ -369,6 +369,16 @@ VG_API long long vg_bn_workspace(long long M, int C);
 VG_API int vg_bn_stats(const float* x, long long M, int C, const float* gamma, const float* beta, float eps, float momentum,
                 float* running_mean, float* running_var, float* mean, float* rstd, float* scale, float* shift,
                 float* work, long long work_elems, void* stream);
+/* Synchronised (cross-rank) BatchNorm statistics, split around the exchange the caller runs between them.
+ * vg_bn_stats_local: this rank's fp64 row [sum x (C) | sum x^2 (C) | M] of x [M][C] (the sums of vg_bn_stats before its
+ * finalize).  work: vg_bn_workspace() floats. */
+VG_API int vg_bn_stats_local(const float* x, long long M, int C, double* row, float* work, long long work_elems, void* stream);
+/* vg_bn_stats_global: rows [world][2C+1] of every rank in rank order, summed in that order in fp64; then vg_bn_stats' finalize
+ * over the global count (mean, rstd, scale, shift; momentum update of the running buffers with the unbiased variance over the
+ * global count, NULL = no update).  count (or NULL): the global row count, as one double, for vg_bn_bwd_global. */
+VG_API int vg_bn_stats_global(const double* rows, int world, int C, const float* gamma, const float* beta, float eps,
+                       float momentum, float* running_mean, float* running_var, float* mean, float* rstd, float* scale,
+                       float* shift, double* count, void* stream);
 /* out = act(raw*scale + shift) (+ res); act 0 none, 1 GELU(erf) */
 VG_API int vg_bn_act(const float* raw, const float* scale, const float* shift, int act, const float* res, float* out,
               long long M, int C, void* stream);
@@ -379,6 +389,18 @@ VG_API int vg_bn_bwd(const float* dOut, const float* raw, const float* scale, co
               const float* rstd, const float* gamma, int act, const float* fgate, const float* fadd,
               long long rows_per_field, long long M, int C, float* dgamma, float* dbeta, float* draw, float* work,
               long long work_elems, void* stream);
+/* Synchronised BatchNorm backward, split around the exchange like the statistics.  vg_bn_bwd_local: this rank's fp64 row
+ * [S1 (C) | S2 (C)] (S1 = sum dpre, S2 = sum dpre*xhat over its M rows, the upstream form and C limits of vg_bn_bwd);
+ * dgamma += S2, dbeta += S1 accumulated from the local sums.  work: vg_bn_workspace() floats. */
+VG_API int vg_bn_bwd_local(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean,
+                    const float* rstd, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M,
+                    int C, float* dgamma, float* dbeta, double* row, float* work, long long work_elems, void* stream);
+/* vg_bn_bwd_global: rows [world][2C] of every rank summed in rank order in fp64, k1 = S1/count, k2 = S2/count (count: the
+ * global row count written by vg_bn_stats_global), then draw [M][C] of this rank's rows as vg_bn_bwd.  work: 2*C floats */
+VG_API int vg_bn_bwd_global(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean,
+                     const float* rstd, const float* gamma, int act, const float* fgate, const float* fadd,
+                     long long rows_per_field, long long M, int C, const double* rows, int world, const double* count,
+                     float* draw, float* work, long long work_elems, void* stream);
 /* BatchNorm with its running statistics (eval mode, frozen) (+ activation) backward, same upstream form as vg_bn_bwd
  * (g = dOut*fgate[n] + fadd[n]) and the same C limits: running_mean, running_rstd = 1/sqrt(running_var + eps), scale / shift
  * the affine folded from them.  draw = g*act'*scale written; dgamma += sum g*act'*(raw - running_mean)*running_rstd and

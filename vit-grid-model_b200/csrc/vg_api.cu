@@ -501,6 +501,17 @@ int vg_bn_stats(const float* x, long long M, int C, const float* gamma, const fl
                       work_elems, (cudaStream_t)stream);
 }
 
+int vg_bn_stats_local(const float* x, long long M, int C, double* row, float* work, long long work_elems, void* stream) {
+  return bn_stats_local_run(x, M, C, row, work, work_elems, (cudaStream_t)stream);
+}
+
+int vg_bn_stats_global(const double* rows, int world, int C, const float* gamma, const float* beta, float eps, float momentum,
+                       float* running_mean, float* running_var, float* mean, float* rstd, float* scale, float* shift, double* count,
+                       void* stream) {
+  return bn_stats_global_run(rows, world, C, gamma, beta, eps, momentum, running_mean, running_var, mean, rstd, scale, shift, count,
+                             (cudaStream_t)stream);
+}
+
 int vg_bn_act(const float* raw, const float* scale, const float* shift, int act, const float* res, float* out,
               long long M, int C, void* stream) {
   return bn_act_run(raw, scale, shift, act, res, out, M, C, (cudaStream_t)stream);
@@ -512,6 +523,21 @@ int vg_bn_bwd(const float* dOut, const float* raw, const float* scale, const flo
               long long work_elems, void* stream) {
   return bn_bwd_run(dOut, raw, scale, shift, mean, rstd, gamma, act, fgate, fadd, rows_per_field, M, C, dgamma, dbeta, draw,
                     work, work_elems, (cudaStream_t)stream);
+}
+
+int vg_bn_bwd_local(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean,
+                    const float* rstd, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
+                    float* dgamma, float* dbeta, double* row, float* work, long long work_elems, void* stream) {
+  return bn_bwd_local_run(dOut, raw, scale, shift, mean, rstd, act, fgate, fadd, rows_per_field, M, C, dgamma, dbeta, row, work,
+                          work_elems, (cudaStream_t)stream);
+}
+
+int vg_bn_bwd_global(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean,
+                     const float* rstd, const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field,
+                     long long M, int C, const double* rows, int world, const double* count, float* draw, float* work,
+                     long long work_elems, void* stream) {
+  return bn_bwd_global_run(dOut, raw, scale, shift, mean, rstd, gamma, act, fgate, fadd, rows_per_field, M, C, rows, world, count,
+                           draw, work, work_elems, (cudaStream_t)stream);
 }
 
 int vg_bn_bwd_frozen(const float* dOut, const float* raw, const float* scale, const float* shift, const float* running_mean,

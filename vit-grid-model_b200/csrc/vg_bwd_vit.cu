@@ -59,16 +59,13 @@ __device__ __forceinline__ void sum_parts2(const float* __restrict__ part, int n
   for (int k = 0; k < 8; ++k) { s1 += red[0][k][l]; s2 += red[1][k][l]; }
 }
 
-// BatchNorm2d training statistics (maxvit.py:89,92,96): biased variance for normalisation, unbiased for the running
-// estimate, momentum update of the running buffers, and the folded per-channel affine  y = raw*scale + shift.
-__global__ void bn_finalize_kernel(const float* __restrict__ part, int nparts, long long M, int C, const float* __restrict__ gamma,
-                                   const float* __restrict__ beta, float eps, float momentum, float* __restrict__ run_mean,
-                                   float* __restrict__ run_var, float* __restrict__ mean, float* __restrict__ rstd,
-                                   float* __restrict__ scale, float* __restrict__ shift) {
-  const int c = blockIdx.x * 32 + (threadIdx.x & 31);       // 256 threads: 32 channels x 8 slices of the partials
-  double s = 0.0, s2 = 0.0;
-  sum_parts2(part, nparts, C, c, s, s2);
-  if (c >= C || threadIdx.x >= 32) return;
+// BatchNorm2d training statistics (maxvit.py:89,92,96) of channel c from its fp64 sums s = Σx, s2 = Σx² over M rows: biased
+// variance for normalisation, unbiased for the running estimate, momentum update of the running buffers, and the folded
+// per-channel affine  y = raw*scale + shift.  Shared by the one-GPU and the synchronised (all ranks' rows) statistics.
+__device__ __forceinline__ void bn_finalize_channel(double s, double s2, long long M, int c, const float* __restrict__ gamma,
+                                                    const float* __restrict__ beta, float eps, float momentum,
+                                                    float* __restrict__ run_mean, float* __restrict__ run_var, float* __restrict__ mean,
+                                                    float* __restrict__ rstd, float* __restrict__ scale, float* __restrict__ shift) {
   const double m = s / (double)M;
   double var = s2 / (double)M - m * m;
   if (var < 0.0) var = 0.0;
@@ -81,6 +78,42 @@ __global__ void bn_finalize_kernel(const float* __restrict__ part, int nparts, l
     run_mean[c] = (1.0f - momentum) * run_mean[c] + momentum * (float)m;
     run_var[c] = (1.0f - momentum) * run_var[c] + momentum * (float)unb;
   }
+}
+
+__global__ void bn_finalize_kernel(const float* __restrict__ part, int nparts, long long M, int C, const float* __restrict__ gamma,
+                                   const float* __restrict__ beta, float eps, float momentum, float* __restrict__ run_mean,
+                                   float* __restrict__ run_var, float* __restrict__ mean, float* __restrict__ rstd,
+                                   float* __restrict__ scale, float* __restrict__ shift) {
+  const int c = blockIdx.x * 32 + (threadIdx.x & 31);       // 256 threads: 32 channels x 8 slices of the partials
+  double s = 0.0, s2 = 0.0;
+  sum_parts2(part, nparts, C, c, s, s2);
+  if (c >= C || threadIdx.x >= 32) return;
+  bn_finalize_channel(s, s2, M, c, gamma, beta, eps, momentum, run_mean, run_var, mean, rstd, scale, shift);
+}
+
+// ---- synchronised (cross-rank) statistics.  A rank's contribution is one fp64 row [Σx (C) | Σx² (C) | M]; the rows of all
+// ranks, gathered in rank order, are summed in that order by every rank, so every rank finalizes the same bits.
+__global__ void bn_stats_local_kernel(const float* __restrict__ part, int nparts, long long M, int C, double* __restrict__ row) {
+  const int c = blockIdx.x * 32 + (threadIdx.x & 31);       // 256 threads: 32 channels x 8 slices of the partials
+  double s = 0.0, s2 = 0.0;
+  sum_parts2(part, nparts, C, c, s, s2);
+  if (blockIdx.x == 0 && threadIdx.x == 0) row[2 * C] = (double)M;
+  if (c >= C || threadIdx.x >= 32) return;
+  row[c] = s; row[C + c] = s2;
+}
+
+__global__ void __launch_bounds__(256) bn_stats_global_kernel(const double* __restrict__ rows, int world, int C,
+                                                              const float* __restrict__ gamma, const float* __restrict__ beta, float eps,
+                                                              float momentum, float* __restrict__ run_mean, float* __restrict__ run_var,
+                                                              float* __restrict__ mean, float* __restrict__ rstd, float* __restrict__ scale,
+                                                              float* __restrict__ shift, double* __restrict__ count) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  const long long stride = 2LL * C + 1;
+  double s = 0.0, s2 = 0.0, m = 0.0;
+  for (int r = 0; r < world; ++r) { s += rows[r * stride + c]; s2 += rows[r * stride + C + c]; m += rows[r * stride + 2 * C]; }
+  if (c == 0 && count) *count = m;
+  bn_finalize_channel(s, s2, (long long)m, c, gamma, beta, eps, momentum, run_mean, run_var, mean, rstd, scale, shift);
 }
 
 // out = act(raw*scale + shift) (+ res)     act: 0 none, 1 GELU(erf)
@@ -192,6 +225,28 @@ __global__ void bn_bwd_finalize_kernel(const float* __restrict__ part, int npart
   if (c >= C || threadIdx.x >= 32) return;
   dbeta[c] += (float)s1; dgamma[c] += (float)s2;
   if (k1) { k1[c] = (float)(s1 / (double)M); k2[c] = (float)(s2 / (double)M); }
+}
+
+// synchronised backward: this rank's fp64 row [S1 (C) | S2 (C)]; dgamma / dbeta accumulate the local sums
+__global__ void bn_bwd_local_kernel(const float* __restrict__ part, int nparts, int C, float* __restrict__ dgamma,
+                                    float* __restrict__ dbeta, double* __restrict__ row) {
+  const int c = blockIdx.x * 32 + (threadIdx.x & 31);       // 256 threads: 32 channels x 8 slices of the partials
+  double s1 = 0.0, s2 = 0.0;
+  sum_parts2(part, nparts, C, c, s1, s2);
+  if (c >= C || threadIdx.x >= 32) return;
+  dbeta[c] += (float)s1; dgamma[c] += (float)s2;
+  row[c] = s1; row[C + c] = s2;
+}
+
+// k1 = ΣS1 / M_global, k2 = ΣS2 / M_global over the gathered rows [world][2C], summed in rank order
+__global__ void __launch_bounds__(256) bn_bwd_global_kernel(const double* __restrict__ rows, int world, int C,
+                                                            const double* __restrict__ count, float* __restrict__ k1, float* __restrict__ k2) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= C) return;
+  double s1 = 0.0, s2 = 0.0;
+  for (int r = 0; r < world; ++r) { s1 += rows[2LL * r * C + c]; s2 += rows[2LL * r * C + C + c]; }
+  const double M = *count;
+  k1[c] = (float)(s1 / M); k2[c] = (float)(s2 / M);
 }
 
 // BatchNorm with running statistics (eval mode, frozen): no batch-mean terms, draw = dpre * scale
@@ -1918,6 +1973,27 @@ int bn_stats_run(const float* X, long long M, int C, const float* gamma, const f
   return check_launch("bn_finalize_kernel");
 }
 
+int bn_stats_local_run(const float* X, long long M, int C, double* row, float* work, long long work_elems, cudaStream_t st) {
+  const int nparts = (int)((M + STAT_ROWS - 1) / STAT_ROWS);
+  if (work_elems < (long long)nparts * 2 * C) return set_error("bn_stats_local: workspace too small");
+  if (nparts > 0) {
+    colstats_kernel<<<nparts, 256, 0, st>>>(X, M, C, work);
+    int rc = check_launch("colstats_kernel");
+    if (rc) return rc;
+  }
+  bn_stats_local_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, M, C, row);
+  return check_launch("bn_stats_local_kernel");
+}
+
+int bn_stats_global_run(const double* rows, int world, int C, const float* gamma, const float* beta, float eps, float momentum,
+                        float* run_mean, float* run_var, float* mean, float* rstd, float* scale, float* shift, double* count,
+                        cudaStream_t st) {
+  if (world < 1) return set_error("bn_stats_global: world=%d", world);
+  bn_stats_global_kernel<<<nblk(C, 256), 256, 0, st>>>(rows, world, C, gamma, beta, eps, momentum, run_mean, run_var, mean, rstd,
+                                                       scale, shift, count);
+  return check_launch("bn_stats_global_kernel");
+}
+
 int bn_act_run(const float* raw, const float* scale, const float* shift, int act, const float* res, float* out, long long M, int C,
                cudaStream_t st) {
   if (C % 4) return set_error("bn_act: C %% 4 != 0");
@@ -1935,21 +2011,59 @@ static int bn_bwd_reduce_launch(const BnBwdParams& p, int nparts, float* work, c
   return check_launch("bn_bwd_reduce_kernel");
 }
 
+static BnBwdParams bn_bwd_params(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean,
+                                 const float* rstd, const float* gamma, int act, const float* fgate, const float* fadd,
+                                 long long rows_per_field, long long M, int C) {
+  BnBwdParams p;
+  p.dOut = dOut; p.raw = raw; p.scale = scale; p.shift = shift; p.mean = mean; p.rstd = rstd; p.gamma = gamma;
+  p.fgate = fgate; p.fadd = fadd; p.rows_per_field = rows_per_field > 0 ? rows_per_field : 1; p.act = act; p.C = C; p.M = M;
+  return p;
+}
+
 int bn_bwd_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
                const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
                float* dgamma, float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st) {
   const int nparts = (int)((M + STAT_ROWS - 1) / STAT_ROWS);
   if (!bn_bwd_width_ok(C)) return set_error("bn_bwd: C=%d must be 4*k with k | 256, or a multiple of 128 up to 2048", C);
   if (work_elems < (long long)nparts * 2 * C + 2 * C) return set_error("bn_bwd: workspace too small");
-  BnBwdParams p;
-  p.dOut = dOut; p.raw = raw; p.scale = scale; p.shift = shift; p.mean = mean; p.rstd = rstd; p.gamma = gamma;
-  p.fgate = fgate; p.fadd = fadd; p.rows_per_field = rows_per_field > 0 ? rows_per_field : 1; p.act = act; p.C = C; p.M = M;
+  const BnBwdParams p = bn_bwd_params(dOut, raw, scale, shift, mean, rstd, gamma, act, fgate, fadd, rows_per_field, M, C);
   float* k1 = work + (long long)nparts * 2 * C; float* k2 = k1 + C;
   int rc = bn_bwd_reduce_launch(p, nparts, work, st);
   if (rc) return rc;
   bn_bwd_finalize_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, M, C, dgamma, dbeta, k1, k2);
   rc = check_launch("bn_bwd_finalize_kernel");
   if (rc) return rc;
+  bn_bwd_apply_kernel<<<nblk(M * (C / 4), 256), 256, 0, st>>>(p, k1, k2, draw);
+  return check_launch("bn_bwd_apply_kernel");
+}
+
+int bn_bwd_local_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
+                     int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C, float* dgamma,
+                     float* dbeta, double* row, float* work, long long work_elems, cudaStream_t st) {
+  const int nparts = (int)((M + STAT_ROWS - 1) / STAT_ROWS);
+  if (!bn_bwd_width_ok(C)) return set_error("bn_bwd_local: C=%d must be 4*k with k | 256, or a multiple of 128 up to 2048", C);
+  if (work_elems < (long long)nparts * 2 * C) return set_error("bn_bwd_local: workspace too small");
+  if (nparts > 0) {
+    const BnBwdParams p = bn_bwd_params(dOut, raw, scale, shift, mean, rstd, nullptr, act, fgate, fadd, rows_per_field, M, C);
+    int rc = bn_bwd_reduce_launch(p, nparts, work, st);
+    if (rc) return rc;
+  }
+  bn_bwd_local_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, C, dgamma, dbeta, row);
+  return check_launch("bn_bwd_local_kernel");
+}
+
+int bn_bwd_global_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
+                      const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
+                      const double* rows, int world, const double* count, float* draw, float* work, long long work_elems,
+                      cudaStream_t st) {
+  if (!bn_bwd_width_ok(C)) return set_error("bn_bwd_global: C=%d must be 4*k with k | 256, or a multiple of 128 up to 2048", C);
+  if (world < 1) return set_error("bn_bwd_global: world=%d", world);
+  if (work_elems < 2LL * C) return set_error("bn_bwd_global: workspace too small");
+  float* k1 = work; float* k2 = work + C;
+  bn_bwd_global_kernel<<<nblk(C, 256), 256, 0, st>>>(rows, world, C, count, k1, k2);
+  int rc = check_launch("bn_bwd_global_kernel");
+  if (rc || M <= 0) return rc;
+  const BnBwdParams p = bn_bwd_params(dOut, raw, scale, shift, mean, rstd, gamma, act, fgate, fadd, rows_per_field, M, C);
   bn_bwd_apply_kernel<<<nblk(M * (C / 4), 256), 256, 0, st>>>(p, k1, k2, draw);
   return check_launch("bn_bwd_apply_kernel");
 }
@@ -1962,9 +2076,7 @@ int bn_bwd_frozen_run(const float* dOut, const float* raw, const float* scale, c
   if (!bn_bwd_width_ok(C)) return set_error("bn_bwd_frozen: C=%d must be 4*k with k | 256, or a multiple of 128 up to 2048", C);
   if (work_elems < (long long)nparts * 2 * C) return set_error("bn_bwd_frozen: workspace too small");
   if (M <= 0) return 0;
-  BnBwdParams p;
-  p.dOut = dOut; p.raw = raw; p.scale = scale; p.shift = shift; p.mean = mean; p.rstd = rstd; p.gamma = nullptr;
-  p.fgate = fgate; p.fadd = fadd; p.rows_per_field = rows_per_field > 0 ? rows_per_field : 1; p.act = act; p.C = C; p.M = M;
+  const BnBwdParams p = bn_bwd_params(dOut, raw, scale, shift, mean, rstd, nullptr, act, fgate, fadd, rows_per_field, M, C);
   int rc = bn_bwd_reduce_launch(p, nparts, work, st);
   if (rc) return rc;
   bn_bwd_finalize_kernel<<<nblk(C, 32), 256, 0, st>>>(work, nparts, M, C, dgamma, dbeta, nullptr, nullptr);

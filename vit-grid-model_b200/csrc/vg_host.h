@@ -153,11 +153,22 @@ long long bn_workspace_elems(long long M, int C);
 int bn_stats_run(const float* X, long long M, int C, const float* gamma, const float* beta, float eps, float momentum,
                  float* run_mean, float* run_var, float* mean, float* rstd, float* scale, float* shift, float* work,
                  long long work_elems, cudaStream_t st);
+int bn_stats_local_run(const float* X, long long M, int C, double* row, float* work, long long work_elems, cudaStream_t st);
+int bn_stats_global_run(const double* rows, int world, int C, const float* gamma, const float* beta, float eps, float momentum,
+                        float* run_mean, float* run_var, float* mean, float* rstd, float* scale, float* shift, double* count,
+                        cudaStream_t st);
 int bn_act_run(const float* raw, const float* scale, const float* shift, int act, const float* res, float* out, long long M, int C,
                cudaStream_t st);
 int bn_bwd_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
                const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
                float* dgamma, float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st);
+int bn_bwd_local_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
+                     int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C, float* dgamma,
+                     float* dbeta, double* row, float* work, long long work_elems, cudaStream_t st);
+int bn_bwd_global_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
+                      const float* gamma, int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C,
+                      const double* rows, int world, const double* count, float* draw, float* work, long long work_elems,
+                      cudaStream_t st);
 int bn_bwd_frozen_run(const float* dOut, const float* raw, const float* scale, const float* shift, const float* mean, const float* rstd,
                       int act, const float* fgate, const float* fadd, long long rows_per_field, long long M, int C, float* dgamma,
                       float* dbeta, float* draw, float* work, long long work_elems, cudaStream_t st);

@@ -259,6 +259,51 @@ def bn_bwd(dOut, raw, st, gamma, act, dgamma, dbeta, fgate=None, fadd=None, rows
     return draw
 
 
+def _exchange_rows(C2, group, dev, fill):
+    """[world][C2] fp64 of every rank's row, in rank order.  Each rank writes its own row of a zeroed buffer (fill) and the
+    buffer is sum-all-reduced on the current stream: x + 0 is exact, so the result is a copy of the rows whatever order the
+    backend adds them in, and every rank holds the same bits."""
+    import torch.distributed as dist
+    rows = torch.zeros(dist.get_world_size(group), C2, dtype=torch.float64, device=dev)
+    fill(rows[dist.get_rank(group)])
+    dist.all_reduce(rows, op=dist.ReduceOp.SUM, group=group)
+    return rows
+
+
+def bn_stats_sync(x2d, bn, group):
+    """bn_stats over the rows of every rank of `group` (torch.nn.SyncBatchNorm semantics): this rank's fp64 column sums and
+    row count, the exchange, then the finalize over the global count.  -> (st, count): count is the global row count
+    (fp64 device scalar) that bn_bwd_sync needs"""
+    M, C = x2d.shape
+    dev = x2d.device
+    work = _f32(_lib.load().vg_bn_workspace(M, C), dev)
+    rows = _exchange_rows(2 * C + 1, group, dev, lambda row: _lib.call("vg_bn_stats_local", x2d.data_ptr(), M, C, row.data_ptr(),
+                                                                    work.data_ptr(), work.numel(), _st()))
+    st = torch.empty(4, C, dtype=torch.float32, device=dev)
+    count = torch.empty(1, dtype=torch.float64, device=dev)
+    _lib.call("vg_bn_stats_global", rows.data_ptr(), rows.shape[0], C, bn.weight.data_ptr(), bn.bias.data_ptr(), float(bn.eps),
+              float(bn.momentum), _p(bn.running_mean), _p(bn.running_var), st[0].data_ptr(), st[1].data_ptr(), st[2].data_ptr(),
+              st[3].data_ptr(), count.data_ptr(), _st())
+    return st, count
+
+
+def bn_bwd_sync(dOut, raw, st, count, group, gamma, act, dgamma, dbeta, fgate=None, fadd=None, rows_per_field=0, out=None):
+    """bn_bwd with S1 = sum dpre and S2 = sum dpre*xhat summed over the rows of every rank of `group`; dgamma / dbeta take
+    this rank's sums (the data-parallel gradient average makes them global)"""
+    M, C = raw.shape
+    dev = raw.device
+    draw = torch.empty_like(raw) if out is None else out
+    work = _f32(max(_lib.load().vg_bn_workspace(M, C), 2 * C), dev)
+    rows = _exchange_rows(2 * C, group, dev, lambda row: _lib.call(
+        "vg_bn_bwd_local", dOut.data_ptr(), raw.data_ptr(), st[2].data_ptr(), st[3].data_ptr(), st[0].data_ptr(), st[1].data_ptr(),
+        int(act), _p(fgate), _p(fadd), int(rows_per_field), M, C, dgamma.data_ptr(), dbeta.data_ptr(), row.data_ptr(),
+        work.data_ptr(), work.numel(), _st()))
+    _lib.call("vg_bn_bwd_global", dOut.data_ptr(), raw.data_ptr(), st[2].data_ptr(), st[3].data_ptr(), st[0].data_ptr(),
+              st[1].data_ptr(), gamma.data_ptr(), int(act), _p(fgate), _p(fadd), int(rows_per_field), M, C, rows.data_ptr(),
+              rows.shape[0], count.data_ptr(), draw.data_ptr(), work.data_ptr(), work.numel(), _st())
+    return draw
+
+
 def bn_frozen_stats(bn):
     """-> (mean, rstd, scale, shift) of an eval-mode BatchNorm: its running statistics, nothing updated"""
     st = torch.empty(4, bn.num_features, dtype=torch.float32, device=bn.running_mean.device)

@@ -1,7 +1,9 @@
 """Data-parallel training, one process per GPU (SURVEY.md §8e): every rank holds a full replica and its own shard of
-the batch (independent CMAQ time steps); the only exchange is the gradient all-reduce, started per finished gradient
-section from inside backward on a side stream so that it overlaps the remaining backward kernels (train.GradSync).
-BatchNorm uses per-rank batch statistics (the DistributedDataParallel default).  Inference needs no collective."""
+the batch (independent CMAQ time steps); the gradient all-reduce is started per finished gradient section from inside
+backward on a side stream so that it overlaps the remaining backward kernels (train.GradSync).
+BatchNorm uses per-rank batch statistics (the DistributedDataParallel default) unless the module was converted with
+``nn.SyncBatchNorm.convert_sync_batchnorm``: a converted BatchNorm takes its train-mode statistics over the rows of every rank
+of its process group (DESIGN.md §5).  Inference needs no collective."""
 from __future__ import annotations
 
 import torch
@@ -24,6 +26,17 @@ class DataParallel(nn.Module):
                     dist.broadcast(t, src=0, group=process_group)
             if hasattr(module, "invalidate_packed"):    # kernel-layout weight copies made before wrapping are stale now
                 module.invalidate_packed()
+        # A NCCL process group runs its collectives in issue order, and GradSync issues the all-reduces of the head, decoder and
+        # ConvTranspose gradients before the MaxViT backward: a statistics exchange in that group would queue behind them and
+        # stall the compute stream.  SyncBatchNorms without a group of their own get a dedicated one over the same ranks
+        # (dist.new_group is collective: every rank constructs DataParallel).
+        unset = [m for m in module.modules() if isinstance(m, nn.SyncBatchNorm) and m.process_group is None]
+        self.stats_group = None
+        if unset:
+            ranks = None if process_group is None else dist.get_process_group_ranks(process_group)
+            self.stats_group = dist.new_group(ranks=ranks)
+            for m in unset:
+                m.process_group = self.stats_group
         module._grad_sync = GradSync(process_group)
 
     def forward(self, *args, **kwargs):

@@ -17,6 +17,8 @@ from __future__ import annotations
 from collections import OrderedDict
 
 import torch
+import torch.distributed as dist
+import torch.nn as nn
 
 from . import _lib, ops, ops_train as ot
 from .maxvit import MBConvResidual
@@ -205,15 +207,32 @@ def dropout_threshold(p: float) -> int:
     return max(0, min(255, int(round(p * 256))))
 
 
+def _bn_sync_group(bn):
+    """the process group whose rows a train-mode BatchNorm's statistics span, or None for this rank's rows alone: the decision
+    of torch.nn.SyncBatchNorm.forward -- a SyncBatchNorm, torch.distributed initialised, its group (WORLD when None) of more
+    than one rank"""
+    if not isinstance(bn, nn.SyncBatchNorm) or not (dist.is_available() and dist.is_initialized()):
+        return None
+    group = bn.process_group if bn.process_group is not None else dist.group.WORLD
+    return group if dist.get_world_size(group) > 1 else None
+
+
 def _bn_stats(bn, raw, frozen):
+    """-> (st, sync): sync = (group, global row count) when the statistics span several ranks (what backward needs), else None"""
     if frozen:
-        return ot.bn_frozen_stats(bn)
-    return ot.bn_stats(raw, bn.weight, bn.bias, bn.eps, bn.momentum, bn.running_mean, bn.running_var)
+        return ot.bn_frozen_stats(bn), None
+    group = _bn_sync_group(bn)
+    if group is not None:
+        st, count = ot.bn_stats_sync(raw, bn, group)
+        return st, (group, count)
+    return ot.bn_stats(raw, bn.weight, bn.bias, bn.eps, bn.momentum, bn.running_mean, bn.running_var), None
 
 
-def _bn_bwd(dOut, raw, st, bn, act, dgamma, dbeta, frozen, **kw):
+def _bn_bwd(dOut, raw, st, sync, bn, act, dgamma, dbeta, frozen, **kw):
     if frozen:
         return ot.bn_bwd_frozen(dOut, raw, st, act, dgamma, dbeta, **kw)
+    if sync is not None:
+        return ot.bn_bwd_sync(dOut, raw, st, sync[1], sync[0], bn.weight, act, dgamma, dbeta, **kw)
     return ot.bn_bwd(dOut, raw, st, bn.weight, act, dgamma, dbeta, **kw)
 
 
@@ -233,21 +252,21 @@ def maxvit_train_forward(vit, x, cond, seed=0, frozen=False):
         bn1, bn2, bn3 = seq[1], seq[4], seq[8]
         h0 = ops.gemm(x2d, P["w_exp"], bias=P["b_exp"], tf32=tf32)
         hid = h0.shape[1]
-        st1 = _bn_stats(bn1, h0, frozen)
+        st1, sy1 = _bn_stats(bn1, h0, frozen)
         h1 = ot.bn_act(h0, st1, 1)
         h2, _ = ot.dw3x3(h1.view(N, H, W, hid), P["w_dw"], P["ones_hid"], P["b_dw"], 0)
-        st2 = _bn_stats(bn2, h2.view(M, hid), frozen)
+        st2, sy2 = _bn_stats(bn2, h2.view(M, hid), frozen)
         h3 = ot.bn_act(h2.view(M, hid), st2, 1).view(N, H, W, hid)
         gate, mean, hidv = ot.se_gate_train(ot.field_sum(h3), H * W, P["se_w1"], P["se_w2"])
         h4 = ot.se_scale_oop(h3, gate)
         y0 = ops.gemm(h4.view(M, hid), P["w_proj"], bias=P["b_proj"], tf32=tf32)
-        st3 = _bn_stats(bn3, y0, frozen)
+        st3, sy3 = _bn_stats(bn3, y0, frozen)
         y = ot.bn_act(y0, st3, 0, res=x2d if P["residual"] else None).view(N, H, W, y0.shape[1])
         if not frozen:
             for bn in (bn1, bn2, bn3):
                 bn.num_batches_tracked += 1
-        sv = dict(x=x, h0=h0, st1=st1, h1=h1, h2=h2, st2=st2, h3=h3, gate=gate, mean=mean, hidv=hidv, h4=h4, y0=y0, st3=st3,
-                  frozen=frozen)
+        sv = dict(x=x, h0=h0, st1=st1, sy1=sy1, h1=h1, h2=h2, st2=st2, sy2=sy2, h3=h3, gate=gate, mean=mean, hidv=hidv, h4=h4,
+                  y0=y0, st3=st3, sy3=sy3, frozen=frozen)
         fb = P["block"]
         film_b = ops.cond_mlp(cond, fb["film_w0"], fb["film_b0"], fb["film_w1"], fb["film_b1"])
         T = 0 if frozen else dropout_threshold(battn.dropout_p)
@@ -286,21 +305,21 @@ def maxvit_train_backward(vit, saved, cond, dcond, dx, G, prefix):
         dy = dx.view(M, C_out)
         bn1, bn2, bn3 = seq[1], seq[4], seq[8]
         fz = sv["frozen"]
-        dy0 = _bn_bwd(dy, sv["y0"], sv["st3"], bn3, 0, G[pm + "8.weight"], G[pm + "8.bias"], fz)
+        dy0 = _bn_bwd(dy, sv["y0"], sv["st3"], sv["sy3"], bn3, 0, G[pm + "8.weight"], G[pm + "8.bias"], fz)
         ot.colsum(dy0, G[pm + "7.bias"])
         ot.wgrad(dy0, sv["h4"].view(M, hid), G[pm + "7.weight"], tf32=tf32)
         dh4 = ops.gemm(dy0, seq[7].weight.detach().flatten(1).t().contiguous(), tf32=tf32)
         del dy0
         dmean = ot.se_bwd(dh4, sv["h3"], sv["gate"], sv["mean"], sv["hidv"], P["se_w1"], P["se_w2"], G[pm + "6.gate.1.weight"],
                           G[pm + "6.gate.3.weight"])
-        dh2 = _bn_bwd(dh4, sv["h2"].view(M, hid), sv["st2"], bn2, 1, G[pm + "4.weight"], G[pm + "4.bias"], fz,
+        dh2 = _bn_bwd(dh4, sv["h2"].view(M, hid), sv["st2"], sv["sy2"], bn2, 1, G[pm + "4.weight"], G[pm + "4.bias"], fz,
                       fgate=sv["gate"], fadd=dmean, rows_per_field=H * W, out=dh4)
         dw9 = torch.zeros(9, hid, dtype=torch.float32, device=dx.device)
         ot.dw3x3_wgrad(sv["h1"].view(N, H, W, hid), dh2.view(N, H, W, hid), dw9, G[pm + "3.bias"])
         G[pm + "3.weight"].view(hid, 9).add_(dw9.t())
         dh1, _ = ot.dw3x3(dh2.view(N, H, W, hid), P["w_dw_flip"], P["ones_hid"], P["zeros_hid"], 0)
         del dh2, dh4
-        dh0 = _bn_bwd(dh1.view(M, hid), sv["h0"], sv["st1"], bn1, 1, G[pm + "1.weight"], G[pm + "1.bias"], fz, out=dh1.view(M, hid))
+        dh0 = _bn_bwd(dh1.view(M, hid), sv["h0"], sv["st1"], sv["sy1"], bn1, 1, G[pm + "1.weight"], G[pm + "1.bias"], fz, out=dh1.view(M, hid))
         ot.colsum(dh0, G[pm + "0.bias"])
         ot.wgrad(dh0, x.view(M, C), G[pm + "0.weight"], tf32=tf32)
         dx = ops.gemm(dh0, seq[0].weight.detach().flatten(1).t().contiguous(), res=dy if P["residual"] else None,
