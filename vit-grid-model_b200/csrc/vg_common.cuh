@@ -281,6 +281,49 @@ __device__ __forceinline__ void tmem_relinquish() { asm volatile("tcgen05.relinq
 __device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t ncols) {
   asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
 }
+// ---- two-CTA (cluster of 2) forms: one MMA of M = 256 reads its A rows and half of B from each CTA's shared memory at the
+// same offsets and accumulates into each CTA's own TMEM; TMEM is allocated in both CTAs at once by one warp of each ----
+__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
+// shared::cluster address of the same variable in CTA `rank` of the cluster
+__device__ __forceinline__ uint32_t mapa_shared(const void* p, uint32_t rank) {
+  uint32_t a;
+  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(smem_u32(p)), "r"(rank));
+  return a;
+}
+// every thread of every CTA of the cluster; orders the threads' memory operations cluster-wide
+__device__ __forceinline__ void cluster_sync() {
+  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+// arrive on an mbarrier of either CTA (cluster address).  CTA-scope release, as for a local arrive: it hands over TMEM, whose
+// reads tcgen05.wait::ld has completed, not memory -- a cluster-scope release would wait for the thread's global stores (MEMBAR.GPU)
+__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_bar) {
+  asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_bar) : "memory");
+}
+// TMA load into this CTA's shared memory that signals an mbarrier of either CTA of the pair (cluster address)
+__device__ __forceinline__ void tma_load_2d_pair(void* dst, const CUtensorMap* m, uint32_t cluster_bar, int c0, int c1) {
+  asm volatile(
+      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
+      ::"r"(smem_u32(dst)), "l"(m), "r"(cluster_bar), "r"(c0), "r"(c1) : "memory");
+}
+__device__ __forceinline__ void tmem_alloc_pair(uint32_t* dst_smem, uint32_t ncols) {
+  asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(ncols) : "memory");
+}
+__device__ __forceinline__ void tmem_relinquish_pair() { asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory"); }
+__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
+  asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(ncols) : "memory");
+}
+// arrives on the mbarrier at this shared-memory offset in both CTAs of the pair when the pair's earlier MMAs retire
+__device__ __forceinline__ void tc_commit_pair(uint64_t* bar) {
+  asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
+               ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
+}
+__device__ __forceinline__ void tc_mma_bf16_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
+}
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
 // One lane of a CONVERGED warp.  Issue tcgen05.mma / tcgen05.commit inside `if (elect_one()) { ... }` with the whole warp

@@ -228,16 +228,28 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__
 // K order: channel block 0 taps 0..8, then channel block 1 taps 0..8, so each A half-buffer is reloaded for the next
 // tile while the other half is being consumed.  L2->SM traffic per 256-pixel tile: 100 KiB (A) + 288 KiB (B)
 // instead of 576 + 288 KiB.
+//
+// The kernel runs as CTA pairs (clusters of 2) on tcgen05's two-CTA MMA.  The two CTAs of pair p own tiles 2p and 2p+1 and
+// each loads its own halo, but only its 64-output-channel half of every weight stage (8 KiB); the leader (rank 0) issues
+// M = 256 MMAs that take 128 rows from the leader's tile and 128 from the peer's, at the same shared-memory offsets (both
+// CTAs build the same halo layout, so the row-shifted A descriptor is valid in both).  Per SM this halves the weight
+// bytes the tensor core reads from shared memory and TMA writes into it (L2->SM traffic per tile: 100 + 144 KiB), and the
+// same 48 KiB hold a 6-stage weight ring.  The accumulator of each CTA's tile lands in that CTA's TMEM with the layout of a
+// one-CTA M = 128 MMA, so the epilogue is per CTA as before; every output element sums its K terms in the same order.
+// Barriers: full / a_full live in the leader and count both CTAs' TMA bytes; empty / a_free / tfull are signalled in both
+// CTAs by multicast commits; the leader's tempty counts the epilogue warps of both CTAs.
 // ------------------------------------------------------------------------------------------------
 constexpr int HALO_MAX_ROWS = 416;                            // HR <= 416 (two TMA boxes of <= 208 rows)
-constexpr int HB_STAGES = 3;                                  // weight ring
+constexpr int HB_STAGES = 6;                                  // weight ring
+constexpr int HB_BYTES = B_BYTES / 2;                         // one CTA's half stage: 64 output channels x 128 B
 constexpr int HALO_RES_BYTES = 8 * 2 * 4096;                  // per epilogue warp: two [32 rows][128 B] fp32 residual chunks (TMA)
 constexpr int HALO_A_BYTES = HALO_MAX_ROWS * 128;             // per channel block
-constexpr int HALO_SMEM_BYTES = 2 * HALO_A_BYTES + HB_STAGES * B_BYTES + HALO_RES_BYTES + PARAM_FLOATS * 4 + 1024 + 256;
+constexpr int HALO_PARAM_FLOATS = 3 * 128;                    // bias | ln_g | ln_b
+constexpr int HALO_SMEM_BYTES = 2 * HALO_A_BYTES + HB_STAGES * HB_BYTES + HALO_RES_BYTES + HALO_PARAM_FLOATS * 4 + 1024 + 512;
 
 struct HaloShape {
   long long M;          // flat pixels (rows of the [q][128] matrices)
-  int num_tiles;        // 256-pixel tiles
+  int num_tiles;        // 256-pixel tiles, rounded up to a whole pair (the odd count's last tile has no rows: row >= M)
   int P;                // row pitch (pixels)
   int HR;               // halo rows loaded per tile (multiple of 16)
   int res_tma;          // the fp32 residual arrives through mapR (else: per-thread global loads)
@@ -253,15 +265,15 @@ __device__ __forceinline__ uint64_t umma_desc_k128_shift(uint32_t tile_addr, int
 // MODE 0: conv + ChanLN / FiLM / ReLU / residual epilogue; 1: the same, saving xhat / rstd / mask for backward; 2: plain fp32 store
 // (+ fp32 residual) -- the DATA GRADIENT of the convolution runs through the same halo pipeline with the tap order flipped
 template <int MODE>
-__global__ void __launch_bounds__(TC_THREADS, 1)
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(TC_THREADS, 1)
 conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
                  const __grid_constant__ CUtensorMap mapR, const __grid_constant__ CUtensorMap mapO, const HaloShape hs, const EpiParams ep) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint8_t* sB = smem + 2 * HALO_A_BYTES;
-  uint8_t* sres = sB + HB_STAGES * B_BYTES;
+  uint8_t* sres = sB + HB_STAGES * HB_BYTES;
   float* sparam = reinterpret_cast<float*>(sres + HALO_RES_BYTES);
-  uint64_t* full = reinterpret_cast<uint64_t*>(sres + HALO_RES_BYTES + PARAM_FLOATS * 4);
+  uint64_t* full = reinterpret_cast<uint64_t*>(sres + HALO_RES_BYTES + HALO_PARAM_FLOATS * 4);
   uint64_t* empty = full + HB_STAGES;
   uint64_t* a_full = empty + HB_STAGES;    // [2]
   uint64_t* a_free = a_full + 2;           // [2]
@@ -272,53 +284,62 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
 
   const int warp = __shfl_sync(0xffffffffu, (int)(threadIdx.x >> 5), 0);
   const int lane = threadIdx.x & 31;
+  const uint32_t rank = cluster_ctarank();                   // tile t = blockIdx.x: rank 0 (the leader) takes the even tile of the pair
 
   if (warp == 0 && lane == 0) { tma_prefetch_desc(&mapA); tma_prefetch_desc(&mapB); if (hs.res_tma) tma_prefetch_desc(&mapR); }
   if (warp == 1 && lane == 0) {
     for (int s = 0; s < HB_STAGES; ++s) { mbar_init(full + s, 1); mbar_init(empty + s, 1); }
-    for (int s = 0; s < 2; ++s) { mbar_init(a_full + s, 1); mbar_init(a_free + s, 1); mbar_init(tfull + s, 1); mbar_init(tempty + s, 8); }
+    for (int s = 0; s < 2; ++s) { mbar_init(a_full + s, 1); mbar_init(a_free + s, 1); mbar_init(tfull + s, 1); mbar_init(tempty + s, 16); }
     for (int s = 0; s < 16; ++s) mbar_init(res_full + s, 1);
     fence_mbar_init();
   }
-  if (warp == 2) { tmem_alloc(tmem_slot, TMEM_COLS); tmem_relinquish(); }
+  if (warp == 2) { tmem_alloc_pair(tmem_slot, TMEM_COLS); tmem_relinquish_pair(); }
   if (MODE != 2) {
     for (int i = threadIdx.x; i < 128; i += TC_THREADS) {
       sparam[i] = ep.bias[i]; sparam[128 + i] = ep.ln_g[i]; sparam[256 + i] = ep.ln_b[i];
     }
   }
   tc_fence_before();
-  __syncthreads();
+  cluster_sync();                                            // both CTAs' barriers are initialised before either signals the other
   tc_fence_after();
   const uint32_t tmem_base = __shfl_sync(0xffffffffu, *tmem_slot, 0);   // warp-uniform: lets the MMA issue use uniform registers (no per-MMA elect/broadcast loop)
   const int halo = hs.P + 1;                                 // rows in front of the tile's first output pixel
   if (warp == 0) {
-    if (lane == 0) {                                         // ===== TMA producer =====
+    if (lane == 0) {                                         // ===== TMA producer (both CTAs): own halo, own half of the weights =====
       int stage = 0; uint32_t phase = 0; uint32_t it = 0;
       const int half_rows = hs.HR / 2;
       for (int t = blockIdx.x; t < hs.num_tiles; t += gridDim.x, ++it) {
         const long long q0 = (long long)t * BM;
         for (int cb = 0; cb < 2; ++cb) {
           mbar_wait(a_free + cb, (it & 1) ^ 1);              // previous tile's taps on this half have retired
-          mbar_arrive_expect_tx(a_full + cb, hs.HR * 128);
+          if (rank == 0) mbar_arrive_expect_tx(a_full + cb, 2 * hs.HR * 128);
+          const uint32_t bar = mapa_shared(a_full + cb, 0);
           uint8_t* sa = smem + cb * HALO_A_BYTES;
-          tma_load_2d(sa, &mapA, a_full + cb, cb * 64, (int)(q0 - halo));
-          tma_load_2d(sa + half_rows * 128, &mapA, a_full + cb, cb * 64, (int)(q0 - halo + half_rows));
+          tma_load_2d_pair(sa, &mapA, bar, cb * 64, (int)(q0 - halo));
+          tma_load_2d_pair(sa + half_rows * 128, &mapA, bar, cb * 64, (int)(q0 - halo + half_rows));
           for (int tap = 0; tap < 9; ++tap) {
             mbar_wait(empty + stage, phase ^ 1);
-            mbar_arrive_expect_tx(full + stage, B_BYTES);
-            tma_load_2d(sB + stage * B_BYTES, &mapB, full + stage, (hs.flip ? 8 - tap : tap) * 128 + cb * 64, 0);
+            if (rank == 0) mbar_arrive_expect_tx(full + stage, 2 * HB_BYTES);
+            tma_load_2d_pair(sB + stage * HB_BYTES, &mapB, mapa_shared(full + stage, 0), (hs.flip ? 8 - tap : tap) * 128 + cb * 64,
+                             (int)rank * 64);
             if (++stage == HB_STAGES) { stage = 0; phase ^= 1; }
           }
         }
       }
+      // the leader's last commits into this CTA's barriers have arrived before the CTA may exit
+      for (int s = 0; s < HB_STAGES; ++s) {
+        mbar_wait(empty + stage, phase ^ 1);
+        if (++stage == HB_STAGES) { stage = 0; phase ^= 1; }
+      }
+      for (int cb = 0; cb < 2; ++cb) mbar_wait(a_free + cb, (it & 1) ^ 1);
     }
   } else if (warp == 1) {
-    {                                                        // ===== MMA issuer: the warp runs converged, an elected lane issues (see elect_one) =====
-      constexpr uint32_t idesc = umma_idesc_bf16(128, BN);
+    if (rank == 0) {                                         // ===== MMA issuer (leader only): the warp runs converged, an elected lane issues (see elect_one) =====
+      constexpr uint32_t idesc = umma_idesc_bf16(2 * 128, BN);
       int stage = 0; uint32_t phase = 0; uint32_t it = 0;
       for (int t = blockIdx.x; t < hs.num_tiles; t += gridDim.x, ++it) {
         const int as = it & 1; const uint32_t aphase = (it >> 1) & 1;
-        mbar_wait(tempty + as, aphase ^ 1);
+        mbar_wait(tempty + as, aphase ^ 1);                  // both CTAs' epilogues have drained this buffer
         tc_fence_after();
         const uint32_t d0 = tmem_base + as * 256, d1 = d0 + 128;
         for (int cb = 0; cb < 2; ++cb) {
@@ -331,17 +352,17 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
             tc_fence_after();
             if (elect_one()) {
               const uint64_t da0 = umma_desc_k128_shift(sa, r0), da1 = umma_desc_k128_shift(sa, r0 + 128);
-              const uint64_t db = umma_desc_k128(smem_u32(sB + stage * B_BYTES));
+              const uint64_t db = umma_desc_k128(smem_u32(sB + stage * HB_BYTES));
 #pragma unroll
               for (int k = 0; k < 4; ++k) {
                 const uint32_t acc = (cb | tap | k) ? 1u : 0u;
-                tc_mma_bf16(d0, da0 + 2 * k, db + 2 * k, idesc, acc);
-                tc_mma_bf16(d1, da1 + 2 * k, db + 2 * k, idesc, acc);
+                tc_mma_bf16_pair(d0, da0 + 2 * k, db + 2 * k, idesc, acc);
+                tc_mma_bf16_pair(d1, da1 + 2 * k, db + 2 * k, idesc, acc);
               }
-              tc_commit(empty + stage);
+              tc_commit_pair(empty + stage);
               if (tap == 8) {
-                tc_commit(a_free + cb);
-                if (cb == 1) tc_commit(tfull + as);
+                tc_commit_pair(a_free + cb);
+                if (cb == 1) tc_commit_pair(tfull + as);
               }
             }
             __syncwarp();
@@ -349,6 +370,8 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
           }
         }
       }
+      // both CTAs' epilogues have released the last two accumulators (the peer's arrivals target this CTA)
+      for (int k = 0; k < 2; ++k, ++it) mbar_wait(tempty + (it & 1), ((it >> 1) & 1) ^ 1);
     }
   } else if (warp >= 4) {                                    // ===== epilogue: 2 x 128 threads, one pixel row each =====
     const int lg = warp & 3;
@@ -384,13 +407,13 @@ conv_halo_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant
       else run_epilogue<MODE == 1 ? EPI_CONV_LN_TRAIN : EPI_CONV_LN, bf16>(ep, cx, row, ok, 0, ld);
       tc_fence_before();
       __syncwarp();
-      if (lane == 0) mbar_arrive(tempty + as);
+      if (lane == 0) mbar_arrive_cluster(mapa_shared(tempty + as, 0));
     }
     if (hs.out2_tma && lane == 0) bulk_wait_all();           // outstanding tensor stores have been performed before the CTA exits
   }
   tc_fence_before();
-  __syncthreads();
-  if (warp == 2) { tc_fence_after(); tmem_dealloc(tmem_base, TMEM_COLS); }
+  cluster_sync();                                            // neither CTA frees TMEM or exits while its peer may still signal it
+  if (warp == 2) { tc_fence_after(); tmem_dealloc_pair(tmem_base, TMEM_COLS); }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -535,6 +558,27 @@ static int launch_simt_epi(const float* scratch, int Ntot, const GemmShape& gs, 
   return check_launch("epilogue_rows_kernel");
 }
 
+// one CTA pair per 2 tiles, persistent over pairs when there are more than the device holds at once
+template <int MODE>
+static int launch_halo(const CUtensorMap& ma, const CUtensorMap& mb, const CUtensorMap& mr, const CUtensorMap& mo, const HaloShape& hs,
+                       const EpiParams& ep, cudaStream_t st) {
+  static int max_pairs[64] = {};                             // co-resident clusters of 2, per device
+  int dev = 0; cudaGetDevice(&dev);
+  int& mp = max_pairs[dev & 63];
+  if (!mp) {
+    cudaError_t e = cudaFuncSetAttribute(conv_halo_kernel<MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, HALO_SMEM_BYTES);
+    if (e == cudaSuccess) {
+      cudaLaunchConfig_t cfg = {};
+      cfg.gridDim = dim3(2); cfg.blockDim = dim3(TC_THREADS); cfg.dynamicSmemBytes = HALO_SMEM_BYTES;
+      e = cudaOccupancyMaxActiveClusters(&mp, conv_halo_kernel<MODE>, &cfg);
+    }
+    if (e != cudaSuccess || mp <= 0) { mp = 0; return set_error("conv_halo: no co-resident CTA pair (%s)", cudaGetErrorString(e)); }
+  }
+  const int pairs = hs.num_tiles / 2;
+  conv_halo_kernel<MODE><<<2 * (pairs < mp ? pairs : mp), TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);
+  return check_launch("conv_halo_kernel");
+}
+
 // bf16 3x3 conv (Cin = Cout = 128) over a PG buffer with halo reuse; returns -1 when the shape does not fit
 int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const EpiParams& ep, int mode_k, int flip, cudaStream_t st);
 
@@ -565,10 +609,10 @@ int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const Ep
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return set_error("conv_halo: A tensor map failed (%d)", (int)r);
   }
-  int rc = make_map_2d(&mb, false, Wt, 9 * 128, 128, BN);
+  int rc = make_map_2d(&mb, false, Wt, 9 * 128, 128, BN / 2);     // each CTA of a pair loads 64 output channels
   if (rc) return rc;
   HaloShape hs;
-  hs.M = M; hs.num_tiles = (int)((hs.M + BM - 1) / BM); hs.P = P; hs.HR = HR; hs.res_tma = res_tma ? 1 : 0;
+  hs.M = M; hs.num_tiles = (int)((hs.M + 2 * BM - 1) / (2 * BM)) * 2; hs.P = P; hs.HR = HR; hs.res_tma = res_tma ? 1 : 0;
   hs.flip = flip;
   // fp32 copy through TMA stores (needs the residual buffers: fp32-residual launches only; the others store it per thread)
   CUtensorMap mo = ma;
@@ -578,21 +622,10 @@ int conv_halo_run_mp(const void* x, const void* Wt, long long M, int P, const Ep
     if (rc2) return rc2;
     hs.out2_tma = 1;
   }
-  static PerDeviceFlag attr_pd;
-  bool& attr_set = attr_pd.cur();
-  if (!attr_set) {
-    cudaError_t e = cudaFuncSetAttribute(conv_halo_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, HALO_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_halo_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, HALO_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(conv_halo_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, HALO_SMEM_BYTES);
-    if (e != cudaSuccess) return set_error("cudaFuncSetAttribute(conv_halo): %s", cudaGetErrorString(e));
-    attr_set = true;
-  }
-  const int grid = hs.num_tiles < num_sms() ? hs.num_tiles : num_sms();
   if (!res_tma) mr = ma;                                     // unused by the kernel
-  if (mode_k == 2) conv_halo_kernel<2><<<grid, TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);
-  else if (train) conv_halo_kernel<1><<<grid, TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);
-  else conv_halo_kernel<0><<<grid, TC_THREADS, HALO_SMEM_BYTES, st>>>(ma, mb, mr, mo, hs, ep);
-  return check_launch("conv_halo_kernel");
+  if (mode_k == 2) return launch_halo<2>(ma, mb, mr, mo, hs, ep, st);
+  if (train) return launch_halo<1>(ma, mb, mr, mo, hs, ep, st);
+  return launch_halo<0>(ma, mb, mr, mo, hs, ep, st);
 }
 
 // The one host entry used by the C ABI (vg_api.cu).  dtype: 0 = bf16 (tcgen05), 1 = fp32 (SIMT FFMA),
